@@ -2,16 +2,20 @@
 """Benchmark of the Langevin posterior-inference path (BASELINE.json metric: latent-steps/s, CIFAR-10 config).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cifar10|svhn|...]
-                    [--batch B] [--mode langevin|train]
+                    [--batch B] [--mode langevin|train] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input: R calls of
 sample_langevin_post_z_with_flow (train.py:307-335), each T = g_l_steps Langevin iterations on B latents per GPU
-(R = `langevin_calls_per_step` is chosen once, after the warm-up, so that the K timed steps last >= 3 s; every call
-gets fresh Philox noise and the L2 is flushed between calls).  value = N * B * T * R * K / time, inputs resident in
+(R = `langevin_calls_per_step` = --calls-per-step, 1 by default, so that K timed steps are K calls; every call gets
+fresh Philox noise and the L2 is flushed between calls).  value = N * B * T * R * K / time, inputs resident in
 HBM, timed with CUDA events, max over ranks.  The primary `value` runs the fp32-equivalent arithmetic (3-pass hi|lo
 forward AND data gradient); `value_bwd1pass` is the opt-in single-fp16-pass data gradient, reported next to it.
 `e2e` is the same metric through the public Python API with pinned HOST buffers, host<->device copies inside the
 timed region.  Prints ONE JSON line (rank 0).
+
+Inputs, parameters and noise seeds depend on the arguments only, so `--dump-outputs DIR` (rank 0) writes the results
+of the same computation on every run: what the last timed call returned, as DIR/<name>.npy (see dump_outputs), for
+comparing two builds output for output.
 """
 from __future__ import annotations
 
@@ -47,7 +51,21 @@ TEST_WORKLOADS = {
 }
 ALL_WORKLOADS = dict(WORKLOADS, **TEST_WORKLOADS)
 ROOFLINE_LATENT_STEPS = {"svhn": 5.98e6, "cifar10": 347e3, "celeba_crop": 971e3, "celeba_hq256": 112e3}  # BASELINE.md s3
-TARGET_TIMED_SECONDS = 3.0
+DUMP_MAX_ELEMENTS = 1 << 20   # per array: a dump of the at most 7 arrays written stays below 64 MB
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array of `arrays` (name -> tensor) as `directory/<name>.npy`, float64 kept, anything else as
+    float32.  An array of more than DUMP_MAX_ELEMENTS elements is replaced by the same seeded sample of that many of
+    its flattened elements (in index order) on every run."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        v = t.detach().cpu().numpy()
+        v = v.astype(np.float64 if v.dtype == np.float64 else np.float32)
+        if v.size > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(v.size, DUMP_MAX_ELEMENTS, replace=False))
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), v)
 
 
 def exact_layer_flops(layers):
@@ -348,7 +366,9 @@ def main():
     sink = _CleanStdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    # 70 timed calls of the default CIFAR-10 workload take about 3 s on a B200: a window long enough that clock and
+    # scheduler noise stay small (`details.timed_region_s` reports it; faster workloads want more steps)
+    ap.add_argument("--steps", type=int, default=70)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cifar10", choices=sorted(ALL_WORKLOADS))
@@ -358,12 +378,17 @@ def main():
     ap.add_argument("--test-steps", type=int, default=None, help="svhn_test: Langevin iterations per chain (400; 8000 = "
                     "the reference's x20 rule)")
     ap.add_argument("--full-50k", action="store_true", help="svhn_test: cover all 50 000 latents (strong scaling)")
-    ap.add_argument("--calls-per-step", type=int, default=None, help="Langevin calls per timed step (default: auto)")
+    ap.add_argument("--calls-per-step", type=int, default=None, help="Langevin calls (--mode train: training "
+                    "iterations) per timed step (default 1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the bwd1pass secondary measurement")
     ap.add_argument("--no-eager-ref", action="store_true", help="skip the eager torch-CUDA reference row")
     ap.add_argument("--stage-table", default=None, help="write the per-stage timing table (json) here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     w = dict(ALL_WORKLOADS[a.workload])
     if a.batch:
         w["B"] = a.batch
@@ -435,19 +460,14 @@ def main():
     for i in range(a.warmup):
         call(i)
     barrier()
-    # R calls per step so that the K timed steps last >= TARGET_TIMED_SECONDS (same R on every rank)
-    if a.calls_per_step:
-        R = a.calls_per_step
-    elif a.full_50k:
-        R = 1
-    else:
-        est_ms = timed_calls(ctx, call, 2) / 2
-        R = max(1, min(64, math.ceil(TARGET_TIMED_SECONDS * 1e3 / (a.steps * est_ms))))
+    R = a.calls_per_step or 1
     sampler.window_begin()
     ms_total = timed_calls(ctx, lambda i: call(a.warmup + i), a.steps * R)
     sampler.window_end()
     clocks = sampler.stop() if rank == 0 else None
     assert torch.isfinite(out).all(), "non-finite latents"
+    if a.dump_outputs and rank == 0:   # before the secondary measurement reuses `out` and `norms`
+        dump_outputs(a.dump_outputs, {"z_T": out, "gnorm_g": norms[0], "gnorm_f": norms[1]})
     value = world * B * T * a.steps * R / (ms_total * 1e-3)
 
     # ---- secondary: the opt-in single-fp16-pass data gradient, same workload, same timing rules ----

@@ -45,20 +45,26 @@ def run_train_bench(a, w, ctx, sink):
     if rank == 0:
         sampler.start()
     for i in range(max(a.warmup, 3)):
-        out = step(i)
+        step(i)
     ctx.barrier()
-    # R training iterations per timed step so that the K steps last >= 3 s (same R on every rank: the estimate is the
-    # max over ranks)
-    import math
-    est_ms = bench.timed_calls(ctx, lambda i: step(50 + i), 2) / 2
-    R = a.calls_per_step or max(1, min(64, math.ceil(bench.TARGET_TIMED_SECONDS * 1e3 / (a.steps * est_ms))))
+    R = a.calls_per_step or 1
     n_iter = a.steps * R
+    last = []
+
+    def timed_step(i):
+        last[:] = step(100 + i)
+
     sampler.window_begin()
-    ms_total = bench.timed_calls(ctx, lambda i: step(100 + i), n_iter)
+    ms_total = bench.timed_calls(ctx, timed_step, n_iter)
     sampler.window_end()
     clocks = sampler.stop() if rank == 0 else None
-    lg, lf, gn, fn, zk = out
+    lg, lf, gn, fn, zk = last
     assert torch.isfinite(zk).all() and torch.isfinite(lg) and torch.isfinite(lf)
+    if a.dump_outputs and rank == 0:   # the parameters as the last timed iteration left them, before the runs below
+        bench.dump_outputs(a.dump_outputs, {
+            "loss_g": lg, "loss_f": lf, "gnorm_g": gn, "gnorm_f": fn, "z_k": zk,
+            "generator_params": torch.cat([p.detach().reshape(-1) for p in netG.parameters()]),
+            "flow_params": torch.cat([p.detach().reshape(-1) for p in netF.parameters()])})
     value = world * B * T * n_iter / (ms_total * 1e-3)
 
     # the same iterations without the collectives (every rank updates from its own shard): what the all-reduces cost

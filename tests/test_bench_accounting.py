@@ -88,3 +88,97 @@ def test_reference_arm_times_one_whole_training_iteration_of_config_1():
     assert d["langevin_call_ms"] > d["updates_ms"] > 0           # SURVEY section 6: 1 467 ms against 110 ms on 8 vCPU
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"] == {"value": line["value"], "unit": "latent-steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_dump_outputs_keeps_small_arrays_and_samples_large_ones_the_same_way(tmp_path):
+    import numpy as np
+    import torch
+    n = bench.DUMP_MAX_ELEMENTS
+    arrays = {"small": torch.arange(6, dtype=torch.float16).reshape(2, 3), "f64": torch.ones(3, dtype=torch.float64),
+              "big": torch.arange(n + 1000, dtype=torch.int32)}
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    small, f64, big = (np.load(tmp_path / "a" / f"{k}.npy") for k in ("small", "f64", "big"))
+    assert small.dtype == np.float32 and small.shape == (2, 3) and np.array_equal(small, np.arange(6).reshape(2, 3))
+    assert f64.dtype == np.float64
+    assert big.dtype == np.float32 and big.shape == (n,) and np.all(np.diff(big) > 0) and big[-1] < n + 1000
+    assert np.array_equal(big, np.load(tmp_path / "b" / "big.npy"))
+
+
+@pytest.mark.gpu
+def test_steps_are_timed_calls_and_the_dump_is_the_last_one(tmp_path):
+    """`--steps K --warmup W` times K Langevin calls, call i with Philox seed 1234 + W + i, and --dump-outputs writes
+    what the last of them returned: what the public API returns for that seed."""
+    import json
+    import subprocess
+    import sys
+    import numpy as np
+    import torch
+    import lsnf_b200
+    from helpers import rel_l2
+    r = subprocess.run([sys.executable, bench.__file__, "--workload", "svhn", "--steps", "2", "--warmup", "3",
+                        "--no-cpu-baseline", "--no-secondary", "--no-eager-ref", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["details"]["langevin_calls_per_step"] == 1
+    w = bench.WORKLOADS["svhn"]
+    dev = torch.device("cuda:0")
+    args, netG, netF, _, _ = bench.build_models(w, dev)
+    x_np, z0_np, _ = synth.inputs(w["B"], w["nz"], 3, w["img"], 1, seed=1)
+    z, gn, fn = lsnf_b200.sample_langevin_post_z_with_flow(torch.from_numpy(z0_np).to(dev), torch.from_numpy(x_np).to(dev),
+                                                           netG, netF, args, seed=1234 + 3 + 1, steps=w["T"])
+    z_T = np.load(tmp_path / "z_T.npy")
+    assert z_T.dtype == np.float32 and z_T.shape == (w["B"], w["nz"])
+    assert rel_l2(z_T, z.reshape(w["B"], w["nz"]).cpu().numpy()) < 1e-6
+    assert float(np.load(tmp_path / "gnorm_g.npy")) == pytest.approx(gn.item(), rel=1e-6)
+    assert float(np.load(tmp_path / "gnorm_f.npy")) == pytest.approx(fn.item(), rel=1e-6)
+
+
+@pytest.mark.gpu
+def test_train_mode_dump_is_the_last_timed_iteration(tmp_path):
+    """`--mode train --steps 1 --warmup 3`: three warm-up iterations (seeds 1000-1002), one timed one (seed 1100),
+    then more iterations for the other rows.  The dump holds the timed iteration's results and the parameters it left:
+    the same as replaying those four iterations here, and the losses the JSON line reports."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    import torch
+    import lsnf_b200
+    from helpers import rel_l2
+    r = subprocess.run([sys.executable, bench.__file__, "--mode", "train", "--workload", "svhn", "--steps", "1",
+                        "--warmup", "3", "--dump-outputs", str(tmp_path / "bench")],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])["details"]
+    assert d["training_iterations_per_step"] == 1
+    assert float(np.load(tmp_path / "bench" / "loss_g.npy")) == d["loss_g"]
+    assert float(np.load(tmp_path / "bench" / "loss_f.npy")) == d["loss_f"]
+    w = bench.WORKLOADS["svhn"]
+    dev = torch.device("cuda:0")
+    args, netG, netF, _, _ = bench.build_models(w, dev)
+    optG, optF = lsnf_b200.make_optimizers(netG, netF, args)
+    x = torch.from_numpy(synth.inputs(w["B"], w["nz"], 3, w["img"], 1, seed=1)[0]).to(dev)
+    for seed in (1000, 1001, 1002, 1100):
+        lg, lf, gn, fn, zk = lsnf_b200.training_iteration(x, netG, netF, optG, optF, args, global_batch=w["B"],
+                                                          sample_offset=0, seed=seed)
+    bench.dump_outputs(str(tmp_path / "here"), {
+        "loss_g": lg, "loss_f": lf, "gnorm_g": gn, "gnorm_f": fn, "z_k": zk,
+        "generator_params": torch.cat([p.detach().reshape(-1) for p in netG.parameters()]),
+        "flow_params": torch.cat([p.detach().reshape(-1) for p in netF.parameters()])})
+    names = sorted(os.listdir(tmp_path / "bench"))
+    assert names == sorted(os.listdir(tmp_path / "here")) and len(names) == 7
+    for f in names:
+        got, want = np.load(tmp_path / "bench" / f), np.load(tmp_path / "here" / f)
+        assert got.dtype == np.float32 and got.shape == want.shape, f
+        assert rel_l2(got, want) < 1e-5, (f, rel_l2(got, want))
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm(tmp_path):
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, bench.__file__, "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr

@@ -1,5 +1,5 @@
 """The oracle restatement against the fixtures written from the reference's own modules
-(oracle/make_golden.py), and -- when /root/reference is present -- against the reference live."""
+(oracle/make_golden.py), and -- when LSNF_REFERENCE names a checkout of the reference -- against the reference live."""
 import os
 import sys
 
@@ -52,6 +52,23 @@ def test_oracle_matches_reference_fixture(name):
     assert rel_err(zN, g["z_T_nonoise"]) < 1e-5
     # the reference's own fp32 error budget against fp64 truth stays far inside the parity tolerance
     assert rel_err(g["z_T"], g["z_T_fp64"]) < 1e-5
+
+
+@pytest.mark.parametrize("name", CASES)
+def test_oracle_forward_passes_match_the_reference_outputs(name):
+    # test_oracle_matches_reference_live's comparison against the reference's outputs stored in the fixtures:
+    # generator_forward against its netG(z), flow_forward against its netF(z) (z1, log-det)
+    g = load_golden(name)
+    c = g["config"]
+    B, nz = c["B"], c["nz"]
+    z = torch.from_numpy(g["z0"])
+    z1, ld = refpath.flow_forward(to_torch(synth.flow_state(nz, c["f_width"], 5, c["coupling"], 2, seed=1)),
+                                  z.reshape(B, nz), torch.zeros(B), 5, c["coupling"])
+    assert rel_err(z1, g["flow_z1"]) < 1e-6 and rel_err(ld, g["flow_logdet"]) < 1e-6
+    if c["dataset"]:
+        gp = to_torch(synth.generator_state(c["dataset"], nz, c["ngf"], 3, seed=1))
+        xh = refpath.generator_forward(gp, z, refpath.generator_layers(c["dataset"], nz, c["ngf"], 3))
+        assert rel_err(xh, g["x_hat"]) < 1e-6
 
 
 def test_parameter_updates_match_the_reference_training_iterations_fixture():
@@ -126,9 +143,13 @@ def test_state_dict_key_inventory():
         assert mine == [str(s) for s in k["gen_" + ds]]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/model.py"), reason="reference tree not present")
+REFERENCE = os.environ.get("LSNF_REFERENCE")
+
+
+@pytest.mark.skipif(not (REFERENCE and os.path.exists(os.path.join(REFERENCE, "model.py"))),
+                    reason="LSNF_REFERENCE does not name a checkout of the reference")
 def test_oracle_matches_reference_live():
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE)
     import model as ref_model
     sys.path.pop(0)
     from oracle.make_golden import ref_args
