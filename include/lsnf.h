@@ -15,6 +15,8 @@
  *   lsnf_generator_param_grads <- loss_g = mse(G(z_k), x) / B; loss_g.backward()  train.py:390-394
  *   lsnf_flow_param_grads    <- loss_f = -ll.mean(); loss_f.backward()    train.py:403-411, model.py:182
  *   lsnf_adam_step           <- optG.step() / optF.step() (torch.optim.Adam) train.py:294-295, :398, :415
+ *   lsnf_generator_vjp       <- backward of netG(z) for any loss (torch.autograd through lsnf_b200.kernel_autograd)
+ *   lsnf_flow_vjp            <- backward of netF(z, objective) for any loss (same)
  *   lsnf_pack_*              <- parameters of _netG / _netF               model.py:48-157, :460-498
  *
  * Conventions: every function returns 0 on success and a negative lsnf_status otherwise;
@@ -188,6 +190,18 @@ int lsnf_flow_param_grads(lsnf_plan* plan, const float* z, int32_t global_batch,
  * `step` is the 1-based count AFTER this update.  grad_scale: nullable device scalar (gradient-norm clipping).
  * grad_kk / grad_inner (nullable): gradient i is stored tap-major [kk][outer][inner] for a parameter laid out
  * [outer][inner][kk] (ConvTranspose2d weights); kk <= 1 means same layout as the parameter.  No plan needed. */
+/* ---- vector-Jacobian products for any loss (autograd through the kernels) ------------------------------ */
+/* dL/dz [B,nz] (nullable) and, on a plan created with train != 0, the parameter gradients (nullable; layout of
+ * lsnf_generator_grad_layout, overwritten) of L for upstream grad_x_hat = dL/dx_hat [B,nc,H,W], at the z of the last
+ * lsnf_generator_forward on this plan.  Runs the data-gradient chain of lsnf_generator_dgrad and the weight-gradient
+ * GEMMs of lsnf_generator_param_grads from the seed grad_x_hat * (1 - x_hat^2), at scale 1.  Needs the 3-pass data
+ * gradient: a plan with bwd_passes == 1 returns LSNF_ERR_UNSUPPORTED.  Deterministic. */
+int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, float* grad_z, float* grads, lsnf_stream stream);
+/* z [B,nz]; upstream grad_z_out [B,nz] and grad_logdet [B] (either nullable = 0) -> grad_z [B,nz] (nullable) and the
+ * flow parameter gradients (nullable; layout of lsnf_flow_grad_layout; needs w_inverse for W). Deterministic. */
+int lsnf_flow_vjp(lsnf_plan* plan, const float* z, const float* grad_z_out, const float* grad_logdet, float* grad_z,
+                  float* grads, lsnf_stream stream);
+
 int lsnf_adam_step(int32_t n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,
                    float* const* exp_avg_sq, const int64_t* sizes, const int32_t* grad_kk, const int32_t* grad_inner,
                    float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,

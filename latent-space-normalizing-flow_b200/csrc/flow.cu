@@ -22,6 +22,10 @@ struct FlowArgs {
   uint32_t ring_floats;  // shared-memory ring that streams the matrices
   float* stash;          // TRAIN instantiation: per-layer, per-sample vectors the parameter gradients are built from
   FlowStash sl;
+  // upstream gradients of the backward (lsnf_flow_vjp): dL/dz_out [B][nz] and dL/dlogdet [B].  Both null: the seeds of
+  // -sum_b log p(z_b), g = z_out and dL/dlogdet = -1; otherwise a null one stands for zero
+  const float* seed_g;
+  const float* seed_ld;
 };
 
 constexpr int FLOW_THREADS = 256;
@@ -398,10 +402,21 @@ __global__ void __launch_bounds__(FLOW_THREADS) flow_forward_kernel(FlowArgs a) 
       if (s < ns) a.z_out[(size_t)(b0 + s) * nz + j] = AT(cur, s, j);
     }
   if (!a.grad) return;
+  // the backward overwrites cur in place (g2p below, with another thread-to-element mapping): every thread must be
+  // done reading it for the z_out store first
+  if (a.z_out) __syncthreads();
 
-  // ---- analytic backward of -sum_b ll_b: seed g = z_out, d/dlogdet = -1 ----
+  // ---- analytic backward of -sum_b ll_b: seed g = z_out, d/dlogdet = -1 (or the caller's seeds) ----
   float* g = cur;  // in place, [nz][S]
   float* g2p = g + S * half;
+  const bool seeded = a.seed_g || a.seed_ld;
+  if (seeded) {
+    for (int i = tid; i < S * nz; i += FLOW_THREADS) {
+      const int s = i / nz, j = i % nz;
+      AT(g, s, j) = (a.seed_g && s < ns) ? a.seed_g[(size_t)(b0 + s) * nz + j] : 0.f;
+    }
+    __syncthreads();
+  }
   for (int L = a.depth - 1; L >= 0; --L) {
     const float* P = fd.next_vec();
     float* st = stash + (size_t)L * S * stash_step;
@@ -411,24 +426,36 @@ __global__ void __launch_bounds__(FLOW_THREADS) flow_forward_kernel(FlowArgs a) 
     const float* xs = sc + S * half;
     // gradient w.r.t. the MLP output h, already multiplied by e3 = exp(3 logs_zeros)
     if (a.coupling == 1) {
-      for (int i = tid; i < S * half; i += FLOW_THREADS) {
-        const int s = i % S, j = i / S;
-        const float g2 = g2p[i], scale = sc[i];
-        const float g_shift = g2 * scale;
-        const float g_scale = g2 * xs[i] - 1.f / scale;
-        const float gh0 = g_shift, gh1 = g_scale * scale * (1.f - scale);
-        AT(ta, s, 2 * j) = gh0 * P[f.e3 + 2 * j];
-        AT(ta, s, 2 * j + 1) = gh1 * P[f.e3 + 2 * j + 1];
-        g2p[i] = g_shift;  // = g_x2
-        if constexpr (TRAIN) {
-          if (s < ns) {   // d/dlogs of h = (p + b) * exp(3 logs) is 3 h (model.py:348)
-            const float* hrow = stash_at(a, L, a.sl.h, n_out, b0 + s, 2 * j);
-            float* gl = stash_at(a, L, a.sl.gl3, n_out, b0 + s, 2 * j);
-            gl[0] = 3.f * gh0 * hrow[0];
-            gl[1] = 3.f * gh1 * hrow[1];
+      // d/dscale of the step's output and of logdet += log(scale) is g2 * x2s - (-dL/dlogdet) / scale.  The default
+      // seed's loop and the caller-seeded one are separate instances of the same expression, so that the default keeps
+      // its own rounding and a caller seed of -1 reproduces it bit for bit.
+      auto coupling_bwd = [&](auto g_scale_of) {
+        for (int i = tid; i < S * half; i += FLOW_THREADS) {
+          const int s = i % S, j = i / S;
+          const float g2 = g2p[i], scale = sc[i];
+          const float g_shift = g2 * scale;
+          const float g_scale = g_scale_of(g2, xs[i], scale, s);
+          const float gh0 = g_shift, gh1 = g_scale * scale * (1.f - scale);
+          AT(ta, s, 2 * j) = gh0 * P[f.e3 + 2 * j];
+          AT(ta, s, 2 * j + 1) = gh1 * P[f.e3 + 2 * j + 1];
+          g2p[i] = g_shift;  // = g_x2
+          if constexpr (TRAIN) {
+            if (s < ns) {   // d/dlogs of h = (p + b) * exp(3 logs) is 3 h (model.py:348)
+              const float* hrow = stash_at(a, L, a.sl.h, n_out, b0 + s, 2 * j);
+              float* gl = stash_at(a, L, a.sl.gl3, n_out, b0 + s, 2 * j);
+              gl[0] = 3.f * gh0 * hrow[0];
+              gl[1] = 3.f * gh1 * hrow[1];
+            }
           }
         }
-      }
+      };
+      if (seeded)
+        coupling_bwd([&](float g2, float x2s, float scale, int s) {
+          const float neg_ld = (a.seed_ld && s < ns) ? -a.seed_ld[b0 + s] : 0.f;
+          return g2 * x2s - neg_ld / scale;
+        });
+      else
+        coupling_bwd([](float g2, float x2s, float scale, int) { return g2 * x2s - 1.f / scale; });
     } else {
       for (int i = tid; i < S * half; i += FLOW_THREADS) {
         const int s = i % S, j = i / S;
@@ -869,6 +896,7 @@ int launch_flow_forward(const lsnf_plan* plan, const float* z, float* z_out, flo
   a.coupling = plan->cfg.f_coupling; a.permutation = plan->cfg.f_permutation;
   a.in = z; a.z_out = z_out; a.logdet = logdet; a.logp = logp; a.grad = grad_z;
   a.stash = nullptr;
+  a.seed_g = a.seed_ld = nullptr;
   return launch_flow_fwd_args(a, s);
 }
 
@@ -878,6 +906,7 @@ int launch_flow_forward(const lsnf_plan* plan, const float* z, float* z_out, flo
 // the batch: matrices dM[k][n] = sum_b X[b][k] G[b][n], vectors = column sums.
 //   d invertible_1x1_conv.w = y^T g_u - B_local * W^-T     (d log|det W| / dW = W^-T, model.py:182)
 //   d actnorm.b = colsum(g_x),  d actnorm.logs = colsum(gl0) - 3 B_local   (logdet += sum 3 logs, model.py:273-276)
+// (with the caller's dL/dlogdet seeds of lsnf_flow_vjp, -B_local becomes sum_b seed_ld[b], summed in a fixed order)
 //   d fc_k.w = in_k^T g_pk,  d fc_k.actnorm.b = colsum(g_pk),  d fc_k.actnorm.logs = colsum(gl_k)   (k = 1, 2)
 //   d fc_zeros.w = a2^T g_p3,  d fc_zeros.b = colsum(g_p3),  d fc_zeros.logs = colsum(gl3)
 // all multiplied by 1 / B_global.  Summation over the batch is in a fixed order: deterministic.
@@ -891,6 +920,8 @@ struct ParamGradArgs {
   const float* logp;     // [B]
   float* grads;          // flat, FlowGradLayout per step
   float* loss;           // -(1 / B_global) sum_b logp_b
+  int seeded;            // lsnf_flow_vjp: the log-det coefficients come from seed_ld (nullable = 0)
+  const float* seed_ld;  // [B]
   FlowLayout fl;
   FlowStash sl;
   FlowGradLayout gl;
@@ -920,6 +951,28 @@ __device__ __forceinline__ void pg_colsum(const float* V, int N, int B, float sc
   }
 }
 
+// sum of v[0..n) over the CTA in a fixed order (strided partial sums, then a tree): deterministic; every thread gets it
+__device__ __forceinline__ float fixed_order_sum(const float* v, int n) {
+  __shared__ float red[256];
+  float acc = 0.f;
+  for (int b = threadIdx.x; b < n; b += blockDim.x) acc += v[b];
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  const float r = red[0];
+  __syncthreads();
+  return r;
+}
+
+// d loss / d logdet summed over the batch: -B for -sum_b ll_b, or sum_b seed_ld[b]
+__device__ __forceinline__ float logdet_coef(const ParamGradArgs& a) {
+  if (!a.seeded) return -(float)a.B;
+  return a.seed_ld ? fixed_order_sum(a.seed_ld, a.B) : 0.f;
+}
+
 __global__ void __launch_bounds__(256) flow_param_grad_kernel(ParamGradArgs a) {
   const int L = blockIdx.y;
   const FlowLayout& f = a.fl;
@@ -931,7 +984,7 @@ __global__ void __launch_bounds__(256) flow_param_grad_kernel(ParamGradArgs a) {
   if (blk < a.blocks_w) {
     if (a.permutation == 2)
       pg_matrix(slot(a.sl.y), nz, slot(a.sl.gu), nz, B, blk * PG_ROWS, a.inv_bg, g + a.gl.off[2],
-                a.params + (size_t)L * f.step_floats + f.Winv, nz, -(float)B);
+                a.params + (size_t)L * f.step_floats + f.Winv, nz, logdet_coef(a));
     return;
   }
   blk -= a.blocks_w;
@@ -952,7 +1005,7 @@ __global__ void __launch_bounds__(256) flow_param_grad_kernel(ParamGradArgs a) {
   blk -= a.blocks_w3;
   if (blk == 0) {
     pg_colsum(slot(a.sl.gx), nz, B, a.inv_bg, 0.f, g + a.gl.off[0]);
-    pg_colsum(slot(a.sl.gl0), nz, B, a.inv_bg, -3.f * (float)B, g + a.gl.off[1]);
+    pg_colsum(slot(a.sl.gl0), nz, B, a.inv_bg, 3.f * logdet_coef(a), g + a.gl.off[1]);
   } else if (blk == 1) {
     pg_colsum(slot(a.sl.gp1), w, B, a.inv_bg, 0.f, g + a.gl.off[4]);
     pg_colsum(slot(a.sl.gl1), w, B, a.inv_bg, 0.f, g + a.gl.off[5]);
@@ -964,34 +1017,30 @@ __global__ void __launch_bounds__(256) flow_param_grad_kernel(ParamGradArgs a) {
     pg_colsum(slot(a.sl.gl3), n_out, B, a.inv_bg, 0.f, g + a.gl.off[11]);
   } else if (L == 0 && a.loss) {
     // loss_f = -mean_b ll_b over the global batch (this rank's partial sum), fixed-order tree
-    __shared__ float red[256];
-    float acc = 0.f;
-    for (int b = threadIdx.x; b < B; b += blockDim.x) acc += a.logp[b];
-    red[threadIdx.x] = acc;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-      if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
-      __syncthreads();
-    }
-    if (threadIdx.x == 0) *a.loss = -red[0] * a.inv_bg;
+    const float sum = fixed_order_sum(a.logp, B);
+    if (threadIdx.x == 0) *a.loss = -sum * a.inv_bg;
   }
 }
 
-int launch_flow_param_grads(const lsnf_plan* plan, const float* z, float inv_global_batch, float* grads, float* loss,
-                            cudaStream_t s) {
+// the TRAIN instantiation of the fused kernel (stash written), then the parameter-gradient reductions
+static int flow_grads(const lsnf_plan* plan, const float* z, const float* seed_g, const float* seed_ld, float* grad_z,
+                      float inv_global_batch, float* grads, float* loss, cudaStream_t s) {
   FlowArgs a;
   a.params = (const float*)(plan->ws + plan->off_flow);
   a.fl = plan->fl; a.depth = plan->cfg.f_depth; a.B = plan->cfg.batch;
   a.coupling = plan->cfg.f_coupling; a.permutation = plan->cfg.f_permutation;
   float* fo = (float*)(plan->ws + plan->off_flow_out);   // z_out [B][nz], logdet [B], logp [B]
   a.in = z; a.z_out = nullptr; a.logdet = nullptr; a.logp = fo + (size_t)a.B * a.fl.nz + a.B;
-  a.grad = (float*)(plan->ws + plan->off_gradf);         // the kernel's backward needs a destination; unused here
+  // the kernel's backward needs a destination even when the caller does not want dL/dz
+  a.grad = grad_z ? grad_z : (float*)(plan->ws + plan->off_gradf);
   a.stash = (float*)(plan->ws + plan->off_fstash);
   a.sl = plan->fstash;
+  a.seed_g = seed_g; a.seed_ld = seed_ld;
   int rc = launch_flow_fwd_args(a, s);
   if (rc) return rc;
   ParamGradArgs p;
   p.stash = a.stash; p.params = a.params; p.logp = a.logp; p.grads = grads; p.loss = loss;
+  p.seeded = (seed_g || seed_ld) ? 1 : 0; p.seed_ld = seed_ld;
   p.fl = plan->fl; p.sl = plan->fstash; p.gl = plan->fgrad;
   p.B = a.B; p.permutation = a.permutation; p.inv_bg = inv_global_batch;
   p.blocks_w = (a.fl.nz + PG_ROWS - 1) / PG_ROWS;
@@ -1004,12 +1053,31 @@ int launch_flow_param_grads(const lsnf_plan* plan, const float* z, float inv_glo
   return LSNF_OK;
 }
 
+int launch_flow_param_grads(const lsnf_plan* plan, const float* z, float inv_global_batch, float* grads, float* loss,
+                            cudaStream_t s) {
+  return flow_grads(plan, z, nullptr, nullptr, nullptr, inv_global_batch, grads, loss, s);
+}
+
+int launch_flow_vjp(const lsnf_plan* plan, const float* z, const float* seed_g, const float* seed_ld, float* grad_z,
+                    float* grads, cudaStream_t s) {
+  if (grads) return flow_grads(plan, z, seed_g, seed_ld, grad_z, 1.f, grads, nullptr, s);
+  FlowArgs a;
+  a.params = (const float*)(plan->ws + plan->off_flow);
+  a.fl = plan->fl; a.depth = plan->cfg.f_depth; a.B = plan->cfg.batch;
+  a.coupling = plan->cfg.f_coupling; a.permutation = plan->cfg.f_permutation;
+  a.in = z; a.z_out = nullptr; a.logdet = nullptr; a.logp = nullptr; a.grad = grad_z;
+  a.stash = nullptr;
+  a.seed_g = seed_g; a.seed_ld = seed_ld;
+  return launch_flow_fwd_args(a, s);
+}
+
 int launch_flow_inverse(const lsnf_plan* plan, const float* eps, float* z, float* negobj, cudaStream_t s) {
   FlowArgs a;
   a.params = (const float*)(plan->ws + plan->off_flow);
   a.fl = plan->fl; a.depth = plan->cfg.f_depth; a.B = plan->cfg.batch;
   a.coupling = plan->cfg.f_coupling; a.permutation = plan->cfg.f_permutation;
   a.in = eps; a.z_out = z; a.logdet = negobj; a.logp = nullptr; a.grad = nullptr; a.stash = nullptr;
+  a.seed_g = a.seed_ld = nullptr;
   const int S = pick_s(a.B);
   const size_t fixed = flow_fixed_floats(a.fl, S, a.depth, false);
   if (flow_ring_floats(a.fl, fixed, a.depth, false, &a.ring_floats)) {

@@ -177,7 +177,9 @@ int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s) {
 // seed of the reconstruction gradient (train.py:313-314):
 //   g[b,c,oy,ox] = (x_hat - x) / sigma^2 * (1 - x_hat^2)          (MSE-sum derivative times tanh')
 // of which only seed_scale = sigma_seed_scale(sigma) <= 16 (a power of two) is applied here; the rest of 1/sigma^2
-// multiplies the fp32 sum of the first layer's split-K partials (langevin_update_kernel / reduce_partial_kernel),
+// multiplies the fp32 sum of the first layer's split-K partials (langevin_update_kernel / reduce_partial_kernel).
+// With upstream != 0, `x` is a caller-supplied dL/dx_hat and the seed is g = x * seed_scale * (1 - x_hat^2) (the
+// vector-Jacobian product of lsnf_generator_vjp, seed_scale 1).  Either seed is
 // written directly as the im2col operand of the last layer's data gradient:
 //   A[b][iy][ix][tap*nc + c] = g[b][c][iy*s - p + ky][ix*s - p + kx]  (0 outside the image), 64 columns.
 // ---------------------------------------------------------------------------------------------------
@@ -189,7 +191,7 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
                                                                 const float* __restrict__ x,
                                                                 uint16_t* __restrict__ a, int B, int nc, int img,
                                                                 int hin, int k, int s, int p, float seed_scale,
-                                                                int fp16) {
+                                                                int fp16, int upstream) {
   extern __shared__ float g[];   // [nc][k][span], span = (seg-1)*s + k
   const int segs = (hin + IM2COL_SEG - 1) / IM2COL_SEG;
   const int seg = blockIdx.x % segs, iy = (blockIdx.x / segs) % hin, b = blockIdx.x / (segs * hin);
@@ -203,7 +205,7 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
     if (oy >= 0 && oy < img && ox >= 0 && ox < img) {
       const size_t o = (((size_t)b * nc + c) * img + oy) * img + ox;
       const float xh = xhat[o];
-      v = (xh - x[o]) * seed_scale * (1.f - xh * xh);
+      v = (upstream ? x[o] : xh - x[o]) * seed_scale * (1.f - xh * xh);
     }
     g[i] = v;
   }
@@ -223,14 +225,14 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
   }
 }
 
-int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float sigma, cudaStream_t s) {
+int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float seed_scale, int upstream, cudaStream_t s) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const int segs = (y.hin + IM2COL_SEG - 1) / IM2COL_SEG;
   const int span = (std::min(IM2COL_SEG, y.hin) - 1) * y.s + y.k;
   const size_t smem = (size_t)plan->cfg.nc * y.k * span * 4;
   recon_grad_im2col_kernel<<<plan->cfg.batch * y.hin * segs, 128, smem, s>>>(
       (const float*)(plan->ws + plan->off_xhat), x, (uint16_t*)(plan->ws + plan->off_im2col), plan->cfg.batch,
-      plan->cfg.nc, plan->img, y.hin, y.k, y.s, y.p, sigma_seed_scale(sigma), plan->cfg.bwd_passes == 1 ? 1 : 0);
+      plan->cfg.nc, plan->img, y.hin, y.k, y.s, y.p, seed_scale, plan->cfg.bwd_passes == 1 ? 1 : 0, upstream);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;
 }

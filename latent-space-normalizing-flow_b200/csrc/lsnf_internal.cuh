@@ -275,7 +275,7 @@ int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);
 int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s);
-int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float sigma, cudaStream_t s);
+int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float seed_scale, int upstream, cudaStream_t s);
 int launch_last_fused(const lsnf_plan* plan, const float* x, float seed_scale, cudaStream_t s);
 int launch_transpose_hl(const TransArgs& a, cudaStream_t s);
 int launch_wgrad_finalize(const FinalizeArgs& a, cudaStream_t s);
@@ -296,6 +296,10 @@ int launch_flow_logdet_inverse(const lsnf_plan* plan, const float* const* params
                                cudaStream_t s);
 int launch_flow_param_grads(const lsnf_plan* plan, const float* z, float inv_global_batch, float* grads, float* loss,
                             cudaStream_t s);
+// lsnf_flow_vjp: the fused forward + backward seeded with seed_g = dL/dz_out and seed_ld = dL/dlogdet (either nullable
+// = 0, not both), then -- when grads != nullptr -- the parameter-gradient reductions at scale 1
+int launch_flow_vjp(const lsnf_plan* plan, const float* z, const float* seed_g, const float* seed_ld, float* grad_z,
+                    float* grads, cudaStream_t s);
 int launch_update(const lsnf_plan* plan, float* z, const float* gg, const float* partial, int nsplit, float gscale,
                   const float* gf, float step, const float* eps, int with_noise, uint64_t seed,
                   uint64_t sample_offset, uint32_t step_idx, const uint64_t* dyn, float* gnorms,

@@ -734,7 +734,7 @@ static int gen_forward(lsnf_plan* p, const float* z, float* x_hat, cudaStream_t 
 
 static int gen_dgrad_partial(lsnf_plan* p, const float* x, float sigma, cudaStream_t s) {
   int rc;
-  if ((rc = launch_recon_grad_im2col(p, x, sigma, s))) return rc;
+  if ((rc = launch_recon_grad_im2col(p, x, sigma_seed_scale(sigma), 0, s))) return rc;
   for (int i = p->n_layers; i < 2 * p->n_layers; ++i)
     if ((rc = run_stage(p, p->stages[i], s))) return rc;
   return LSNF_OK;
@@ -792,6 +792,36 @@ extern "C" int lsnf_generator_grad_layout(const lsnf_plan* plan, int64_t* offset
   return LSNF_OK;
 }
 
+// LSNF_SYNC_DEBUG=1: synchronise after every step of the generator's parameter gradients and name the one that failed
+static int sync_check(cudaStream_t s, const char* what, int l) {
+  static const bool dbg = [] { const char* e = getenv("LSNF_SYNC_DEBUG"); return e && e[0] == '1'; }();
+  if (!dbg) return 0;
+  cudaError_t e = cudaStreamSynchronize(s);
+  if (e == cudaSuccess) return 0;
+  set_error(std::string("CUDA error: ") + cudaGetErrorString(e) + " after " + what + " of layer " + std::to_string(l));
+  return LSNF_ERR_CUDA;
+}
+
+// weight and bias gradient of layer l from the activations and the data-gradient tensors in the workspace, times scale
+static int gen_layer_grads(lsnf_plan* plan, int l, float* grads, float scale, cudaStream_t s) {
+  const int L = plan->n_layers;
+  int rc;
+  WgradLayer& w = plan->wg[l];
+  TransArgs ta = w.ta, tg = w.tg;
+  ta.src = (const uint16_t*)(plan->ws + (l == 0 ? plan->off_zhl : plan->off_act[l - 1]));
+  tg.src = (const uint16_t*)(plan->ws + (l == L - 1 ? plan->off_im2col : plan->off_gpre[l]));
+  if ((rc = launch_transpose_hl(ta, s)) || (rc = sync_check(s, "activation transpose", l))) return rc;
+  if ((rc = launch_transpose_hl(tg, s)) || (rc = sync_check(s, "gradient transpose", l))) return rc;
+  if ((rc = launch_tapgemm_tc(w.st, s)) || (rc = sync_check(s, "weight-gradient tap-GEMM", l))) return rc;
+  FinalizeArgs f = w.fin;
+  f.out = grads + w.grad_w_off; f.scale = scale;
+  if ((rc = launch_wgrad_finalize(f, s)) || (rc = sync_check(s, "finalize", l))) return rc;
+  RowSumArgs r = w.rs;
+  r.out = grads + w.grad_b_off; r.scale = scale;
+  if ((rc = launch_bias_rowsum(r, s)) || (rc = sync_check(s, "bias row sums", l))) return rc;
+  return LSNF_OK;
+}
+
 extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const float* x, int32_t global_batch,
                                           float* grads, float* loss, int32_t part, lsnf_stream stream) {
   int rc = need(plan, true, false);
@@ -804,19 +834,10 @@ extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const
   const lsnf_config& c = plan->cfg;
   const int L = plan->n_layers;
   const bool prologue = part < 0, layers_all = part == -1;
-  // LSNF_SYNC_DEBUG=1: synchronise after every step and name the one that failed
-  static const bool dbg = [] { const char* e = getenv("LSNF_SYNC_DEBUG"); return e && e[0] == '1'; }();
-  auto check = [&](const char* what, int l) -> int {
-    if (!dbg) return 0;
-    cudaError_t e = cudaStreamSynchronize(s);
-    if (e == cudaSuccess) return 0;
-    set_error(std::string("CUDA error: ") + cudaGetErrorString(e) + " after " + what + " of layer " + std::to_string(l));
-    return LSNF_ERR_CUDA;
-  };
   if (prologue) {
     // x_hat = G(z_k) (train.py:392) and loss_g = mse_sum / B (train.py:393)
     if ((rc = gen_forward(plan, z, nullptr, s, true))) return rc;
-    if ((rc = check("generator forward", -1))) return rc;
+    if ((rc = sync_check(s, "generator forward", -1))) return rc;
     const long long npix = (long long)c.batch * c.nc * plan->img * plan->img;
     // partial sums in the (idle) norm scratch of the update kernel, ticket next to its own
     if (loss && (rc = launch_mse_sum((const float*)(plan->ws + plan->off_xhat), x, npix, 1.f / (float)global_batch,
@@ -828,7 +849,7 @@ extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const
     if ((rc = launch_last_fused(plan, x, 1.f, s))) return rc;
     for (int i = L; i < 2 * L - 1; ++i)
       if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
-    if ((rc = check("data-gradient chain", -1))) return rc;
+    if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
     plan->wg_ready = true;
     if (!layers_all) return LSNF_OK;
   }
@@ -837,20 +858,35 @@ extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const
   const float scale = 2.f / (float)global_batch;
   for (int l = L - 1; l >= 0; --l) {
     if (!layers_all && l != part) continue;
-    WgradLayer& w = plan->wg[l];
-    TransArgs ta = w.ta, tg = w.tg;
-    ta.src = (const uint16_t*)(plan->ws + (l == 0 ? plan->off_zhl : plan->off_act[l - 1]));
-    tg.src = (const uint16_t*)(plan->ws + (l == L - 1 ? plan->off_im2col : plan->off_gpre[l]));
-    if ((rc = launch_transpose_hl(ta, s)) || (rc = check("activation transpose", l))) return rc;
-    if ((rc = launch_transpose_hl(tg, s)) || (rc = check("gradient transpose", l))) return rc;
-    if ((rc = launch_tapgemm_tc(w.st, s)) || (rc = check("weight-gradient tap-GEMM", l))) return rc;
-    FinalizeArgs f = w.fin;
-    f.out = grads + w.grad_w_off; f.scale = scale;
-    if ((rc = launch_wgrad_finalize(f, s)) || (rc = check("finalize", l))) return rc;
-    RowSumArgs r = w.rs;
-    r.out = grads + w.grad_b_off; r.scale = scale;
-    if ((rc = launch_bias_rowsum(r, s)) || (rc = check("bias row sums", l))) return rc;
+    if ((rc = gen_layer_grads(plan, l, grads, scale, s))) return rc;
   }
+  return LSNF_OK;
+}
+
+extern "C" int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, float* grad_z, float* grads,
+                                  lsnf_stream stream) {
+  int rc = need(plan, true, false);
+  if (rc) return rc;
+  if (!grad_x_hat) return fail(LSNF_ERR_INVALID, "null grad_x_hat");
+  if (plan->cfg.bwd_passes == 1)
+    return fail(LSNF_ERR_UNSUPPORTED, "the vector-Jacobian product needs the 3-pass bf16 data gradient (bwd_passes 1 "
+                                      "has fp16's range, too narrow for an arbitrary upstream gradient)");
+  if (grads && plan->wg.empty()) return fail(LSNF_ERR_STATE, "plan was created without lsnf_config.train");
+  if (grads && plan->cfg.gemm_impl != LSNF_GEMM_TCGEN05)
+    return fail(LSNF_ERR_UNSUPPORTED, "weight gradients need the tcgen05 path");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int L = plan->n_layers;
+  // seed g = dL/dx_hat * (1 - x_hat^2) at scale 1 (bf16 keeps fp32's exponent range), x_hat of the last forward pass
+  if ((rc = launch_recon_grad_im2col(plan, grad_x_hat, 1.f, 1, s))) return rc;
+  const int end = grad_z ? 2 * L : 2 * L - 1;   // the first layer's data gradient only feeds dL/dz
+  for (int i = L; i < end; ++i)
+    if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
+  if (grad_z && (rc = launch_reduce_partial(plan, grad_z, 1.f, s))) return rc;
+  // the gradient tensors no longer hold the part = -2 state of lsnf_generator_param_grads
+  plan->wg_ready = false;
+  if (grads)
+    for (int l = L - 1; l >= 0; --l)
+      if ((rc = gen_layer_grads(plan, l, grads, 1.f, s))) return rc;
   return LSNF_OK;
 }
 
@@ -876,6 +912,24 @@ extern "C" int lsnf_flow_param_grads(lsnf_plan* plan, const float* z, int32_t gl
   if (plan->cfg.f_permutation == 2 && !plan->have_winv)
     return fail(LSNF_ERR_STATE, "flow weights were packed without w_inverse (needed for d log|det W| / dW = W^-T)");
   return launch_flow_param_grads(plan, z, 1.f / (float)global_batch, grads, loss, (cudaStream_t)stream);
+}
+
+extern "C" int lsnf_flow_vjp(lsnf_plan* plan, const float* z, const float* grad_z_out, const float* grad_logdet,
+                             float* grad_z, float* grads, lsnf_stream stream) {
+  int rc = need(plan, false, true);
+  if (rc) return rc;
+  if (!z) return fail(LSNF_ERR_INVALID, "null z");
+  if (grads && plan->cfg.f_permutation == 2 && !plan->have_winv)
+    return fail(LSNF_ERR_STATE, "flow weights were packed without w_inverse (needed for d log|det W| / dW = W^-T)");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!grad_z_out && !grad_logdet) {
+    // a zero upstream gradient (the fused kernel reads two null seeds as those of -sum_b log p)
+    if (grad_z) LSNF_CUDA(cudaMemsetAsync(grad_z, 0, (size_t)plan->cfg.batch * plan->cfg.nz * 4, s));
+    if (grads) LSNF_CUDA(cudaMemsetAsync(grads, 0, lsnf_flow_grad_floats(plan) * 4, s));
+    return LSNF_OK;
+  }
+  if (!grad_z && !grads) return LSNF_OK;
+  return launch_flow_vjp(plan, z, grad_z_out, grad_logdet, grad_z, grads, s);
 }
 
 extern "C" int lsnf_adam_step(int32_t n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,

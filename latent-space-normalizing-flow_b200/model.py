@@ -9,6 +9,8 @@ Execution:
     run as ordinary differentiable torch ops, so code written against the reference modules (including its own
     autograd-based Langevin closure) keeps working.  That branch is not part of the Langevin path:
     ``sample_langevin_post_z_with_flow`` and ``train.training_iteration`` never take it.
+  * Under ``lsnf_b200.kernel_autograd()`` such calls on float32 CUDA tensors instead run the kernels forward and
+    their vector-Jacobian products backward (``autograd_fns``); CPU tensors and the reverse flow pass stay eager.
 """
 from __future__ import annotations
 
@@ -17,7 +19,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import synth
+from . import autograd_fns, synth
 from .plan import get_plan
 
 
@@ -46,6 +48,11 @@ def _autograd_needed(module: nn.Module, *tensors) -> bool:
     if any(t.requires_grad for t in tensors if isinstance(t, torch.Tensor)):
         return True
     return module.training and any(p.requires_grad for p in module.parameters())
+
+
+def _kernel_autograd(z) -> bool:
+    """A differentiable call takes the kernels' autograd Functions: ``kernel_autograd`` is on and z is float32 CUDA."""
+    return autograd_fns.is_enabled() and z.is_cuda and z.dtype == torch.float32
 
 
 class _netG(nn.Module):
@@ -93,6 +100,8 @@ class _netG(nn.Module):
 
     def forward(self, z):
         if _autograd_needed(self, z):
+            if _kernel_autograd(z):
+                return autograd_fns.generator_apply(self, z)
             return self.gen(z)
         return self.generate(z)
 
@@ -284,6 +293,10 @@ class _netF(nn.Module):
         if init:
             raise NotImplementedError("data-dependent actnorm init is never enabled upstream (train.py:316,406,614)")
         if _autograd_needed(self, z, objective):
+            if not reverse and _kernel_autograd(z):
+                assert len(z.shape) == 2                                # model.py:237
+                z_out, logdet = autograd_fns.flow_apply(self, z)
+                return z_out, objective + logdet, []                   # model.py:483
             z, objective = self._eager(z, objective, reverse)
             if not reverse:
                 return z, objective, []

@@ -71,6 +71,9 @@ class Plan:
         self._f_sig = None
         self._f_has_inv = False
         self._keep = []  # tensors referenced by in-flight pack kernels
+        # bumped by every call that overwrites the generator activations in the workspace (and by a re-pack, which
+        # makes them stale): a backward pass that finds it moved re-runs its forward pass before lsnf_generator_vjp
+        self.act_epoch = 0
         from .synth import image_size
         self.img = image_size(arch) if arch != "none" else 0
 
@@ -92,6 +95,7 @@ class Plan:
         return out
 
     def run_stage(self, index: int) -> None:
+        self.act_epoch += 1
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.lsnf_plan_run_stage(self.handle, int(index), _stream(self.device)), "lsnf_plan_run_stage")
 
@@ -137,6 +141,7 @@ class Plan:
             _cabi.check(self.lib.lsnf_pack_generator_weights(self.handle, wp, bp, len(ws), C.c_void_p(_stream(self.device))),
                         "lsnf_pack_generator_weights")
         self._g_sig = sig
+        self.act_epoch += 1
 
     def ensure_flow(self, netF, need_inverse: bool = False) -> None:
         steps = netF.revnet2d_s[0].revnet2d_step_s
@@ -187,6 +192,7 @@ class Plan:
     def generator_forward(self, z: torch.Tensor) -> torch.Tensor:
         _check_tensor(z, "z", self.device, (self.batch, self.nz))
         out = torch.empty(self.batch, self.nc, self.img, self.img, dtype=torch.float32, device=self.device)
+        self.act_epoch += 1
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.lsnf_generator_forward(self.handle, z.data_ptr(), out.data_ptr(), _stream(self.device)),
                         "lsnf_generator_forward")
@@ -199,6 +205,43 @@ class Plan:
             _cabi.check(self.lib.lsnf_generator_dgrad(self.handle, x.data_ptr(), float(sigma), g.data_ptr(),
                                                       _stream(self.device)), "lsnf_generator_dgrad")
         return g
+
+    def generator_vjp(self, grad_x_hat: torch.Tensor, want_z: bool = True, want_params: bool = False):
+        """(dL/dz [B,nz] or None, flat parameter-gradient buffer or None) for upstream dL/dx_hat, at the z of the last
+        ``generator_forward`` on this plan (``act_epoch`` tells whether that is still the one in the workspace).
+        ``want_params`` needs ``train=True``; the buffer has the layout of ``generator_grad_layout``."""
+        _check_tensor(grad_x_hat, "grad_x_hat", self.device, (self.batch, self.nc, self.img, self.img))
+        g = torch.empty(self.batch, self.nz, dtype=torch.float32, device=self.device) if want_z else None
+        flat = None
+        if want_params:
+            flat = torch.empty(int(self.lib.lsnf_generator_grad_floats(self.handle)), dtype=torch.float32,
+                               device=self.device)
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_generator_vjp(self.handle, grad_x_hat.data_ptr(), g.data_ptr() if want_z else None,
+                                                    flat.data_ptr() if want_params else None, _stream(self.device)),
+                        "lsnf_generator_vjp")
+        return g, flat
+
+    def flow_vjp(self, z: torch.Tensor, grad_z_out: Optional[torch.Tensor], grad_logdet: Optional[torch.Tensor],
+                 want_z: bool = True, want_params: bool = False):
+        """(dL/dz [B,nz] or None, flat parameter-gradient buffer or None) of the forward flow at z for upstream
+        dL/dz_out [B,nz] and dL/dlogdet [B] (either None = 0).  The buffer has the layout of ``flow_grad_layout``;
+        ``want_params`` needs ``ensure_flow(netF, need_inverse=True)``."""
+        _check_tensor(z, "z", self.device, (self.batch, self.nz))
+        if grad_z_out is not None:
+            _check_tensor(grad_z_out, "grad_z_out", self.device, (self.batch, self.nz))
+        if grad_logdet is not None:
+            _check_tensor(grad_logdet, "grad_logdet", self.device, (self.batch,))
+        g = torch.empty_like(z) if want_z else None
+        flat = None
+        if want_params:
+            flat = torch.zeros(int(self.lib.lsnf_flow_grad_floats(self.handle)), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_flow_vjp(
+                self.handle, z.data_ptr(), grad_z_out.data_ptr() if grad_z_out is not None else None,
+                grad_logdet.data_ptr() if grad_logdet is not None else None, g.data_ptr() if want_z else None,
+                flat.data_ptr() if want_params else None, _stream(self.device)), "lsnf_flow_vjp")
+        return g, flat
 
     def flow_forward(self, z: torch.Tensor, want_grad: bool = False):
         _check_tensor(z, "z", self.device, (self.batch, self.nz))
@@ -226,6 +269,7 @@ class Plan:
         _check_tensor(eps, "eps", self.device, (self.batch, self.nz))
         x = torch.empty(self.batch, self.nc, self.img, self.img, dtype=torch.float32, device=self.device)
         z = torch.empty_like(eps) if want_z else None
+        self.act_epoch += 1
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.lsnf_sample_prior(self.handle, eps.data_ptr(), x.data_ptr(),
                                                    z.data_ptr() if want_z else None, int(bool(to_unit_range)),
@@ -255,6 +299,7 @@ class Plan:
         _check_tensor(flat, "flat gradient buffer", self.device, (n,))
         if loss is None:
             loss = torch.empty((), dtype=torch.float32, device=self.device)
+        self.act_epoch += 1
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.lsnf_generator_param_grads(self.handle, z.data_ptr(), x.data_ptr(), int(global_batch),
                                                             flat.data_ptr(), loss.data_ptr(), int(part),
@@ -309,6 +354,7 @@ class Plan:
             out = torch.empty_like(z0)
         if norms is None:
             norms = torch.zeros(2, dtype=torch.float32, device=self.device)
+        self.act_epoch += 1
         with torch.cuda.device(self.device):
             _cabi.check(self.lib.lsnf_langevin_run(
                 self.handle, z0.data_ptr(), x.data_ptr(), int(steps), float(step_size), float(sigma),
