@@ -74,11 +74,18 @@ typedef enum lsnf_gemm_impl {
 typedef struct lsnf_config {
   int32_t arch;          /* lsnf_arch */
   int32_t batch;         /* samples held by this plan (this rank's shard) */
-  int32_t nz;            /* --nz, even (model.py:383) */
+  int32_t nz;            /* --nz, a multiple of 4 in 4..256 (even: model.py:383) */
   int32_t ngf;           /* --ngf */
   int32_t nc;            /* --nc (3) */
-  int32_t f_depth;       /* --f_depth */
-  int32_t f_width;       /* --f_width */
+  int32_t f_depth;       /* --f_depth, 1..32 */
+  int32_t f_width;       /* --f_width, a multiple of 4 in 4..256.  Accepted flow range: one step of the fused flow kernels
+                            must fit the 227 KB of shared memory of one CTA at one sample per CTA -- its largest matrix
+                            (f_width^2 floats, or nz^2 with f_flow_permutation 2) plus f_depth * (2 f_width + nz) floats of
+                            activations plus ~3 KB.  So f_width <= 232 (192 at nz 100, f_depth 32); with
+                            f_flow_permutation 2 nz <= 228 (224 at f_width 64, f_depth 5; 204 at f_depth 32); the shuffle
+                            permutation takes every nz up to 256 (f_width <= 196 there).  lsnf_plan_create refuses a
+                            configuration outside it with LSNF_ERR_INVALID.  A configuration it accepts runs at every batch:
+                            the kernels take fewer samples per CTA where the preferred number does not fit. */
   int32_t f_permutation; /* --f_flow_permutation: 2 = invertible 1x1 (default), 1 = fixed shuffle */
   int32_t f_coupling;    /* --f_flow_coupling: 1 = affine (default), 0 = additive */
   float leak;            /* --g_activation_leak of the LeakyReLU (0.2) */

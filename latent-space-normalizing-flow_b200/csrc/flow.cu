@@ -798,8 +798,9 @@ int launch_flow_pack(lsnf_plan* plan, const float* const* params, const int32_t*
   return LSNF_OK;
 }
 
-// samples per CTA: every CTA streams all the parameters (~1.3 MB per pass) through its shared memory, so a few
-// samples share one stream; 4 keeps the reference batch of 100 on 25 SMs for ~20 us
+// preferred samples per CTA: every CTA streams all the parameters (~1.3 MB per pass) through its shared memory, so a
+// few samples share one stream; 4 keeps the reference batch of 100 on 25 SMs for ~20 us.  Where that tier's shared
+// memory does not fit, the launchers take the next smaller one (fitting_s)
 static int pick_s(int B) {
   if (B <= 32) return 1;
   if (B <= 64) return 2;
@@ -819,14 +820,24 @@ static size_t flow_fixed_floats(const FlowLayout& f, int S, int depth, bool stas
 }
 
 // ring size: everything one pass streams if it fits, else whatever the 227 KB budget leaves (>= the largest matrix)
-static int flow_ring_floats(const FlowLayout& f, size_t fixed, int depth, bool both_passes, uint32_t* ring) {
-  const size_t budget = (size_t)227 * 1024 / 4;
+int flow_smem(const FlowLayout& f, int S, int depth, bool stash, bool both_passes, uint32_t* ring_floats,
+              size_t* smem_bytes) {
+  const size_t budget = (size_t)FLOW_SMEM_BYTES / 4;
+  const size_t fixed = flow_fixed_floats(f, S, depth, stash);
   if (fixed + f.max_mat > budget) return -1;
-  const size_t per_step = (size_t)f.nz * f.nz + (size_t)f.half * f.w + (size_t)f.w * f.w + (size_t)f.w * f.n_out;
-  const size_t want = per_step * depth * (both_passes ? 2 : 1);
+  const size_t want = f.step_mat * depth * (both_passes ? 2 : 1);
   size_t r = std::min(budget - fixed, want + 4);
   r = std::max(r, f.max_mat) / 4 * 4;
-  *ring = (uint32_t)r;
+  *ring_floats = (uint32_t)r;
+  *smem_bytes = (fixed + r) * 4;
+  return 0;
+}
+
+// the largest samples-per-CTA tier <= pick_s(B) whose footprint fits (0: none, not even S = 1)
+static int fitting_s(const FlowArgs& a, bool stash, bool both_passes, uint32_t* ring_floats, size_t* smem_bytes) {
+  for (int S = pick_s(a.B); S >= 1; S /= 2)
+    if (flow_smem(a.fl, S, a.depth, stash, both_passes, ring_floats, smem_bytes) == 0) return S;
+  set_error("flow kernel shared memory budget exceeded");
   return 0;
 }
 
@@ -847,14 +858,10 @@ static int launch_inv_t(const FlowArgs& a, size_t smem, cudaStream_t s) {
 }
 
 static int launch_flow_fwd_args(FlowArgs& a, cudaStream_t s) {
-  const int S = pick_s(a.B);
-  const size_t fixed = flow_fixed_floats(a.fl, S, a.depth, true);
-  if (flow_ring_floats(a.fl, fixed, a.depth, a.grad != nullptr, &a.ring_floats)) {
-    set_error("flow kernel shared memory budget exceeded");
-    return LSNF_ERR_INVALID;
-  }
-  const size_t smem = (fixed + a.ring_floats) * 4;
+  size_t smem;
+  const int S = fitting_s(a, true, a.grad != nullptr, &a.ring_floats, &smem);
   switch (S) {
+    case 0: return LSNF_ERR_INVALID;
     case 1: return launch_fwd_t<1>(a, smem, s);
     case 2: return launch_fwd_t<2>(a, smem, s);
     case 4: return launch_fwd_t<4>(a, smem, s);
@@ -1078,14 +1085,10 @@ int launch_flow_inverse(const lsnf_plan* plan, const float* eps, float* z, float
   a.coupling = plan->cfg.f_coupling; a.permutation = plan->cfg.f_permutation;
   a.in = eps; a.z_out = z; a.logdet = negobj; a.logp = nullptr; a.grad = nullptr; a.stash = nullptr;
   a.seed_g = a.seed_ld = nullptr;
-  const int S = pick_s(a.B);
-  const size_t fixed = flow_fixed_floats(a.fl, S, a.depth, false);
-  if (flow_ring_floats(a.fl, fixed, a.depth, false, &a.ring_floats)) {
-    set_error("flow kernel shared memory budget exceeded");
-    return LSNF_ERR_INVALID;
-  }
-  const size_t smem = (fixed + a.ring_floats) * 4;
+  size_t smem;
+  const int S = fitting_s(a, false, false, &a.ring_floats, &smem);
   switch (S) {
+    case 0: return LSNF_ERR_INVALID;
     case 1: return launch_inv_t<1>(a, smem, s);
     case 2: return launch_inv_t<2>(a, smem, s);
     case 4: return launch_inv_t<4>(a, smem, s);

@@ -93,7 +93,8 @@ struct FlowLayout {
   size_t an_b, an_e, an_ei, W, WT, Winv, W1, W1T, b1, e1, W2, W2T, b2, e2, W3, W3T, b3, e3, perm, perm_inv, ld_const;
   size_t step_floats;
   size_t vec_floats;  // the per-step vectors come first in a step's block, [0, vec_floats)
-  size_t max_mat;     // floats of the largest matrix
+  size_t max_mat;     // floats of the largest matrix a flow kernel streams (W counts only with the 1x1 permutation)
+  size_t step_mat;    // floats of the matrices one step streams in one pass (likewise)
 };
 
 // Training stash of the flow prior (flow parameter update, train.py:403-415): per step, per slot a [B][dim] block.
@@ -289,6 +290,13 @@ int launch_flow_pack(lsnf_plan* plan, const float* const* params, const int32_t*
 int launch_flow_forward(const lsnf_plan* plan, const float* z, float* z_out, float* logdet, float* logp,
                         float* grad_z, cudaStream_t s);
 int launch_flow_inverse(const lsnf_plan* plan, const float* eps, float* z, float* negobj, cudaStream_t s);
+// Dynamic shared memory of one fused flow launch at S samples per CTA: the fixed part (with the forward kernel's
+// per-step activation stash when `stash`) plus the matrix ring (sized for both passes when `both_passes`).  Returns 0
+// and sets *ring_floats and *smem_bytes when that fits the 227 KB a CTA may opt in to, -1 otherwise.  The launchers
+// and lsnf_plan_create both decide with it.
+int flow_smem(const FlowLayout& f, int S, int depth, bool stash, bool both_passes, uint32_t* ring_floats,
+              size_t* smem_bytes);
+constexpr int FLOW_SMEM_BYTES = 227 * 1024;
 int launch_adam(int n, float* const* params, const float* const* grads, float* const* m, float* const* v,
                 const int64_t* sizes, const int32_t* grad_kk, const int32_t* grad_inner, float lr, float beta1,
                 float beta2, float eps, float weight_decay, int64_t step, const float* grad_scale, cudaStream_t s);

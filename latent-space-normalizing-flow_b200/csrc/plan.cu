@@ -221,8 +221,23 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     f.W1 = tk((size_t)f.half * f.w); f.W1T = tk((size_t)f.half * f.w);
     f.W2 = tk((size_t)f.w * f.w); f.W2T = tk((size_t)f.w * f.w);
     f.W3 = tk((size_t)f.w * f.n_out); f.W3T = tk((size_t)f.w * f.n_out);
-    f.max_mat = std::max({(size_t)f.nz * f.nz, (size_t)f.half * f.w, (size_t)f.w * f.w, (size_t)f.w * f.n_out});
+    // what the flow kernels stream: the shuffle permutation has no matrix
+    const size_t w_floats = c.f_permutation == 2 ? (size_t)f.nz * f.nz : 0;
+    f.max_mat = std::max({w_floats, (size_t)f.half * f.w, (size_t)f.w * f.w, (size_t)f.w * f.n_out});
+    f.step_mat = w_floats + (size_t)f.half * f.w + (size_t)f.w * f.w + (size_t)f.w * f.n_out;
     f.step_floats = o;
+    // every flow entry point must be able to launch: the forward kernel (with its activation stash, both passes) at
+    // one sample per CTA is the largest footprint; the inverse kernel needs less
+    uint32_t ring_floats;
+    size_t smem_bytes;
+    if (flow_smem(f, 1, c.f_depth, true, true, &ring_floats, &smem_bytes)) {
+      delete p;
+      return fail(LSNF_ERR_INVALID,
+                  "flow prior exceeds the " + std::to_string(FLOW_SMEM_BYTES / 1024) +
+                      " KB of shared memory of one CTA even at one sample per CTA: its largest matrix (f_width^2, or "
+                      "nz^2 with f_flow_permutation 2) plus f_depth * (2 f_width + nz) stashed activations must fit "
+                      "(include/lsnf.h, lsnf_config)");
+    }
     p->off_flow = take(f.step_floats * 4 * c.f_depth);
     // training stash and flat gradient layout of the flow parameter update (train.py:403-415)
     FlowStash& t = p->fstash;
