@@ -15,6 +15,7 @@
  *   lsnf_generator_param_grads <- loss_g = mse(G(z_k), x) / B; loss_g.backward()  train.py:390-394
  *   lsnf_flow_param_grads    <- loss_f = -ll.mean(); loss_f.backward()    train.py:403-411, model.py:182
  *   lsnf_adam_step           <- optG.step() / optF.step() (torch.optim.Adam) train.py:294-295, :398, :415
+ *   lsnf_*_masked            <- the same three generator-loss entry points with a per-pixel likelihood weight
  *   lsnf_generator_vjp       <- backward of netG(z) for any loss (torch.autograd through lsnf_b200.kernel_autograd)
  *   lsnf_flow_vjp            <- backward of netF(z, objective) for any loss (same)
  *   lsnf_pack_*              <- parameters of _netG / _netF               model.py:48-157, :460-498
@@ -204,6 +205,30 @@ int lsnf_flow_param_grads(lsnf_plan* plan, const float* z, int32_t global_batch,
  * GEMMs of lsnf_generator_param_grads from the seed grad_x_hat * (1 - x_hat^2), at scale 1.  Needs the 3-pass data
  * gradient: a plan with bwd_passes == 1 returns LSNF_ERR_UNSUPPORTED.  Deterministic. */
 int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, float* grad_z, float* grads, lsnf_stream stream);
+
+/* ---- masked reconstruction loss (inpainting, occluded pixels, images with missing regions) -------------- */
+/* The three calls below are lsnf_langevin_run, lsnf_generator_dgrad and lsnf_generator_param_grads with a nullable
+ * `mask`: fp32 [B,nc,H,W], the layout of x, a per-pixel likelihood weight m (1 = observed, 0 = missing, fractions
+ * allowed).  mask == NULL is exactly the unmasked call (which is implemented as this call with NULL).
+ *   Langevin energy  1/(2 sigma^2) sum m (G(z) - x)^2 - log p(z)     (so m_i = sigma^2 / sigma_i^2 is a per-pixel
+ *                                                                      noise precision)
+ *   generator loss   loss_g = sum m (G(z) - x)^2 / global_batch      (the flow prior and its update are unchanged)
+ * The weight multiplies (G(z) - x) before any other factor, so an all-ones mask reproduces the unmasked results bit
+ * for bit.  The gradient norms of lsnf_langevin_run_masked are those of the masked gradient.  Supported weights lie in
+ * [0, 1]: the data-gradient tensors are sized for that range (a larger common weight can be folded into sigma).  The
+ * library does not read device values, so it does not check this.
+ * lsnf_langevin_run_masked: a call that replays a CUDA graph first copies the mask into the workspace (as it does x),
+ * so the mask's contents and address may change between calls; masked and unmasked loops never share a graph.
+ * lsnf_generator_param_grads_masked: the mask is read by the part -1 and -2 calls only (the forward pass, the loss and
+ * the data-gradient chain); a layer's call (part >= 0) ignores it. */
+int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const float* x, const float* mask, int32_t steps,
+                             float step_size, float sigma, int32_t with_noise, const float* eps, uint64_t seed,
+                             uint64_t sample_offset, float* z_out, float* gnorms, lsnf_stream stream);
+int lsnf_generator_dgrad_masked(lsnf_plan* plan, const float* x, const float* mask, float sigma, float* grad_z,
+                                lsnf_stream stream);
+int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z, const float* x, const float* mask,
+                                      int32_t global_batch, float* grads, float* loss, int32_t part,
+                                      lsnf_stream stream);
 /* z [B,nz]; upstream grad_z_out [B,nz] and grad_logdet [B] (either nullable = 0) -> grad_z [B,nz] (nullable) and the
  * flow parameter gradients (nullable; layout of lsnf_flow_grad_layout; needs w_inverse for W). Deterministic. */
 int lsnf_flow_vjp(lsnf_plan* plan, const float* z, const float* grad_z_out, const float* grad_logdet, float* grad_z,

@@ -80,6 +80,12 @@ EXPORTS = {
     "lsnf_flow_grad_floats": (C.c_size_t, [C.c_void_p]),
     "lsnf_flow_grad_layout": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "lsnf_flow_param_grads": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lsnf_langevin_run_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float,
+                                           C.c_float, C.c_int32, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                                           C.c_void_p, C.c_void_p]),
+    "lsnf_generator_dgrad_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
+    "lsnf_generator_param_grads_masked": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "lsnf_generator_vjp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lsnf_flow_vjp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lsnf_adam_step": (C.c_int, [C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),

@@ -179,7 +179,10 @@ int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s) {
 // of which only seed_scale = sigma_seed_scale(sigma) <= 16 (a power of two) is applied here; the rest of 1/sigma^2
 // multiplies the fp32 sum of the first layer's split-K partials (langevin_update_kernel / reduce_partial_kernel).
 // With upstream != 0, `x` is a caller-supplied dL/dx_hat and the seed is g = x * seed_scale * (1 - x_hat^2) (the
-// vector-Jacobian product of lsnf_generator_vjp, seed_scale 1).  Either seed is
+// vector-Jacobian product of lsnf_generator_vjp, seed_scale 1).  With upstream == 0 and a likelihood mask m (nullable,
+// [B,nc,H,W] like x) the loss is the weighted 1/(2 sigma^2) sum m (x_hat - x)^2 and the seed (m * (x_hat - x)) * ...:
+// the weight multiplies the difference before any other factor, so an all-ones mask reproduces the unmasked seed bit
+// for bit.  Either seed is
 // written directly as the im2col operand of the last layer's data gradient:
 //   A[b][iy][ix][tap*nc + c] = g[b][c][iy*s - p + ky][ix*s - p + kx]  (0 outside the image), 64 columns.
 // ---------------------------------------------------------------------------------------------------
@@ -189,6 +192,7 @@ int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s) {
 constexpr int IM2COL_SEG = 32;
 __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __restrict__ xhat,
                                                                 const float* __restrict__ x,
+                                                                const float* __restrict__ mask,
                                                                 uint16_t* __restrict__ a, int B, int nc, int img,
                                                                 int hin, int k, int s, int p, float seed_scale,
                                                                 int fp16, int upstream) {
@@ -205,7 +209,9 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
     if (oy >= 0 && oy < img && ox >= 0 && ox < img) {
       const size_t o = (((size_t)b * nc + c) * img + oy) * img + ox;
       const float xh = xhat[o];
-      v = (upstream ? x[o] : xh - x[o]) * seed_scale * (1.f - xh * xh);
+      float d = upstream ? x[o] : xh - x[o];
+      if (mask) d = mask[o] * d;   // read only with upstream == 0 (the launcher passes null otherwise)
+      v = d * seed_scale * (1.f - xh * xh);
     }
     g[i] = v;
   }
@@ -225,14 +231,15 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
   }
 }
 
-int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float seed_scale, int upstream, cudaStream_t s) {
+int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
+                             cudaStream_t s) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const int segs = (y.hin + IM2COL_SEG - 1) / IM2COL_SEG;
   const int span = (std::min(IM2COL_SEG, y.hin) - 1) * y.s + y.k;
   const size_t smem = (size_t)plan->cfg.nc * y.k * span * 4;
   recon_grad_im2col_kernel<<<plan->cfg.batch * y.hin * segs, 128, smem, s>>>(
-      (const float*)(plan->ws + plan->off_xhat), x, (uint16_t*)(plan->ws + plan->off_im2col), plan->cfg.batch,
-      plan->cfg.nc, plan->img, y.hin, y.k, y.s, y.p, seed_scale, plan->cfg.bwd_passes == 1 ? 1 : 0, upstream);
+      (const float*)(plan->ws + plan->off_xhat), x, upstream ? nullptr : mask, (uint16_t*)(plan->ws + plan->off_im2col),
+      plan->cfg.batch, plan->cfg.nc, plan->img, y.hin, y.k, y.s, y.p, seed_scale, plan->cfg.bwd_passes == 1 ? 1 : 0, upstream);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;
 }
@@ -243,7 +250,9 @@ int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float seed_s
 // (coalesced 128-bit reads; the per-position stride is padded to an odd word count so the tap gathers that follow
 // are bank-conflict free), computes x_hat and the loss-gradient seed for the output window the tile's taps touch,
 // and writes the tile's 64-column im2col rows.  x_hat is written by the tile that owns pixel (oy/s, ox/s); the tap
-// summation order equals last_gather_tanh_kernel's, so x_hat is bit-identical to the unfused path.
+// summation order equals last_gather_tanh_kernel's, so x_hat is bit-identical to the unfused path.  With a mask
+// (nullable) the CTA also stages the mask window next to the x window and weights the seed as
+// recon_grad_im2col_kernel does.
 // ---------------------------------------------------------------------------------------------------
 constexpr int FUSE_HALO = 2;   // ceil((k-1)/s) for both supported geometries (k3/s1, k4/s2)
 // x / d for the small index ranges of this kernel (x * d < 2^32) as one multiply-high: the kernel is all index
@@ -256,8 +265,9 @@ struct FastDiv {
 
 template <int K, int S>
 __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict__ d, const float* __restrict__ bias,
-                                                         const float* __restrict__ x, float* __restrict__ xhat,
-                                                         uint16_t* __restrict__ a, int B, int nc, int img, int hin,
+                                                         const float* __restrict__ x, const float* __restrict__ mask,
+                                                         float* __restrict__ xhat, uint16_t* __restrict__ a, int B,
+                                                         int nc, int img, int hin,
                                                          int p, int n_pad, int TR, int TC, float seed_scale, int fp16,
                                                          int write_lo) {
   extern __shared__ float fs[];
@@ -272,6 +282,7 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
   const int GH = (TR - 1) * S + K, GW = (TC - 1) * S + K;
   float* Dt = fs;                         // [DH][DW][PS]
   float* G = fs + (size_t)DH * DW * PS;   // [nc][GH][GW]
+  float* M = G + (size_t)nc * GH * GW;    // [nc][GH][GW], mask window (only with a mask)
   const int tid = threadIdx.x;
   const int qs = n_pad == 32 ? 3 : 4;     // log2 of the float4 count per position (n_pad is 32 or 64)
   const int dr0 = max(0, r0 - FUSE_HALO), dr1 = min(hin, r0 + nr + FUSE_HALO);
@@ -300,6 +311,24 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
       if (i < nwin) G[i] = xv[u];
     }
   }
+  if (mask) {
+    for (int i0 = tid; i0 < nwin; i0 += U * blockDim.x) {
+      float mv[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int i = i0 + u * blockDim.x;
+        const int c = by_gwh.div(i), rem = i - c * GW * GH, yy = by_gw.div(rem), xx = rem - yy * GW;
+        const int oy = oy_lo + yy, ox = ox_lo + xx;
+        mv[u] = (i < nwin && oy >= 0 && oy < img && ox >= 0 && ox < img)
+                    ? __ldg(mask + (((size_t)b * nc + c) * img + oy) * img + ox) : 0.f;
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int i = i0 + u * blockDim.x;
+        if (i < nwin) M[i] = mv[u];
+      }
+    }
+  }
   const int nd = ((dr1 - dr0) * dwc) << qs;
   const float* dbase = d + ((size_t)b * hin * hin) * n_pad;
   for (int i0 = tid; i0 < nd; i0 += U * blockDim.x) {
@@ -326,7 +355,7 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
     }
   }
   __syncthreads();
-  // ---- x_hat and the seed g = (x_hat - x) / sigma^2 * (1 - x_hat^2) on the output window of the tile ----
+  // ---- x_hat and the seed g = (m * (x_hat - x)) / sigma^2 * (1 - x_hat^2) on the output window of the tile ----
   for (int i = tid; i < nwin; i += blockDim.x) {
     const int c = by_gwh.div(i), rem = i - c * GW * GH, yy = by_gw.div(rem), xx = rem - yy * GW;
     const int oy = oy_lo + yy, ox = ox_lo + xx;
@@ -354,7 +383,9 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
       const int iyo = oy / S, ixo = ox / S;   // the tile that owns this pixel writes x_hat
       if (iyo >= r0 && iyo < r0 + nr && ixo >= c0 && ixo < c0 + ncol)
         xhat[(((size_t)b * nc + c) * img + oy) * img + ox] = xh;
-      g = (xh - G[i]) * seed_scale * (1.f - xh * xh);
+      float dv = xh - G[i];
+      if (mask) dv = M[i] * dv;
+      g = dv * seed_scale * (1.f - xh * xh);
     }
     G[i] = g;
   }
@@ -383,13 +414,13 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
   }
 }
 
-int launch_last_fused(const lsnf_plan* plan, const float* x, float seed_scale, cudaStream_t s) {
+int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, cudaStream_t s) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const int n_pad = plan->dlast_pad;
   const int TC = std::min(32, y.hin), TR = std::min(n_pad <= 32 ? 8 : 4, y.hin);
   const int DW = TC + 2 * FUSE_HALO, DH = TR + 2 * FUSE_HALO;
   const int GH = (TR - 1) * y.s + y.k, GW = (TC - 1) * y.s + y.k;
-  const size_t smem = ((size_t)DH * DW * (n_pad + 1) + (size_t)plan->cfg.nc * GH * GW) * 4;
+  const size_t smem = ((size_t)DH * DW * (n_pad + 1) + (size_t)plan->cfg.nc * GH * GW * (mask ? 2 : 1)) * 4;
   const int tiles = ((y.hin + TR - 1) / TR) * ((y.hin + TC - 1) / TC);
   const float* d = (const float*)(plan->ws + plan->off_dlast);
   const float* bias = (const float*)(plan->ws + plan->off_bias[plan->n_layers - 1]);
@@ -399,11 +430,11 @@ int launch_last_fused(const lsnf_plan* plan, const float* x, float seed_scale, c
   if (smem > 160 * 1024) { set_error("fused last-layer kernel: tile does not fit shared memory"); return LSNF_ERR_INVALID; }
   const dim3 grid(plan->cfg.batch * tiles), block(256);
   if (y.k == 3 && y.s == 1)
-    LSNF_CUDA(launch_k(last_fused_kernel<3, 1>, grid, block, smem, s, d, bias, x, xh, a, plan->cfg.batch, plan->cfg.nc,
-                       plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
+    LSNF_CUDA(launch_k(last_fused_kernel<3, 1>, grid, block, smem, s, d, bias, x, mask, xh, a, plan->cfg.batch,
+                       plan->cfg.nc, plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
   else
-    LSNF_CUDA(launch_k(last_fused_kernel<4, 2>, grid, block, smem, s, d, bias, x, xh, a, plan->cfg.batch, plan->cfg.nc,
-                       plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
+    LSNF_CUDA(launch_k(last_fused_kernel<4, 2>, grid, block, smem, s, d, bias, x, mask, xh, a, plan->cfg.batch,
+                       plan->cfg.nc, plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
   return LSNF_OK;
 }
 

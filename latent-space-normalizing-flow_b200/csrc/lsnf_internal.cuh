@@ -191,14 +191,14 @@ struct lsnf_plan {
   // concurrently with the generator stages
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  // CUDA graphs of the whole g_l_steps loop, keyed by (steps, step_size, sigma, with_noise); per-call values
+  // CUDA graphs of the whole g_l_steps loop, keyed by (steps, step_size, sigma, with_noise, masked); per-call values
   // (seed, sample offset) are read from device memory, inputs are staged into the workspace
   // A graph holds one CHUNK of at most `graph_chunk` iterations; the step index of its first iteration is read
   // from device memory (dyn[2]), so a chain of any length replays the same few graphs (train.py:606: 8 000 steps).
-  struct LoopGraph { int steps; float step_size, sigma; int with_noise; cudaGraphExec_t exec; };
+  struct LoopGraph { int steps; float step_size, sigma; int with_noise; bool masked; cudaGraphExec_t exec; };
   std::vector<LoopGraph> graphs;
   cudaStream_t cap_stream = nullptr;
-  size_t off_x = 0, off_gnorms = 0, off_dyn = 0, off_sk_slots = 0, off_sk_flags = 0;
+  size_t off_x = 0, off_mask = 0, off_gnorms = 0, off_dyn = 0, off_sk_slots = 0, off_sk_flags = 0;
   long long runs = 0;
   bool use_graphs = true;
   int graph_chunk = 40;
@@ -276,13 +276,15 @@ int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);
 int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s);
-int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, float seed_scale, int upstream, cudaStream_t s);
-int launch_last_fused(const lsnf_plan* plan, const float* x, float seed_scale, cudaStream_t s);
+// mask (nullable): per-pixel likelihood weight [B,nc,H,W] of the loss-gradient seed (ignored with upstream != 0)
+int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
+                             cudaStream_t s);
+int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, cudaStream_t s);
 int launch_transpose_hl(const TransArgs& a, cudaStream_t s);
 int launch_wgrad_finalize(const FinalizeArgs& a, cudaStream_t s);
 int launch_bias_rowsum(const RowSumArgs& a, cudaStream_t s);
-int launch_mse_sum(const float* xh, const float* x, long long n, float scale, float* partial, unsigned int* ticket,
-                   float* out, cudaStream_t s);
+int launch_mse_sum(const float* xh, const float* x, const float* mask, long long n, float scale, float* partial,
+                   unsigned int* ticket, float* out, cudaStream_t s);
 int launch_reduce_partial(const lsnf_plan* plan, float* grad_z, float scale, cudaStream_t s);
 int launch_flow_pack(lsnf_plan* plan, const float* const* params, const int32_t* const* perm,
                      const int32_t* const* perm_inv, const float* log_abs_det, const float* const* winv,

@@ -264,6 +264,7 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     p->off_sk_slots = take((size_t)160 * 128 * 256 * 4);   // stream-K partial accumulators (<= 160 CTAs)
     p->off_sk_flags = take((size_t)160 * 8 * 4);
     p->off_x = take((size_t)B * c.nc * p->img * p->img * 4);
+    p->off_mask = take((size_t)B * c.nc * p->img * p->img * 4);   // the graph-replayed loop's copy of a mask
     for (int l = 0; l < L - 1; ++l) {
       const auto& y = p->layers[l];
       const size_t bytes = (size_t)B * y.hout * y.hout * 2 * y.co * 2;
@@ -747,9 +748,9 @@ static int gen_forward(lsnf_plan* p, const float* z, float* x_hat, cudaStream_t 
   return LSNF_OK;
 }
 
-static int gen_dgrad_partial(lsnf_plan* p, const float* x, float sigma, cudaStream_t s) {
+static int gen_dgrad_partial(lsnf_plan* p, const float* x, const float* mask, float sigma, cudaStream_t s) {
   int rc;
-  if ((rc = launch_recon_grad_im2col(p, x, sigma_seed_scale(sigma), 0, s))) return rc;
+  if ((rc = launch_recon_grad_im2col(p, x, mask, sigma_seed_scale(sigma), 0, s))) return rc;
   for (int i = p->n_layers; i < 2 * p->n_layers; ++i)
     if ((rc = run_stage(p, p->stages[i], s))) return rc;
   return LSNF_OK;
@@ -769,13 +770,18 @@ extern "C" int lsnf_generator_forward(lsnf_plan* plan, const float* z, float* x_
   return gen_forward(plan, z, x_hat, (cudaStream_t)stream, true);
 }
 
-extern "C" int lsnf_generator_dgrad(lsnf_plan* plan, const float* x, float sigma, float* grad_z, lsnf_stream stream) {
+extern "C" int lsnf_generator_dgrad_masked(lsnf_plan* plan, const float* x, const float* mask, float sigma,
+                                           float* grad_z, lsnf_stream stream) {
   int rc = need(plan, true, false);
   if (rc) return rc;
   if (!x || !grad_z || !(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "bad argument");
   cudaStream_t s = (cudaStream_t)stream;
-  if ((rc = gen_dgrad_partial(plan, x, sigma, s))) return rc;
+  if ((rc = gen_dgrad_partial(plan, x, mask, sigma, s))) return rc;
   return launch_reduce_partial(plan, grad_z, sigma_post_scale(sigma), s);
+}
+
+extern "C" int lsnf_generator_dgrad(lsnf_plan* plan, const float* x, float sigma, float* grad_z, lsnf_stream stream) {
+  return lsnf_generator_dgrad_masked(plan, x, nullptr, sigma, grad_z, stream);
 }
 
 extern "C" int lsnf_flow_forward(lsnf_plan* plan, const float* z, float* z_out, float* logdet, float* logp,
@@ -837,8 +843,9 @@ static int gen_layer_grads(lsnf_plan* plan, int l, float* grads, float scale, cu
   return LSNF_OK;
 }
 
-extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const float* x, int32_t global_batch,
-                                          float* grads, float* loss, int32_t part, lsnf_stream stream) {
+extern "C" int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z, const float* x, const float* mask,
+                                                 int32_t global_batch, float* grads, float* loss, int32_t part,
+                                                 lsnf_stream stream) {
   int rc = need(plan, true, false);
   if (rc) return rc;
   if (plan->wg.empty()) return fail(LSNF_ERR_STATE, "plan was created without lsnf_config.train");
@@ -855,13 +862,13 @@ extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const
     if ((rc = sync_check(s, "generator forward", -1))) return rc;
     const long long npix = (long long)c.batch * c.nc * plan->img * plan->img;
     // partial sums in the (idle) norm scratch of the update kernel, ticket next to its own
-    if (loss && (rc = launch_mse_sum((const float*)(plan->ws + plan->off_xhat), x, npix, 1.f / (float)global_batch,
+    if (loss && (rc = launch_mse_sum((const float*)(plan->ws + plan->off_xhat), x, mask, npix, 1.f / (float)global_batch,
                                      (float*)(plan->ws + plan->off_flow_out),
                                      (unsigned int*)(plan->ws + plan->off_scalars + 64), loss, s)))
       return rc;
     // backward through the generator: seed (x_hat - x)(1 - x_hat^2) unscaled; the factor 2 / B of the loss is applied
     // in fp32 when the gradients are finalized.  The first layer's data gradient is not needed.
-    if ((rc = launch_last_fused(plan, x, 1.f, s))) return rc;
+    if ((rc = launch_last_fused(plan, x, mask, 1.f, s))) return rc;
     for (int i = L; i < 2 * L - 1; ++i)
       if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
     if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
@@ -878,6 +885,11 @@ extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const
   return LSNF_OK;
 }
 
+extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const float* x, int32_t global_batch,
+                                          float* grads, float* loss, int32_t part, lsnf_stream stream) {
+  return lsnf_generator_param_grads_masked(plan, z, x, nullptr, global_batch, grads, loss, part, stream);
+}
+
 extern "C" int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, float* grad_z, float* grads,
                                   lsnf_stream stream) {
   int rc = need(plan, true, false);
@@ -892,7 +904,7 @@ extern "C" int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, floa
   cudaStream_t s = (cudaStream_t)stream;
   const int L = plan->n_layers;
   // seed g = dL/dx_hat * (1 - x_hat^2) at scale 1 (bf16 keeps fp32's exponent range), x_hat of the last forward pass
-  if ((rc = launch_recon_grad_im2col(plan, grad_x_hat, 1.f, 1, s))) return rc;
+  if ((rc = launch_recon_grad_im2col(plan, grad_x_hat, nullptr, 1.f, 1, s))) return rc;
   const int end = grad_z ? 2 * L : 2 * L - 1;   // the first layer's data gradient only feeds dL/dz
   for (int i = L; i < end; ++i)
     if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
@@ -991,7 +1003,7 @@ extern "C" int lsnf_langevin_launch_count(const lsnf_plan* plan, int32_t steps) 
   return 1 + steps * (2 * plan->n_layers + 3) + chunks;
 }
 
-// the g_l_steps loop on stream s: inputs are the workspace copies of z and x
+// the g_l_steps loop on stream s: inputs are the workspace copies of z and x (and of the mask, nullable)
 // LSNF_TRACE=1: time every launch of the second iteration in situ with CUDA events and print the table to stderr
 struct LoopTrace {
   std::vector<cudaEvent_t> ev;
@@ -1023,7 +1035,8 @@ struct LoopTrace {
   }
 };
 
-static int langevin_loop(lsnf_plan* plan, const float* x, int steps, float step_size, float sigma, int with_noise,
+static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int steps, float step_size, float sigma,
+                         int with_noise,
                          const float* eps, uint64_t seed, uint64_t sample_offset, const uint64_t* dyn, float* gnorms,
                          cudaStream_t s) {
   const float gscale = sigma_post_scale(sigma);
@@ -1075,7 +1088,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, int steps, float step_
     }
     {
       PdlScope pdl(pdl_ok(false));
-      if ((rc = launch_last_fused(plan, x, sigma_seed_scale(sigma), s))) return rc;
+      if ((rc = launch_last_fused(plan, x, mask, sigma_seed_scale(sigma), s))) return rc;
     }
     tr.mark("gather + tanh + recon grad + im2col");
     for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i) {
@@ -1098,9 +1111,10 @@ static int langevin_loop(lsnf_plan* plan, const float* x, int steps, float step_
   return LSNF_OK;
 }
 
-extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* x, int32_t steps, float step_size,
-                                 float sigma, int32_t with_noise, const float* eps, uint64_t seed,
-                                 uint64_t sample_offset, float* z_out, float* gnorms, lsnf_stream stream) {
+extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const float* x, const float* mask,
+                                        int32_t steps, float step_size, float sigma, int32_t with_noise,
+                                        const float* eps, uint64_t seed, uint64_t sample_offset, float* z_out,
+                                        float* gnorms, lsnf_stream stream) {
   int rc = need(plan, true, true);
   if (rc) return rc;
   if (!z0 || !x || !z_out || steps < 0 || !(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "bad argument");
@@ -1116,26 +1130,34 @@ extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* 
   const bool graph_ok = plan->use_graphs && !eps && steps > 0 && plan->runs > 0;
   plan->runs++;
   if (!graph_ok) {
-    if ((rc = langevin_loop(plan, x, steps, step_size, sigma, with_noise, eps, seed, sample_offset, nullptr, gnorms, s)))
+    if ((rc = langevin_loop(plan, x, mask, steps, step_size, sigma, with_noise, eps, seed, sample_offset, nullptr,
+                            gnorms, s)))
       return rc;
   } else {
     // The chain is replayed in chunks of at most `graph_chunk` iterations: one graph per chunk length, the index of
     // a chunk's first iteration (Philox counter) is read from device memory, so test mode's 8 000-step chains
     // (train.py:606) reuse one 40-iteration graph 200 times instead of instantiating 88 000 kernel nodes.
+    // A masked call's graph reads the workspace copy of the mask, so masked and unmasked loops never share a graph.
     float* x_ws = (float*)(plan->ws + plan->off_x);
+    float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
+    const bool masked = mask != nullptr;
     float* gn_ws = (float*)(plan->ws + plan->off_gnorms);
     const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
-    LSNF_CUDA(cudaMemcpyAsync(x_ws, x, (size_t)c.batch * c.nc * plan->img * plan->img * 4, cudaMemcpyDeviceToDevice, s));
+    const size_t xbytes = (size_t)c.batch * c.nc * plan->img * plan->img * 4;
+    LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
+    if (masked) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
     for (int done = 0; done < steps;) {
       const int n = std::min(steps - done, plan->graph_chunk);
       cudaGraphExec_t exec = nullptr;
       for (auto& g : plan->graphs)
-        if (g.steps == n && g.step_size == step_size && g.sigma == sigma && g.with_noise == with_noise) exec = g.exec;
+        if (g.steps == n && g.step_size == step_size && g.sigma == sigma && g.with_noise == with_noise &&
+            g.masked == masked)
+          exec = g.exec;
       if (!exec) {
         cudaGraph_t graph = nullptr;
         cudaStream_t cs = plan->cap_stream;
         LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-        rc = langevin_loop(plan, x_ws, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs);
+        rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs);
         cudaError_t ce = cudaStreamEndCapture(cs, &graph);
         if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
         if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
@@ -1143,7 +1165,7 @@ extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* 
         cudaGraphDestroy(graph);
         if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
         if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
-        plan->graphs.push_back({n, step_size, sigma, with_noise, exec});
+        plan->graphs.push_back({n, step_size, sigma, with_noise, masked, exec});
       }
       if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s))) return rc;
       LSNF_CUDA(cudaGraphLaunch(exec, s));
@@ -1153,4 +1175,11 @@ extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* 
   }
   LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
   return LSNF_OK;
+}
+
+extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* x, int32_t steps, float step_size,
+                                 float sigma, int32_t with_noise, const float* eps, uint64_t seed,
+                                 uint64_t sample_offset, float* z_out, float* gnorms, lsnf_stream stream) {
+  return lsnf_langevin_run_masked(plan, z0, x, nullptr, steps, step_size, sigma, with_noise, eps, seed, sample_offset,
+                                  z_out, gnorms, stream);
 }

@@ -196,19 +196,20 @@ int launch_bias_rowsum(const RowSumArgs& a, cudaStream_t s) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// loss_g = scale * sum (x_hat - x)^2 (train.py:393): 64 CTAs leave fixed-order partial sums, the last one to finish adds
-// them in index order (deterministic)
+// loss_g = scale * sum (x_hat - x)^2 (train.py:393), or scale * sum m (x_hat - x)^2 with a mask (nullable): 64 CTAs leave
+// fixed-order partial sums, the last one to finish adds them in index order (deterministic).  fmaf(m*d, d, acc) equals
+// fmaf(d, d, acc) for m = 1, so an all-ones mask reproduces the unmasked loss bit for bit.
 // ---------------------------------------------------------------------------------------------------
 constexpr int MSE_CTAS = 64;
 __global__ void __launch_bounds__(256) mse_sum_kernel(const float* __restrict__ xh, const float* __restrict__ x,
-                                                      long long n, float scale, float* __restrict__ partial,
+                                                      const float* __restrict__ mask, long long n, float scale, float* __restrict__ partial,
                                                       unsigned int* __restrict__ ticket, float* __restrict__ out) {
   __shared__ float red[256];
   __shared__ bool last;
   float acc = 0.f;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float d = xh[i] - x[i];
-    acc = fmaf(d, d, acc);
+    acc = fmaf(mask ? mask[i] * d : d, d, acc);
   }
   red[threadIdx.x] = acc;
   __syncthreads();
@@ -232,9 +233,9 @@ __global__ void __launch_bounds__(256) mse_sum_kernel(const float* __restrict__ 
   }
 }
 
-int launch_mse_sum(const float* xh, const float* x, long long n, float scale, float* partial, unsigned int* ticket,
-                   float* out, cudaStream_t s) {
-  mse_sum_kernel<<<MSE_CTAS, 256, 0, s>>>(xh, x, n, scale, partial, ticket, out);
+int launch_mse_sum(const float* xh, const float* x, const float* mask, long long n, float scale, float* partial,
+                   unsigned int* ticket, float* out, cudaStream_t s) {
+  mse_sum_kernel<<<MSE_CTAS, 256, 0, s>>>(xh, x, mask, n, scale, partial, ticket, out);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;
 }

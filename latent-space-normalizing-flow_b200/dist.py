@@ -22,17 +22,21 @@ def shard_batch(t: torch.Tensor, rank: int, world: int) -> torch.Tensor:
 
 
 def langevin_sharded(z_global, x_global, netG, netF, args, *, seed: int, rank: int = None, world: int = None,
-                     gather: bool = False, **kw):
+                     gather: bool = False, mask=None, **kw):
     """Run this rank's shard of a global batch.  Noise is keyed by the GLOBAL sample index, so every rank draws
     exactly the noise the single-GPU run draws for its samples (the latents then agree up to fp32 summation order:
     split-K / stream-K cut points depend on the tile count).  Returns (z_shard or gathered z, |grad_g|, |grad_f|)
-    with the two diagnostics averaged over the global batch when ``gather``."""
+    with the two diagnostics averaged over the global batch when ``gather``.  ``mask`` (per-pixel likelihood weight of
+    the global batch, ``plan.as_mask``) is sharded like x; a mask without a batch axis of the global batch's size
+    (e.g. [1,1,H,W] or [H,W]) is shared by every sample and passed to each rank whole."""
     from .langevin import sample_langevin_post_z_with_flow
     rank = dist.get_rank() if rank is None else rank
     world = dist.get_world_size() if world is None else world
     a, b = shard_range(z_global.shape[0], rank, world)
+    if mask is not None and mask.dim() == x_global.dim() and mask.shape[0] == x_global.shape[0]:
+        mask = mask[a:b]
     z, gn, fn = sample_langevin_post_z_with_flow(z_global[a:b], x_global[a:b], netG, netF, args, seed=seed,
-                                                 sample_offset=a, **kw)
+                                                 sample_offset=a, mask=mask, **kw)
     if not gather:
         return z, gn, fn
     sizes = [shard_range(z_global.shape[0], r, world) for r in range(world)]

@@ -44,7 +44,8 @@ def langevin_plan(netG: _netG, netF: _netF, batch: int, device, bwd_passes: Opti
 def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbose: bool = False, *,
                                      eps: Optional[torch.Tensor] = None, steps: Optional[int] = None,
                                      with_noise: Optional[bool] = None, seed: Optional[int] = None,
-                                     sample_offset: int = 0, bwd_passes: Optional[int] = None, train: bool = False):
+                                     sample_offset: int = 0, bwd_passes: Optional[int] = None, train: bool = False,
+                                     mask: Optional[torch.Tensor] = None):
     """z [B,nz,1,1], x [B,nc,H,W] -> (z_k [B,nz,1,1], mean_b|grad_g|, mean_b|grad_f|) as train.py:335 returns them.
 
     ``args`` supplies g_l_steps, g_l_step_size, g_l_with_noise, g_llhd_sigma (train.py:311-326).  ``eps``
@@ -54,6 +55,10 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
     diagnostics use the real batch size (the reference's ``view(args.batch_size, -1)`` breaks on a ragged batch).
     ``bwd_passes``: tensor-core passes of the reconstruction-gradient GEMMs: 3 (fp32-equivalent hi|lo split) unless
     the caller opts in to the single fp16 pass with 1 (``plan.default_bwd_passes``).
+    ``mask``: per-pixel likelihood weight m for partly observed images (inpainting, occluded pixels): the energy
+    becomes 1/(2 sigma^2) sum m (G(z) - x)^2 - log p(z), with 1 = observed, 0 = missing and fractions in [0, 1]
+    allowed.  Any shape that broadcasts to x's, any real or bool dtype (``plan.as_mask``).  |grad_g| is then the
+    norm of the masked gradient.
     """
     if not isinstance(netG, _netG) or not isinstance(netF, _netF):
         raise TypeError("netG / netF must be lsnf_b200._netG / _netF instances")
@@ -80,7 +85,7 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
     plan.ensure_generator(netG)
     plan.ensure_flow(netF)
     out, norms = plan.langevin_run(z2, xx, T, s, sigma, with_noise=noise, eps=e, seed=seed,
-                                   sample_offset=sample_offset)
+                                   sample_offset=sample_offset, mask=mask)
     if verbose:
         print("Langevin posterior: z_grad_g_grad_norm={:8.3f}, z_grad_f_grad_norm={:8.3f}".format(
             norms[0].item(), norms[1].item()))
@@ -88,15 +93,17 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
 
 
 def make_sampler(args, test_mode: bool = False):
-    """Closure with the reference's exact signature ``f(z, x, netG, netF, verbose=False)``.
+    """Closure with the reference's exact signature ``f(z, x, netG, netF, verbose=False)``, plus the keyword-only
+    ``mask`` of ``sample_langevin_post_z_with_flow``.
 
     ``test_mode=True`` reproduces the test variant: ``g_l_steps * 20`` iterations and no noise
     (train.py:606, :623-625)."""
-    def sampler(z, x, netG, netF, verbose=False):
+    def sampler(z, x, netG, netF, verbose=False, *, mask=None):
         if test_mode:
             return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose,
-                                                    steps=int(_get(args, "g_l_steps", 20)) * 20, with_noise=False)
-        return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose)
+                                                    steps=int(_get(args, "g_l_steps", 20)) * 20, with_noise=False,
+                                                    mask=mask)
+        return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose, mask=mask)
     return sampler
 
 

@@ -44,6 +44,29 @@ def _check_tensor(t: torch.Tensor, name: str, device, shape=None):
         raise RuntimeError(f"{name} has shape {tuple(t.shape)}, expected {tuple(shape)}")
 
 
+def as_mask(mask, x: torch.Tensor) -> torch.Tensor:
+    """The per-pixel likelihood weight ``mask`` of a masked reconstruction loss as the library reads it: an fp32
+    contiguous tensor of x's shape [B,nc,H,W] on x's device.  ``mask`` may have any shape that broadcasts to x's
+    ([B,1,H,W], [1,1,H,W], [H,W], ...) and any real or bool dtype (True = 1 = observed, 0 = missing; fractional weights
+    in [0, 1] are allowed).  A mask on the CPU raises RuntimeError, as x does; a shape that does not broadcast to x's
+    raises ValueError."""
+    if not isinstance(mask, torch.Tensor):
+        raise TypeError("mask must be a torch.Tensor")
+    try:
+        shape = torch.broadcast_shapes(tuple(mask.shape), tuple(x.shape))
+    except RuntimeError:
+        shape = None
+    if shape != tuple(x.shape):
+        raise ValueError(f"mask of shape {tuple(mask.shape)} does not broadcast to x's shape {tuple(x.shape)}")
+    if mask.device.type == "cpu":
+        raise RuntimeError("mask must be a CUDA tensor: the Langevin path has no CPU fallback")
+    if mask.device != x.device:
+        raise RuntimeError(f"mask is on {mask.device}, x is on {x.device}")
+    if mask.is_complex():
+        raise ValueError("mask must be real")
+    return mask.detach().to(torch.float32).expand(x.shape).contiguous()
+
+
 class Plan:
     def __init__(self, *, arch: str, batch: int, nz: int, ngf: int, nc: int, f_depth: int, f_width: int,
                  f_permutation: int, f_coupling: int, leak: float, device, gemm_impl: int = _cabi.GEMM_TCGEN05,
@@ -198,12 +221,16 @@ class Plan:
                         "lsnf_generator_forward")
         return out
 
-    def generator_dgrad(self, x: torch.Tensor, sigma: float) -> torch.Tensor:
+    def generator_dgrad(self, x: torch.Tensor, sigma: float, *, mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """d/dz [1/(2 sigma^2) sum m (G(z) - x)^2] at the z of the last ``generator_forward``; m = ``mask`` (see
+        ``as_mask``), or 1 without one."""
         _check_tensor(x, "x", self.device, (self.batch, self.nc, self.img, self.img))
+        m = as_mask(mask, x) if mask is not None else None
         g = torch.empty(self.batch, self.nz, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.lsnf_generator_dgrad(self.handle, x.data_ptr(), float(sigma), g.data_ptr(),
-                                                      _stream(self.device)), "lsnf_generator_dgrad")
+            _cabi.check(self.lib.lsnf_generator_dgrad_masked(self.handle, x.data_ptr(), m.data_ptr() if m is not None
+                                                             else None, float(sigma), g.data_ptr(), _stream(self.device)),
+                        "lsnf_generator_dgrad_masked")
         return g
 
     def generator_vjp(self, grad_x_hat: torch.Tensor, want_z: bool = True, want_params: bool = False):
@@ -286,13 +313,16 @@ class Plan:
         return [(int(off[i]), int(size[i])) for i in range(n)]
 
     def generator_param_grads(self, z: torch.Tensor, x: torch.Tensor, global_batch: int,
-                              flat: Optional[torch.Tensor] = None, part: int = -1, loss: Optional[torch.Tensor] = None):
+                              flat: Optional[torch.Tensor] = None, part: int = -1, loss: Optional[torch.Tensor] = None,
+                              *, mask: Optional[torch.Tensor] = None):
         """Gradients of loss_g = mse_sum(G(z), x) / global_batch w.r.t. every generator weight and bias into one
         flat fp32 buffer (returned with this rank's share of loss_g).  Needs ``train=True`` at plan creation and
         ``ensure_generator`` on the current parameters.  ``part``: -1 everything; -2 forward + loss + data-gradient
-        chain only; l >= 0 only layer l's gradients (include/lsnf.h)."""
+        chain only; l >= 0 only layer l's gradients (include/lsnf.h).  ``mask`` (see ``as_mask``) weights the loss
+        per pixel, loss_g = sum m (G(z) - x)^2 / global_batch; only the part -1 and -2 calls read it."""
         _check_tensor(z, "z", self.device, (self.batch, self.nz))
         _check_tensor(x, "x", self.device, (self.batch, self.nc, self.img, self.img))
+        m = as_mask(mask, x) if mask is not None else None
         n = int(self.lib.lsnf_generator_grad_floats(self.handle))
         if flat is None:
             flat = torch.zeros(n, dtype=torch.float32, device=self.device)
@@ -301,9 +331,9 @@ class Plan:
             loss = torch.empty((), dtype=torch.float32, device=self.device)
         self.act_epoch += 1
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.lsnf_generator_param_grads(self.handle, z.data_ptr(), x.data_ptr(), int(global_batch),
-                                                            flat.data_ptr(), loss.data_ptr(), int(part),
-                                                            _stream(self.device)), "lsnf_generator_param_grads")
+            _cabi.check(self.lib.lsnf_generator_param_grads_masked(
+                self.handle, z.data_ptr(), x.data_ptr(), m.data_ptr() if m is not None else None, int(global_batch),
+                flat.data_ptr(), loss.data_ptr(), int(part), _stream(self.device)), "lsnf_generator_param_grads_masked")
         return flat, loss
 
     # ---- flow parameter update (train.py:403-415) ----------------------------------------------------
@@ -345,9 +375,13 @@ class Plan:
         return norms
 
     def langevin_run(self, z0, x, steps, step_size, sigma, with_noise=True, eps=None, seed=0, sample_offset=0,
-                     out: Optional[torch.Tensor] = None, norms: Optional[torch.Tensor] = None):
+                     out: Optional[torch.Tensor] = None, norms: Optional[torch.Tensor] = None, *,
+                     mask: Optional[torch.Tensor] = None):
+        """``steps`` Langevin iterations from z0 on the energy 1/(2 sigma^2) sum m (G(z) - x)^2 - log p(z), with
+        m = ``mask`` (see ``as_mask``) or 1 without one.  Returns (z_T, [mean |grad_g|, mean |grad_f|])."""
         _check_tensor(z0, "z", self.device, (self.batch, self.nz))
         _check_tensor(x, "x", self.device, (self.batch, self.nc, self.img, self.img))
+        m = as_mask(mask, x) if mask is not None else None
         if eps is not None:
             _check_tensor(eps, "eps", self.device, (steps, self.batch, self.nz))
         if out is None:
@@ -356,10 +390,11 @@ class Plan:
             norms = torch.zeros(2, dtype=torch.float32, device=self.device)
         self.act_epoch += 1
         with torch.cuda.device(self.device):
-            _cabi.check(self.lib.lsnf_langevin_run(
-                self.handle, z0.data_ptr(), x.data_ptr(), int(steps), float(step_size), float(sigma),
-                int(bool(with_noise)), eps.data_ptr() if eps is not None else None, int(seed) & (2 ** 64 - 1),
-                int(sample_offset), out.data_ptr(), norms.data_ptr(), _stream(self.device)), "lsnf_langevin_run")
+            _cabi.check(self.lib.lsnf_langevin_run_masked(
+                self.handle, z0.data_ptr(), x.data_ptr(), m.data_ptr() if m is not None else None, int(steps),
+                float(step_size), float(sigma), int(bool(with_noise)), eps.data_ptr() if eps is not None else None,
+                int(seed) & (2 ** 64 - 1), int(sample_offset), out.data_ptr(), norms.data_ptr(), _stream(self.device)),
+                "lsnf_langevin_run_masked")
         return out, norms
 
 

@@ -14,7 +14,7 @@ import torch.distributed as dist
 
 from .langevin import sample_langevin_post_z_with_flow
 from .optim import FusedAdam
-from .plan import flow_step_params
+from .plan import as_mask, flow_step_params
 
 
 def make_optimizers(netG, netF, args):
@@ -40,10 +40,11 @@ def _comm_stream(device):
     return _comm_streams[key]
 
 
-def _gen_plan_and_buffers(netG, z_k, x, plan):
+def _gen_plan_and_buffers(netG, z_k, x, plan, mask=None):
     b = z_k.shape[0]
     z2 = z_k.detach().reshape(b, netG.nz).contiguous().float()
     xx = x.detach().contiguous().float()
+    m = as_mask(mask, xx) if mask is not None else None
     if plan is None:
         plan = netG._plan(b, z2.device, train=True)
     plan.ensure_generator(netG)
@@ -55,15 +56,16 @@ def _gen_plan_and_buffers(netG, z_k, x, plan):
     params = [p for m in convs for p in (m.weight, m.bias)]
     layout = plan.generator_grad_layout()
     pairs = [(p, flat[off:off + size].view_as(p)) for (off, size), p in zip(layout, params)]
-    return plan, z2, xx, flat, layout, pairs
+    return plan, z2, xx, m, flat, layout, pairs
 
 
-def generator_gradients(netG, z_k, x, global_batch, plan=None):
+def generator_gradients(netG, z_k, x, global_batch, plan=None, *, mask=None):
     """(flat gradient buffer, [(parameter, gradient view)], this rank's share of loss_g) of
     loss_g = mse_sum(G(z_k), x) / global_batch (train.py:392-394) through ``lsnf_generator_param_grads``: forward,
-    data-gradient chain and one weight-gradient tap-GEMM per layer on the tensor cores."""
-    plan, z2, xx, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan)
-    flat, loss = plan.generator_param_grads(z2, xx, global_batch, flat)
+    data-gradient chain and one weight-gradient tap-GEMM per layer on the tensor cores.  With ``mask`` (per-pixel
+    weight m, ``plan.as_mask``) loss_g = sum m (G(z_k) - x)^2 / global_batch."""
+    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask)
+    flat, loss = plan.generator_param_grads(z2, xx, global_batch, flat, mask=m)
     return flat, pairs, loss
 
 
@@ -91,19 +93,20 @@ class _PendingGeneratorUpdate:
         return self.loss
 
 
-def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None):
+def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None):
     """First half of the generator step of train.py:390-398: gradients, and with several ranks their all-reduce
     started layer by layer (bucket = one layer's weight + bias gradient, last layer first) on a comm stream while the
-    main stream computes the next layer's weight gradient.  ``.finish()`` completes the step."""
+    main stream computes the next layer's weight gradient.  ``.finish()`` completes the step.  ``mask``: per-pixel
+    weight of the loss, as in ``generator_gradients``."""
     b_global = z_k.shape[0] if global_batch is None else int(global_batch)
-    plan, z2, xx, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan)
+    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask)
     if world <= 1:
-        flat, loss = plan.generator_param_grads(z2, xx, b_global, flat)
+        flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, mask=m)
         return _PendingGeneratorUpdate(netG, optG, args, flat, pairs, loss, [])
     comm = _comm_stream(z2.device)
     main = torch.cuda.current_stream(z2.device)
     handles = []
-    flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, part=-2)
+    flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, part=-2, mask=m)
 
     def reduce_async(t):
         ev = torch.cuda.Event()
@@ -122,10 +125,10 @@ def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group
     return _PendingGeneratorUpdate(netG, optG, args, flat, pairs, loss, handles)
 
 
-def generator_update(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None):
+def generator_update(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None):
     """The generator step of train.py:390-398 without autograd.  Returns loss_g."""
     return generator_update_begin(netG, optG, z_k, x, args, global_batch=global_batch, group=group, world=world,
-                                  plan=plan).finish()
+                                  plan=plan, mask=mask).finish()
 
 
 def flow_params_in_order(netF):
@@ -181,8 +184,10 @@ _iter_counter = [0]
 
 
 def training_iteration(x, netG, netF, optG, optF, args, *, global_batch=None, sample_offset=None, seed=None,
-                       z0=None, group=None, data_parallel=None):
+                       z0=None, group=None, data_parallel=None, mask=None):
     """x: this rank's shard [B_local, nc, H, W] on the GPU.  Returns (loss_g, loss_f, |grad_g|, |grad_f|, z_k).
+    ``mask``: this rank's shard of a per-pixel likelihood weight (any shape that broadcasts to x's, ``plan.as_mask``)
+    for training on partly observed images: both the Langevin energy and loss_g weight (G(z) - x)^2 by it.
 
     Mirrors train.py:378-415: z_0 ~ N(0, I); z_k = Langevin(z_0, x); generator step on mse_sum(G(z_k), x) / B;
     flow step on -mean log p(z_k) (with the f_is_grad_clamp / f_max_norm clipping of train.py:411-412).  With several
@@ -222,13 +227,14 @@ def training_iteration(x, netG, netF, optG, optF, args, *, global_batch=None, sa
         gen = torch.Generator(x.device).manual_seed(int(seed) & (2 ** 63 - 1))
         z0 = torch.randn(b_global, netG.nz, 1, 1, device=x.device, generator=gen)[sample_offset:sample_offset + b_local]
     z_k, gn, fn = sample_langevin_post_z_with_flow(z0, x, netG, netF, args, seed=seed,
-                                                   sample_offset=sample_offset, train=True)   # train.py:387
+                                                   sample_offset=sample_offset, train=True, mask=mask)   # train.py:387
     from .langevin import langevin_plan
     from .plan import default_bwd_passes
     plan = langevin_plan(netG, netF, b_local, x.device, default_bwd_passes(), train=True)  # the plan that call used
     # generator update (train.py:390-398): weight-gradient tap-GEMMs, per-layer all-reduces on the comm stream ...
+    masked = {} if mask is None else {"mask": mask}   # an unmasked iteration makes exactly the unmasked call
     pending = generator_update_begin(netG, optG, z_k, x, args, global_batch=b_global, group=group, world=world,
-                                     plan=plan)
+                                     plan=plan, **masked)
     # ... overlapped with the flow update (train.py:403-415): gradient kernels + one flat all-reduce + fused Adam.
     # The two updates are independent (neither reads the other network's parameters), so finishing the generator's
     # Adam step after the flow's changes nothing.
