@@ -234,6 +234,31 @@ int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z, const flo
 int lsnf_flow_vjp(lsnf_plan* plan, const float* z, const float* grad_z_out, const float* grad_logdet, float* grad_z,
                   float* grads, lsnf_stream stream);
 
+/* ---- annealed importance sampling (AIS) with Metropolis-adjusted Langevin transitions ------------------ */
+/* Estimates log p(x) = log int p(x|z) p(z) dz.  With l(z) = -sum m (G(z) - x)^2 / (2 sigma^2) (m = mask, NULL = 1) and
+ * pi_beta(z) ~ p(z) exp(beta l(z)), every chain b runs, for t = 1..steps:
+ *   log w += (betas[t] - betas[t-1]) l(z_{t-1})                                  (fp64 accumulator)
+ *   z_t = one MALA step on pi_{betas[t]} from z_{t-1}: proposal z' = z - (s^2/2) grad U(z) + s eps, accepted iff
+ *         log u < U(z) - U(z') - |z - z' + (s^2/2) grad U(z')|^2 / (2 s^2) + |eps|^2 / 2   (NaN / inf energies reject)
+ * with U = -log p - beta l.  Forward AIS (betas 0 -> 1, z0 exact prior samples) gives a stochastic lower bound:
+ * log p(x) >= E[log w] + C, C = -1/2 sum_{m_i > 0} log(2 pi sigma^2 / m_i), which the caller adds.  A decreasing
+ * schedule started from an exact posterior sample is BDMC's reverse chain, whose -log w bounds from above.  With a
+ * constant schedule of ones the call is a Metropolis-adjusted posterior sampler.
+ *   z0 [B,nz], x and mask [B,nc,H,W], betas: device array of steps + 1 values in [0, 1] (not checked: the library
+ *   does not read device values on the host); steps >= 1; step_size > 0 is the initial step s of every chain; with
+ *   target_accept > 0 each chain adapts it after every decision, log s += 0.05 (min(1, alpha) - target_accept), s
+ *   clamped to [1e-5, 10]; target_accept <= 0 keeps it fixed.
+ *   eps [steps,B,nz] (the t-th proposal's noise) and u [steps,B] (the t-th decision's uniform), both nullable: Philox
+ *   keyed by (seed, sample_offset + b, iteration) otherwise.  Injected noise runs eagerly; other calls after a plan's
+ *   first replay CUDA graphs of the loop (the schedule, x and mask are copied into the workspace before each replay).
+ *   Outputs: z_out [B,nz] the last state, log_w [B] without C, accept_rate [B] accepted / steps.
+ * Each proposal is stored rounded to the fp16 hi|lo value the first generator layer reads, so the generator, the
+ * flow and the acceptance test all see the same z.  steps transitions take steps + 1 loop iterations. */
+int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, const float* betas,
+                 int32_t steps, float step_size, float target_accept, float sigma, const float* eps, const float* u,
+                 uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w, float* accept_rate,
+                 lsnf_stream stream);
+
 int lsnf_adam_step(int32_t n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,
                    float* const* exp_avg_sq, const int64_t* sizes, const int32_t* grad_kk, const int32_t* grad_inner,
                    float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,

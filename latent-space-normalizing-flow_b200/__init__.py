@@ -5,6 +5,7 @@ module interfaces and checkpoint keys (model.py), ``sample_langevin_post_z_with_
 train.py:307-335.  All device work is hand-written sm_100a CUDA behind the C ABI of ``include/lsnf.h``.
 """
 from . import synth  # noqa: F401
+from .ais import ais_log_likelihood, bdmc  # noqa: F401
 from .autograd_fns import kernel_autograd  # noqa: F401
 from .cli import parse_args  # noqa: F401
 from .langevin import (AttrDict, langevin_plan, make_args, make_sampler, sample_langevin_post_z_with_flow,  # noqa: F401
@@ -17,4 +18,4 @@ from .train import (flow_gradients, flow_update, generator_gradients, generator_
 
 __all__ = ["_netG", "_netF", "weights_init_xavier", "sample_langevin_post_z_with_flow", "make_sampler", "make_args",
            "sample_x", "training_iteration", "make_optimizers", "flow_update", "flow_gradients", "generator_update", "generator_gradients", "FusedAdam", "Plan", "get_plan", "clear_plans", "invalidate_plans", "langevin_plan", "AttrDict", "synth",
-           "parse_args", "reconstruction_error", "kernel_autograd"]
+           "parse_args", "reconstruction_error", "kernel_autograd", "ais_log_likelihood", "bdmc"]

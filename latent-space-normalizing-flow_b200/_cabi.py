@@ -88,6 +88,9 @@ EXPORTS = {
                                                     C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "lsnf_generator_vjp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lsnf_flow_vjp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lsnf_ais_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float,
+                               C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                               C.c_void_p, C.c_void_p, C.c_void_p]),
     "lsnf_adam_step": (C.c_int, [C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                  C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32),
                                  C.POINTER(C.c_int32), C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,

@@ -266,6 +266,7 @@ struct FastDiv {
 template <int K, int S>
 __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict__ d, const float* __restrict__ bias,
                                                          const float* __restrict__ x, const float* __restrict__ mask,
+                                                         float* __restrict__ epart,
                                                          float* __restrict__ xhat, uint16_t* __restrict__ a, int B,
                                                          int nc, int img, int hin,
                                                          int p, int n_pad, int TR, int TC, float seed_scale, int fp16,
@@ -356,6 +357,7 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
   }
   __syncthreads();
   // ---- x_hat and the seed g = (m * (x_hat - x)) / sigma^2 * (1 - x_hat^2) on the output window of the tile ----
+  float esum = 0.f;   // sum m (x_hat - x)^2 over the pixels this thread visits that the tile owns (epart only)
   for (int i = tid; i < nwin; i += blockDim.x) {
     const int c = by_gwh.div(i), rem = i - c * GW * GH, yy = by_gw.div(rem), xx = rem - yy * GW;
     const int oy = oy_lo + yy, ox = ox_lo + xx;
@@ -381,13 +383,28 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
       for (int t = 0; t < T * T; ++t) acc += v[t];
       const float xh = tanhf(acc);
       const int iyo = oy / S, ixo = ox / S;   // the tile that owns this pixel writes x_hat
-      if (iyo >= r0 && iyo < r0 + nr && ixo >= c0 && ixo < c0 + ncol)
-        xhat[(((size_t)b * nc + c) * img + oy) * img + ox] = xh;
-      float dv = xh - G[i];
+      const bool own = iyo >= r0 && iyo < r0 + nr && ixo >= c0 && ixo < c0 + ncol;
+      if (own) xhat[(((size_t)b * nc + c) * img + oy) * img + ox] = xh;
+      const float d0 = xh - G[i];
+      float dv = d0;
       if (mask) dv = M[i] * dv;
+      if (own) esum += dv * d0;
       g = dv * seed_scale * (1.f - xh * xh);
     }
     G[i] = g;
+  }
+  if (epart) {
+    // per-sample energy partial of the tile (annealed importance sampling): a fixed-order block sum, one float per CTA
+    __shared__ float ered[8];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) esum += __shfl_xor_sync(0xffffffffu, esum, o);
+    if ((tid & 31) == 0) ered[tid >> 5] = esum;
+    __syncthreads();
+    if (tid == 0) {
+      float e = 0.f;
+      for (int w = 0; w < (int)(blockDim.x >> 5); ++w) e += ered[w];
+      epart[blockIdx.x] = e;
+    }
   }
   __syncthreads();
   // ---- im2col rows of the tile: A[pos][tap*nc + c] = g[c][iy*s - p + ky][ix*s - p + kx] ----
@@ -414,14 +431,22 @@ __global__ void __launch_bounds__(256) last_fused_kernel(const float* __restrict
   }
 }
 
-int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, cudaStream_t s) {
+int last_fused_tiles(const lsnf_plan* plan, int* TR, int* TC) {
+  const auto& y = plan->layers[plan->n_layers - 1];
+  *TC = std::min(32, y.hin);
+  *TR = std::min(plan->dlast_pad <= 32 ? 8 : 4, y.hin);
+  return ((y.hin + *TR - 1) / *TR) * ((y.hin + *TC - 1) / *TC);
+}
+
+int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float* epart, float seed_scale,
+                      cudaStream_t s) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const int n_pad = plan->dlast_pad;
-  const int TC = std::min(32, y.hin), TR = std::min(n_pad <= 32 ? 8 : 4, y.hin);
+  int TR, TC;
+  const int tiles = last_fused_tiles(plan, &TR, &TC);
   const int DW = TC + 2 * FUSE_HALO, DH = TR + 2 * FUSE_HALO;
   const int GH = (TR - 1) * y.s + y.k, GW = (TC - 1) * y.s + y.k;
   const size_t smem = ((size_t)DH * DW * (n_pad + 1) + (size_t)plan->cfg.nc * GH * GW * (mask ? 2 : 1)) * 4;
-  const int tiles = ((y.hin + TR - 1) / TR) * ((y.hin + TC - 1) / TC);
   const float* d = (const float*)(plan->ws + plan->off_dlast);
   const float* bias = (const float*)(plan->ws + plan->off_bias[plan->n_layers - 1]);
   float* xh = (float*)(plan->ws + plan->off_xhat);
@@ -430,10 +455,10 @@ int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, 
   if (smem > 160 * 1024) { set_error("fused last-layer kernel: tile does not fit shared memory"); return LSNF_ERR_INVALID; }
   const dim3 grid(plan->cfg.batch * tiles), block(256);
   if (y.k == 3 && y.s == 1)
-    LSNF_CUDA(launch_k(last_fused_kernel<3, 1>, grid, block, smem, s, d, bias, x, mask, xh, a, plan->cfg.batch,
+    LSNF_CUDA(launch_k(last_fused_kernel<3, 1>, grid, block, smem, s, d, bias, x, mask, epart, xh, a, plan->cfg.batch,
                        plan->cfg.nc, plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
   else
-    LSNF_CUDA(launch_k(last_fused_kernel<4, 2>, grid, block, smem, s, d, bias, x, mask, xh, a, plan->cfg.batch,
+    LSNF_CUDA(launch_k(last_fused_kernel<4, 2>, grid, block, smem, s, d, bias, x, mask, epart, xh, a, plan->cfg.batch,
                        plan->cfg.nc, plan->img, y.hin, y.p, n_pad, TR, TC, seed_scale, one, !one));
   return LSNF_OK;
 }
@@ -611,12 +636,231 @@ int launch_update(const lsnf_plan* plan, float* z, const float* gg, const float*
   return LSNF_OK;
 }
 
-__global__ void set_dyn_kernel(uint64_t* dyn, uint64_t seed, uint64_t sample_offset, uint64_t base_step) {
-  dyn[0] = seed; dyn[1] = sample_offset; dyn[2] = base_step;
+__global__ void set_dyn_kernel(uint64_t* dyn, uint64_t seed, uint64_t sample_offset, uint64_t base_step,
+                               uint64_t total) {
+  dyn[0] = seed; dyn[1] = sample_offset; dyn[2] = base_step; dyn[3] = total;
 }
 
-int launch_set_dyn(const lsnf_plan* plan, uint64_t seed, uint64_t sample_offset, uint32_t base_step, cudaStream_t s) {
-  set_dyn_kernel<<<1, 1, 0, s>>>((uint64_t*)(plan->ws + plan->off_dyn), seed, sample_offset, base_step);
+int launch_set_dyn(const lsnf_plan* plan, uint64_t seed, uint64_t sample_offset, uint32_t base_step, cudaStream_t s,
+                   uint32_t total) {
+  set_dyn_kernel<<<1, 1, 0, s>>>((uint64_t*)(plan->ws + plan->off_dyn), seed, sample_offset, base_step, total);
+  LSNF_CUDA(cudaGetLastError());
+  return LSNF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Annealed importance sampling with Metropolis-adjusted Langevin (MALA) transitions (lsnf_ais_run).
+// The loop evaluates, at the point z the generator saw, l(z) = -sum m (G(z) - x)^2 / (2 sigma^2) (from the fused
+// last-layer kernel's per-tile partials), log p(z) and both gradients; this kernel keeps the chain's state and
+//   iteration k = 0      initialises the state with the evaluated point,
+//   iteration 1 <= k     accepts or rejects the proposal of step k (target pi_{beta_k}),
+//   iteration k < T      adds (beta_{k+1} - beta_k) l(z_k) to log w and proposes step k+1 on pi_{beta_{k+1}},
+// so T transitions take T+1 iterations.  k is the global iteration index (dyn[2] + t under graph replay) and T is
+// read from dyn[3] there.  The proposal is stored rounded to its fp16 hi|lo value, the point the first generator layer
+// reads, so that G, the flow and the Metropolis-Hastings test all see the same z.  The same stored gradient proposes
+// and enters the acceptance density, so the test is exact with respect to the computed energies.
+// ---------------------------------------------------------------------------------------------------
+__global__ void ais_begin_kernel(float* __restrict__ z, uint16_t* __restrict__ zhl, int B, int nz, int kp) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B * kp) return;
+  const int b = i / kp, j = i % kp;
+  const float v = j < nz ? z[(size_t)b * nz + j] : 0.f;
+  uint16_t hi, lo;
+  split16(v, true, hi, lo);
+  zhl[(size_t)b * 2 * kp + j] = hi;
+  zhl[(size_t)b * 2 * kp + kp + j] = lo;
+  if (j < nz) z[(size_t)b * nz + j] = join16(hi, lo, true);
+}
+
+int launch_ais_begin(const lsnf_plan* plan, float* z, cudaStream_t s) {
+  const int n = plan->cfg.batch * plan->kp;
+  ais_begin_kernel<<<(n + 255) / 256, 256, 0, s>>>(z, (uint16_t*)(plan->ws + plan->off_zhl), plan->cfg.batch,
+                                                   plan->cfg.nz, plan->kp);
+  LSNF_CUDA(cudaGetLastError());
+  return LSNF_OK;
+}
+
+// fixed-order sum over the 256 threads of a CTA (every thread gets the result)
+__device__ __forceinline__ float block_sum256(float v, float* red) {
+  __syncthreads();
+  red[threadIdx.x] = v;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  return red[0];
+}
+
+__device__ __forceinline__ float4 f4_fma(float4 a, float s, float4 b) {   // a + s * b
+  return make_float4(a.x + s * b.x, a.y + s * b.y, a.z + s * b.z, a.w + s * b.w);
+}
+
+__global__ void __launch_bounds__(256) ais_update_kernel(
+    AisArgs A, float* __restrict__ z, uint16_t* __restrict__ zhl, const float* __restrict__ partial, int nsplit,
+    int nzp, float gscale, const float* __restrict__ gf, int B, int nz, int kp, uint64_t seed, uint64_t sample_offset,
+    uint32_t t, const uint64_t* __restrict__ dyn) {
+  __shared__ float4 part[8][64];
+  __shared__ float red[256];
+  __shared__ int s_accept;
+  __shared__ float s_step;
+  pdl_wait();
+  pdl_trigger();
+  uint32_t k = t, total = (uint32_t)A.total;
+  if (dyn) { seed = dyn[0]; sample_offset = dyn[1]; k += (uint32_t)dyn[2]; total = (uint32_t)dyn[3]; }
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const int nq = nz / 4;
+  const int grp = tid >> 5, lane = tid & 31;
+  for (int q = lane; q < nq; q += 32) {
+    float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 4
+    for (int s = grp; s < nsplit; s += 8) {
+      const float4 p = __ldcg(reinterpret_cast<const float4*>(partial + ((size_t)s * B + b) * nzp + 4 * q));
+      g.x += p.x; g.y += p.y; g.z += p.z; g.w += p.w;
+    }
+    part[grp][q] = g;
+  }
+  __syncthreads();
+  const bool act = tid < nq;
+  const size_t o = (size_t)b * nz + 4 * (act ? tid : 0);
+  float4 gr1 = make_float4(0.f, 0.f, 0.f, 0.f), gp1 = gr1, z1 = gr1;   // the point evaluated by this iteration
+  if (act) {
+    gr1 = part[0][tid];
+#pragma unroll
+    for (int j = 1; j < 8; ++j) {
+      const float4 p = part[j][tid];
+      gr1.x += p.x; gr1.y += p.y; gr1.z += p.z; gr1.w += p.w;
+    }
+    gr1.x *= gscale; gr1.y *= gscale; gr1.z *= gscale; gr1.w *= gscale;   // -dl/dz
+    gp1 = *reinterpret_cast<const float4*>(gf + o);                         // -dlog p/dz
+    z1 = *reinterpret_cast<const float4*>(z + o);
+  }
+  float* ell = A.scal;              // state: l(z)
+  float* lp = A.scal + B;           //        log p(z) (the flow's, with its constant)
+  float* stp = A.scal + 2 * B;      //        step size
+  float* acc = A.scal + 3 * B;      //        accepted proposals
+  float* e2 = A.scal + 4 * B;       //        |eps|^2 / 2 of the pending proposal
+  float ell_cur = 0.f;              // thread 0 only
+  float4 zc = z1, grc = gr1, gpc = gp1;
+  float step;
+  if (k == 0) {
+    if (act) {
+      *reinterpret_cast<float4*>(A.zc + o) = z1;
+      *reinterpret_cast<float4*>(A.gr + o) = gr1;
+      *reinterpret_cast<float4*>(A.gp + o) = gp1;
+    }
+    step = A.step0;
+    if (tid == 0) {
+      float e = 0.f;
+      for (int i = 0; i < A.tiles; ++i) e += A.epart[(size_t)b * A.tiles + i];
+      ell_cur = -e * A.inv2s2;
+      ell[b] = ell_cur; lp[b] = A.logp[b]; stp[b] = step; acc[b] = 0.f; A.logw[b] = 0.0;
+    }
+  } else {
+    const float beta = A.betas[t];
+    step = stp[b];
+    if (act) {
+      zc = *reinterpret_cast<const float4*>(A.zc + o);
+      grc = *reinterpret_cast<const float4*>(A.gr + o);
+      gpc = *reinterpret_cast<const float4*>(A.gp + o);
+    }
+    // reverse-move density: |z - z' + (s^2/2) grad U(z')|^2 / (2 s^2)
+    const float h = 0.5f * step * step;
+    float rk = 0.f;
+    if (act) {
+      const float4 gu = f4_fma(gp1, beta, gr1);
+      const float4 r = f4_fma(make_float4(zc.x - z1.x, zc.y - z1.y, zc.z - z1.z, zc.w - z1.w), h, gu);
+      rk = r.x * r.x + r.y * r.y + r.z * r.z + r.w * r.w;
+    }
+    rk = block_sum256(rk, red);
+    if (tid == 0) {
+      float e = 0.f;
+      for (int i = 0; i < A.tiles; ++i) e += A.epart[(size_t)b * A.tiles + i];
+      const float ell1 = -e * A.inv2s2, lp1 = A.logp[b];
+      const double u0 = -(double)lp[b] - (double)beta * ell[b], u1 = -(double)lp1 - (double)beta * ell1;
+      const double la = u0 - u1 - (double)rk / (2.0 * (double)step * step) + (double)e2[b];
+      float u;
+      if (A.u) {
+        u = A.u[(size_t)(k - 1) * B + b];
+      } else {
+        const uint64_t sample = sample_offset + (uint64_t)b;
+        uint32_t r[4];
+        philox4x32_10((uint32_t)sample, (uint32_t)(sample >> 32), k, 0xFFFFFFFFu, (uint32_t)seed,
+                      (uint32_t)(seed >> 32), r);
+        u = ((float)(r[0] >> 8) + 0.5f) * 5.9604644775390625e-8f;
+      }
+      const bool ok = isfinite(u1) && isfinite(la) && log((double)u) < la;
+      ell_cur = ok ? ell1 : ell[b];
+      if (ok) { ell[b] = ell1; lp[b] = lp1; acc[b] += 1.f; }
+      double sn = step;
+      if (A.target > 0.f) {
+        const double a = isfinite(u1) && !isnan(la) ? (la >= 0.0 ? 1.0 : exp(la)) : 0.0;
+        sn = fmin(fmax(sn * exp(AIS_KAPPA * (a - (double)A.target)), AIS_STEP_MIN), AIS_STEP_MAX);
+      }
+      s_accept = ok ? 1 : 0;
+      s_step = (float)sn;
+      stp[b] = (float)sn;
+    }
+    __syncthreads();
+    step = s_step;
+    if (s_accept) {
+      zc = z1; grc = gr1; gpc = gp1;
+      if (act) {
+        *reinterpret_cast<float4*>(A.zc + o) = z1;
+        *reinterpret_cast<float4*>(A.gr + o) = gr1;
+        *reinterpret_cast<float4*>(A.gp + o) = gp1;
+      }
+    }
+  }
+  if (k >= total) {
+    // the chain's result: z_T in the workspace latent, log w and the acceptance rate in the output rows
+    if (act) *reinterpret_cast<float4*>(z + o) = zc;
+    if (tid == 0) {
+      A.scal[5 * B + b] = (float)A.logw[b];
+      A.scal[6 * B + b] = acc[b] / (float)total;
+    }
+    return;
+  }
+  const float beta0 = A.betas[t], beta1 = A.betas[t + 1];
+  if (tid == 0) A.logw[b] += ((double)beta1 - (double)beta0) * (double)ell_cur;
+  // proposal of step k+1 on pi_{beta_{k+1}}: z' = z - (s^2/2) grad U(z) + s eps, rounded to its fp16 hi|lo value
+  float4 e = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (act) {
+    if (A.eps) {
+      e = *reinterpret_cast<const float4*>(A.eps + (size_t)k * B * nz + o);
+    } else {
+      const uint64_t sample = sample_offset + (uint64_t)b;
+      uint32_t r[4];
+      philox4x32_10((uint32_t)sample, (uint32_t)(sample >> 32), k, (uint32_t)tid, (uint32_t)seed,
+                    (uint32_t)(seed >> 32), r);
+      box_muller(r[0], r[1], e.x, e.y);
+      box_muller(r[2], r[3], e.z, e.w);
+    }
+    const float h = 0.5f * step * step;
+    const float4 gu = f4_fma(gpc, beta1, grc);
+    float v[4] = {zc.x - h * gu.x + step * e.x, zc.y - h * gu.y + step * e.y, zc.z - h * gu.z + step * e.z,
+                  zc.w - h * gu.w + step * e.w};
+    __align__(8) uint16_t hi[4], lo[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      split16(v[j], true, hi[j], lo[j]);
+      v[j] = join16(hi[j], lo[j], true);
+    }
+    *reinterpret_cast<float4*>(z + o) = make_float4(v[0], v[1], v[2], v[3]);
+    uint16_t* row = zhl + (size_t)b * 2 * kp;
+    *reinterpret_cast<uint2*>(row + 4 * tid) = *reinterpret_cast<uint2*>(hi);
+    *reinterpret_cast<uint2*>(row + kp + 4 * tid) = *reinterpret_cast<uint2*>(lo);
+  }
+  const float ee = block_sum256(e.x * e.x + e.y * e.y + e.z * e.z + e.w * e.w, red);
+  if (tid == 0) e2[b] = 0.5f * ee;
+}
+
+int launch_ais_update(const lsnf_plan* plan, const AisArgs& a, const float* gf, float gscale, uint64_t seed,
+                      uint64_t sample_offset, uint32_t t, const uint64_t* dyn, cudaStream_t s) {
+  ais_update_kernel<<<plan->cfg.batch, 256, 0, s>>>(
+      a, (float*)(plan->ws + plan->off_z), (uint16_t*)(plan->ws + plan->off_zhl),
+      (const float*)(plan->ws + plan->off_partial), plan->ksplit_first, plan->nzp, gscale, gf, plan->cfg.batch,
+      plan->cfg.nz, plan->kp, seed, sample_offset, t, dyn);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;
 }

@@ -158,6 +158,29 @@ struct WgradLayer {
   RowSumArgs rs;
 };
 
+// State and per-call values of annealed importance sampling (lsnf_ais_run, ais_update_kernel).  The state lives in the
+// plan's workspace: the chain's current point z, its reconstruction gradient -dl/dz and its prior gradient
+// -dlog p/dz kept apart (so that grad U_beta = gp + beta gr can be formed for any beta), [B][nz] each; log w (fp64);
+// and the rows of `scal` [7][B]: l(z), log p(z), step size, accepted proposals, |eps|^2/2 of the pending proposal, and
+// the outputs float log w and acceptance rate.
+struct AisArgs {
+  float* zc;
+  float* gr;
+  float* gp;
+  float* scal;
+  double* logw;
+  float* epart;          // [B][tiles]: sum m (G(z) - x)^2 over the pixels of one fused last-layer tile
+  float* logp;           // [B]: log p(z) from the flow kernel
+  const float* betas;    // betas[t] is the schedule value of the call's (or replayed chunk's) iteration t
+  const float* eps;      // injected proposal noise [T][B][nz] (eager calls only), or null: Philox
+  const float* u;        // injected uniforms of the decisions [T][B] (eager calls only), or null: Philox
+  int tiles, total;      // tiles per sample; T (eager calls; a replayed graph reads it from dyn[3])
+  float step0, target, inv2s2;   // initial step size, target acceptance rate (<= 0: fixed step), 1 / (2 sigma^2)
+};
+// step-size adaptation after every decision: log s += AIS_KAPPA (min(1, alpha) - target), s clamped
+constexpr double AIS_KAPPA = 0.05, AIS_STEP_MIN = 1e-5, AIS_STEP_MAX = 10.0;
+constexpr int AIS_BETA_FLOATS = 1024;   // workspace copy of a replayed chunk's schedule values (<= 1023 iterations)
+
 }  // namespace lsnf
 
 struct lsnf_plan {
@@ -195,10 +218,18 @@ struct lsnf_plan {
   // (seed, sample offset) are read from device memory, inputs are staged into the workspace
   // A graph holds one CHUNK of at most `graph_chunk` iterations; the step index of its first iteration is read
   // from device memory (dyn[2]), so a chain of any length replays the same few graphs (train.py:606: 8 000 steps).
-  struct LoopGraph { int steps; float step_size, sigma; int with_noise; bool masked; cudaGraphExec_t exec; };
+  // AIS graphs (lsnf_ais_run) carry the flag `ais` and their target acceptance rate, so that they never mix with the
+  // Langevin loops of the same plan.
+  struct LoopGraph {
+    int steps; float step_size, sigma; int with_noise; bool masked; bool ais; float target; cudaGraphExec_t exec;
+  };
   std::vector<LoopGraph> graphs;
   cudaStream_t cap_stream = nullptr;
   size_t off_x = 0, off_mask = 0, off_gnorms = 0, off_dyn = 0, off_sk_slots = 0, off_sk_flags = 0;
+  // annealed importance sampling (lsnf::AisArgs): chain state, energy partials, log p, schedule copy of a replay
+  size_t off_ais_z = 0, off_ais_gr = 0, off_ais_gp = 0, off_ais_logw = 0, off_ais_scal = 0, off_ais_epart = 0,
+         off_ais_logp = 0, off_ais_beta = 0;
+  int fused_tiles = 0;   // CTAs of the fused last-layer kernel per sample
   long long runs = 0;
   bool use_graphs = true;
   int graph_chunk = 40;
@@ -279,7 +310,13 @@ int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cud
 // mask (nullable): per-pixel likelihood weight [B,nc,H,W] of the loss-gradient seed (ignored with upstream != 0)
 int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
                              cudaStream_t s);
-int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, cudaStream_t s);
+// epart (nullable): [B][tiles] sum m (x_hat - x)^2 over the pixels each CTA owns (tiles = last_fused_tiles)
+int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float* epart, float seed_scale,
+                      cudaStream_t s);
+int last_fused_tiles(const lsnf_plan* plan, int* TR, int* TC);
+int launch_ais_begin(const lsnf_plan* plan, float* z, cudaStream_t s);
+int launch_ais_update(const lsnf_plan* plan, const AisArgs& a, const float* gf, float gscale, uint64_t seed,
+                      uint64_t sample_offset, uint32_t t, const uint64_t* dyn, cudaStream_t s);
 int launch_transpose_hl(const TransArgs& a, cudaStream_t s);
 int launch_wgrad_finalize(const FinalizeArgs& a, cudaStream_t s);
 int launch_bias_rowsum(const RowSumArgs& a, cudaStream_t s);
@@ -314,7 +351,9 @@ int launch_update(const lsnf_plan* plan, float* z, const float* gg, const float*
                   const float* gf, float step, const float* eps, int with_noise, uint64_t seed,
                   uint64_t sample_offset, uint32_t step_idx, const uint64_t* dyn, float* gnorms,
                   int write_zhl, cudaStream_t s);
-int launch_set_dyn(const lsnf_plan* plan, uint64_t seed, uint64_t sample_offset, uint32_t base_step, cudaStream_t s);
+// dyn[0..3] = (seed, sample offset, first iteration of the replayed chunk, total iterations of an AIS run)
+int launch_set_dyn(const lsnf_plan* plan, uint64_t seed, uint64_t sample_offset, uint32_t base_step, cudaStream_t s,
+                   uint32_t total = 0);
 // Per-device one-time setup (opt-in shared-memory limits of every kernel instantiation).  Called by
 // lsnf_plan_bind for the plan's device; thread-safe; nothing on the launch path touches function attributes.
 int tc_prepare_device(int device);

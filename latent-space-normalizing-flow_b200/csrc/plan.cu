@@ -556,6 +556,18 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     }
     p->gen_grad_floats = goff;
   }
+  if (L > 0) {   // annealed importance sampling (lsnf_ais_run): chain state and energies, after every other region
+    int tr, tc;
+    p->fused_tiles = last_fused_tiles(p, &tr, &tc);
+    p->off_ais_z = take((size_t)B * c.nz * 4);
+    p->off_ais_gr = take((size_t)B * c.nz * 4);
+    p->off_ais_gp = take((size_t)B * c.nz * 4);
+    p->off_ais_logw = take((size_t)B * 8);
+    p->off_ais_scal = take((size_t)7 * B * 4);
+    p->off_ais_epart = take((size_t)B * p->fused_tiles * 4);
+    p->off_ais_logp = take((size_t)B * 4);
+    p->off_ais_beta = take((size_t)AIS_BETA_FLOATS * 4);
+  }
   p->ws_bytes = off;
   *out = p;
   return LSNF_OK;
@@ -868,7 +880,7 @@ extern "C" int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z
       return rc;
     // backward through the generator: seed (x_hat - x)(1 - x_hat^2) unscaled; the factor 2 / B of the loss is applied
     // in fp32 when the gradients are finalized.  The first layer's data gradient is not needed.
-    if ((rc = launch_last_fused(plan, x, mask, 1.f, s))) return rc;
+    if ((rc = launch_last_fused(plan, x, mask, nullptr, 1.f, s))) return rc;
     for (int i = L; i < 2 * L - 1; ++i)
       if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
     if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
@@ -1035,10 +1047,12 @@ struct LoopTrace {
   }
 };
 
+// With `ais` (lsnf_ais_run) the same stages also write the per-tile energy partials and log p(z), and the iteration
+// ends with the AIS update instead of the Langevin update.
 static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int steps, float step_size, float sigma,
                          int with_noise,
                          const float* eps, uint64_t seed, uint64_t sample_offset, const uint64_t* dyn, float* gnorms,
-                         cudaStream_t s) {
+                         cudaStream_t s, const AisArgs* ais = nullptr) {
   const float gscale = sigma_post_scale(sigma);
   int rc;
   static int trace_env = -1;
@@ -1077,7 +1091,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
       if (l == fork_at) {
         LSNF_CUDA(cudaEventRecord(plan->ev_fork, s));
         LSNF_CUDA(cudaStreamWaitEvent(plan->side, plan->ev_fork, 0));
-        if ((rc = launch_flow_forward(plan, z, nullptr, nullptr, nullptr, gf, plan->side))) return rc;
+        if ((rc = launch_flow_forward(plan, z, nullptr, nullptr, ais ? ais->logp : nullptr, gf, plan->side))) return rc;
         LSNF_CUDA(cudaEventRecord(plan->ev_join, plan->side));
       }
       {
@@ -1088,7 +1102,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
     }
     {
       PdlScope pdl(pdl_ok(false));
-      if ((rc = launch_last_fused(plan, x, mask, sigma_seed_scale(sigma), s))) return rc;
+      if ((rc = launch_last_fused(plan, x, mask, ais ? ais->epart : nullptr, sigma_seed_scale(sigma), s))) return rc;
     }
     tr.mark("gather + tanh + recon grad + im2col");
     for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i) {
@@ -1101,9 +1115,12 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
     LSNF_CUDA(cudaStreamWaitEvent(s, plan->ev_join, 0));
     tr.mark("join flow prior");
     const float* e = eps ? eps + (size_t)t * c.batch * c.nz : nullptr;
-    if ((rc = launch_update(plan, z, nullptr, partial, plan->ksplit_first, gscale, gf, step_size, e, with_noise, seed,
-                            sample_offset, (uint32_t)t, dyn, t == steps - 1 ? gnorms : nullptr, 1, s)))
+    if (ais) {
+      if ((rc = launch_ais_update(plan, *ais, gf, gscale, seed, sample_offset, (uint32_t)t, dyn, s))) return rc;
+    } else if ((rc = launch_update(plan, z, nullptr, partial, plan->ksplit_first, gscale, gf, step_size, e, with_noise,
+                                   seed, sample_offset, (uint32_t)t, dyn, t == steps - 1 ? gnorms : nullptr, 1, s))) {
       return rc;
+    }
     prev_pair = false;   // the update kernel precedes the next iteration's first layer
     tr.mark("update");
     tr.report();
@@ -1151,7 +1168,7 @@ extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const 
       cudaGraphExec_t exec = nullptr;
       for (auto& g : plan->graphs)
         if (g.steps == n && g.step_size == step_size && g.sigma == sigma && g.with_noise == with_noise &&
-            g.masked == masked)
+            g.masked == masked && !g.ais)
           exec = g.exec;
       if (!exec) {
         cudaGraph_t graph = nullptr;
@@ -1165,7 +1182,7 @@ extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const 
         cudaGraphDestroy(graph);
         if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
         if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
-        plan->graphs.push_back({n, step_size, sigma, with_noise, masked, exec});
+        plan->graphs.push_back({n, step_size, sigma, with_noise, masked, false, 0.f, exec});
       }
       if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s))) return rc;
       LSNF_CUDA(cudaGraphLaunch(exec, s));
@@ -1182,4 +1199,88 @@ extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* 
                                  uint64_t sample_offset, float* z_out, float* gnorms, lsnf_stream stream) {
   return lsnf_langevin_run_masked(plan, z0, x, nullptr, steps, step_size, sigma, with_noise, eps, seed, sample_offset,
                                   z_out, gnorms, stream);
+}
+
+extern "C" int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, const float* betas,
+                            int32_t steps, float step_size, float target_accept, float sigma, const float* eps,
+                            const float* u, uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w,
+                            float* accept_rate, lsnf_stream stream) {
+  int rc = need(plan, true, true);
+  if (rc) return rc;
+  if (!z0 || !x || !betas || !z_out || !log_w || !accept_rate) return fail(LSNF_ERR_INVALID, "null argument");
+  if (steps < 1) return fail(LSNF_ERR_INVALID, "steps must be at least 1");
+  if (!(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "sigma must be positive");
+  if (!(step_size > 0.f)) return fail(LSNF_ERR_INVALID, "step_size must be positive");
+  cudaStream_t s = (cudaStream_t)stream;
+  const lsnf_config& c = plan->cfg;
+  const int B = c.batch;
+  float* z = (float*)(plan->ws + plan->off_z);
+  const size_t zbytes = (size_t)B * c.nz * 4;
+  LSNF_CUDA(cudaMemcpyAsync(z, z0, zbytes, cudaMemcpyDeviceToDevice, s));
+  if ((rc = launch_ais_begin(plan, z, s))) return rc;
+  AisArgs a;
+  a.zc = (float*)(plan->ws + plan->off_ais_z);
+  a.gr = (float*)(plan->ws + plan->off_ais_gr);
+  a.gp = (float*)(plan->ws + plan->off_ais_gp);
+  a.scal = (float*)(plan->ws + plan->off_ais_scal);
+  a.logw = (double*)(plan->ws + plan->off_ais_logw);
+  a.epart = (float*)(plan->ws + plan->off_ais_epart);
+  a.logp = (float*)(plan->ws + plan->off_ais_logp);
+  a.betas = betas; a.eps = eps; a.u = u;
+  a.tiles = plan->fused_tiles; a.total = steps;
+  a.step0 = step_size; a.target = target_accept > 0.f ? target_accept : 0.f;
+  a.inv2s2 = 0.5f / (sigma * sigma);
+  const int iters = steps + 1;   // iteration 0 only initialises and proposes, the last one only decides
+  const bool graph_ok = plan->use_graphs && !eps && !u && plan->runs > 0;
+  plan->runs++;
+  if (!graph_ok) {
+    if ((rc = langevin_loop(plan, x, mask, iters, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, nullptr, s,
+                            &a)))
+      return rc;
+  } else {
+    // As lsnf_langevin_run_masked: chunks of at most graph_chunk iterations, inputs staged into the workspace.  The
+    // schedule is not captured either: before each replay, the chunk's values are copied into the workspace.
+    float* x_ws = (float*)(plan->ws + plan->off_x);
+    float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
+    float* beta_ws = (float*)(plan->ws + plan->off_ais_beta);
+    const bool masked = mask != nullptr;
+    const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
+    const size_t xbytes = (size_t)B * c.nc * plan->img * plan->img * 4;
+    LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
+    if (masked) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
+    AisArgs ag = a;
+    ag.betas = beta_ws;
+    const int chunk = std::min(plan->graph_chunk, AIS_BETA_FLOATS - 1);
+    for (int done = 0; done < iters;) {
+      const int n = std::min(iters - done, chunk);
+      cudaGraphExec_t exec = nullptr;
+      for (auto& g : plan->graphs)
+        if (g.ais && g.steps == n && g.step_size == step_size && g.sigma == sigma && g.masked == masked &&
+            g.target == a.target)
+          exec = g.exec;
+      if (!exec) {
+        cudaGraph_t graph = nullptr;
+        cudaStream_t cs = plan->cap_stream;
+        LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
+        rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, 1, nullptr, 0, 0, dyn, nullptr, cs, &ag);
+        cudaError_t ce = cudaStreamEndCapture(cs, &graph);
+        if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
+        if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
+        ce = cudaGraphInstantiate(&exec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
+        if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
+        plan->graphs.push_back({n, step_size, sigma, 1, masked, true, a.target, exec});
+      }
+      const int nb = std::min(n + 1, iters - done);   // the last iteration reads no next value
+      LSNF_CUDA(cudaMemcpyAsync(beta_ws, betas + done, (size_t)nb * 4, cudaMemcpyDeviceToDevice, s));
+      if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s, (uint32_t)steps))) return rc;
+      LSNF_CUDA(cudaGraphLaunch(exec, s));
+      done += n;
+    }
+  }
+  LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
+  LSNF_CUDA(cudaMemcpyAsync(log_w, a.scal + 5 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
+  LSNF_CUDA(cudaMemcpyAsync(accept_rate, a.scal + 6 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
+  return LSNF_OK;
 }

@@ -397,6 +397,35 @@ class Plan:
                 "lsnf_langevin_run_masked")
         return out, norms
 
+    def ais_run(self, z0, x, betas, steps, step_size, sigma, *, target_accept: float = 0.0,
+                mask: Optional[torch.Tensor] = None, eps: Optional[torch.Tensor] = None,
+                u: Optional[torch.Tensor] = None, seed: int = 0, sample_offset: int = 0):
+        """Annealed importance sampling with MALA transitions from z0 along the schedule ``betas`` [steps+1] (fp32, on
+        the plan's device) on pi_beta(z) ~ p(z) exp(-beta sum m (G(z) - x)^2 / (2 sigma^2)) (include/lsnf.h:
+        lsnf_ais_run).  ``target_accept`` > 0 adapts each chain's step size, <= 0 keeps ``step_size``.  ``eps``
+        [steps,B,nz] and ``u`` [steps,B] inject the noise.  Returns (z_T [B,nz], log w [B] without the likelihood's
+        normalising constant, acceptance rate [B])."""
+        _check_tensor(z0, "z", self.device, (self.batch, self.nz))
+        _check_tensor(x, "x", self.device, (self.batch, self.nc, self.img, self.img))
+        _check_tensor(betas, "betas", self.device, (int(steps) + 1,))
+        m = as_mask(mask, x) if mask is not None else None
+        if eps is not None:
+            _check_tensor(eps, "eps", self.device, (steps, self.batch, self.nz))
+        if u is not None:
+            _check_tensor(u, "u", self.device, (steps, self.batch))
+        z_out = torch.empty_like(z0)
+        log_w = torch.empty(self.batch, dtype=torch.float32, device=self.device)
+        rate = torch.empty_like(log_w)
+        self.act_epoch += 1
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_ais_run(
+                self.handle, z0.data_ptr(), x.data_ptr(), m.data_ptr() if m is not None else None, betas.data_ptr(),
+                int(steps), float(step_size), float(target_accept), float(sigma),
+                eps.data_ptr() if eps is not None else None, u.data_ptr() if u is not None else None,
+                int(seed) & (2 ** 64 - 1), int(sample_offset), z_out.data_ptr(), log_w.data_ptr(), rate.data_ptr(),
+                _stream(self.device)), "lsnf_ais_run")
+        return z_out, log_w, rate
+
 
 _PLANS: Dict[Tuple, Plan] = {}
 
