@@ -214,15 +214,21 @@ struct lsnf_plan {
   // concurrently with the generator stages
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  // CUDA graphs of the whole g_l_steps loop, keyed by (steps, step_size, sigma, with_noise, masked); per-call values
-  // (seed, sample offset) are read from device memory, inputs are staged into the workspace
-  // A graph holds one CHUNK of at most `graph_chunk` iterations; the step index of its first iteration is read
-  // from device memory (dyn[2]), so a chain of any length replays the same few graphs (train.py:606: 8 000 steps).
-  // AIS graphs (lsnf_ais_run) carry the flag `ais` and their target acceptance rate, so that they never mix with the
-  // Langevin loops of the same plan.
-  struct LoopGraph {
-    int steps; float step_size, sigma; int with_noise; bool masked; bool ais; float target; cudaGraphExec_t exec;
+  // CUDA graphs of the g_l_steps loop, one per chunk length of at most `graph_chunk` (plan.cu) iterations.  Per-call
+  // values (seed, sample offset, the step index of the chunk's first iteration) are read from device memory (dyn) and
+  // inputs are staged into the workspace, so a chain of any length replays the same few graphs (train.py:606: 8 000
+  // steps).
+  // Every value a captured launch bakes in must be part of the key.  An AIS run's step count is not baked in:
+  // ais_update_kernel reads it from dyn[3] under replay.  A Langevin loop keys with target = 0, an AIS loop
+  // (lsnf_ais_run) with with_noise = 1, and `ais` keeps the two apart.
+  struct LoopKey {
+    int steps; float step_size, sigma; int with_noise; bool masked, ais; float target;
+    bool operator==(const LoopKey& o) const {
+      return steps == o.steps && step_size == o.step_size && sigma == o.sigma && with_noise == o.with_noise &&
+             masked == o.masked && ais == o.ais && target == o.target;
+    }
   };
+  struct LoopGraph { LoopKey key; cudaGraphExec_t exec; };
   std::vector<LoopGraph> graphs;
   cudaStream_t cap_stream = nullptr;
   size_t off_x = 0, off_mask = 0, off_gnorms = 0, off_dyn = 0, off_sk_slots = 0, off_sk_flags = 0;
@@ -232,7 +238,6 @@ struct lsnf_plan {
   int fused_tiles = 0;   // CTAs of the fused last-layer kernel per sample
   long long runs = 0;
   bool use_graphs = true;
-  int graph_chunk = 40;
 };
 
 namespace lsnf {
@@ -302,7 +307,6 @@ int launch_tapgemm_simt(const StageHost& st, cudaStream_t s);
 int launch_tapgemm_tc(const StageHost& st, cudaStream_t s);
 int tc_encode_maps(lsnf_plan* plan, StageHost& st);
 void tc_launch_info(const StageHost& st, int num_sms, lsnf_launch_info* out);
-bool tc_stage_is_pair(const StageHost& st);   // the stage runs on the persistent CTA-pair kernel
 int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w, cudaStream_t s);
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);

@@ -7,10 +7,6 @@
 
 #include "lsnf_internal.cuh"
 
-#ifndef LSNF_PDL_DEFAULT
-#define LSNF_PDL_DEFAULT 1
-#endif
-
 namespace lsnf {
 
 thread_local int g_launch_pdl = 0;   // see lsnf_internal.cuh
@@ -681,8 +677,6 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
   {
     const char* e = getenv("LSNF_NO_GRAPH");
     plan->use_graphs = !(e && e[0] == '1');
-    const char* c = getenv("LSNF_GRAPH_CHUNK");
-    if (c && atoi(c) > 0) plan->graph_chunk = atoi(c);
   }
   plan->bound = true;
   plan->g_packed = plan->f_packed = false;
@@ -1007,11 +1001,15 @@ extern "C" int lsnf_langevin_update(lsnf_plan* plan, float* z, const float* grad
                        nullptr, gnorms, 0, (cudaStream_t)stream);
 }
 
+// Loop iterations per captured graph.  An AIS chunk reads graph_chunk + 1 schedule values from the workspace.
+constexpr int graph_chunk = 40;
+static_assert(graph_chunk < AIS_BETA_FLOATS, "the workspace schedule copy must hold a chunk's values");
+
 extern "C" int lsnf_langevin_launch_count(const lsnf_plan* plan, int32_t steps) {
   if (!plan) return 0;
   // per step: L forward + fused gather/tanh/seed/im2col + L data-gradient + flow + update; once: split_z; per
   // replayed graph chunk: the kernel that sets (seed, sample offset, first step index) in device memory
-  const int chunks = steps > 0 ? (steps + plan->graph_chunk - 1) / plan->graph_chunk : 0;
+  const int chunks = steps > 0 ? (steps + graph_chunk - 1) / graph_chunk : 0;
   return 1 + steps * (2 * plan->n_layers + 3) + chunks;
 }
 
@@ -1052,7 +1050,7 @@ struct LoopTrace {
 static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int steps, float step_size, float sigma,
                          int with_noise,
                          const float* eps, uint64_t seed, uint64_t sample_offset, const uint64_t* dyn, float* gnorms,
-                         cudaStream_t s, const AisArgs* ais = nullptr) {
+                         cudaStream_t s, const AisArgs* ais) {
   const float gscale = sigma_post_scale(sigma);
   int rc;
   static int trace_env = -1;
@@ -1063,22 +1061,11 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
   float* z = (float*)(plan->ws + plan->off_z);
   float* gf = (float*)(plan->ws + plan->off_gradf);
   const float* partial = (const float*)(plan->ws + plan->off_partial);
-  // Programmatic dependent launch across the kernel boundaries of the loop's main stream (lsnf_internal.cuh).
-  // LSNF_PDL: 0 off, 1 every boundary, 2 only boundaries with no CTA-pair kernel on either side, 3 / 4 not into / not
-  // out of a CTA-pair kernel.  The update kernel is never launched this way (it also waits for the flow prior's
+  // Programmatic dependent launch across the kernel boundaries of the loop's main stream (lsnf_internal.cuh), on the
+  // tcgen05 path unless LSNF_PDL=0.  The update kernel is never launched this way (it also waits for the flow prior's
   // stream), nor is the first kernel of a call or of a captured graph (no kernel precedes it there).
-  static const int pdl_mode = [] { const char* e = getenv("LSNF_PDL"); return e ? atoi(e) : LSNF_PDL_DEFAULT; }();
-  const bool tc_path = c.gemm_impl == LSNF_GEMM_TCGEN05;
-  bool prev_pair = false, have_prev = false;
-  auto pdl_ok = [&](bool this_pair) {
-    bool ok = tc_path && have_prev && pdl_mode != 0;
-    if (pdl_mode == 2) ok = ok && !this_pair && !prev_pair;
-    if (pdl_mode == 3) ok = ok && !this_pair;
-    if (pdl_mode == 4) ok = ok && !prev_pair;
-    have_prev = true;
-    prev_pair = this_pair;
-    return ok;
-  };
+  static const bool pdl_env = [] { const char* e = getenv("LSNF_PDL"); return !(e && strcmp(e, "0") == 0); }();
+  const bool use_pdl = pdl_env && c.gemm_impl == LSNF_GEMM_TCGEN05;
   for (int t = 0; t < steps; ++t) {
     tr.on = trace_env == 1 && t == 1 && !dyn;
     tr.mark("start");
@@ -1095,19 +1082,19 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
         LSNF_CUDA(cudaEventRecord(plan->ev_join, plan->side));
       }
       {
-        PdlScope pdl(pdl_ok(tc_path && tc_stage_is_pair(plan->stages[l])));
+        PdlScope pdl(use_pdl && (t > 0 || l > 0));
         if ((rc = run_stage(plan, plan->stages[l], s))) return rc;
       }
       tr.mark(("forward layer " + std::to_string(l)).c_str());
     }
     {
-      PdlScope pdl(pdl_ok(false));
+      PdlScope pdl(use_pdl);
       if ((rc = launch_last_fused(plan, x, mask, ais ? ais->epart : nullptr, sigma_seed_scale(sigma), s))) return rc;
     }
     tr.mark("gather + tanh + recon grad + im2col");
     for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i) {
       {
-        PdlScope pdl(pdl_ok(tc_path && tc_stage_is_pair(plan->stages[i])));
+        PdlScope pdl(use_pdl);
         if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
       }
       tr.mark(("dgrad layer " + std::to_string(plan->stages[i].layer)).c_str());
@@ -1121,10 +1108,71 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
                                    seed, sample_offset, (uint32_t)t, dyn, t == steps - 1 ? gnorms : nullptr, 1, s))) {
       return rc;
     }
-    prev_pair = false;   // the update kernel precedes the next iteration's first layer
     tr.mark("update");
     tr.report();
   }
+  return LSNF_OK;
+}
+
+// Runs `iters` loop iterations on the workspace z, with the Langevin update or, with `ais`, the AIS update.  The
+// first call of a plan runs eagerly (module load, kernel attributes), and so do calls with injected noise: parity
+// runs pass a different eps pointer every time.  Later calls replay CUDA graphs of the loop in chunks of at most
+// graph_chunk iterations: one graph per chunk length, the index of a chunk's first iteration (Philox counter) read
+// from device memory, so test mode's 8 000-step chains (train.py:606) reuse one 40-iteration graph 200 times instead
+// of instantiating 88 000 kernel nodes.  Graphs read the workspace copies of x and the mask, and an AIS graph that of
+// its chunk's schedule values, which are staged before each replay.
+static int run_chain(lsnf_plan* plan, const float* x, const float* mask, int iters, float step_size, float sigma,
+                     int with_noise, const float* eps, uint64_t seed, uint64_t sample_offset, float* gnorms,
+                     cudaStream_t s, const AisArgs* ais = nullptr) {
+  const bool injected = eps || (ais && (ais->eps || ais->u));
+  const bool graph_ok = plan->use_graphs && !injected && iters > 0 && plan->runs > 0;
+  plan->runs++;
+  if (!graph_ok)
+    return langevin_loop(plan, x, mask, iters, step_size, sigma, with_noise, eps, seed, sample_offset, nullptr, gnorms,
+                         s, ais);
+  const lsnf_config& c = plan->cfg;
+  float* x_ws = (float*)(plan->ws + plan->off_x);
+  float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
+  float* gn_ws = (float*)(plan->ws + plan->off_gnorms);
+  float* beta_ws = (float*)(plan->ws + plan->off_ais_beta);
+  const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
+  const size_t xbytes = (size_t)c.batch * c.nc * plan->img * plan->img * 4;
+  LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
+  if (mask) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
+  AisArgs ag = {};
+  if (ais) { ag = *ais; ag.betas = beta_ws; }
+  int rc;
+  for (int done = 0; done < iters;) {
+    const int n = std::min(iters - done, graph_chunk);
+    const lsnf_plan::LoopKey key = {n, step_size, sigma, with_noise, mask != nullptr, ais != nullptr,
+                                    ais ? ais->target : 0.f};
+    cudaGraphExec_t exec = nullptr;
+    for (auto& g : plan->graphs)
+      if (g.key == key) exec = g.exec;
+    if (!exec) {
+      cudaGraph_t graph = nullptr;
+      cudaStream_t cs = plan->cap_stream;
+      LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
+      rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs,
+                         ais ? &ag : nullptr);
+      cudaError_t ce = cudaStreamEndCapture(cs, &graph);
+      if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
+      if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
+      ce = cudaGraphInstantiate(&exec, graph, 0);
+      cudaGraphDestroy(graph);
+      if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
+      if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
+      plan->graphs.push_back({key, exec});
+    }
+    if (ais) {
+      const int nb = std::min(n + 1, iters - done);   // the last iteration reads no next value
+      LSNF_CUDA(cudaMemcpyAsync(beta_ws, ais->betas + done, (size_t)nb * 4, cudaMemcpyDeviceToDevice, s));
+    }
+    if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s, ais ? (uint32_t)ais->total : 0))) return rc;
+    LSNF_CUDA(cudaGraphLaunch(exec, s));
+    done += n;
+  }
+  if (gnorms) LSNF_CUDA(cudaMemcpyAsync(gnorms, gn_ws, 8, cudaMemcpyDeviceToDevice, s));
   return LSNF_OK;
 }
 
@@ -1141,55 +1189,8 @@ extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const 
   const size_t zbytes = (size_t)c.batch * c.nz * 4;
   LSNF_CUDA(cudaMemcpyAsync(z, z0, zbytes, cudaMemcpyDeviceToDevice, s));
   if ((rc = launch_split_z(plan, z, s))) return rc;
-  // The first call of a plan runs eagerly (module load, kernel attributes); later noise-free / Philox calls replay
-  // a CUDA graph of the whole loop.  Injected-noise calls (parity runs) pass a different eps pointer every time
-  // and stay eager.
-  const bool graph_ok = plan->use_graphs && !eps && steps > 0 && plan->runs > 0;
-  plan->runs++;
-  if (!graph_ok) {
-    if ((rc = langevin_loop(plan, x, mask, steps, step_size, sigma, with_noise, eps, seed, sample_offset, nullptr,
-                            gnorms, s)))
-      return rc;
-  } else {
-    // The chain is replayed in chunks of at most `graph_chunk` iterations: one graph per chunk length, the index of
-    // a chunk's first iteration (Philox counter) is read from device memory, so test mode's 8 000-step chains
-    // (train.py:606) reuse one 40-iteration graph 200 times instead of instantiating 88 000 kernel nodes.
-    // A masked call's graph reads the workspace copy of the mask, so masked and unmasked loops never share a graph.
-    float* x_ws = (float*)(plan->ws + plan->off_x);
-    float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
-    const bool masked = mask != nullptr;
-    float* gn_ws = (float*)(plan->ws + plan->off_gnorms);
-    const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
-    const size_t xbytes = (size_t)c.batch * c.nc * plan->img * plan->img * 4;
-    LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
-    if (masked) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
-    for (int done = 0; done < steps;) {
-      const int n = std::min(steps - done, plan->graph_chunk);
-      cudaGraphExec_t exec = nullptr;
-      for (auto& g : plan->graphs)
-        if (g.steps == n && g.step_size == step_size && g.sigma == sigma && g.with_noise == with_noise &&
-            g.masked == masked && !g.ais)
-          exec = g.exec;
-      if (!exec) {
-        cudaGraph_t graph = nullptr;
-        cudaStream_t cs = plan->cap_stream;
-        LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-        rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs);
-        cudaError_t ce = cudaStreamEndCapture(cs, &graph);
-        if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-        if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
-        ce = cudaGraphInstantiate(&exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
-        if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
-        plan->graphs.push_back({n, step_size, sigma, with_noise, masked, false, 0.f, exec});
-      }
-      if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s))) return rc;
-      LSNF_CUDA(cudaGraphLaunch(exec, s));
-      done += n;
-    }
-    if (gnorms) LSNF_CUDA(cudaMemcpyAsync(gnorms, gn_ws, 8, cudaMemcpyDeviceToDevice, s));
-  }
+  if ((rc = run_chain(plan, x, mask, steps, step_size, sigma, with_noise, eps, seed, sample_offset, gnorms, s)))
+    return rc;
   LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
   return LSNF_OK;
 }
@@ -1230,55 +1231,9 @@ extern "C" int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, co
   a.tiles = plan->fused_tiles; a.total = steps;
   a.step0 = step_size; a.target = target_accept > 0.f ? target_accept : 0.f;
   a.inv2s2 = 0.5f / (sigma * sigma);
-  const int iters = steps + 1;   // iteration 0 only initialises and proposes, the last one only decides
-  const bool graph_ok = plan->use_graphs && !eps && !u && plan->runs > 0;
-  plan->runs++;
-  if (!graph_ok) {
-    if ((rc = langevin_loop(plan, x, mask, iters, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, nullptr, s,
-                            &a)))
-      return rc;
-  } else {
-    // As lsnf_langevin_run_masked: chunks of at most graph_chunk iterations, inputs staged into the workspace.  The
-    // schedule is not captured either: before each replay, the chunk's values are copied into the workspace.
-    float* x_ws = (float*)(plan->ws + plan->off_x);
-    float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
-    float* beta_ws = (float*)(plan->ws + plan->off_ais_beta);
-    const bool masked = mask != nullptr;
-    const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
-    const size_t xbytes = (size_t)B * c.nc * plan->img * plan->img * 4;
-    LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
-    if (masked) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
-    AisArgs ag = a;
-    ag.betas = beta_ws;
-    const int chunk = std::min(plan->graph_chunk, AIS_BETA_FLOATS - 1);
-    for (int done = 0; done < iters;) {
-      const int n = std::min(iters - done, chunk);
-      cudaGraphExec_t exec = nullptr;
-      for (auto& g : plan->graphs)
-        if (g.ais && g.steps == n && g.step_size == step_size && g.sigma == sigma && g.masked == masked &&
-            g.target == a.target)
-          exec = g.exec;
-      if (!exec) {
-        cudaGraph_t graph = nullptr;
-        cudaStream_t cs = plan->cap_stream;
-        LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-        rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, 1, nullptr, 0, 0, dyn, nullptr, cs, &ag);
-        cudaError_t ce = cudaStreamEndCapture(cs, &graph);
-        if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
-        if (ce != cudaSuccess) return cuda_fail(ce, "cudaStreamEndCapture");
-        ce = cudaGraphInstantiate(&exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (ce != cudaSuccess) return cuda_fail(ce, "cudaGraphInstantiate");
-        if (plan->graphs.size() >= 8) { cudaGraphExecDestroy(plan->graphs.front().exec); plan->graphs.erase(plan->graphs.begin()); }
-        plan->graphs.push_back({n, step_size, sigma, 1, masked, true, a.target, exec});
-      }
-      const int nb = std::min(n + 1, iters - done);   // the last iteration reads no next value
-      LSNF_CUDA(cudaMemcpyAsync(beta_ws, betas + done, (size_t)nb * 4, cudaMemcpyDeviceToDevice, s));
-      if ((rc = launch_set_dyn(plan, seed, sample_offset, (uint32_t)done, s, (uint32_t)steps))) return rc;
-      LSNF_CUDA(cudaGraphLaunch(exec, s));
-      done += n;
-    }
-  }
+  // steps + 1 iterations: iteration 0 only initialises and proposes, the last one only decides
+  if ((rc = run_chain(plan, x, mask, steps + 1, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, s, &a)))
+    return rc;
   LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
   LSNF_CUDA(cudaMemcpyAsync(log_w, a.scal + 5 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
   LSNF_CUDA(cudaMemcpyAsync(accept_rate, a.scal + 6 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));

@@ -15,7 +15,6 @@
 //   tapgemm_tc2_kernel<DEEP> (persistent cta_group::2 pairs for the 256-wide stages); the host picks per stage
 //   (use_pair, ring_geometry, out_tma_kind, pair_stream_k -- mirrored by lsnf_plan_stage_launch_info).
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <type_traits>
 
@@ -23,9 +22,6 @@
 
 namespace lsnf {
 
-#ifndef LSNF_EXP_FWD2PASS
-#define LSNF_EXP_FWD2PASS 0   // 1: forward stages use weights' hi halves only; 2: activations' hi halves only
-#endif
 constexpr int TC_EPI_WARPS = 8;                       // two warps per TMEM lane quarter, each owning half the columns
 constexpr int TC_THREADS = 64 + 32 * TC_EPI_WARPS;
 constexpr int A_TILE_BYTES = BLOCK_M * BLOCK_K * 2;  // 16 KiB per hi or lo half
@@ -429,14 +425,6 @@ tapgemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             const uint64_t a_hi = da + 2 * k, a_lo = a_hi + (A_TILE_BYTES >> 4);
             const uint64_t b_hi = db + 2 * k, b_lo = b_hi + (Cfg::B_TILE_BYTES >> 4);
             if (three) {
-#if LSNF_EXP_FWD2PASS   // experiment builds only (tools/run_fwd2pass_ab.sh): drop one cross term of the forward stages
-              if (st.fp16) {
-                if (LSNF_EXP_FWD2PASS == 1) umma_bf16(tmem_base, a_lo, b_hi, idesc, (it > it0 || k > 0) ? 1u : 0u);
-                else umma_bf16(tmem_base, a_hi, b_lo, idesc, (it > it0 || k > 0) ? 1u : 0u);
-                umma_bf16(tmem_base, a_hi, b_hi, idesc, 1u);
-                continue;
-              }
-#endif
               umma_bf16(tmem_base, a_lo, b_hi, idesc, (it > it0 || k > 0) ? 1u : 0u);
               umma_bf16(tmem_base, a_hi, b_lo, idesc, 1u);
               umma_bf16(tmem_base, a_hi, b_hi, idesc, 1u);
@@ -897,14 +885,6 @@ tapgemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
               const uint64_t a_hi = da + 2 * k, a_lo = a_hi + (A_TILE_BYTES >> 4);
               const uint64_t b_hi = db + 2 * k, b_lo = b_hi + (P_B_TILE_BYTES >> 4);
               if (three) {
-#if LSNF_EXP_FWD2PASS
-                if (st.fp16) {
-                  if (LSNF_EXP_FWD2PASS == 1) umma2_bf16(d_tmem, a_lo, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
-                  else umma2_bf16(d_tmem, a_hi, b_lo, idesc, (it > w.ka || k > 0) ? 1u : 0u);
-                  umma2_bf16(d_tmem, a_hi, b_hi, idesc, 1u);
-                  continue;
-                }
-#endif
                 umma2_bf16(d_tmem, a_lo, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
                 umma2_bf16(d_tmem, a_hi, b_lo, idesc, 1u);
                 umma2_bf16(d_tmem, a_hi, b_hi, idesc, 1u);
@@ -978,11 +958,6 @@ static EncodeTiledFn get_encode() {
   return fn;
 }
 
-static bool pair_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("LSNF_NO_PAIR"); v = (e && e[0] == '1') ? 0 : 1; }
-  return v == 1;
-}
 // The CTA-pair kernel serves every stage with 256-wide N tiles.  A stage with a single M tile still uses it: the
 // second CTA of each pair then owns an all-padding tile (its A boxes are out of bounds -> zero fill, no traffic; its
 // stores are clipped), which wastes half of a tensor pipe that such weight-streaming stages leave idle anyway, and
@@ -995,11 +970,9 @@ static bool use_pair(const StageHost& sh) {
   const StageDev& d = sh.dev;
   const int mtiles = d.tiles_b * d.tiles_h * d.tiles_w;
   const int total = d.ph[0].ntaps * (d.Ka / BLOCK_K);
-  return pair_enabled() && !d.wgrad && d.block_n == 256 && d.n_pad % 256 == 0 && d.ksplit == 1 && total >= 3 &&
+  return !d.wgrad && d.block_n == 256 && d.n_pad % 256 == 0 && d.ksplit == 1 && total >= 3 &&
          (mtiles >= 2 || total >= 8);
 }
-
-bool tc_stage_is_pair(const StageHost& sh) { return use_pair(sh); }
 
 // Ring of the 1-CTA kernel for one launch: stage bytes, depth, dynamic shared memory to request.
 struct RingGeom { int nst; size_t stage_bytes, smem; };
@@ -1023,18 +996,12 @@ static RingGeom ring_geometry(const StageDev& d) {
   return {nst, stage, smem};
 }
 
-static bool tma_store_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("LSNF_NO_TMA_STORE"); v = (e && e[0] == '1') ? 0 : 1; }
-  return v == 1;
-}
-
 // Which tensor-store map the 16-bit output of a stage gets: 1 stride-2 forward [B][2H][2W][2C], 2 first layer
 // [B][k*k][2C], 3 plain gradient [B][H][W][2C], 4 phase-split gradient; 0 = per-thread stores.
 static int out_tma_kind(const StageHost& sh) {
   const StageDev& d = sh.dev;
   const bool wide_single = d.block_n >= 128 && d.n_pad % d.block_n == 0 && d.ksplit == 1;   // 1-CTA kernel, wide N tile
-  if (!(use_pair(sh) || wide_single) || !(d.epi == EPI_ACT_HL || d.epi == EPI_GRAD_HL) || !tma_store_enabled()) return 0;
+  if (!(use_pair(sh) || wide_single) || !(d.epi == EPI_ACT_HL || d.epi == EPI_GRAD_HL)) return 0;
   if (d.epi == EPI_ACT_HL && sh.first) return 2;
   if (d.epi == EPI_ACT_HL && d.ms == 2) return 1;
   if (d.epi == EPI_GRAD_HL && !d.split) return 3;
@@ -1149,9 +1116,7 @@ static bool pair_stream_k(const StageDev& st, int max_pairs) {
   const int rounds = (num_tiles + max_pairs - 1) / max_pairs;
   const long long static_units = (long long)rounds * total;                        // critical path, whole tiles
   const long long sk_units = ((long long)num_tiles * total + max_pairs - 1) / max_pairs + 35;
-  static int sk_env = -1;
-  if (sk_env < 0) { const char* e = getenv("LSNF_STREAMK"); sk_env = e ? atoi(e) : 2; }   // 0 off, 1 always, 2 auto
-  return (sk_env == 1 || (sk_env == 2 && sk_units < static_units)) && total >= 8 &&
+  return sk_units < static_units && total >= 8 &&
          (long long)num_tiles * total >= 4LL * max_pairs && max_pairs <= 80;
 }
 

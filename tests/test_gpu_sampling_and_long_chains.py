@@ -173,16 +173,16 @@ np.save({out!r}, np.stack(outs))   # [eager first call, graph replay]
 
 
 def test_programmatic_dependent_launch_changes_no_bit(tmp_path):
-    # DESIGN.md 4.7: the kernels of the loop chain by programmatic dependent launch (LSNF_PDL, read once per process).
-    # It moves launches and kernel set-up earlier and nothing else, so processes with it on (the default: every
-    # boundary), off and restricted around the CTA-pair kernels must produce the same bits -- at SVHN's true width and
-    # batch, where the loop mixes 1-CTA, CTA-pair / stream-K and CUDA-core kernels, eagerly and from the replayed graph.
+    # DESIGN.md 4.7: the kernels of the loop chain by programmatic dependent launch (LSNF_PDL=0 turns it off, read once
+    # per process).  It moves launches and kernel set-up earlier and nothing else, so processes with it on (the
+    # default) and off must produce the same bits -- at SVHN's true width and batch, where the loop mixes 1-CTA,
+    # CTA-pair / stream-K and CUDA-core kernels, eagerly and from the replayed graph.
     import os
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     got = {}
-    for mode in ("0", "1", "2"):
+    for mode in ("0", "1"):
         out = str(tmp_path / f"z_pdl{mode}.npy")
         env = dict(os.environ, LSNF_PDL=mode)
         subprocess.run([sys.executable, "-c", _PDL_SCRIPT.format(root=root, tests=os.path.join(root, "tests"), out=out)],
@@ -190,4 +190,4 @@ def test_programmatic_dependent_launch_changes_no_bit(tmp_path):
         got[mode] = np.load(out)
         assert np.isfinite(got[mode]).all()
         assert np.array_equal(got[mode][0], got[mode][1])        # eager == replay within one process
-    assert np.array_equal(got["0"], got["1"]) and np.array_equal(got["0"], got["2"])
+    assert np.array_equal(got["0"], got["1"])

@@ -252,6 +252,32 @@ def test_launch_geometry_scales_with_the_sm_count():
     lib.lsnf_plan_destroy(h)
 
 
+def baseline_launch_records():
+    """Every field of lsnf_plan_stage_launch_info, per stage of every BASELINE configuration."""
+    recs = []
+    for arch, nz, ngf, batch in BASELINE_CONFIGS:
+        lib, h = make_plan(arch, nz, ngf, batch)
+        recs.append([[getattr(li, f) for f, _ in li._fields_ if f != "reserved"] for li in launch_infos(lib, h)])
+        lib.lsnf_plan_destroy(h)
+    return recs
+
+
+def test_launch_records_do_not_depend_on_the_environment():
+    # How a stage launches depends on the stage and the SM count alone: variables that once forced the 1-CTA
+    # kernel, per-thread epilogue stores or no stream-K change no record.
+    import json
+    import os
+    import subprocess
+    import sys
+    tests = os.path.dirname(os.path.abspath(__file__))
+    script = (f"import sys, json; sys.path[:0] = [{os.path.dirname(tests)!r}, {tests!r}]; import test_plan_tables as t; "
+              "print(json.dumps(t.baseline_launch_records()))")
+    env = dict(os.environ, LSNF_NO_PAIR="1", LSNF_NO_TMA_STORE="1", LSNF_STREAMK="0")
+    out = subprocess.run([sys.executable, "-c", script], env=env, check=True, capture_output=True, text=True,
+                         timeout=600).stdout
+    assert json.loads(out.splitlines()[-1]) == baseline_launch_records()
+
+
 def test_multiply_high_division_of_the_fused_last_layer_kernel_is_exact():
     # gen_aux.cu FastDiv: x / d == umulhi(x, floor((2^32 - 1) / d) + 1) whenever x * d < 2^32; the kernel divides
     # tile-local indices (< 2^16) by tile extents (< 2^11)
