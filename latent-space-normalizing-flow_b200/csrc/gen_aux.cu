@@ -43,16 +43,14 @@ __global__ void pack_stage_kernel(const float* __restrict__ w, uint16_t* __restr
 }
 
 int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w, cudaStream_t s) {
-  PackGeom g;
-  g.kind = st.kind; g.first = st.first; g.last = st.last; g.k = st.k; g.ci = st.ci; g.co = st.co;
-  g.n_pad = st.info.n_pad; g.ka = st.info.b_k;
+  const PackGeom g = geom_of(st);
   const int rows = st.info.b_rows;
   const long long total = (long long)rows * g.ka;
   const int threads = 256;
   const int blocks = (int)std::min<long long>((total + threads - 1) / threads, 148 * 16);
-  const float* scale = (st.kind == 0 || plan->cfg.bwd_passes == 1)
-                           ? (const float*)(plan->ws + plan->off_wscale + (size_t)st.layer * 16 + 4) : nullptr;
-  pack_stage_kernel<<<blocks, threads, 0, s>>>(w, (uint16_t*)(plan->ws + st.b_off), g, rows, st.ci,
+  const float* scale = (st.info.kind == 0 || plan->cfg.bwd_passes == 1)
+                           ? (const float*)(plan->ws + plan->off_wscale + (size_t)st.info.layer * 16 + 4) : nullptr;
+  pack_stage_kernel<<<blocks, threads, 0, s>>>(w, (uint16_t*)(plan->ws + st.info.b_offset), g, rows, st.ci,
                                                st.info.operand_fp16, scale);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;

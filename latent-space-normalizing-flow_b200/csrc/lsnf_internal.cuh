@@ -73,18 +73,24 @@ struct StageDev {
   PhaseDev ph[LSNF_MAX_PHASES];
 };
 
+// How one tap-GEMM stage launches on a device with a given SM count: decided by tc_plan_launch (tapgemm_tc.cu) alone.
+using TcKernel = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, StageDev);
+struct TcLaunch {
+  TcKernel kernel = nullptr;   // tapgemm_tc2_kernel<passes == 1> or tapgemm_tc_kernel<block_n>; null: no such N tile
+  lsnf_launch_info info;       // what lsnf_plan_stage_launch_info reports: grid, block, shared memory, ring depth,
+                               // stream-K, tensor-store kind, TMEM columns
+};
+
 struct StageHost {
-  lsnf_stage_info info;
-  StageDev dev;
+  lsnf_stage_info info;   // layer, kind (0 forward, 1 data gradient, 2 weight gradient), workspace offsets, tables
+  StageDev dev;           // derived from info by fill_dev (plan.cu); lsnf_plan_bind adds the workspace pointers and
+                          // nst, sk_enable and out_tma from `launch`
+  TcLaunch launch;        // for the plan's device (lsnf_plan_bind)
   CUtensorMap tmA, tmB, tmO;
   bool maps_ready = false;
-  int layer = 0;
-  int kind = 0;      // 0 fwd, 1 bwd
   int k = 0, s = 0, p = 0, ci = 0, co = 0;  // the ConvTranspose2d this stage belongs to
-  size_t a_off = 0, b_off = 0, out_off = 0, mbits_off = 0, bias_off = 0;
-  size_t b_bytes = 0;
   bool last = false, first = false;
-  int num_sms = 148;   // SM count of the plan's device (set by lsnf_plan_bind): persistent grids, stream-K shares
+  size_t mbits_off = 0, bias_off = 0;       // workspace offsets of the sign bits and the bias, where the stage has them
 };
 
 struct FlowLayout {
@@ -306,7 +312,8 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
 int launch_tapgemm_simt(const StageHost& st, cudaStream_t s);
 int launch_tapgemm_tc(const StageHost& st, cudaStream_t s);
 int tc_encode_maps(lsnf_plan* plan, StageHost& st);
-void tc_launch_info(const StageHost& st, int num_sms, lsnf_launch_info* out);
+// What launch_tapgemm_tc does for this stage on a device with `num_sms` SMs (no device needed)
+TcLaunch tc_plan_launch(const StageHost& st, int num_sms);
 int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w, cudaStream_t s);
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);
@@ -404,6 +411,10 @@ __host__ __device__ inline bool pack_index(const PackGeom& g, int ci, int co, in
     }
   }
   return true;
+}
+
+inline PackGeom geom_of(const StageHost& st) {
+  return {st.info.kind, st.first, st.last, st.k, st.ci, st.co, st.info.n_pad, st.info.b_k};
 }
 
 }  // namespace lsnf

@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 
 #include "lsnf_internal.cuh"
 
@@ -109,29 +110,36 @@ static int up2_bwd_taps(int n_pad, lsnf_tap* t) {
   return n;
 }
 
-static void fill_dev(lsnf_plan* p, StageHost& st) {
+// The kernel parameter of a stage, derived from its record for all three kinds; lsnf_plan_bind adds only the workspace
+// pointers and nst, sk_enable and out_tma of the launch record.
+static void fill_dev(const lsnf_plan* p, StageHost& st) {
   const lsnf_stage_info& I = st.info;
+  const lsnf_plan::Layer& y = p->layers[I.layer];
+  const bool wg = I.kind == 2;   // weight gradient: one M axis of C_in rows; every blockIdx.z slice is one tap
   StageDev& d = st.dev;
   memset(&d, 0, sizeof(d));
-  d.aP = I.a_planes; d.B = p->cfg.batch; d.Hg = I.grid_h; d.Wg = I.grid_w; d.Ka = I.k_per_tap;
+  d.aP = I.a_planes; d.B = wg ? 1 : p->cfg.batch; d.Hg = I.grid_h; d.Wg = I.grid_w; d.Ka = I.k_per_tap;
   d.bB = I.box_b; d.bH = I.box_h; d.bW = I.box_w;
   d.aH = I.a_h; d.aW = I.a_w; d.tap_gen = I.tap_gen_k; d.b_k = I.b_k; d.b_rows = I.b_rows;
-  d.tiles_b = (d.B + d.bB - 1) / d.bB; d.tiles_h = d.Hg / d.bH; d.tiles_w = d.Wg / d.bW;
+  // (the C_in rows of a weight-gradient stage need not fill its last tile)
+  d.tiles_b = (d.B + d.bB - 1) / d.bB; d.tiles_h = d.Hg / d.bH; d.tiles_w = (d.Wg + d.bW - 1) / d.bW;
   d.n_valid = I.n_valid; d.n_pad = I.n_pad; d.block_n = I.block_n;
   d.nphase = I.n_phases; d.ksplit = I.k_splits;
   {
     const int ntaps0 = I.tap_gen_k ? I.tap_gen_k * I.tap_gen_k : I.n_taps[0];
-    const int total = ntaps0 * (I.k_per_tap / BLOCK_K);
+    const int total = (wg ? 1 : ntaps0) * (I.k_per_tap / BLOCK_K);
     d.it_per_split = (total + I.k_splits - 1) / I.k_splits;
   }
-  d.epi = I.epilogue; d.oC = I.out_channels; d.ms = I.out_mul; d.split = I.out_phase_split;
+  d.epi = I.epilogue; d.bias_mod = I.kind == 0 ? y.co : 0; d.oC = I.out_channels; d.ms = I.out_mul;
+  d.split = I.out_phase_split;
   d.leak = p->cfg.leak;
   d.fp16 = I.operand_fp16; d.passes = I.passes;
   // single-pass data gradients carry fp16 tensors (hi half only) end to end
   const bool single_bwd = p->cfg.bwd_passes == 1;
   d.out_fp16 = (I.epilogue == EPI_ACT_HL || single_bwd) ? 1 : 0;
   d.out_single = (I.epilogue == EPI_GRAD_HL && single_bwd) ? 1 : 0;
-  d.rows_total = (int64_t)p->cfg.batch * I.grid_h * I.grid_w;
+  d.rows_total = (int64_t)d.B * I.grid_h * I.grid_w;
+  d.wgrad = wg ? 1 : 0;
   for (int ph = 0; ph < I.n_phases; ++ph) {
     d.ph[ph].ntaps = I.tap_gen_k ? I.tap_gen_k * I.tap_gen_k : I.n_taps[ph];
     d.ph[ph].mo = I.out_off_y[ph]; d.ph[ph].no = I.out_off_x[ph];
@@ -140,18 +148,40 @@ static void fill_dev(lsnf_plan* p, StageHost& st) {
       d.ph[ph].taps[t] = {(int16_t)s.dy, (int16_t)s.dx, (int16_t)s.plane, 0, s.brow};
     }
   }
+  if (I.kind == 0 && st.last) {
+    d.nc = p->cfg.nc; d.Ho = y.hout; d.Wo = y.hout;
+  } else if (I.kind == 0) {
+    d.sW = 2 * y.co; d.sH = (int64_t)y.hout * d.sW; d.sB = (int64_t)y.hout * d.sH; d.sPos = d.sW;
+  } else if (I.kind == 1 && !st.first) {
+    const int hg = I.grid_h;
+    d.sW = 2 * y.ci;
+    if (I.out_phase_split) {
+      d.sH = (int64_t)(hg / 2) * d.sW; d.sB = (int64_t)(hg / 2) * d.sH; d.sP = (int64_t)d.B * d.sB;
+    } else {
+      d.sH = (int64_t)hg * d.sW; d.sB = (int64_t)hg * d.sH;
+    }
+  } else if (wg && !st.first && !st.last) {
+    // plane and (dy, dx) of every tap: brow = plane * C_out in the transposed gradient, its as-is or column-shifted
+    // copy by dx (TransArgs::xvar); dy shifts the K range by dy zero-haloed rows of Wp positions
+    lsnf_tap tp[16];
+    up2_bwd_taps(y.co, tp);
+    const int wp = p->wg[I.layer].tg.Wp;
+    for (int t = 0; t < 16; ++t)
+      d.ph[0].taps[t] = {0, 0, 0, (int16_t)(tp[t].dy * wp), (tp[t].plane * 2 + (tp[t].dx != 0 ? 1 : 0)) * y.co};
+  }
 }
 
-}  // namespace lsnf
+// Next 1024-byte aligned workspace region; ws_bytes is the running total.
+static size_t take(lsnf_plan* p, size_t bytes) {
+  const size_t o = p->ws_bytes;
+  p->ws_bytes = align_up(o + bytes, 1024);
+  return o;
+}
 
-using namespace lsnf;
-
-extern "C" int lsnf_abi_version(void) { return LSNF_ABI_VERSION; }
-extern "C" const char* lsnf_last_error(void) { return g_err.c_str(); }
-
-extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
-  if (!cfg || !out) return fail(LSNF_ERR_INVALID, "null argument");
-  const lsnf_config& c = *cfg;
+// Checks the config, then the generator's geometry, in this order.  Derives what the checks read: the layer table
+// (with image size, kp, nzp) and the flow layout.
+static int check_config(lsnf_plan* p) {
+  const lsnf_config& c = p->cfg;
   if (c.batch <= 0) return fail(LSNF_ERR_INVALID, "batch must be positive");
   if (c.nz <= 0 || (c.nz & 1)) return fail(LSNF_ERR_INVALID, "nz must be even (model.py:383)");
   if (c.nz % 4) return fail(LSNF_ERR_INVALID, "nz must be a multiple of 4 (128-bit latent rows)");
@@ -165,44 +195,27 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
   if (c.gemm_impl != LSNF_GEMM_TCGEN05 && c.gemm_impl != LSNF_GEMM_SIMT) return fail(LSNF_ERR_INVALID, "bad gemm_impl");
   if (c.bwd_passes != 0 && c.bwd_passes != 1 && c.bwd_passes != 3) return fail(LSNF_ERR_INVALID, "bwd_passes must be 0, 1 or 3");
 
-  lsnf_plan* p = new lsnf_plan();
-  p->cfg = c;
   const int L = arch_layers(c, p->layers);
-  if (L < 0) { delete p; return fail(LSNF_ERR_INVALID, "unknown arch (model.py:154 raises ValueError)"); }
+  if (L < 0) return fail(LSNF_ERR_INVALID, "unknown arch (model.py:154 raises ValueError)");
   p->n_layers = L;
   p->kp = (int)align_up(c.nz, BLOCK_K);
   p->nzp = (int)align_up(c.nz, 128);
-  const int B = c.batch;
-
   if (L > 0) {
-    if (c.nc <= 0 || c.nc > 4) { delete p; return fail(LSNF_ERR_INVALID, "nc must be in 1..4"); }
-    if (c.ngf <= 0) { delete p; return fail(LSNF_ERR_INVALID, "ngf must be positive"); }
+    if (c.nc <= 0 || c.nc > 4) return fail(LSNF_ERR_INVALID, "nc must be in 1..4");
+    if (c.ngf <= 0) return fail(LSNF_ERR_INVALID, "ngf must be positive");
     int h = 1;
     for (int l = 0; l < L; ++l) {
       auto& y = p->layers[l];
       y.hin = h;
       y.hout = (h - 1) * y.s - 2 * y.p + y.k;
       h = y.hout;
-      if (l < L - 1 && y.co % BLOCK_K) {
-        delete p;
+      if (l < L - 1 && y.co % BLOCK_K)
         return fail(LSNF_ERR_INVALID, "hidden generator channel counts must be multiples of 64 (raise --ngf)");
-      }
-      if (y.hin > 128) { delete p; return fail(LSNF_ERR_INVALID, "layer grid wider than 128 not supported"); }
+      if (y.hin > 128) return fail(LSNF_ERR_INVALID, "layer grid wider than 128 not supported");
     }
     p->img = h;
   }
 
-  // ---- workspace layout ----
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
-  p->off_z = take((size_t)B * c.nz * 4);
-  p->off_gradg = take((size_t)B * c.nz * 4);
-  p->off_gradf = take((size_t)B * c.nz * 4);
-  p->off_scalars = take(256);
-  p->off_dyn = take(64);
-  p->off_gnorms = take(64);
-  p->off_norms = take((size_t)2 * B * 4);
-  p->off_flow_out = take((size_t)B * (c.nz + 2) * 4);
   {  // flow parameter block (floats)
     FlowLayout& f = p->fl;
     f.nz = c.nz; f.w = c.f_width; f.half = c.nz / 2; f.n_out = c.f_coupling ? c.nz : c.nz / 2;
@@ -226,16 +239,47 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     // one sample per CTA is the largest footprint; the inverse kernel needs less
     uint32_t ring_floats;
     size_t smem_bytes;
-    if (flow_smem(f, 1, c.f_depth, true, true, &ring_floats, &smem_bytes)) {
-      delete p;
+    if (flow_smem(f, 1, c.f_depth, true, true, &ring_floats, &smem_bytes))
       return fail(LSNF_ERR_INVALID,
                   "flow prior exceeds the " + std::to_string(FLOW_SMEM_BYTES / 1024) +
                       " KB of shared memory of one CTA even at one sample per CTA: its largest matrix (f_width^2, or "
                       "nz^2 with f_flow_permutation 2) plus f_depth * (2 f_width + nz) stashed activations must fit "
                       "(include/lsnf.h, lsnf_config)");
-    }
-    p->off_flow = take(f.step_floats * 4 * c.f_depth);
-    // training stash and flat gradient layout of the flow parameter update (train.py:403-415)
+  }
+
+  // the ConvTranspose2d geometries the stage builders implement: forward stages first, then data gradients
+  for (int l = 0; l < L; ++l) {
+    const auto& y = p->layers[l];
+    const bool up2 = y.k == 4 && y.s == 2 && y.p == 1, same = y.k == 3 && y.s == 1 && y.p == 1;
+    if (l == 0 && !(y.s == 1 && y.p == 0)) return fail(LSNF_ERR_INVALID, "first layer must be s1 p0");
+    if (l == 0 && L == 1) return fail(LSNF_ERR_INVALID, "single-layer generator not supported");
+    if (l > 0 && !(up2 || same))
+      return fail(LSNF_ERR_INVALID, l == L - 1 ? "unsupported last-layer geometry" : "unsupported ConvTranspose2d geometry");
+  }
+  for (int l = L - 1; l >= 0; --l) {
+    const auto& y = p->layers[l];
+    if (l == L - 1 && y.k * y.k * y.co > BLOCK_K) return fail(LSNF_ERR_INVALID, "k*k*nc must be <= 64");
+    if (l > 0 && l < L - 1 && !(y.k == 4 && y.s == 2 && y.p == 1))
+      return fail(LSNF_ERR_INVALID, "unsupported hidden layer geometry");
+  }
+  return LSNF_OK;
+}
+
+// Every region but the tap-GEMM operands and results of the stage builders and the AIS state.
+static void take_regions(lsnf_plan* p) {
+  const lsnf_config& c = p->cfg;
+  const int L = p->n_layers, B = c.batch;
+  const FlowLayout& f = p->fl;
+  p->off_z = take(p, (size_t)B * c.nz * 4);
+  p->off_gradg = take(p, (size_t)B * c.nz * 4);
+  p->off_gradf = take(p, (size_t)B * c.nz * 4);
+  p->off_scalars = take(p, 256);
+  p->off_dyn = take(p, 64);
+  p->off_gnorms = take(p, 64);
+  p->off_norms = take(p, (size_t)2 * B * 4);
+  p->off_flow_out = take(p, (size_t)B * (c.nz + 2) * 4);
+  p->off_flow = take(p, f.step_floats * 4 * c.f_depth);
+  {  // training stash and flat gradient layout of the flow parameter update (train.py:403-415)
     FlowStash& t = p->fstash;
     size_t so = 0;
     auto ts = [&](size_t n) { size_t r = so; so += n; return r; };
@@ -243,9 +287,9 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     t.gu = ts(f.nz); t.gp1 = ts(f.w); t.gp2 = ts(f.w); t.gp3 = ts(f.n_out); t.gx = ts(f.nz);
     t.gl0 = ts(f.nz); t.gl1 = ts(f.w); t.gl2 = ts(f.w); t.gl3 = ts(f.n_out);
     t.layer_floats = so;
-    p->off_fstash = take(so * 4 * (size_t)B * c.f_depth);
+    p->off_fstash = take(p, so * 4 * (size_t)B * c.f_depth);
     // W^-1 [f_depth][nz][nz] and log|det W| [f_depth] when the library evaluates them itself
-    p->off_flinalg = take(((size_t)c.f_depth * f.nz * f.nz + 32) * 4);
+    p->off_flinalg = take(p, ((size_t)c.f_depth * f.nz * f.nz + 32) * 4);
     FlowGradLayout& gl = p->fgrad;
     const size_t sizes[LSNF_FLOW_PTRS_PER_STEP] = {
         (size_t)f.nz, (size_t)f.nz, (size_t)f.nz * f.nz, (size_t)f.half * f.w, (size_t)f.w, (size_t)f.w,
@@ -254,318 +298,300 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
     for (int i = 0; i < LSNF_FLOW_PTRS_PER_STEP; ++i) { gl.off[i] = go; gl.size[i] = sizes[i]; go += (sizes[i] + 3) / 4 * 4; }
     gl.step_floats = go;
   }
+  if (L == 0) return;
+  p->off_zhl = take(p, (size_t)B * 2 * p->kp * 2);
+  p->off_sk_slots = take(p, (size_t)160 * 128 * 256 * 4);   // stream-K partial accumulators (<= 160 CTAs)
+  p->off_sk_flags = take(p, (size_t)160 * 8 * 4);
+  p->off_x = take(p, (size_t)B * c.nc * p->img * p->img * 4);
+  p->off_mask = take(p, (size_t)B * c.nc * p->img * p->img * 4);   // the graph-replayed loop's copy of a mask
+  for (int l = 0; l < L - 1; ++l) {
+    const auto& y = p->layers[l];
+    const size_t bytes = (size_t)B * y.hout * y.hout * 2 * y.co * 2;
+    p->off_act[l] = take(p, bytes);
+    p->off_gpre[l] = take(p, bytes);
+    p->off_mbits[l] = take(p, (size_t)B * y.hout * y.hout * y.co / 8);   // LeakyReLU sign bits of act[l]
+  }
+  for (int l = 0; l < L; ++l) p->off_bias[l] = take(p, (size_t)p->layers[l].co * 4);
+  p->off_xhat = take(p, (size_t)B * c.nc * p->img * p->img * 4);
+  p->off_wscale = take(p, (size_t)L * 16);   // per layer: |w|max bits, scale 2^k, descale 2^-k
+  const auto& yl = p->layers[L - 1];
+  const int kk = yl.k * yl.k * yl.co;
+  p->off_dlast = take(p, (size_t)B * yl.hin * yl.hin * (kk <= 32 ? 32 : 64) * 4);
+  p->off_im2col = take(p, (size_t)B * yl.hin * yl.hin * 2 * BLOCK_K * 2);
+}
 
+// A cleared record of `kind` for layer l, and the ConvTranspose2d it belongs to.
+static void set_conv(StageHost& st, const lsnf_plan* p, int kind, int l) {
+  const auto& y = p->layers[l];
+  memset(&st.info, 0, sizeof(st.info));
+  st.info.kind = kind; st.info.layer = l;
+  st.k = y.k; st.s = y.s; st.p = y.p; st.ci = y.ci; st.co = y.co;
+  st.first = l == 0; st.last = l == p->n_layers - 1;
+}
+
+// Forward stage of layer l (train.py:312): stages[l].
+static void build_forward_stage(lsnf_plan* p, int l) {
+  const lsnf_config& c = p->cfg;
+  const int B = c.batch;
+  const auto& y = p->layers[l];
+  StageHost& st = p->stages[l];
+  set_conv(st, p, 0, l);
+  lsnf_stage_info& I = st.info;
+  I.a_planes = 1;
+  I.k_splits = 1;
+  if (st.first) {
+    I.grid_h = I.grid_w = 1;
+    I.k_per_tap = p->kp;
+    I.n_valid = y.k * y.k * y.co; I.n_pad = I.n_valid; I.block_n = pick_block_n(y.co);
+    I.n_phases = 1; I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
+    I.out_mul = 1; I.out_channels = y.co; I.epilogue = EPI_ACT_HL;
+    I.a_offset = p->off_zhl;
+  } else {
+    I.grid_h = I.grid_w = y.hin;
+    I.k_per_tap = y.ci;
+    I.out_channels = y.co;
+    if (st.last) {
+      // direct product D[pos][(tap, c)] = act[pos][:] . W[:, c, tap]; last_gather_tanh sums the taps that land
+      // on each output pixel (col2im without atomics), adds the bias and applies tanh
+      I.n_valid = y.k * y.k * y.co; I.n_pad = I.n_valid <= 32 ? 32 : 64; I.block_n = I.n_pad;
+      I.epilogue = EPI_PARTIAL; I.out_channels = I.n_pad;
+      I.n_phases = 1; I.out_mul = 1; I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
+      p->dlast_pad = I.n_pad;
+    } else {
+      I.n_valid = I.n_pad = y.co; I.epilogue = EPI_ACT_HL;
+      I.block_n = pick_block_n_hidden(y.co, B * y.hin * y.hin, (y.k == 4 && y.s == 2) ? 4 : 1,
+                                      ((y.k == 4 && y.s == 2) ? 4 : y.k * y.k) * (y.ci / BLOCK_K));
+      if (y.k == 4 && y.s == 2 && y.p == 1) {
+        I.n_phases = 4; I.out_mul = 2;
+        for (int ph = 0; ph < 4; ++ph) {
+          I.n_taps[ph] = up2_fwd_taps(ph >> 1, ph & 1, I.n_pad, I.taps[ph]);
+          I.out_off_y[ph] = ph >> 1; I.out_off_x[ph] = ph & 1;
+        }
+      } else {   // k3 s1 p1
+        I.n_phases = 1; I.out_mul = 1; I.n_taps[0] = 9;
+        for (int ky = 0; ky < 3; ++ky)
+          for (int kx = 0; kx < 3; ++kx) I.taps[0][ky * 3 + kx] = {1 - ky, 1 - kx, 0, (ky * 3 + kx) * I.n_pad};
+      }
+    }
+    I.a_offset = p->off_act[l - 1];
+  }
+  make_box(I.grid_h, I.grid_w, &I.box_b, &I.box_h, &I.box_w);
+  const size_t b_rows = (st.first || st.last) ? (size_t)I.n_pad : (size_t)y.k * y.k * I.n_pad;
+  I.operand_fp16 = 1; I.passes = 3;
+  I.a_h = I.grid_h; I.a_w = I.grid_w; I.tap_gen_k = 0; I.b_k = I.k_per_tap; I.b_rows = (int)b_rows;
+  I.b_offset = take(p, b_rows * 2 * I.k_per_tap * 2);
+  I.out_offset = st.last ? p->off_dlast : p->off_act[l];
+  st.mbits_off = st.last ? 0 : p->off_mbits[l];
+  st.bias_off = p->off_bias[l];
+  int taps_sum = 0;
+  for (int ph = 0; ph < I.n_phases; ++ph) taps_sum += I.n_taps[ph];
+  I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)I.n_valid * I.k_per_tap * taps_sum;
+  if (st.first) I.flops = 2LL * B * (long long)I.n_valid * c.nz;
+  if (st.last) I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)y.k * y.k * y.co * y.ci;
+  fill_dev(p, st);
+}
+
+// Data-gradient stage of layer l (train.py:314): stages[L + (L - 1 - l)], run from the last layer down to the first.
+// The first layer's stage writes split-K partials whose region lsnf_plan_create takes after all data-gradient stages.
+static void build_dgrad_stage(lsnf_plan* p, int l) {
+  const lsnf_config& c = p->cfg;
+  const int L = p->n_layers, B = c.batch;
+  const auto& y = p->layers[l];
+  StageHost& st = p->stages[L + (L - 1 - l)];
+  set_conv(st, p, 1, l);
+  lsnf_stage_info& I = st.info;
+  I.a_planes = 1; I.k_splits = 1;
+  I.n_phases = 1; I.out_mul = 1;
+  size_t b_rows;
+  if (st.last) {
+    I.grid_h = I.grid_w = y.hin;
+    I.k_per_tap = BLOCK_K;
+    I.n_valid = I.n_pad = y.ci; I.block_n = pick_block_n(y.ci);
+    I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
+    I.a_offset = p->off_im2col;
+    b_rows = I.n_pad;
+  } else if (st.first) {
+    I.grid_h = I.grid_w = 1;
+    I.k_per_tap = y.co;           // per output position of the first layer; taps run over the k*k positions
+    I.n_valid = c.nz; I.n_pad = p->nzp; I.block_n = 128;
+    I.n_taps[0] = 0;              // generated: tap t -> (dy, dx) = (t / k, t % k), B column offset t*co
+    I.a_offset = p->off_gpre[0];
+    b_rows = I.n_pad;
+    const int kblocks = y.k * y.k * y.co / BLOCK_K;
+    const int mtiles = (B + BLOCK_M - 1) / BLOCK_M;
+    int want = std::max(1, (148 + mtiles - 1) / mtiles);   // about one wave of CTAs
+    int per = std::max(2, (kblocks + want - 1) / want);
+    I.k_splits = (kblocks + per - 1) / per;
+    per = (kblocks + I.k_splits - 1) / I.k_splits;       // what the kernels use (it_per_split)
+    I.k_splits = (kblocks + per - 1) / per;               // every split is non-empty
+    p->ksplit_first = I.k_splits;
+  } else {   // k4 s2 p1
+    I.grid_h = I.grid_w = y.hin;
+    I.k_per_tap = y.co;
+    I.n_valid = I.n_pad = y.ci; I.block_n = pick_block_n_hidden(y.ci, B * y.hin * y.hin, 1, 16 * (y.co / BLOCK_K));
+    I.a_planes = 4;
+    I.n_taps[0] = up2_bwd_taps(I.n_pad, I.taps[0]);
+    I.a_offset = p->off_gpre[l];
+    b_rows = (size_t)16 * I.n_pad;
+  }
+  make_box(I.grid_h, I.grid_w, &I.box_b, &I.box_h, &I.box_w);
+  const size_t b_k = st.first ? (size_t)y.k * y.k * y.co : (size_t)I.k_per_tap;
+  I.operand_fp16 = c.bwd_passes == 1 ? 1 : 0; I.passes = c.bwd_passes == 1 ? 1 : 3;
+  I.a_h = st.first ? y.k : I.grid_h; I.a_w = st.first ? y.k : I.grid_w;
+  I.tap_gen_k = st.first ? y.k : 0; I.b_k = (int)b_k; I.b_rows = (int)b_rows;
+  I.b_offset = take(p, b_rows * 2 * b_k * 2);
+  if (st.first) {
+    I.epilogue = EPI_PARTIAL; I.out_channels = I.n_pad;
+  } else {
+    I.epilogue = EPI_GRAD_HL; I.out_channels = y.ci;
+    // the consumer (data gradient of layer l-1) reads phase-split when it is a stride-2 layer
+    I.out_phase_split = (l - 1 > 0) ? 1 : 0;
+    I.out_offset = p->off_gpre[l - 1];
+    st.mbits_off = p->off_mbits[l - 1];
+  }
+  I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)I.n_valid *
+            (st.last ? y.k * y.k * y.co : (st.first ? (long long)y.k * y.k * y.co : 16LL * y.co));
+  fill_dev(p, st);
+}
+
+// Generator parameter update of layer l (train.py:390-394): transposed operands, the weight-gradient tap-GEMM and where
+// its results go in the flat gradient buffer (gen_grad_floats is the running total).
+static void build_wgrad_layer(lsnf_plan* p, int l) {
+  const lsnf_config& c = p->cfg;
+  const int L = p->n_layers, B = c.batch;
+  const auto& y = p->layers[l];
+  WgradLayer& w = p->wg[l];
+  const bool first = (l == 0), last = (l == L - 1);
+  const int kk = y.k * y.k;
+  const bool single = c.bwd_passes == 1;   // gradient tensors hold fp16 hi halves only
+  w.kk = kk;
+  int n_cols, hp, wp, halo, block_n;
+  TransArgs& ta = w.ta;
+  TransArgs& tg = w.tg;
+  memset(&ta, 0, sizeof(ta)); memset(&tg, 0, sizeof(tg));
+  if (first) {
+    // dW0[ci][(tap, co)] = sum_b z[b][ci] * gpre_0[b][tap][co]
+    w.a_rows = (int)align_up(c.nz, 128); hp = wp = 1; halo = 0;
+    w.Kp = (long long)align_up(B, BLOCK_K);
+    w.planes = 1; w.g_rows = kk * y.co; w.ntaps = 1; n_cols = kk * y.co; block_n = pick_block_n(n_cols);
+    ta.P = 1; ta.B = B; ta.H = ta.W = 1; ta.C = p->kp; ta.s_b = 2 * p->kp; ta.src_fp16 = 1; ta.c_rows = w.a_rows;
+    tg.P = kk; tg.B = B; tg.H = tg.W = 1; tg.C = y.co; tg.s_plane = 2 * y.co; tg.s_b = (long long)kk * 2 * y.co;
+    tg.c_rows = y.co;
+  } else if (last) {
+    // dW[ci][(tap, c)] = sum_pos act[pos][ci] * im2col_seed[pos][(tap, c)]   (the seed already holds the taps)
+    w.a_rows = y.ci; hp = wp = y.hin; halo = 0;
+    w.Kp = (long long)align_up((size_t)B * y.hin * y.hin, BLOCK_K);
+    w.planes = 1; w.g_rows = BLOCK_K; w.ntaps = 1; n_cols = BLOCK_K; block_n = 64;
+    ta.P = 1; ta.B = B; ta.H = ta.W = y.hin; ta.C = y.ci; ta.s_w = 2 * y.ci; ta.s_h = (long long)y.hin * ta.s_w;
+    ta.s_b = (long long)y.hin * ta.s_h; ta.src_fp16 = 1; ta.c_rows = y.ci;
+    tg.P = 1; tg.B = B; tg.H = tg.W = y.hin; tg.C = BLOCK_K; tg.s_w = 2 * BLOCK_K; tg.s_h = (long long)y.hin * tg.s_w;
+    tg.s_b = (long long)y.hin * tg.s_h; tg.c_rows = BLOCK_K;
+  } else {
+    // k4/s2/p1: per tap, dW[ci][co] = sum_pos act[pos][ci] * gpre[plane_tap][pos + (dy, dx)][co].  One zero halo
+    // row above and below every sample (dy becomes the K offset dy * Wp, a multiple of 8 elements = 16 bytes as
+    // TMA box origins must be); dx picks the as-is or the column-shifted copy of the phase plane (TransArgs::xvar)
+    w.a_rows = y.ci; hp = y.hin + 2; wp = (int)align_up(y.hin, 8); halo = 1;
+    w.Kp = (long long)align_up((size_t)B * hp * wp, BLOCK_K);
+    w.planes = 8; w.g_rows = y.co; w.ntaps = 16; n_cols = y.co; block_n = pick_block_n(y.co);
+    ta.P = 1; ta.B = B; ta.H = ta.W = y.hin; ta.C = y.ci; ta.s_w = 2 * y.ci; ta.s_h = (long long)y.hin * ta.s_w;
+    ta.s_b = (long long)y.hin * ta.s_h; ta.src_fp16 = 1; ta.c_rows = y.ci;
+    tg.P = 4; tg.B = B; tg.H = tg.W = y.hin; tg.C = y.co; tg.s_w = 2 * y.co; tg.s_h = (long long)y.hin * tg.s_w;
+    tg.s_b = (long long)y.hin * tg.s_h; tg.s_plane = (long long)B * tg.s_b; tg.c_rows = y.co; tg.xvar = 1;
+  }
+  ta.Hp = tg.Hp = hp; ta.Wp = tg.Wp = wp; ta.halo = tg.halo = halo; ta.Kp = tg.Kp = w.Kp;
+  tg.src_fp16 = single ? 1 : 0; tg.src_single = single ? 1 : 0;
+  w.off_aT = take(p, (size_t)w.a_rows * 2 * w.Kp * 2);
+  w.off_gT = take(p, (size_t)w.planes * w.g_rows * 2 * w.Kp * 2);
+  // the tap-GEMM: rows = C_in, columns = C_out (or (tap, co) / the 64 seed columns), K = flattened positions
+  StageHost& st = w.st;
+  set_conv(st, p, 2, l);
+  lsnf_stage_info& I = st.info;
+  I.grid_h = 1; I.grid_w = w.a_rows; I.box_b = 1; I.box_h = 1; I.box_w = BLOCK_M;
+  I.k_per_tap = (int)w.Kp; I.n_valid = n_cols; I.block_n = block_n; I.n_pad = (int)align_up(n_cols, block_n);
+  I.n_phases = 1; I.n_taps[0] = w.ntaps; I.out_mul = 1; I.out_channels = I.n_pad; I.epilogue = EPI_PARTIAL;
+  I.a_planes = 1; I.a_h = 1; I.a_w = w.a_rows; I.b_k = (int)w.Kp; I.b_rows = w.planes * w.g_rows;
+  I.operand_fp16 = 0; I.passes = 3;
+  const int kblocks = (int)(w.Kp / BLOCK_K);
+  const int tiles = ((w.a_rows + BLOCK_M - 1) / BLOCK_M) * (I.n_pad / block_n) * w.ntaps;
+  int want = std::max(1, (2 * 148 + tiles - 1) / tiles);
+  want = std::min(want, std::max(1, kblocks / 4));          // at least four K blocks per split
+  const int per = (kblocks + want - 1) / want;
+  w.ksplit = (kblocks + per - 1) / per;                     // every split is non-empty: it_per_split = per
+  I.k_splits = w.ksplit;
+  for (int t = 0; t < w.ntaps; ++t) I.taps[0][t] = {0, 0, 0, 0};
+  I.flops = 2LL * w.a_rows * (long long)n_cols * w.Kp * w.ntaps;
+  I.a_offset = w.off_aT; I.b_offset = w.off_gT;
+  w.off_part = take(p, (size_t)w.ntaps * w.ksplit * w.a_rows * I.n_pad * 4);
+  I.out_offset = w.off_part;
+  fill_dev(p, st);
+  // results: dW in the parameter's own layout, then db
+  w.grad_w_off = p->gen_grad_floats; p->gen_grad_floats += align_up((size_t)y.ci * y.co * kk, 4);
+  w.grad_b_off = p->gen_grad_floats; p->gen_grad_floats += align_up((size_t)y.co, 4);
+  FinalizeArgs& f = w.fin;
+  memset(&f, 0, sizeof(f));
+  f.ksplit = w.ksplit; f.kk = kk; f.C_in = y.ci; f.C_out = y.co;
+  if (first) { f.s_tap = y.co; f.s_split = 0; f.s_ci = I.n_pad; f.ksplit = 1; }
+  else if (last) { f.s_tap = y.co; f.s_split = (long long)w.a_rows * I.n_pad; f.s_ci = I.n_pad; }
+  else { f.s_tap = (long long)w.ksplit * w.a_rows * I.n_pad; f.s_split = (long long)w.a_rows * I.n_pad; f.s_ci = I.n_pad; }
+  RowSumArgs& r = w.rs;
+  memset(&r, 0, sizeof(r));
+  r.Kp = w.Kp; r.C = y.co;
+  if (first) { r.nsel = kk; for (int t = 0; t < kk; ++t) r.sel[t] = t * y.co; }
+  else if (last) {
+    // every output pixel is produced by exactly one of these taps (oy = iy*s - p + ky covers each oy once)
+    r.nsel = 0;
+    for (int ky = 0; ky < y.k; ++ky)
+      for (int kx = 0; kx < y.k; ++kx) {
+        const bool once_y = y.s == 1 ? ky == y.p : (ky == 1 || ky == 2);
+        const bool once_x = y.s == 1 ? kx == y.p : (kx == 1 || kx == 2);
+        if (once_y && once_x) r.sel[r.nsel++] = (ky * y.k + kx) * y.co;
+      }
+  } else { r.nsel = 4; for (int q = 0; q < 4; ++q) r.sel[q] = 2 * q * y.co; }   // the as-is copy of every plane
+}
+
+// Annealed importance sampling (lsnf_ais_run): chain state and energies, after every other region.
+static void take_ais_regions(lsnf_plan* p) {
+  const int B = p->cfg.batch, nz = p->cfg.nz;
+  int tr, tc;
+  p->fused_tiles = last_fused_tiles(p, &tr, &tc);
+  p->off_ais_z = take(p, (size_t)B * nz * 4);
+  p->off_ais_gr = take(p, (size_t)B * nz * 4);
+  p->off_ais_gp = take(p, (size_t)B * nz * 4);
+  p->off_ais_logw = take(p, (size_t)B * 8);
+  p->off_ais_scal = take(p, (size_t)7 * B * 4);
+  p->off_ais_epart = take(p, (size_t)B * p->fused_tiles * 4);
+  p->off_ais_logp = take(p, (size_t)B * 4);
+  p->off_ais_beta = take(p, (size_t)AIS_BETA_FLOATS * 4);
+}
+
+}  // namespace lsnf
+
+using namespace lsnf;
+
+extern "C" int lsnf_abi_version(void) { return LSNF_ABI_VERSION; }
+extern "C" const char* lsnf_last_error(void) { return g_err.c_str(); }
+
+extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
+  if (!cfg || !out) return fail(LSNF_ERR_INVALID, "null argument");
+  std::unique_ptr<lsnf_plan> p(new lsnf_plan());
+  p->cfg = *cfg;
+  if (int rc = check_config(p.get())) return rc;
+  take_regions(p.get());
+  const int L = p->n_layers;
   if (L > 0) {
-    p->off_zhl = take((size_t)B * 2 * p->kp * 2);
-    p->off_sk_slots = take((size_t)160 * 128 * 256 * 4);   // stream-K partial accumulators (<= 160 CTAs)
-    p->off_sk_flags = take((size_t)160 * 8 * 4);
-    p->off_x = take((size_t)B * c.nc * p->img * p->img * 4);
-    p->off_mask = take((size_t)B * c.nc * p->img * p->img * 4);   // the graph-replayed loop's copy of a mask
-    for (int l = 0; l < L - 1; ++l) {
-      const auto& y = p->layers[l];
-      const size_t bytes = (size_t)B * y.hout * y.hout * 2 * y.co * 2;
-      p->off_act[l] = take(bytes);
-      p->off_gpre[l] = take(bytes);
-      p->off_mbits[l] = take((size_t)B * y.hout * y.hout * y.co / 8);   // LeakyReLU sign bits of act[l]
-    }
-    for (int l = 0; l < L; ++l) p->off_bias[l] = take((size_t)p->layers[l].co * 4);
-    p->off_xhat = take((size_t)B * c.nc * p->img * p->img * 4);
-    p->off_wscale = take((size_t)L * 16);   // per layer: |w|max bits, scale 2^k, descale 2^-k
-    {
-      const auto& ylast = p->layers[L - 1];
-      const int kk = ylast.k * ylast.k * ylast.co;
-      p->off_dlast = take((size_t)B * ylast.hin * ylast.hin * (kk <= 32 ? 32 : 64) * 4);
-    }
-    const auto& yl = p->layers[L - 1];
-    p->off_im2col = take((size_t)B * yl.hin * yl.hin * 2 * BLOCK_K * 2);
-
     p->stages.resize(2 * L);
-    // ---- forward stages ----
-    for (int l = 0; l < L; ++l) {
-      const auto& y = p->layers[l];
-      StageHost& st = p->stages[l];
-      lsnf_stage_info& I = st.info;
-      memset(&I, 0, sizeof(I));
-      st.layer = l; st.kind = 0; st.k = y.k; st.s = y.s; st.p = y.p; st.ci = y.ci; st.co = y.co;
-      st.first = (l == 0); st.last = (l == L - 1);
-      I.kind = 0; I.layer = l;
-      I.a_planes = 1;
-      I.k_splits = 1;
-      if (st.first) {
-        if (!(y.s == 1 && y.p == 0)) { delete p; return fail(LSNF_ERR_INVALID, "first layer must be s1 p0"); }
-        if (st.last) { delete p; return fail(LSNF_ERR_INVALID, "single-layer generator not supported"); }
-        I.grid_h = I.grid_w = 1;
-        I.k_per_tap = p->kp;
-        I.n_valid = y.k * y.k * y.co; I.n_pad = I.n_valid; I.block_n = pick_block_n(y.co);
-        I.n_phases = 1; I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
-        I.out_mul = 1; I.out_channels = y.co; I.epilogue = EPI_ACT_HL;
-        st.a_off = p->off_zhl;
-      } else {
-        I.grid_h = I.grid_w = y.hin;
-        I.k_per_tap = y.ci;
-        I.out_channels = y.co;
-        if (st.last) {
-          // direct product D[pos][(tap, c)] = act[pos][:] . W[:, c, tap]; last_gather_tanh sums the taps that land
-          // on each output pixel (col2im without atomics), adds the bias and applies tanh
-          if (!((y.k == 4 && y.s == 2 && y.p == 1) || (y.k == 3 && y.s == 1 && y.p == 1))) {
-            delete p; return fail(LSNF_ERR_INVALID, "unsupported last-layer geometry");
-          }
-          I.n_valid = y.k * y.k * y.co; I.n_pad = I.n_valid <= 32 ? 32 : 64; I.block_n = I.n_pad;
-          I.epilogue = EPI_PARTIAL; I.out_channels = I.n_pad;
-          I.n_phases = 1; I.out_mul = 1; I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
-          p->dlast_pad = I.n_pad;
-        } else {
-          I.n_valid = I.n_pad = y.co; I.epilogue = EPI_ACT_HL;
-          I.block_n = pick_block_n_hidden(y.co, B * y.hin * y.hin, (y.k == 4 && y.s == 2) ? 4 : 1,
-                                          ((y.k == 4 && y.s == 2) ? 4 : y.k * y.k) * (y.ci / BLOCK_K));
-        }
-        if (st.last) {
-          // taps already set (single centre tap)
-        } else if (y.k == 4 && y.s == 2 && y.p == 1) {
-          I.n_phases = 4; I.out_mul = 2;
-          for (int ph = 0; ph < 4; ++ph) {
-            I.n_taps[ph] = up2_fwd_taps(ph >> 1, ph & 1, I.n_pad, I.taps[ph]);
-            I.out_off_y[ph] = ph >> 1; I.out_off_x[ph] = ph & 1;
-          }
-        } else if (y.k == 3 && y.s == 1 && y.p == 1) {
-          I.n_phases = 1; I.out_mul = 1; I.n_taps[0] = 9;
-          for (int ky = 0; ky < 3; ++ky)
-            for (int kx = 0; kx < 3; ++kx) I.taps[0][ky * 3 + kx] = {1 - ky, 1 - kx, 0, (ky * 3 + kx) * I.n_pad};
-        } else { delete p; return fail(LSNF_ERR_INVALID, "unsupported ConvTranspose2d geometry"); }
-        st.a_off = p->off_act[l - 1];
-      }
-      make_box(I.grid_h, I.grid_w, &I.box_b, &I.box_h, &I.box_w);
-      const int total_taps = (st.first || st.last) ? 1 : y.k * y.k;
-      const size_t b_rows = (st.first || st.last) ? (size_t)I.n_pad : (size_t)total_taps * I.n_pad;
-      I.operand_fp16 = 1; I.passes = 3;
-      I.a_h = I.grid_h; I.a_w = I.grid_w; I.tap_gen_k = 0; I.b_k = I.k_per_tap; I.b_rows = (int)b_rows;
-      st.b_bytes = b_rows * 2 * I.k_per_tap * 2;
-      st.b_off = take(st.b_bytes);
-      st.out_off = st.last ? p->off_dlast : p->off_act[l];
-      st.mbits_off = st.last ? 0 : p->off_mbits[l];
-      st.bias_off = p->off_bias[l];
-      I.a_offset = st.a_off; I.b_offset = st.b_off; I.out_offset = st.out_off;
-      int taps_sum = 0;
-      for (int ph = 0; ph < I.n_phases; ++ph) taps_sum += I.n_taps[ph];
-      I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)I.n_valid * I.k_per_tap * taps_sum;
-      if (st.first) I.flops = 2LL * B * (long long)I.n_valid * c.nz;
-      if (st.last) I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)y.k * y.k * y.co * y.ci;
-      fill_dev(p, st);
-      StageDev& d = st.dev;
-      d.bias_mod = y.co;
-      if (st.last) {
-        d.nc = c.nc; d.Ho = y.hout; d.Wo = y.hout;
-        d.bias = nullptr;
-      } else {
-        d.sW = 2 * y.co; d.sH = (int64_t)y.hout * d.sW; d.sB = (int64_t)y.hout * d.sH; d.sPos = d.sW; d.sP = 0;
-      }
-    }
-    // ---- data-gradient stages (executed from the last layer down to the first) ----
-    for (int l = L - 1; l >= 0; --l) {
-      const auto& y = p->layers[l];
-      StageHost& st = p->stages[L + (L - 1 - l)];
-      lsnf_stage_info& I = st.info;
-      memset(&I, 0, sizeof(I));
-      st.layer = l; st.kind = 1; st.k = y.k; st.s = y.s; st.p = y.p; st.ci = y.ci; st.co = y.co;
-      st.first = (l == 0); st.last = (l == L - 1);
-      I.kind = 1; I.layer = l; I.a_planes = 1; I.k_splits = 1;
-      I.n_phases = 1; I.out_mul = 1;
-      size_t b_rows;
-      if (st.last) {
-        if (y.k * y.k * y.co > BLOCK_K) { delete p; return fail(LSNF_ERR_INVALID, "k*k*nc must be <= 64"); }
-        I.grid_h = I.grid_w = y.hin;
-        I.k_per_tap = BLOCK_K;
-        I.n_valid = I.n_pad = y.ci; I.block_n = pick_block_n(y.ci);
-        I.n_taps[0] = 1; I.taps[0][0] = {0, 0, 0, 0};
-        st.a_off = p->off_im2col;
-        b_rows = I.n_pad;
-      } else if (st.first) {
-        I.grid_h = I.grid_w = 1;
-        I.k_per_tap = y.co;           // per output position of the first layer; taps run over the k*k positions
-        I.n_valid = c.nz; I.n_pad = p->nzp; I.block_n = 128;
-        I.n_taps[0] = 0;              // generated: tap t -> (dy, dx) = (t / k, t % k), B column offset t*co
-        st.a_off = p->off_gpre[0];
-        b_rows = I.n_pad;
-        const int kblocks = y.k * y.k * y.co / BLOCK_K;
-        const int mtiles = (B + BLOCK_M - 1) / BLOCK_M;
-        int want = std::max(1, (148 + mtiles - 1) / mtiles);   // about one wave of CTAs
-        int per = std::max(2, (kblocks + want - 1) / want);
-        I.k_splits = (kblocks + per - 1) / per;
-        per = (kblocks + I.k_splits - 1) / I.k_splits;       // what the kernels use (it_per_split)
-        I.k_splits = (kblocks + per - 1) / per;               // every split is non-empty
-        p->ksplit_first = I.k_splits;
-      } else {
-        if (!(y.k == 4 && y.s == 2 && y.p == 1)) { delete p; return fail(LSNF_ERR_INVALID, "unsupported hidden layer geometry"); }
-        I.grid_h = I.grid_w = y.hin;
-        I.k_per_tap = y.co;
-        I.n_valid = I.n_pad = y.ci; I.block_n = pick_block_n_hidden(y.ci, B * y.hin * y.hin, 1, 16 * (y.co / BLOCK_K));
-        I.a_planes = 4;
-        I.n_taps[0] = up2_bwd_taps(I.n_pad, I.taps[0]);
-        st.a_off = p->off_gpre[l];
-        b_rows = (size_t)16 * I.n_pad;
-      }
-      make_box(I.grid_h, I.grid_w, &I.box_b, &I.box_h, &I.box_w);
-      const size_t b_k = st.first ? (size_t)y.k * y.k * y.co : (size_t)I.k_per_tap;
-      I.operand_fp16 = c.bwd_passes == 1 ? 1 : 0; I.passes = c.bwd_passes == 1 ? 1 : 3;
-      I.a_h = st.first ? y.k : I.grid_h; I.a_w = st.first ? y.k : I.grid_w;
-      I.tap_gen_k = st.first ? y.k : 0; I.b_k = (int)b_k; I.b_rows = (int)b_rows;
-      st.b_bytes = b_rows * 2 * b_k * 2;
-      st.b_off = take(st.b_bytes);
-      if (st.first) {
-        I.epilogue = EPI_PARTIAL; I.out_channels = I.n_pad;
-      } else {
-        I.epilogue = EPI_GRAD_HL; I.out_channels = y.ci;
-        // the consumer (data gradient of layer l-1) reads phase-split when it is a stride-2 layer
-        I.out_phase_split = (l - 1 > 0) ? 1 : 0;
-        st.out_off = p->off_gpre[l - 1];
-        st.mbits_off = p->off_mbits[l - 1];
-      }
-      I.a_offset = st.a_off; I.b_offset = st.b_off; I.out_offset = st.out_off;
-      I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)I.n_valid *
-                (st.last ? y.k * y.k * y.co : (st.first ? (long long)y.k * y.k * y.co : 16LL * y.co));
-      fill_dev(p, st);
-      StageDev& d = st.dev;
-      if (!st.first) {
-        const int hg = I.grid_h;
-        d.sW = 2 * y.ci;
-        if (I.out_phase_split) {
-          d.sH = (int64_t)(hg / 2) * d.sW; d.sB = (int64_t)(hg / 2) * d.sH; d.sP = (int64_t)B * d.sB;
-        } else {
-          d.sH = (int64_t)hg * d.sW; d.sB = (int64_t)hg * d.sH; d.sP = 0;
-        }
-      }
-    }
+    for (int l = 0; l < L; ++l) build_forward_stage(p.get(), l);
+    for (int l = L - 1; l >= 0; --l) build_dgrad_stage(p.get(), l);
     // partial sums of the first layer's split-K data gradient
-    p->off_partial = take((size_t)p->ksplit_first * B * p->nzp * 4);
-    p->stages[2 * L - 1].out_off = p->off_partial;
+    p->off_partial = take(p.get(), (size_t)p->ksplit_first * p->cfg.batch * p->nzp * 4);
     p->stages[2 * L - 1].info.out_offset = p->off_partial;
-  }
-  // ---- generator parameter update (train.py:390-394): transposed operands + weight-gradient tap-GEMMs ----
-  if (L > 0 && c.train) {
-    p->wg.resize(L);
-    size_t goff = 0;
-    for (int l = 0; l < L; ++l) {
-      const auto& y = p->layers[l];
-      WgradLayer& w = p->wg[l];
-      const bool first = (l == 0), last = (l == L - 1);
-      const int kk = y.k * y.k;
-      const bool single = c.bwd_passes == 1;   // gradient tensors hold fp16 hi halves only
-      w.kk = kk;
-      int n_cols, hp, wp, halo, block_n;
-      TransArgs& ta = w.ta;
-      TransArgs& tg = w.tg;
-      memset(&ta, 0, sizeof(ta)); memset(&tg, 0, sizeof(tg));
-      if (first) {
-        // dW0[ci][(tap, co)] = sum_b z[b][ci] * gpre_0[b][tap][co]
-        w.a_rows = (int)align_up(c.nz, 128); hp = wp = 1; halo = 0;
-        w.Kp = (long long)align_up(B, BLOCK_K);
-        w.planes = 1; w.g_rows = kk * y.co; w.ntaps = 1; n_cols = kk * y.co; block_n = pick_block_n(n_cols);
-        ta.P = 1; ta.B = B; ta.H = ta.W = 1; ta.C = p->kp; ta.s_b = 2 * p->kp; ta.src_fp16 = 1; ta.c_rows = w.a_rows;
-        tg.P = kk; tg.B = B; tg.H = tg.W = 1; tg.C = y.co; tg.s_plane = 2 * y.co; tg.s_b = (long long)kk * 2 * y.co;
-        tg.c_rows = y.co;
-      } else if (last) {
-        // dW[ci][(tap, c)] = sum_pos act[pos][ci] * im2col_seed[pos][(tap, c)]   (the seed already holds the taps)
-        w.a_rows = y.ci; hp = wp = y.hin; halo = 0;
-        w.Kp = (long long)align_up((size_t)B * y.hin * y.hin, BLOCK_K);
-        w.planes = 1; w.g_rows = BLOCK_K; w.ntaps = 1; n_cols = BLOCK_K; block_n = 64;
-        ta.P = 1; ta.B = B; ta.H = ta.W = y.hin; ta.C = y.ci; ta.s_w = 2 * y.ci; ta.s_h = (long long)y.hin * ta.s_w;
-        ta.s_b = (long long)y.hin * ta.s_h; ta.src_fp16 = 1; ta.c_rows = y.ci;
-        tg.P = 1; tg.B = B; tg.H = tg.W = y.hin; tg.C = BLOCK_K; tg.s_w = 2 * BLOCK_K; tg.s_h = (long long)y.hin * tg.s_w;
-        tg.s_b = (long long)y.hin * tg.s_h; tg.c_rows = BLOCK_K;
-      } else {
-        // k4/s2/p1: per tap, dW[ci][co] = sum_pos act[pos][ci] * gpre[plane_tap][pos + (dy, dx)][co].  One zero halo
-        // row above and below every sample (dy becomes the K offset dy * Wp, a multiple of 8 elements = 16 bytes as
-        // TMA box origins must be); dx picks the as-is or the column-shifted copy of the phase plane (TransArgs::xvar)
-        w.a_rows = y.ci; hp = y.hin + 2; wp = (int)align_up(y.hin, 8); halo = 1;
-        w.Kp = (long long)align_up((size_t)B * hp * wp, BLOCK_K);
-        w.planes = 8; w.g_rows = y.co; w.ntaps = 16; n_cols = y.co; block_n = pick_block_n(y.co);
-        ta.P = 1; ta.B = B; ta.H = ta.W = y.hin; ta.C = y.ci; ta.s_w = 2 * y.ci; ta.s_h = (long long)y.hin * ta.s_w;
-        ta.s_b = (long long)y.hin * ta.s_h; ta.src_fp16 = 1; ta.c_rows = y.ci;
-        tg.P = 4; tg.B = B; tg.H = tg.W = y.hin; tg.C = y.co; tg.s_w = 2 * y.co; tg.s_h = (long long)y.hin * tg.s_w;
-        tg.s_b = (long long)y.hin * tg.s_h; tg.s_plane = (long long)B * tg.s_b; tg.c_rows = y.co; tg.xvar = 1;
-      }
-      ta.Hp = tg.Hp = hp; ta.Wp = tg.Wp = wp; ta.halo = tg.halo = halo; ta.Kp = tg.Kp = w.Kp;
-      tg.src_fp16 = single ? 1 : 0; tg.src_single = single ? 1 : 0;
-      w.off_aT = take((size_t)w.a_rows * 2 * w.Kp * 2);
-      w.off_gT = take((size_t)w.planes * w.g_rows * 2 * w.Kp * 2);
-      // the tap-GEMM: rows = C_in, columns = C_out (or (tap, co) / the 64 seed columns), K = flattened positions
-      StageHost& st = w.st;
-      lsnf_stage_info& I = st.info;
-      memset(&I, 0, sizeof(I));
-      st.layer = l; st.kind = 2; st.k = y.k; st.s = y.s; st.p = y.p; st.ci = y.ci; st.co = y.co;
-      st.first = first; st.last = last;
-      I.kind = 2; I.layer = l; I.grid_h = 1; I.grid_w = w.a_rows; I.box_b = 1; I.box_h = 1; I.box_w = BLOCK_M;
-      I.k_per_tap = (int)w.Kp; I.n_valid = n_cols; I.block_n = block_n; I.n_pad = (int)align_up(n_cols, block_n);
-      I.n_phases = 1; I.n_taps[0] = w.ntaps; I.out_mul = 1; I.out_channels = I.n_pad; I.epilogue = EPI_PARTIAL;
-      I.a_planes = 1; I.a_h = 1; I.a_w = w.a_rows; I.b_k = (int)w.Kp; I.b_rows = w.planes * w.g_rows;
-      I.operand_fp16 = 0; I.passes = 3;
-      const int kblocks = (int)(w.Kp / BLOCK_K);
-      const int tiles = ((w.a_rows + BLOCK_M - 1) / BLOCK_M) * (I.n_pad / block_n) * w.ntaps;
-      int want = std::max(1, (2 * 148 + tiles - 1) / tiles);
-      want = std::min(want, std::max(1, kblocks / 4));          // at least four K blocks per split
-      int per = (kblocks + want - 1) / want;
-      w.ksplit = (kblocks + per - 1) / per;
-      I.k_splits = w.ksplit;
-      for (int t = 0; t < w.ntaps; ++t) I.taps[0][t] = {0, 0, 0, 0};
-      I.flops = 2LL * w.a_rows * (long long)n_cols * w.Kp * w.ntaps;
-      st.a_off = w.off_aT; st.b_off = w.off_gT;
-      w.off_part = take((size_t)w.ntaps * w.ksplit * w.a_rows * I.n_pad * 4);
-      st.out_off = w.off_part;
-      I.a_offset = st.a_off; I.b_offset = st.b_off; I.out_offset = st.out_off;
-      fill_dev(p, st);
-      StageDev& d = st.dev;
-      d.B = 1; d.tiles_b = 1; d.tiles_h = 1; d.tiles_w = (w.a_rows + BLOCK_M - 1) / BLOCK_M;
-      d.rows_total = w.a_rows; d.wgrad = 1; d.it_per_split = per;
-      if (!first && !last) {
-        lsnf_tap tp[16];
-        up2_bwd_taps(y.co, tp);   // plane and (dy, dx) of every tap; brow = plane * C_out in the transposed gradient
-        for (int t = 0; t < 16; ++t) {
-          d.ph[0].taps[t].dy = 0; d.ph[0].taps[t].dx = 0; d.ph[0].taps[t].plane = 0;
-          d.ph[0].taps[t].bsh = (int16_t)(tp[t].dy * wp);
-          d.ph[0].taps[t].brow = (tp[t].plane * 2 + (tp[t].dx != 0 ? 1 : 0)) * y.co;
-        }
-      }
-      // results: dW in the parameter's own layout, then db
-      w.grad_w_off = goff; goff += align_up((size_t)y.ci * y.co * kk, 4);
-      w.grad_b_off = goff; goff += align_up((size_t)y.co, 4);
-      FinalizeArgs& f = w.fin;
-      memset(&f, 0, sizeof(f));
-      f.ksplit = w.ksplit; f.kk = kk; f.C_in = y.ci; f.C_out = y.co;
-      if (first) { f.s_tap = y.co; f.s_split = 0; f.s_ci = I.n_pad; f.ksplit = 1; }
-      else if (last) { f.s_tap = y.co; f.s_split = (long long)w.a_rows * I.n_pad; f.s_ci = I.n_pad; }
-      else { f.s_tap = (long long)w.ksplit * w.a_rows * I.n_pad; f.s_split = (long long)w.a_rows * I.n_pad; f.s_ci = I.n_pad; }
-      RowSumArgs& r = w.rs;
-      memset(&r, 0, sizeof(r));
-      r.Kp = w.Kp; r.C = y.co;
-      if (first) { r.nsel = kk; for (int t = 0; t < kk; ++t) r.sel[t] = t * y.co; }
-      else if (last) {
-        // every output pixel is produced by exactly one of these taps (oy = iy*s - p + ky covers each oy once)
-        r.nsel = 0;
-        for (int ky = 0; ky < y.k; ++ky)
-          for (int kx = 0; kx < y.k; ++kx) {
-            const bool once_y = y.s == 1 ? ky == y.p : (ky == 1 || ky == 2);
-            const bool once_x = y.s == 1 ? kx == y.p : (kx == 1 || kx == 2);
-            if (once_y && once_x) r.sel[r.nsel++] = (ky * y.k + kx) * y.co;
-          }
-      } else { r.nsel = 4; for (int q = 0; q < 4; ++q) r.sel[q] = 2 * q * y.co; }   // the as-is copy of every plane
-      if (first && w.ksplit != 1) { /* K = batch only: never split */ }
+    if (p->cfg.train) {
+      p->wg.resize(L);
+      for (int l = 0; l < L; ++l) build_wgrad_layer(p.get(), l);
     }
-    p->gen_grad_floats = goff;
+    take_ais_regions(p.get());
   }
-  if (L > 0) {   // annealed importance sampling (lsnf_ais_run): chain state and energies, after every other region
-    int tr, tc;
-    p->fused_tiles = last_fused_tiles(p, &tr, &tc);
-    p->off_ais_z = take((size_t)B * c.nz * 4);
-    p->off_ais_gr = take((size_t)B * c.nz * 4);
-    p->off_ais_gp = take((size_t)B * c.nz * 4);
-    p->off_ais_logw = take((size_t)B * 8);
-    p->off_ais_scal = take((size_t)7 * B * 4);
-    p->off_ais_epart = take((size_t)B * p->fused_tiles * 4);
-    p->off_ais_logp = take((size_t)B * 4);
-    p->off_ais_beta = take((size_t)AIS_BETA_FLOATS * 4);
-  }
-  p->ws_bytes = off;
-  *out = p;
+  *out = p.release();
   return LSNF_OK;
 }
 
@@ -593,16 +619,8 @@ extern "C" int lsnf_plan_stage_launch_info(const lsnf_plan* plan, int32_t index,
                                            lsnf_launch_info* out) {
   if (!plan || !out || index < 0 || index >= (int)plan->stages.size()) return fail(LSNF_ERR_INVALID, "bad stage index");
   if (num_sms < 2) return fail(LSNF_ERR_INVALID, "num_sms must be at least 2");
-  tc_launch_info(plan->stages[index], num_sms, out);
+  *out = tc_plan_launch(plan->stages[index], num_sms).info;
   return LSNF_OK;
-}
-
-static PackGeom geom_of(const StageHost& st) {
-  PackGeom g;
-  g.kind = st.kind; g.first = st.first; g.last = st.last; g.k = st.k; g.ci = st.ci; g.co = st.co;
-  g.n_pad = st.info.n_pad;
-  g.ka = st.info.b_k;
-  return g;
 }
 
 extern "C" int lsnf_plan_pack_index(const lsnf_plan* plan, int32_t index, int32_t ci, int32_t co, int32_t ky,
@@ -615,6 +633,20 @@ extern "C" int lsnf_plan_pack_index(const lsnf_plan* plan, int32_t index, int32_
   pack_index(geom_of(st), ci, co, ky, kx, &r, &c);
   *row = r; *col = c;
   return LSNF_OK;
+}
+
+// Operand and output pointers of a stage in the bound workspace, and its launch on the plan's device; with
+// `encode`, its tensor maps.
+static int bind_stage(lsnf_plan* plan, StageHost& st, bool encode) {
+  StageDev& d = st.dev;
+  d.a = (const __nv_bfloat16*)(plan->ws + st.info.a_offset);
+  d.b = (const __nv_bfloat16*)(plan->ws + st.info.b_offset);
+  d.out = plan->ws + st.info.out_offset;
+  st.launch = tc_plan_launch(st, plan->num_sms);
+  d.nst = st.launch.info.ring_stages;
+  d.sk_enable = st.launch.info.stream_k;
+  d.out_tma = st.launch.info.tma_store;
+  return encode ? tc_encode_maps(plan, st) : LSNF_OK;
 }
 
 extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
@@ -634,31 +666,18 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
     if ((rc = tc_prepare_device(dev)) || (rc = aux_prepare_device(dev)) || (rc = flow_prepare_device(dev))) return rc;
   }
   for (auto& st : plan->stages) {
+    const lsnf_stage_info& I = st.info;
     StageDev& d = st.dev;
-    st.num_sms = plan->num_sms;
-    d.a = (const __nv_bfloat16*)(plan->ws + st.a_off);
-    d.b = (const __nv_bfloat16*)(plan->ws + st.b_off);
-    d.out = plan->ws + st.out_off;
-    d.bias = (st.kind == 0 && !st.last) ? (const float*)(plan->ws + st.bias_off) : nullptr;
+    d.bias = (I.kind == 0 && !st.last) ? (const float*)(plan->ws + st.bias_off) : nullptr;
     d.sk_slots = (float*)(plan->ws + plan->off_sk_slots);
     d.sk_flags = (int32_t*)(plan->ws + plan->off_sk_flags);
-    d.descale = (st.kind == 0 || plan->cfg.bwd_passes == 1) ? (const float*)(plan->ws + plan->off_wscale + (size_t)st.layer * 16 + 8) : nullptr;
-    d.mbits = ((st.kind == 0 && !st.last) || (st.kind == 1 && !st.first)) ? (uint32_t*)(plan->ws + st.mbits_off) : nullptr;
-    if (plan->cfg.gemm_impl == LSNF_GEMM_TCGEN05) {
-      int rc = tc_encode_maps(plan, st);
-      if (rc) return rc;
-    }
+    d.descale = (I.kind == 0 || plan->cfg.bwd_passes == 1) ? (const float*)(plan->ws + plan->off_wscale + (size_t)I.layer * 16 + 8) : nullptr;
+    d.mbits = ((I.kind == 0 && !st.last) || (I.kind == 1 && !st.first)) ? (uint32_t*)(plan->ws + st.mbits_off) : nullptr;
+    int rc = bind_stage(plan, st, plan->cfg.gemm_impl == LSNF_GEMM_TCGEN05);
+    if (rc) return rc;
   }
   for (auto& w : plan->wg) {
-    StageHost& st = w.st;
-    StageDev& d = st.dev;
-    st.num_sms = plan->num_sms;
-    d.a = (const __nv_bfloat16*)(plan->ws + st.a_off);
-    d.b = (const __nv_bfloat16*)(plan->ws + st.b_off);
-    d.out = plan->ws + st.out_off;
-    d.bias = nullptr; d.descale = nullptr; d.mbits = nullptr;
-    d.sk_slots = nullptr; d.sk_flags = nullptr;
-    int rc = tc_encode_maps(plan, st);
+    int rc = bind_stage(plan, w.st, true);
     if (rc) return rc;
     w.ta.dst = (uint16_t*)(plan->ws + w.off_aT);
     w.tg.dst = (uint16_t*)(plan->ws + w.off_gT);
@@ -706,7 +725,7 @@ extern "C" int lsnf_pack_generator_weights(lsnf_plan* plan, const float* const* 
     if (rc) return rc;
   }
   for (auto& st : plan->stages) {
-    int rc = launch_pack_stage(plan, st, weights[st.layer], s);
+    int rc = launch_pack_stage(plan, st, weights[st.info.layer], s);
     if (rc) return rc;
   }
   for (int l = 0; l < plan->n_layers; ++l)
@@ -1097,7 +1116,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
         PdlScope pdl(use_pdl);
         if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
       }
-      tr.mark(("dgrad layer " + std::to_string(plan->stages[i].layer)).c_str());
+      tr.mark(("dgrad layer " + std::to_string(plan->stages[i].info.layer)).c_str());
     }
     LSNF_CUDA(cudaStreamWaitEvent(s, plan->ev_join, 0));
     tr.mark("join flow prior");

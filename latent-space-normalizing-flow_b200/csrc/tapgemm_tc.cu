@@ -12,8 +12,9 @@
 // * Warp roles: warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..9 = epilogue
 //   (tcgen05.ld -> bias / LeakyReLU / LeakyReLU' from bit-packed signs -> 16-bit hi|lo through TMA tensor stores,
 //   or fp32 rows).  Two kernels: tapgemm_tc_kernel<BN> (one CTA per tile, ring sized per launch) and
-//   tapgemm_tc2_kernel<DEEP> (persistent cta_group::2 pairs for the 256-wide stages); the host picks per stage
-//   (use_pair, ring_geometry, out_tma_kind, pair_stream_k -- mirrored by lsnf_plan_stage_launch_info).
+//   tapgemm_tc2_kernel<DEEP> (persistent cta_group::2 pairs for the 256-wide stages).  tc_plan_launch picks the
+//   kernel, grid, ring and epilogue of each stage; lsnf_plan_bind stores that record and launch_tapgemm_tc launches
+//   from it, and lsnf_plan_stage_launch_info reports it.
 #include <algorithm>
 #include <mutex>
 #include <type_traits>
@@ -966,8 +967,7 @@ static EncodeTiledFn get_encode() {
 // prologue and epilogue: they run on the 1-CTA kernel with shallow rings and several CTAs per SM instead (measured in
 // round 2: the last layer's data gradient at CIFAR-10, one K block per tile, takes 64 us on the pair kernel against
 // 44 us here).
-static bool use_pair(const StageHost& sh) {
-  const StageDev& d = sh.dev;
+static bool use_pair(const StageDev& d) {
   const int mtiles = d.tiles_b * d.tiles_h * d.tiles_w;
   const int total = d.ph[0].ntaps * (d.Ka / BLOCK_K);
   return !d.wgrad && d.block_n == 256 && d.n_pad % 256 == 0 && d.ksplit == 1 && total >= 3 &&
@@ -976,7 +976,7 @@ static bool use_pair(const StageHost& sh) {
 
 // Ring of the 1-CTA kernel for one launch: stage bytes, depth, dynamic shared memory to request.
 struct RingGeom { int nst; size_t stage_bytes, smem; };
-static RingGeom ring_geometry(const StageDev& d) {
+static RingGeom ring_geometry(const StageDev& d, int out_tma) {
   const bool three = d.passes != 1;
   const size_t stage = (size_t)(three ? 2 : 1) * (A_TILE_BYTES + (size_t)d.block_n * BLOCK_K * 2);
   const int total = d.ph[0].ntaps * (d.Ka / BLOCK_K);
@@ -987,7 +987,7 @@ static RingGeom ring_geometry(const StageDev& d) {
   const size_t budget = (iters <= 4 ? TC_SMEM_MAX / 2 : TC_SMEM_MAX) - TC_SMEM_EXTRA;
   int nst = (int)std::min<size_t>(budget / stage, (size_t)std::min(iters, TC_MAX_STAGES));
   nst = std::max(nst, 1);
-  while (d.out_tma && nst * stage < 32768) ++nst;   // the tensor-store epilogue stages 32 KiB in the idle ring
+  while (out_tma && nst * stage < 32768) ++nst;   // the tensor-store epilogue stages 32 KiB in the idle ring
   size_t smem = nst * stage + TC_SMEM_EXTRA;
   // never more resident CTAs than tensor memory can hold (the allocation of one more would spin)
   const int tmem_cols = d.block_n < 32 ? 32 : d.block_n;
@@ -998,112 +998,15 @@ static RingGeom ring_geometry(const StageDev& d) {
 
 // Which tensor-store map the 16-bit output of a stage gets: 1 stride-2 forward [B][2H][2W][2C], 2 first layer
 // [B][k*k][2C], 3 plain gradient [B][H][W][2C], 4 phase-split gradient; 0 = per-thread stores.
-static int out_tma_kind(const StageHost& sh) {
+static int out_tma_kind(const StageHost& sh, bool pair) {
   const StageDev& d = sh.dev;
   const bool wide_single = d.block_n >= 128 && d.n_pad % d.block_n == 0 && d.ksplit == 1;   // 1-CTA kernel, wide N tile
-  if (!(use_pair(sh) || wide_single) || !(d.epi == EPI_ACT_HL || d.epi == EPI_GRAD_HL)) return 0;
+  if (!(pair || wide_single) || !(d.epi == EPI_ACT_HL || d.epi == EPI_GRAD_HL)) return 0;
   if (d.epi == EPI_ACT_HL && sh.first) return 2;
   if (d.epi == EPI_ACT_HL && d.ms == 2) return 1;
   if (d.epi == EPI_GRAD_HL && !d.split) return 3;
   if (d.epi == EPI_GRAD_HL && d.split && d.bW >= 2 && d.bH >= 2 && (d.bH % 2) == 0) return 4;
   return 0;
-}
-
-int tc_encode_maps(lsnf_plan* plan, StageHost& sh) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point not available"); return LSNF_ERR_CUDA; }
-  const StageDev& d = sh.dev;
-  {
-    const cuuint64_t row = (cuuint64_t)2 * d.Ka * 2;  // bytes per position (hi|lo)
-    cuuint64_t dims[5] = {(cuuint64_t)2 * d.Ka, (cuuint64_t)d.aW, (cuuint64_t)d.aH, (cuuint64_t)d.B, (cuuint64_t)d.aP};
-    cuuint64_t strides[4] = {row, row * d.aW, row * d.aW * d.aH, row * d.aW * d.aH * d.B};
-    cuuint32_t box[5] = {BLOCK_K, (cuuint32_t)d.bW, (cuuint32_t)d.bH, (cuuint32_t)d.bB, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    CUresult r = enc(&sh.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)d.a, dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled(A) failed with code " + std::to_string((int)r) + " for stage layer " +
-                std::to_string(sh.layer) + " kind " + std::to_string(sh.kind));
-      return LSNF_ERR_CUDA;
-    }
-  }
-  {
-    cuuint64_t dims[2] = {(cuuint64_t)2 * d.b_k, (cuuint64_t)d.b_rows};
-    cuuint64_t strides[1] = {(cuuint64_t)2 * d.b_k * 2};
-    const bool pair = use_pair(sh);
-    cuuint32_t box[2] = {BLOCK_K, (cuuint32_t)(pair ? d.block_n / 2 : d.block_n)};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = enc(&sh.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)d.b, dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled(B) failed with code " + std::to_string((int)r) + " for stage layer " +
-                std::to_string(sh.layer) + " kind " + std::to_string(sh.kind));
-      return LSNF_ERR_CUDA;
-    }
-  }
-  // output map of the 16-bit epilogues (tensor stores)
-  sh.dev.out_tma = 0;
-  const int want_kind = out_tma_kind(sh);
-  if (want_kind) {
-    const cuuint64_t C2 = (cuuint64_t)2 * d.oC, eb = 2;   // channels per position (hi|lo), bytes per element
-    cuuint64_t dims[5], strides[4];
-    cuuint32_t box[5], es[5] = {1, 1, 1, 1, 1};
-    int kind = 0;
-    if (want_kind == 2) {                                  // [B][k*k][2C]
-      const cuuint64_t kk = (cuuint64_t)sh.k * sh.k;
-      dims[0] = C2; dims[1] = kk; dims[2] = 1; dims[3] = 1; dims[4] = d.B;
-      strides[0] = C2 * eb; strides[1] = C2 * kk * eb; strides[2] = C2 * kk * eb; strides[3] = C2 * kk * eb;
-      box[0] = 64; box[1] = 1; box[2] = 1; box[3] = 1; box[4] = 128;
-      kind = 2;
-    } else if (want_kind == 1) {                           // [B][2H][2W][2C] as (c, px, w, py, b*H + h)
-      const cuuint64_t W = d.Wg, H = d.Hg;
-      dims[0] = C2; dims[1] = 2; dims[2] = W; dims[3] = 2; dims[4] = (cuuint64_t)d.B * H;
-      strides[0] = C2 * eb; strides[1] = 2 * C2 * eb; strides[2] = 2 * W * C2 * eb; strides[3] = 4 * W * C2 * eb;
-      box[0] = 64; box[1] = 1; box[2] = d.bW; box[3] = 1; box[4] = d.bB * d.bH;
-      kind = 1;
-    } else if (want_kind == 3) {                           // [B][H][W][2C]
-      const cuuint64_t W = d.Wg, H = d.Hg;
-      dims[0] = C2; dims[1] = W; dims[2] = H; dims[3] = d.B; dims[4] = 1;
-      strides[0] = C2 * eb; strides[1] = W * C2 * eb; strides[2] = H * W * C2 * eb; strides[3] = (cuuint64_t)d.B * H * W * C2 * eb;
-      box[0] = 64; box[1] = d.bW; box[2] = d.bH; box[3] = d.bB; box[4] = 1;
-      kind = 3;
-    } else if (want_kind == 4) {
-      // [4 = (py,px)][B][H/2][W/2][2C] as (c, w/2, b*(H/2) + h/2, px, py): strides increase monotonically; the
-      // epilogue permutes its staging rows accordingly
-      const cuuint64_t Wh = d.Wg / 2, Hh = d.Hg / 2;
-      const cuuint64_t plane = (cuuint64_t)d.B * Hh * Wh * C2;
-      dims[0] = C2; dims[1] = Wh; dims[2] = (cuuint64_t)d.B * Hh; dims[3] = 2; dims[4] = 2;
-      strides[0] = C2 * eb; strides[1] = Wh * C2 * eb; strides[2] = plane * eb; strides[3] = 2 * plane * eb;
-      box[0] = 64; box[1] = d.bW / 2; box[2] = d.bB * d.bH / 2; box[3] = 2; box[4] = 2;
-      kind = 4;
-    }
-    if (kind) {
-      CUresult r = enc(&sh.tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.out, dims, strides, box, es,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled(out) failed with code " + std::to_string((int)r) + " for stage layer " +
-                  std::to_string(sh.layer) + " kind " + std::to_string(sh.kind));
-        return LSNF_ERR_CUDA;
-      }
-      sh.dev.out_tma = kind;
-    }
-  }
-  if (!sh.dev.out_tma) sh.tmO = sh.tmA;   // placeholder, never dereferenced
-  sh.maps_ready = true;
-  return LSNF_OK;
-}
-
-template <int BN>
-static int launch_bn(const StageHost& sh, cudaStream_t s) {
-  StageDev st = sh.dev;
-  const RingGeom g = ring_geometry(st);
-  st.nst = g.nst;
-  dim3 grid(st.tiles_b * st.tiles_h * st.tiles_w, st.n_pad / BN, (st.wgrad ? st.ph[0].ntaps : st.nphase) * st.ksplit);
-  LSNF_CUDA(launch_k(tapgemm_tc_kernel<BN>, grid, dim3(TC_THREADS), g.smem, s, sh.tmA, sh.tmB, sh.tmO, st));
-  return LSNF_OK;
 }
 
 // Stream-K (equal shares of tiles x K blocks per pair, partial accumulators exchanged through L2) pays only when
@@ -1120,54 +1023,121 @@ static bool pair_stream_k(const StageDev& st, int max_pairs) {
          (long long)num_tiles * total >= 4LL * max_pairs && max_pairs <= 80;
 }
 
-static int launch_pair(const StageHost& sh, cudaStream_t s) {
-  const StageDev& st = sh.dev;
-  const int mtiles = st.tiles_b * st.tiles_h * st.tiles_w;
-  const int num_tiles = (mtiles + 1) / 2 * (st.n_pad / P_BN) * st.nphase;   // an odd tail pairs with an empty tile
-  const int max_pairs = sh.num_sms / 2;   // of the plan's device (lsnf_plan_bind)
-  StageDev launch_st = st;
-  launch_st.sk_enable = pair_stream_k(st, max_pairs);
-  const int pairs = launch_st.sk_enable ? max_pairs : std::min(num_tiles, max_pairs);
-  dim3 grid(2 * pairs, 1, 1);
-  if (st.passes == 1)
-    LSNF_CUDA(launch_k(tapgemm_tc2_kernel<true>, grid, dim3(TC_THREADS), P_SMEM_BYTES, s, sh.tmA, sh.tmB, sh.tmO, launch_st));
-  else
-    LSNF_CUDA(launch_k(tapgemm_tc2_kernel<false>, grid, dim3(TC_THREADS), P_SMEM_BYTES, s, sh.tmA, sh.tmB, sh.tmO, launch_st));
-  return LSNF_OK;
-}
-
-// What launch_tapgemm_tc would do for this stage on a device with `num_sms` SMs (no device needed).
-void tc_launch_info(const StageHost& sh_in, int num_sms, lsnf_launch_info* out) {
-  StageHost sh = sh_in;
-  sh.dev.out_tma = out_tma_kind(sh);
+TcLaunch tc_plan_launch(const StageHost& sh, int num_sms) {
   const StageDev& d = sh.dev;
+  const bool pair = use_pair(d);
   const int mtiles = d.tiles_b * d.tiles_h * d.tiles_w;
-  memset(out, 0, sizeof(*out));
-  out->block = TC_THREADS;
-  out->tma_store = d.out_tma;
-  out->tmem_columns = use_pair(sh) ? 512 : (d.block_n < 32 ? 32 : d.block_n);
-  if (use_pair(sh)) {
+  TcLaunch l;
+  lsnf_launch_info& o = l.info;
+  memset(&o, 0, sizeof(o));
+  o.block = TC_THREADS;
+  o.tma_store = out_tma_kind(sh, pair);   // before the ring: the tensor-store epilogue stages in it
+  if (pair) {
     const int max_pairs = num_sms / 2;
-    const int num_tiles = (mtiles + 1) / 2 * (d.n_pad / P_BN) * d.nphase;
-    out->kernel = LSNF_KERNEL_PAIR;
-    out->stream_k = pair_stream_k(d, max_pairs) ? 1 : 0;
-    out->grid_x = 2 * (out->stream_k ? max_pairs : std::min(num_tiles, max_pairs));
-    out->grid_y = out->grid_z = 1;
-    out->ring_stages = d.passes == 1 ? P_MAX_STAGES : P_STAGES;
-    out->stage_bytes = d.passes == 1 ? P_STAGE_BYTES / 2 : P_STAGE_BYTES;
-    out->smem_bytes = P_SMEM_BYTES;
-    out->ctas_per_sm = 1;
+    const int num_tiles = (mtiles + 1) / 2 * (d.n_pad / P_BN) * d.nphase;   // an odd tail pairs with an empty tile
+    l.kernel = d.passes == 1 ? &tapgemm_tc2_kernel<true> : &tapgemm_tc2_kernel<false>;
+    o.kernel = LSNF_KERNEL_PAIR;
+    o.stream_k = pair_stream_k(d, max_pairs) ? 1 : 0;
+    o.grid_x = 2 * (o.stream_k ? max_pairs : std::min(num_tiles, max_pairs));
+    o.grid_y = o.grid_z = 1;
+    o.ring_stages = d.passes == 1 ? P_MAX_STAGES : P_STAGES;
+    o.stage_bytes = d.passes == 1 ? P_STAGE_BYTES / 2 : P_STAGE_BYTES;
+    o.smem_bytes = P_SMEM_BYTES;
+    o.ctas_per_sm = 1;
+    o.tmem_columns = 512;
   } else {
-    const RingGeom g = ring_geometry(d);
-    out->kernel = LSNF_KERNEL_SINGLE;
-    out->grid_x = mtiles; out->grid_y = d.n_pad / d.block_n; out->grid_z = d.nphase * d.ksplit;
-    out->ring_stages = g.nst;
-    out->stage_bytes = (int32_t)g.stage_bytes;
-    out->smem_bytes = (int32_t)g.smem;
+    switch (d.block_n) {
+      case 256: l.kernel = &tapgemm_tc_kernel<256>; break;
+      case 128: l.kernel = &tapgemm_tc_kernel<128>; break;
+      case 64: l.kernel = &tapgemm_tc_kernel<64>; break;
+      case 32: l.kernel = &tapgemm_tc_kernel<32>; break;
+      case 16: l.kernel = &tapgemm_tc_kernel<16>; break;
+    }
+    const RingGeom g = ring_geometry(d, o.tma_store);
+    o.kernel = LSNF_KERNEL_SINGLE;
+    // every blockIdx.z slice of a weight-gradient stage is one tap (x split)
+    o.grid_x = mtiles; o.grid_y = d.n_pad / d.block_n; o.grid_z = (d.wgrad ? d.ph[0].ntaps : d.nphase) * d.ksplit;
+    o.ring_stages = g.nst;
+    o.stage_bytes = (int32_t)g.stage_bytes;
+    o.smem_bytes = (int32_t)g.smem;
     // shared memory (1 KiB per CTA is reserved by the system), the 2048-thread and 64 Ki-register limits
     const int by_smem = (TC_SMEM_MAX + 1024) / ((int)g.smem + 1024);
-    out->ctas_per_sm = std::max(1, std::min(by_smem, 2048 / TC_THREADS));
+    o.ctas_per_sm = std::max(1, std::min(by_smem, 2048 / TC_THREADS));
+    o.tmem_columns = d.block_n < 32 ? 32 : d.block_n;
   }
+  return l;
+}
+
+int tc_encode_maps(lsnf_plan* plan, StageHost& sh) {
+  EncodeTiledFn enc = get_encode();
+  if (!enc) { set_error("cuTensorMapEncodeTiled entry point not available"); return LSNF_ERR_CUDA; }
+  const StageDev& d = sh.dev;
+  const lsnf_launch_info& li = sh.launch.info;
+  auto failed = [&](const char* map, CUresult r) {
+    set_error(std::string("cuTensorMapEncodeTiled(") + map + ") failed with code " + std::to_string((int)r) +
+              " for stage layer " + std::to_string(sh.info.layer) + " kind " + std::to_string(sh.info.kind));
+    return LSNF_ERR_CUDA;
+  };
+  {
+    const cuuint64_t row = (cuuint64_t)2 * d.Ka * 2;  // bytes per position (hi|lo)
+    cuuint64_t dims[5] = {(cuuint64_t)2 * d.Ka, (cuuint64_t)d.aW, (cuuint64_t)d.aH, (cuuint64_t)d.B, (cuuint64_t)d.aP};
+    cuuint64_t strides[4] = {row, row * d.aW, row * d.aW * d.aH, row * d.aW * d.aH * d.B};
+    cuuint32_t box[5] = {BLOCK_K, (cuuint32_t)d.bW, (cuuint32_t)d.bH, (cuuint32_t)d.bB, 1};
+    cuuint32_t es[5] = {1, 1, 1, 1, 1};
+    CUresult r = enc(&sh.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)d.a, dims, strides, box, es,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return failed("A", r);
+  }
+  {
+    cuuint64_t dims[2] = {(cuuint64_t)2 * d.b_k, (cuuint64_t)d.b_rows};
+    cuuint64_t strides[1] = {(cuuint64_t)2 * d.b_k * 2};
+    const bool pair = li.kernel == LSNF_KERNEL_PAIR;   // each CTA of a pair loads half the N tile
+    cuuint32_t box[2] = {BLOCK_K, (cuuint32_t)(pair ? d.block_n / 2 : d.block_n)};
+    cuuint32_t es[2] = {1, 1};
+    CUresult r = enc(&sh.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)d.b, dims, strides, box, es,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return failed("B", r);
+  }
+  // output map of the 16-bit epilogues (tensor stores)
+  if (li.tma_store) {
+    const cuuint64_t C2 = (cuuint64_t)2 * d.oC, eb = 2;   // channels per position (hi|lo), bytes per element
+    cuuint64_t dims[5], strides[4];
+    cuuint32_t box[5], es[5] = {1, 1, 1, 1, 1};
+    if (li.tma_store == 2) {                               // [B][k*k][2C]
+      const cuuint64_t kk = (cuuint64_t)sh.k * sh.k;
+      dims[0] = C2; dims[1] = kk; dims[2] = 1; dims[3] = 1; dims[4] = d.B;
+      strides[0] = C2 * eb; strides[1] = C2 * kk * eb; strides[2] = C2 * kk * eb; strides[3] = C2 * kk * eb;
+      box[0] = 64; box[1] = 1; box[2] = 1; box[3] = 1; box[4] = 128;
+    } else if (li.tma_store == 1) {                        // [B][2H][2W][2C] as (c, px, w, py, b*H + h)
+      const cuuint64_t W = d.Wg, H = d.Hg;
+      dims[0] = C2; dims[1] = 2; dims[2] = W; dims[3] = 2; dims[4] = (cuuint64_t)d.B * H;
+      strides[0] = C2 * eb; strides[1] = 2 * C2 * eb; strides[2] = 2 * W * C2 * eb; strides[3] = 4 * W * C2 * eb;
+      box[0] = 64; box[1] = 1; box[2] = d.bW; box[3] = 1; box[4] = d.bB * d.bH;
+    } else if (li.tma_store == 3) {                        // [B][H][W][2C]
+      const cuuint64_t W = d.Wg, H = d.Hg;
+      dims[0] = C2; dims[1] = W; dims[2] = H; dims[3] = d.B; dims[4] = 1;
+      strides[0] = C2 * eb; strides[1] = W * C2 * eb; strides[2] = H * W * C2 * eb; strides[3] = (cuuint64_t)d.B * H * W * C2 * eb;
+      box[0] = 64; box[1] = d.bW; box[2] = d.bH; box[3] = d.bB; box[4] = 1;
+    } else {
+      // 4: [4 = (py,px)][B][H/2][W/2][2C] as (c, w/2, b*(H/2) + h/2, px, py): strides increase monotonically; the
+      // epilogue permutes its staging rows accordingly
+      const cuuint64_t Wh = d.Wg / 2, Hh = d.Hg / 2;
+      const cuuint64_t plane = (cuuint64_t)d.B * Hh * Wh * C2;
+      dims[0] = C2; dims[1] = Wh; dims[2] = (cuuint64_t)d.B * Hh; dims[3] = 2; dims[4] = 2;
+      strides[0] = C2 * eb; strides[1] = Wh * C2 * eb; strides[2] = plane * eb; strides[3] = 2 * plane * eb;
+      box[0] = 64; box[1] = d.bW / 2; box[2] = d.bB * d.bH / 2; box[3] = 2; box[4] = 2;
+    }
+    CUresult r = enc(&sh.tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.out, dims, strides, box, es,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) return failed("out", r);
+  } else {
+    sh.tmO = sh.tmA;   // placeholder, never dereferenced
+  }
+  sh.maps_ready = true;
+  return LSNF_OK;
 }
 
 // opt-in shared-memory limit of every instantiation, once per device (lsnf_plan_bind); function attributes are per
@@ -1191,15 +1161,11 @@ int tc_prepare_device(int device) {
 
 int launch_tapgemm_tc(const StageHost& sh, cudaStream_t s) {
   if (!sh.maps_ready) { set_error("tensor maps not encoded"); return LSNF_ERR_STATE; }
-  if (use_pair(sh)) return launch_pair(sh, s);
-  switch (sh.dev.block_n) {
-    case 256: return launch_bn<256>(sh, s);
-    case 128: return launch_bn<128>(sh, s);
-    case 64: return launch_bn<64>(sh, s);
-    case 32: return launch_bn<32>(sh, s);
-    case 16: return launch_bn<16>(sh, s);
-    default: set_error("unsupported N tile"); return LSNF_ERR_INVALID;
-  }
+  const TcLaunch& l = sh.launch;
+  if (!l.kernel) { set_error("unsupported N tile"); return LSNF_ERR_INVALID; }
+  LSNF_CUDA(launch_k(l.kernel, dim3(l.info.grid_x, l.info.grid_y, l.info.grid_z), dim3(l.info.block),
+                     l.info.smem_bytes, s, sh.tmA, sh.tmB, sh.tmO, sh.dev));
+  return LSNF_OK;
 }
 
 }  // namespace lsnf
