@@ -265,7 +265,9 @@ int lsnf_adam_step(int32_t n_tensors, float* const* params, const float* const* 
                    const float* grad_scale, lsnf_stream stream);
 
 /* Launches generator stage `index` alone (0..L-1 forward, L..2L-1 data gradient) on the buffers currently in the
- * workspace.  Profiling / test hook: bench.py times the dominant tap-GEMM with CUDA events through it. */
+ * workspace.  Profiling / test hook: bench.py times the dominant tap-GEMM with CUDA events through it.  A stage whose
+ * launch record has cross_fp8 set reads the e4m3 operand the last data-gradient call converted (the conversion is
+ * not part of the stage), and no stage run this way changes the scales a later call uses. */
 int lsnf_plan_run_stage(lsnf_plan* plan, int32_t index, lsnf_stream stream);
 /* how many kernels one lsnf_langevin_run of `steps` iterations launches (for bench.py's gpu_launches). */
 int lsnf_langevin_launch_count(const lsnf_plan* plan, int32_t steps);
@@ -333,7 +335,8 @@ typedef struct lsnf_launch_info {
   int32_t tmem_columns;           /* TMEM columns one CTA allocates */
   int32_t tma_store;              /* 0 per-thread stores, 1..4 tensor-store map kind of the 16-bit output */
   int32_t stream_k;               /* 1 if the K range of tiles is split across CTA pairs */
-  int32_t reserved[4];
+  int32_t cross_fp8;              /* 1 if the cross terms run as one e4m3 stream (fp16 hi*hi + kind::f8f6f4) */
+  int32_t reserved[3];
 } lsnf_launch_info;
 int lsnf_plan_stage_launch_info(const lsnf_plan* plan, int32_t index, int32_t num_sms, lsnf_launch_info* out);
 

@@ -46,7 +46,8 @@ class LaunchInfo(C.Structure):
     _fields_ = [("kernel", C.c_int32), ("grid_x", C.c_int32), ("grid_y", C.c_int32), ("grid_z", C.c_int32),
                 ("block", C.c_int32), ("ring_stages", C.c_int32), ("stage_bytes", C.c_int32),
                 ("smem_bytes", C.c_int32), ("ctas_per_sm", C.c_int32), ("tmem_columns", C.c_int32),
-                ("tma_store", C.c_int32), ("stream_k", C.c_int32), ("reserved", C.c_int32 * 4)]
+                ("tma_store", C.c_int32), ("stream_k", C.c_int32), ("cross_fp8", C.c_int32),
+                ("reserved", C.c_int32 * 3)]
 
 
 KERNEL_SINGLE, KERNEL_PAIR = 0, 1

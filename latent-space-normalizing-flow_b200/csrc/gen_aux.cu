@@ -1,5 +1,7 @@
 // Small HBM-bound kernels around the generator tap-GEMMs: weight packing, latent splitting, the
 // reconstruction-gradient seed (with its im2col), split-K reduction and the fused Langevin update.
+#include <cuda_fp8.h>
+
 #include <mutex>
 
 #include "lsnf_internal.cuh"
@@ -15,9 +17,18 @@ __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bflo
 // weight packing: ConvTranspose2d weight [ci][co][k][k] fp32 -> K-major bf16 hi|lo operand of one stage
 // (model.py:57-149 weights; layouts documented at pack_index in lsnf_internal.cuh)
 // ---------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint8_t e4m3(float v) {   // round to nearest, out of range -> +-448
+  return (uint8_t)__nv_cvt_float_to_fp8(v, __NV_SATFINITE, __NV_E4M3);
+}
+
+// cross8 stages (tc_cross_fp8) split w 2^kw (kw: the e4m3 scale of the layer's max |w|, `wmax`) into fp16 halves
+// w_hi + w_lo and take, per 64-column K block of a row, w_hi 2^6 in the hi half's columns and the 128 bytes
+// [w_lo8 x 64 | w_hi8 x 64] in the lo half's, w_hi8 = e4m3(w_hi), w_lo8 = e4m3(w_lo 2^11).
 __global__ void pack_stage_kernel(const float* __restrict__ w, uint16_t* __restrict__ out, PackGeom g, int rows,
-                                  int nz_valid, int fp16, const float* __restrict__ scale) {
+                                  int nz_valid, int fp16, const float* __restrict__ scale,
+                                  const unsigned int* __restrict__ wmax) {
   const float sc = scale ? *scale : 1.f;
+  const int kw = wmax ? fp8_scale_exp(__uint_as_float(*wmax)) : 0;
   const long long total = (long long)rows * g.ka;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -36,6 +47,15 @@ __global__ void pack_stage_kernel(const float* __restrict__ w, uint16_t* __restr
     if (ci < g.ci && co < g.co && tap < g.k * g.k && ci < nz_valid)
       v = w[((long long)ci * g.co + co) * g.k * g.k + tap] * sc;
     uint16_t hi, lo;
+    if (wmax) {
+      split16(ldexpf(v, kw), true, hi, lo);
+      const float h = __half2float(__ushort_as_half(hi)), l = __half2float(__ushort_as_half(lo));
+      out[(long long)row * 2 * g.ka + col] = __half_as_ushort(__float2half_rn(h * 64.f));
+      uint8_t* x8 = reinterpret_cast<uint8_t*>(out + (long long)row * 2 * g.ka + g.ka) + (col / 64) * 128 + col % 64;
+      x8[0] = e4m3(l * 2048.f);
+      x8[64] = e4m3(h);
+      continue;
+    }
     split16(v, fp16 != 0, hi, lo);
     out[(long long)row * 2 * g.ka + col] = hi;
     out[(long long)row * 2 * g.ka + g.ka + col] = lo;
@@ -50,9 +70,73 @@ int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w
   const int blocks = (int)std::min<long long>((total + threads - 1) / threads, 148 * 16);
   const float* scale = (st.info.kind == 0 || plan->cfg.bwd_passes == 1)
                            ? (const float*)(plan->ws + plan->off_wscale + (size_t)st.info.layer * 16 + 4) : nullptr;
+  const unsigned int* wmax =
+      st.dev.cross8 ? (const unsigned int*)(plan->ws + plan->off_wscale + (size_t)st.info.layer * 16) : nullptr;
   pack_stage_kernel<<<blocks, threads, 0, s>>>(w, (uint16_t*)(plan->ws + st.info.b_offset), g, rows, st.ci,
-                                               st.info.operand_fp16, scale);
+                                               st.info.operand_fp16, scale, wmax);
   LSNF_CUDA(cudaGetLastError());
+  return LSNF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// A operand of a cross8 stage from the bf16 hi|lo gradient its producer wrote, element by element (the phase-split
+// layout is kept): the value (hi + lo, exact in fp32) times 2^ka is split into fp16 halves a_hi + a_lo, and each
+// 64-channel block of a position holds a_hi 2^5 in the hi half's place and the 128 bytes [a_hi8 x 64 | a_lo8 x 64] in
+// the lo half's, a_hi8 = e4m3(a_hi), a_lo8 = e4m3(a_lo 2^11); ka is the e4m3 scale of the gradient's max |value|
+// (atomicMax-ed by the producer's epilogue).  With the weights' 2^kw and lifts (pack_stage_kernel) every product of
+// the stage carries 2^(ka+kw+11): hi*hi as (a_hi 2^5)(w_hi 2^6), which fp16 holds (2^8 * 2^6 < 65504), the cross
+// terms as a_hi8 w_lo8 and a_lo8 w_hi8.  One thread writes 2^-(ka+kw+11) to the stage's descale word; the stage
+// zeroes the amax word.
+// ---------------------------------------------------------------------------------------------------
+// One thread per 16 channels of a position (two 64-channel blocks fill a warp's 512-byte reads), threadIdx.y picks
+// the position: every load and store is a 16-byte vector and no index needs a division.
+__global__ void __launch_bounds__(256) convert_fp8_kernel(const uint16_t* __restrict__ src, uint16_t* __restrict__ dst,
+                                                          int rows, int C, const unsigned int* amax,
+                                                          const unsigned int* __restrict__ wmax, float* descale) {
+  pdl_wait();
+  pdl_trigger();
+  const int ka = fp8_scale_exp(__uint_as_float(*amax));
+  if (blockIdx.x == 0 && threadIdx.x == 0 && threadIdx.y == 0)
+    *descale = ldexpf(1.f, -(ka + fp8_scale_exp(__uint_as_float(*wmax)) + 11));
+  const int row = blockIdx.x * blockDim.y + threadIdx.y;
+  if (row >= rows) return;
+  const float sa = ldexpf(1.f, ka);
+  const int c = threadIdx.x * 16;
+  const uint16_t* in = src + (size_t)row * 2 * C + c;
+  __align__(16) uint16_t h16[16], l16[16];
+  *reinterpret_cast<uint4*>(h16) = __ldcs(reinterpret_cast<const uint4*>(in));
+  *reinterpret_cast<uint4*>(h16 + 8) = __ldcs(reinterpret_cast<const uint4*>(in + 8));
+  *reinterpret_cast<uint4*>(l16) = __ldcs(reinterpret_cast<const uint4*>(in + C));
+  *reinterpret_cast<uint4*>(l16 + 8) = __ldcs(reinterpret_cast<const uint4*>(in + C + 8));
+  __align__(16) uint16_t hs[16];
+  __align__(16) uint8_t h8[16], l8[16];
+#pragma unroll
+  for (int q = 0; q < 16; ++q) {
+    const float v = (__bfloat162float(__ushort_as_bfloat16(h16[q])) + __bfloat162float(__ushort_as_bfloat16(l16[q]))) * sa;
+    const float h = __half2float(__float2half_rn(v)), l = v - h;
+    hs[q] = __half_as_ushort(__float2half_rn(h * 32.f));
+    h8[q] = e4m3(h);
+    l8[q] = e4m3(l * 2048.f);
+  }
+  uint16_t* o = dst + (size_t)row * 2 * C;
+  *reinterpret_cast<uint4*>(o + c) = *reinterpret_cast<const uint4*>(hs);
+  *reinterpret_cast<uint4*>(o + c + 8) = *reinterpret_cast<const uint4*>(hs + 8);
+  uint8_t* x8 = reinterpret_cast<uint8_t*>(o + C) + (c / 64) * 128 + c % 64;
+  *reinterpret_cast<uint4*>(x8) = *reinterpret_cast<const uint4*>(h8);
+  *reinterpret_cast<uint4*>(x8 + 64) = *reinterpret_cast<const uint4*>(l8);
+}
+
+int launch_convert_fp8(const lsnf_plan* plan, const StageHost& st, cudaStream_t s) {
+  const lsnf_plan::Layer& y = plan->layers[st.info.layer];
+  const int C = st.info.k_per_tap;   // a multiple of 64
+  const int rows = plan->cfg.batch * y.hout * y.hout;
+  const dim3 block(C / 16, std::max(1, 256 / (C / 16)));
+  uint32_t* words = (uint32_t*)(plan->ws + st.x8_off);
+  LSNF_CUDA(launch_k(convert_fp8_kernel, dim3((rows + block.y - 1) / block.y), block, 0, s,
+                     (const uint16_t*)(plan->ws + st.x8_src_off), (uint16_t*)(plan->ws + st.info.a_offset), rows, C,
+                     (const unsigned int*)words,
+                     (const unsigned int*)(plan->ws + plan->off_wscale + (size_t)st.info.layer * 16),
+                     (float*)(words + 1)));
   return LSNF_OK;
 }
 

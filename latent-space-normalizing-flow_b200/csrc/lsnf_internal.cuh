@@ -70,6 +70,12 @@ struct StageDev {
   int32_t out_tma, nst;               // hi|lo output written by TMA tensor stores (1 up2 forward, 2 first layer,
                                       // 3 plain gradient, 4 phase-split gradient; 0 = per-thread stores); ring depth
                                       // of this launch (1-CTA kernel)
+  int32_t cross8;                     // operands are an fp16 hi half plus an e4m3 cross-term half (see
+                                      // tc_cross_fp8, tapgemm_tc.cu); 0 = 16-bit hi|lo halves
+  uint32_t* amax_out;                 // the epilogue atomicMax-es max |output| (fp32 bits) into this word: the
+                                      // consumer stage converts the output to e4m3 with that scale; or null
+  uint32_t* amax_reset;               // this stage's input amax word, zeroed once the conversion that read it is
+                                      // complete; or null
   PhaseDev ph[LSNF_MAX_PHASES];
 };
 
@@ -91,6 +97,9 @@ struct StageHost {
   int k = 0, s = 0, p = 0, ci = 0, co = 0;  // the ConvTranspose2d this stage belongs to
   bool last = false, first = false;
   size_t mbits_off = 0, bias_off = 0;       // workspace offsets of the sign bits and the bias, where the stage has them
+  // cross8 stages: workspace offsets of the bf16 hi|lo gradient the conversion reads (the converted operand is at
+  // info.a_offset) and of the two words [amax bits of that gradient, descale of the accumulator]
+  size_t x8_src_off = 0, x8_off = 0;
 };
 
 struct FlowLayout {
@@ -263,6 +272,15 @@ __device__ __forceinline__ void split16(float v, bool fp16, uint16_t& hi, uint16
     hi = __bfloat16_as_ushort(h); lo = __bfloat16_as_ushort(l);
   }
 }
+// e4m3 scale of a tensor whose max |value| is amax: the exponent k with amax * 2^k in [128, 256) (e4m3 reaches 448),
+// clamped so that every power of two the cross8 stages build from it stays a normal fp32 number; 0 for zeros
+__host__ __device__ inline int fp8_scale_exp(float amax) {
+  if (!(amax > 0.f) || !(amax <= 3.4e38f)) return 0;
+  int e = 0;
+  frexpf(amax, &e);   // amax = f * 2^e, f in [0.5, 1)
+  const int k = 8 - e;
+  return k < -40 ? -40 : (k > 40 ? 40 : k);
+}
 __device__ __forceinline__ float join16(uint16_t hi, uint16_t lo, bool fp16) {
   if (fp16) return __half2float(__ushort_as_half(hi)) + __half2float(__ushort_as_half(lo));
   return __bfloat162float(__ushort_as_bfloat16(hi)) + __bfloat162float(__ushort_as_bfloat16(lo));
@@ -314,6 +332,10 @@ int launch_tapgemm_tc(const StageHost& st, cudaStream_t s);
 int tc_encode_maps(lsnf_plan* plan, StageHost& st);
 // What launch_tapgemm_tc does for this stage on a device with `num_sms` SMs (no device needed)
 TcLaunch tc_plan_launch(const StageHost& st, int num_sms);
+// Whether a 3-pass bf16 data-gradient stage runs its cross terms as one e4m3 stream (operand format of the stage)
+bool tc_cross_fp8(const StageDev& d);
+// bf16 hi|lo gradient -> the hi16 / e4m3 operand of a cross8 stage, and the stage's descale word
+int launch_convert_fp8(const lsnf_plan* plan, const StageHost& st, cudaStream_t s);
 int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w, cudaStream_t s);
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);

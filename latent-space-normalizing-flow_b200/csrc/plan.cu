@@ -452,6 +452,14 @@ static void build_dgrad_stage(lsnf_plan* p, int l) {
   I.flops = 2LL * B * I.grid_h * I.grid_w * (long long)I.n_valid *
             (st.last ? y.k * y.k * y.co : (st.first ? (long long)y.k * y.k * y.co : 16LL * y.co));
   fill_dev(p, st);
+  // the tcgen05 path runs this stage's cross terms in e4m3: it reads gpre[l] converted to the hi16 / e4m3 format
+  // (launch_convert_fp8) from a region of its own, and keeps gpre[l]'s amax and its accumulator descale beside it
+  if (c.gemm_impl == LSNF_GEMM_TCGEN05 && tc_cross_fp8(st.dev)) {
+    st.dev.cross8 = 1;
+    st.x8_src_off = I.a_offset;
+    I.a_offset = take(p, (size_t)B * y.hout * y.hout * 2 * y.co * 2);
+    st.x8_off = take(p, 16);
+  }
 }
 
 // Generator parameter update of layer l (train.py:390-394): transposed operands, the weight-gradient tap-GEMM and where
@@ -665,13 +673,19 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
     int rc;
     if ((rc = tc_prepare_device(dev)) || (rc = aux_prepare_device(dev)) || (rc = flow_prepare_device(dev))) return rc;
   }
-  for (auto& st : plan->stages) {
+  for (size_t i = 0; i < plan->stages.size(); ++i) {
+    StageHost& st = plan->stages[i];
     const lsnf_stage_info& I = st.info;
     StageDev& d = st.dev;
     d.bias = (I.kind == 0 && !st.last) ? (const float*)(plan->ws + st.bias_off) : nullptr;
     d.sk_slots = (float*)(plan->ws + plan->off_sk_slots);
     d.sk_flags = (int32_t*)(plan->ws + plan->off_sk_flags);
     d.descale = (I.kind == 0 || plan->cfg.bwd_passes == 1) ? (const float*)(plan->ws + plan->off_wscale + (size_t)I.layer * 16 + 8) : nullptr;
+    if (d.cross8) d.descale = (const float*)(plan->ws + st.x8_off + 4);
+    d.amax_reset = d.cross8 ? (uint32_t*)(plan->ws + st.x8_off) : nullptr;
+    // the data-gradient stage before a cross8 stage writes that stage's input
+    const bool feeds8 = i + 1 < plan->stages.size() && plan->stages[i + 1].dev.cross8;
+    d.amax_out = feeds8 ? (uint32_t*)(plan->ws + plan->stages[i + 1].x8_off) : nullptr;
     d.mbits = ((I.kind == 0 && !st.last) || (I.kind == 1 && !st.first)) ? (uint32_t*)(plan->ws + st.mbits_off) : nullptr;
     int rc = bind_stage(plan, st, plan->cfg.gemm_impl == LSNF_GEMM_TCGEN05);
     if (rc) return rc;
@@ -715,6 +729,16 @@ static int run_stage(const lsnf_plan* p, const StageHost& st, cudaStream_t s) {
   return p->cfg.gemm_impl == LSNF_GEMM_TCGEN05 ? launch_tapgemm_tc(st, s) : launch_tapgemm_simt(st, s);
 }
 
+// A data-gradient stage of a chain: a cross8 stage first converts the gradient its predecessor just wrote.
+// (lsnf_plan_run_stage runs the tap-GEMM alone, on the operand the last chain call converted.)
+static int run_dgrad_stage(const lsnf_plan* p, const StageHost& st, cudaStream_t s) {
+  if (st.dev.cross8) {
+    const int rc = launch_convert_fp8(p, st, s);
+    if (rc) return rc;
+  }
+  return run_stage(p, st, s);
+}
+
 extern "C" int lsnf_pack_generator_weights(lsnf_plan* plan, const float* const* weights, const float* const* biases,
                                            int32_t n_layers, lsnf_stream stream) {
   if (!plan || !plan->bound) return fail(LSNF_ERR_STATE, "plan not bound");
@@ -727,6 +751,8 @@ extern "C" int lsnf_pack_generator_weights(lsnf_plan* plan, const float* const* 
   for (auto& st : plan->stages) {
     int rc = launch_pack_stage(plan, st, weights[st.info.layer], s);
     if (rc) return rc;
+    // a cross8 stage's input amax starts at 0; from then on the stage zeroes it after each conversion
+    if (st.dev.cross8) LSNF_CUDA(cudaMemsetAsync(plan->ws + st.x8_off, 0, 16, s));
   }
   for (int l = 0; l < plan->n_layers; ++l)
     LSNF_CUDA(cudaMemcpyAsync(plan->ws + plan->off_bias[l], biases[l], (size_t)plan->layers[l].co * 4,
@@ -777,7 +803,7 @@ static int gen_dgrad_partial(lsnf_plan* p, const float* x, const float* mask, fl
   int rc;
   if ((rc = launch_recon_grad_im2col(p, x, mask, sigma_seed_scale(sigma), 0, s))) return rc;
   for (int i = p->n_layers; i < 2 * p->n_layers; ++i)
-    if ((rc = run_stage(p, p->stages[i], s))) return rc;
+    if ((rc = run_dgrad_stage(p, p->stages[i], s))) return rc;
   return LSNF_OK;
 }
 
@@ -785,7 +811,11 @@ extern "C" int lsnf_plan_run_stage(lsnf_plan* plan, int32_t index, lsnf_stream s
   int rc = need(plan, true, false);
   if (rc) return rc;
   if (index < 0 || index >= (int)plan->stages.size()) return fail(LSNF_ERR_INVALID, "bad stage index");
-  return run_stage(plan, plan->stages[index], (cudaStream_t)stream);
+  // a stage run alone leaves the amax words of the chain alone: the next chain call's e4m3 scales depend on that
+  // call's gradients only
+  StageHost alone = plan->stages[index];
+  alone.dev.amax_out = alone.dev.amax_reset = nullptr;
+  return run_stage(plan, alone, (cudaStream_t)stream);
 }
 
 extern "C" int lsnf_generator_forward(lsnf_plan* plan, const float* z, float* x_hat, lsnf_stream stream) {
@@ -895,7 +925,7 @@ extern "C" int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z
     // in fp32 when the gradients are finalized.  The first layer's data gradient is not needed.
     if ((rc = launch_last_fused(plan, x, mask, nullptr, 1.f, s))) return rc;
     for (int i = L; i < 2 * L - 1; ++i)
-      if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
+      if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
     if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
     plan->wg_ready = true;
     if (!layers_all) return LSNF_OK;
@@ -932,7 +962,7 @@ extern "C" int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, floa
   if ((rc = launch_recon_grad_im2col(plan, grad_x_hat, nullptr, 1.f, 1, s))) return rc;
   const int end = grad_z ? 2 * L : 2 * L - 1;   // the first layer's data gradient only feeds dL/dz
   for (int i = L; i < end; ++i)
-    if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
+    if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
   if (grad_z && (rc = launch_reduce_partial(plan, grad_z, 1.f, s))) return rc;
   // the gradient tensors no longer hold the part = -2 state of lsnf_generator_param_grads
   plan->wg_ready = false;
@@ -1026,10 +1056,13 @@ static_assert(graph_chunk < AIS_BETA_FLOATS, "the workspace schedule copy must h
 
 extern "C" int lsnf_langevin_launch_count(const lsnf_plan* plan, int32_t steps) {
   if (!plan) return 0;
-  // per step: L forward + fused gather/tanh/seed/im2col + L data-gradient + flow + update; once: split_z; per
-  // replayed graph chunk: the kernel that sets (seed, sample offset, first step index) in device memory
+  // per step: L forward + fused gather/tanh/seed/im2col + L data-gradient (each cross8 stage with its operand
+  // conversion) + flow + update; once: split_z; per replayed graph chunk: the kernel that sets (seed, sample offset,
+  // first step index) in device memory
   const int chunks = steps > 0 ? (steps + graph_chunk - 1) / graph_chunk : 0;
-  return 1 + steps * (2 * plan->n_layers + 3) + chunks;
+  int conversions = 0;
+  for (const auto& st : plan->stages) conversions += st.dev.cross8;
+  return 1 + steps * (2 * plan->n_layers + 3 + conversions) + chunks;
 }
 
 // the g_l_steps loop on stream s: inputs are the workspace copies of z and x (and of the mask, nullable)
@@ -1114,7 +1147,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
     for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i) {
       {
         PdlScope pdl(use_pdl);
-        if ((rc = run_stage(plan, plan->stages[i], s))) return rc;
+        if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
       }
       tr.mark(("dgrad layer " + std::to_string(plan->stages[i].info.layer)).c_str());
     }

@@ -8,7 +8,9 @@
 // * Operands are 16-bit hi|lo pairs (value = hi + lo; fp16 for the forward pass, bf16 for 3-pass data gradients); each
 //   K step issues three tcgen05.mma (lo*hi, hi*lo, hi*hi) into one fp32 TMEM accumulator -- the 3-pass split that
 //   keeps z_T within the 1e-4 parity budget.  Single-pass stages (passes == 1: the data gradient of noisy chains)
-//   load and multiply the hi halves only.
+//   load and multiply the hi halves only.  The wide 3-pass data-gradient stages (cross8, tc_cross_fp8) instead hold an
+//   fp16 hi half and, in the lo half's bytes, the two cross terms as e4m3 along K: per K block one kind::f16 pass on
+//   the hi halves and one kind::f8f6f4 pass (twice the 16-bit rate) over the 128-element e4m3 row.
 // * Warp roles: warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..9 = epilogue
 //   (tcgen05.ld -> bias / LeakyReLU / LeakyReLU' from bit-packed signs -> 16-bit hi|lo through TMA tensor stores,
 //   or fp32 rows).  Two kernels: tapgemm_tc_kernel<BN> (one CTA per tile, ring sized per launch) and
@@ -149,6 +151,13 @@ __device__ __forceinline__ void epi_bar_sync() {   // the 8 epilogue warps only
   asm volatile("bar.sync 1, %0;" ::"n"(32 * TC_EPI_WARPS) : "memory");
 }
 
+// max |value| of a warp's gradient outputs into the consumer's amax word (non-negative floats order like their bits)
+__device__ __forceinline__ void warp_amax(uint32_t* word, float m, int lane) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if (lane == 0) atomicMax(word, __float_as_uint(m));
+}
+
 // element i of a small register array without dynamic indexing (which would push the array to local memory)
 template <int N>
 __device__ __forceinline__ uint32_t pick_word(const uint32_t (&a)[N], int i) {
@@ -259,6 +268,7 @@ __device__ __forceinline__ void tc_epilogue(const StageDev& st, int mtile, int n
     __syncwarp();
     __threadfence();
   }
+  float amax = 0.f;
 #pragma unroll 1
   for (int cc = 0; cc < SPAN; cc += CH) {
     uint32_t v[CH];
@@ -301,6 +311,7 @@ __device__ __forceinline__ void tc_epilogue(const StageDev& st, int mtile, int n
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
           const float t = ((mw >> q) & 1u) ? f[q] * leak : f[q];   // sign of the saved activation
+          amax = fmaxf(amax, fabsf(t));
           split16(t, out16, hi[q], lo[q]);
         }
         *reinterpret_cast<uint4*>(o16 + cc + j) = *reinterpret_cast<uint4*>(hi);
@@ -314,6 +325,7 @@ __device__ __forceinline__ void tc_epilogue(const StageDev& st, int mtile, int n
       if (epi == EPI_ACT_HL) obits[cc >> 5] = signs;   // hidden widths are multiples of 64: whole words
     }
   }
+  if (epi == EPI_GRAD_HL && st.amax_out) warp_amax(st.amax_out, amax, lane);
   if (sk_mode == 2) {
     __syncwarp();
     if (lane == 0)
@@ -504,6 +516,15 @@ __device__ __forceinline__ void umma2_bf16(uint32_t tmem_d, uint64_t da, uint64_
       "}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accum)
       : "memory");
 }
+__device__ __forceinline__ void umma2_f8(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accum) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accum)
+      : "memory");
+}
 __device__ __forceinline__ void umma2_commit_both(uint32_t bar) {
   asm volatile(
       "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
@@ -613,6 +634,7 @@ __device__ __forceinline__ void tc_epilogue_tma(const StageDev& st, const CUtens
     __syncwarp();
     __threadfence();
   }
+  float amax = 0.f;
 #pragma unroll 1
   for (int ch = 0; ch < NCH; ++ch) {
     const int col = ch * 64 + half * 32;   // column of the accumulator tile
@@ -654,6 +676,7 @@ __device__ __forceinline__ void tc_epilogue_tma(const StageDev& st, const CUtens
         for (int q = 0; q < 8; ++q) {
           const float a = __uint_as_float(v[j + q]) * descale;
           t[q] = ((mw >> q) & 1u) ? a * leak : a;   // sign of the saved activation
+          amax = fmaxf(amax, fabsf(t[q]));
         }
       }
       // row r of the slab is 128 B; the 16-byte chunk index is XORed with (row % 8) -- the 128-byte TMA swizzle
@@ -688,6 +711,7 @@ __device__ __forceinline__ void tc_epilogue_tma(const StageDev& st, const CUtens
     }
     if (obits) obits[2 * ch] = signs;   // after the barrier: the store's latency stays off the slab's critical path
   }
+  if (epi == EPI_GRAD_HL && st.amax_out) warp_amax(st.amax_out, amax, lane);
   if (sk_mode == 2) {
     __syncwarp();
     if (lane == 0)
@@ -822,6 +846,8 @@ tapgemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   const uint32_t tmem_base = *tmem_slot_ptr;
   pdl_wait();      // see lsnf_internal.cuh: the set-up above overlaps the tail of the previous kernel
   pdl_trigger();
+  // the conversion that read this stage's input amax is complete: zero the word for the next producer
+  if (st.amax_reset && blockIdx.x == 0 && threadIdx.x == 0) *st.amax_reset = 0u;
 
   if (warp == 0) {
     {
@@ -865,8 +891,11 @@ tapgemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   } else if (warp == 1) {
     if (leader) {
       // ===== MMA issuer (leader CTA only): M = 256 over both CTAs, N = 256 =====
-      const uint32_t fmt = st.fp16 ? 0u : 1u;
+      const bool cross8 = st.cross8 != 0;
+      const uint32_t fmt = (st.fp16 || cross8) ? 0u : 1u;   // the hi halves of a cross8 stage are fp16
       const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(P_BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+      // kind::f8f6f4 with E4M3 (format 0) A and B, fp32 accumulator
+      const uint32_t idesc8 = (1u << 4) | ((uint32_t)(P_BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
       uint32_t s = 0, par = 0, sa = tiles;
       for (int j = 0; j < sk.n_items; ++j) {
         const SkItem w = sk.item(j);
@@ -881,16 +910,27 @@ tapgemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           // descriptors differ only in their 16-byte-unit address field: K step k starts 32 bytes further
           const uint64_t da = umma_desc(sa), db = umma_desc(sa + b_off);
           if (elect_one()) {
+            if (three && cross8) {
+              // hi*hi on the fp16 halves (K = 16 per MMA), then the e4m3 rows [a_hi8 | a_lo8] . [w_lo8 | w_hi8]
+              // (K = 32 per MMA): the same 32-byte descriptor steps cover the 128-byte rows
 #pragma unroll
-            for (int k = 0; k < BLOCK_K / 16; ++k) {
-              const uint64_t a_hi = da + 2 * k, a_lo = a_hi + (A_TILE_BYTES >> 4);
-              const uint64_t b_hi = db + 2 * k, b_lo = b_hi + (P_B_TILE_BYTES >> 4);
-              if (three) {
-                umma2_bf16(d_tmem, a_lo, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
-                umma2_bf16(d_tmem, a_hi, b_lo, idesc, 1u);
-                umma2_bf16(d_tmem, a_hi, b_hi, idesc, 1u);
-              } else {
-                umma2_bf16(d_tmem, a_hi, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
+              for (int k = 0; k < BLOCK_K / 16; ++k)
+                umma2_bf16(d_tmem, da + 2 * k, db + 2 * k, idesc, (it > w.ka || k > 0) ? 1u : 0u);
+#pragma unroll
+              for (int k = 0; k < BLOCK_K / 16; ++k)
+                umma2_f8(d_tmem, da + (A_TILE_BYTES >> 4) + 2 * k, db + (P_B_TILE_BYTES >> 4) + 2 * k, idesc8, 1u);
+            } else {
+#pragma unroll
+              for (int k = 0; k < BLOCK_K / 16; ++k) {
+                const uint64_t a_hi = da + 2 * k, a_lo = a_hi + (A_TILE_BYTES >> 4);
+                const uint64_t b_hi = db + 2 * k, b_lo = b_hi + (P_B_TILE_BYTES >> 4);
+                if (three) {
+                  umma2_bf16(d_tmem, a_lo, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
+                  umma2_bf16(d_tmem, a_hi, b_lo, idesc, 1u);
+                  umma2_bf16(d_tmem, a_hi, b_hi, idesc, 1u);
+                } else {
+                  umma2_bf16(d_tmem, a_hi, b_hi, idesc, (it > w.ka || k > 0) ? 1u : 0u);
+                }
               }
             }
             umma2_commit_both(empty_bar(s));      // frees the slot in both CTAs
@@ -974,6 +1014,17 @@ static bool use_pair(const StageDev& d) {
          (mtiles >= 2 || total >= 8);
 }
 
+// The 3-pass bf16 data-gradient stages that run on the pair kernel with at least 8 M tiles take the fp16 / e4m3
+// cross-term operands (DESIGN.md section 4.1): two pass-equivalents per K block instead of three.  With fewer rows
+// (CelebA-HQ256 B=8: 1 and 4 M tiles, 128 and 512 rows) a stage streams far more weight bytes than it multiplies
+// (2048 x 1024 x 16 taps for 128 rows), fewer MMA passes buy little, and the operand conversion costs more than they
+// save.  lsnf_plan_create gives a selected stage that operand format (StageDev::cross8) and the conversion of its
+// input; the pair kernel's main loop follows it.
+bool tc_cross_fp8(const StageDev& d) {
+  const int mtiles = d.tiles_b * d.tiles_h * d.tiles_w;
+  return use_pair(d) && d.epi == EPI_GRAD_HL && d.passes == 3 && !d.fp16 && mtiles >= 8;
+}
+
 // Ring of the 1-CTA kernel for one launch: stage bytes, depth, dynamic shared memory to request.
 struct RingGeom { int nst; size_t stage_bytes, smem; };
 static RingGeom ring_geometry(const StageDev& d, int out_tma) {
@@ -1045,6 +1096,7 @@ TcLaunch tc_plan_launch(const StageHost& sh, int num_sms) {
     o.smem_bytes = P_SMEM_BYTES;
     o.ctas_per_sm = 1;
     o.tmem_columns = 512;
+    o.cross_fp8 = d.cross8;
   } else {
     switch (d.block_n) {
       case 256: l.kernel = &tapgemm_tc_kernel<256>; break;

@@ -42,6 +42,13 @@ def pow2_floor(v: float) -> float:
     return 2.0 ** math.floor(math.log2(v)) if v > 0 else 1.0
 
 
+def fp8_scale_exp(m: float) -> int:
+    """k with m * 2^k in [128, 256), clamped to [-40, 40]; 0 for m = 0 (csrc/lsnf_internal.cuh fp8_scale_exp)."""
+    if not m > 0:
+        return 0
+    return max(-40, min(40, 8 - math.frexp(m)[1]))
+
+
 def split(t: torch.Tensor, dt: torch.dtype):
     """t ~= hi + lo with both halves representable in ``dt`` (what split_z / the stage epilogues store)."""
     hi = t.to(dt).float()
@@ -82,6 +89,9 @@ class Scheme:
        "16"  - the 16-bit halves themselves (the shipped 3-pass kernels)
        "f8t" - both operands of the cross term re-rounded to e4m3, one scale per tensor
        "f8b" - e4m3 with a power-of-two scale per 32 elements along K (kind::mxf8f6f4)
+       "f8x" - what the wide data-gradient stages build: each operand times its power-of-two scale 2^k
+               (max |tensor| * 2^k in [128, 256)) split into fp16 halves, hi*hi in fp16, both cross terms in
+               e4m3 (round to nearest) with the lo halves lifted by 2^11; ``base`` is ignored
     passes: tensor-pipe cost in units of one 16-bit pass (fp8 runs at twice the 16-bit rate)."""
 
     def __init__(self, name, base, cross=(), cross_fmt="16", scale_w=True):
@@ -93,6 +103,13 @@ class Scheme:
         if self.base is None:
             return op(a, w)
         k = 1.0
+        if self.cross_fmt == "f8x":
+            sa, sw = 2.0 ** fp8_scale_exp(float(a.abs().max())), 2.0 ** fp8_scale_exp(float(w.abs().max()))
+            ah, al = split(a * sa, F16)
+            wh, wl = split(w * sw, F16)
+            e = lambda t: t.to(F8).float()   # noqa: E731
+            lift = 2.0 ** 11
+            return (op(ah, wh) + (op(e(ah), e(wl * lift)) + op(e(al * lift), e(wh))) / lift) / (sa * sw)
         if self.scale_w:   # per-layer power-of-two weight scale (max |w| -> [1, 2)), undone exactly afterwards
             k = 1.0 / pow2_floor(float(w.abs().max()))
         ah, al = split(a, self.base)
@@ -202,6 +219,8 @@ BWD = {
     "f16x1": Scheme("fp16 single pass (shipped opt-in)", F16, (), scale_w=False),
     "f16+f8t": Scheme("fp16 hi*hi + cross terms in e4m3, per-tensor scale", F16, BOTH, "f8t"),
     "f16+f8b": Scheme("fp16 hi*hi + cross terms in e4m3, scale per 32 K", F16, BOTH, "f8b"),
+    "f16+f8x": Scheme("fp16 hi*hi + cross terms as one e4m3 stream, power-of-two scale per tensor (shipped on the "
+                      "wide stages)", F16, BOTH, "f8x", scale_w=False),
 }
 # (forward, data gradient, z_T error measured on a B200 at B=100 or None)
 COMBOS = [
@@ -217,6 +236,7 @@ COMBOS = [
     ("f16+f8b", "f16x1", None),
     ("f16x3", "f16+f8b", None),
     ("f16x3", "f16+f8t", None),
+    ("f16x3", "f16+f8x", None),
 ]
 
 

@@ -14,7 +14,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "latent-space-normalizing-flow_b200", "_lib", "liblsnf_b200.so")
-WATCH = ["UTCHMMA", "UTCHMMA.2CTA", "UTCBAR", "LDTM", "STTM", "UTMALDG", "UTMASTG", "UTMAPF", "UBLKCP", "SYNCS", "ELECT",
+WATCH = ["UTCHMMA", "UTCHMMA.2CTA", "UTCQMMA", "UTCQMMA.2CTA", "UTCBAR", "LDTM", "STTM", "UTMALDG", "UTMASTG", "UTMAPF", "UBLKCP", "SYNCS", "ELECT",
          "ACQBULK", "PREEXIT", "HMMA", "FFMA", "MUFU", "BAR.SYNC", "LDG", "STG", "LDS", "STS", "RED", "ATOM"]
 
 
