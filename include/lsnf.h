@@ -97,7 +97,11 @@ typedef struct lsnf_config {
                             reduced-precision mode, measured margins in DESIGN.md section 4.1 */
   int32_t train;         /* != 0: the workspace also holds the buffers of lsnf_generator_param_grads (transposed
                             operands and split-K partials of the weight-gradient GEMMs); 0 for inference-only plans */
-  int32_t reserved[3];
+  int32_t meas_rows;     /* m > 0: rows of a dense linear measurement operator A [m, nc*H*W] (lsnf_*_measured below);
+                            the workspace then also holds A packed twice (about 8 m n bytes, n = nc*H*W) plus the
+                            split-K partials of its two GEMMs.  0 = no operator: the plan is exactly that of a config
+                            without this field */
+  int32_t reserved[2];
 } lsnf_config;
 
 /* number of per-step flow parameter pointers expected by lsnf_pack_flow_weights, in this order:
@@ -259,12 +263,42 @@ int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* 
                  uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w, float* accept_rate,
                  lsnf_stream stream);
 
+/* ---- linear measurements y = A vec(G(z)) + sigma noise (compressed sensing, super-resolution, deblurring) ------- */
+/* A plan created with lsnf_config.meas_rows = m > 0 runs the energy
+ *   U(z) = |A vec(x_hat) - y|^2 / (2 sigma^2) - log p(z),   x_hat = G(z),
+ * with vec the NCHW flattening of x_hat [B,nc,H,W] (n = nc*H*W elements per sample; torch's x.view(B, -1)), A a dense
+ * fp32 [m, n] row-major device matrix and y [B, m].  Heteroscedastic noise needs nothing extra: scaling row i of A and
+ * of y by sigma / sigma_i gives the same energy.
+ * Workspace: A is kept as two K-major 16-bit hi|lo copies, about 8 m n bytes, plus fp32 split-K partials of
+ * A x_hat and A^T r (r = A x_hat - y).  A dense operator grows fast with the image: at CelebA-HQ256 (n = 196 608) a
+ * 4x-downsampling A (m = n / 16) takes 19 GB.
+ * lsnf_pack_measurement: packs A (read once; the caller may free or change it afterwards) into both copies, with one
+ *   power-of-two scale computed on the device for the fp16 copy of the forward product, undone exactly in fp32.
+ *   Pack again after A changes.
+ * lsnf_langevin_run_measured, lsnf_generator_dgrad_measured and lsnf_ais_run_measured have the contracts of
+ *   lsnf_langevin_run, lsnf_generator_dgrad and lsnf_ais_run (injected noise, Philox keying, gradient norms, graph
+ *   replay with y copied into the workspace before each replay; measured and unmeasured loops never share a graph)
+ *   with y [B, m] in place of x (and the mask).  For AIS, l(z) = -|A vec(G(z)) - y|^2 / (2 sigma^2) and the caller adds
+ *   C = -(m/2) log(2 pi sigma^2).
+ * The three return LSNF_ERR_UNSUPPORTED on a plan with meas_rows == 0 or bwd_passes == 1 (the single-pass data
+ * gradient writes an fp16 seed and A^T r has no bounded range), and LSNF_ERR_INVALID until an operator is packed. */
+int lsnf_pack_measurement(lsnf_plan* plan, const float* A, lsnf_stream stream);
+int lsnf_langevin_run_measured(lsnf_plan* plan, const float* z0, const float* y, int32_t steps, float step_size,
+                               float sigma, int32_t with_noise, const float* eps, uint64_t seed, uint64_t sample_offset,
+                               float* z_out, float* gnorms, lsnf_stream stream);
+int lsnf_generator_dgrad_measured(lsnf_plan* plan, const float* y, float sigma, float* grad_z, lsnf_stream stream);
+int lsnf_ais_run_measured(lsnf_plan* plan, const float* z0, const float* y, const float* betas, int32_t steps,
+                          float step_size, float target_accept, float sigma, const float* eps, const float* u,
+                          uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w, float* accept_rate,
+                          lsnf_stream stream);
+
 int lsnf_adam_step(int32_t n_tensors, float* const* params, const float* const* grads, float* const* exp_avg,
                    float* const* exp_avg_sq, const int64_t* sizes, const int32_t* grad_kk, const int32_t* grad_inner,
                    float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
                    const float* grad_scale, lsnf_stream stream);
 
-/* Launches generator stage `index` alone (0..L-1 forward, L..2L-1 data gradient) on the buffers currently in the
+/* Launches generator stage `index` alone (0..L-1 forward, L..2L-1 data gradient, and on a plan with meas_rows > 0
+ * 2L = A x_hat, 2L+1 = A^T r) on the buffers currently in the
  * workspace.  Profiling / test hook: bench.py times the dominant tap-GEMM with CUDA events through it.  A stage whose
  * launch record has cross_fp8 set reads the e4m3 operand the last data-gradient call converted (the conversion is
  * not part of the stage), and no stage run this way changes the scales a later call uses. */
@@ -283,7 +317,7 @@ typedef struct lsnf_tap {
 } lsnf_tap;
 
 typedef struct lsnf_stage_info {
-  int32_t kind;          /* 0 forward, 1 data-gradient */
+  int32_t kind;          /* 0 forward, 1 data-gradient, 3 measurement operator (A x_hat or A^T r; layer = the last) */
   int32_t layer;         /* generator layer index */
   int32_t grid_h, grid_w;/* row grid: M = batch * grid_h * grid_w */
   int32_t box_b, box_h, box_w; /* M tile = box_b*box_h*box_w = 128 rows */

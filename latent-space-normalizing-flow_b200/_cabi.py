@@ -22,7 +22,7 @@ class Config(C.Structure):
     _fields_ = [("arch", C.c_int32), ("batch", C.c_int32), ("nz", C.c_int32), ("ngf", C.c_int32), ("nc", C.c_int32),
                 ("f_depth", C.c_int32), ("f_width", C.c_int32), ("f_permutation", C.c_int32),
                 ("f_coupling", C.c_int32), ("leak", C.c_float), ("gemm_impl", C.c_int32),
-                ("bwd_passes", C.c_int32), ("train", C.c_int32), ("reserved", C.c_int32 * 3)]
+                ("bwd_passes", C.c_int32), ("train", C.c_int32), ("meas_rows", C.c_int32), ("reserved", C.c_int32 * 2)]
 
 
 class Tap(C.Structure):
@@ -92,6 +92,14 @@ EXPORTS = {
     "lsnf_ais_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float,
                                C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
                                C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lsnf_pack_measurement": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lsnf_langevin_run_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_float,
+                                             C.c_int32, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
+                                             C.c_void_p]),
+    "lsnf_generator_dgrad_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
+    "lsnf_ais_run_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float,
+                                        C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lsnf_adam_step": (C.c_int, [C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                  C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int32),
                                  C.POINTER(C.c_int32), C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,

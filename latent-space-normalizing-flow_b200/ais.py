@@ -32,10 +32,15 @@ def sigmoid_schedule(steps: int, delta: float = 4.0) -> np.ndarray:
     return b
 
 
-def log_likelihood_constant(sigma: float, shape, mask: Optional[torch.Tensor] = None) -> np.ndarray:
+def log_likelihood_constant(sigma: float, shape, mask: Optional[torch.Tensor] = None,
+                            operator: Optional[torch.Tensor] = None) -> np.ndarray:
     """C = -1/2 sum_{i: m_i > 0} log(2 pi sigma^2 / m_i) per image, fp64 [B]: the normaliser of the Gaussian likelihood
-    p(x|z) with per-pixel precision m_i / sigma^2 (-(D/2) log(2 pi sigma^2) without a mask).  ``shape`` is x's."""
+    p(x|z) with per-pixel precision m_i / sigma^2 (-(D/2) log(2 pi sigma^2) without a mask).  ``shape`` is x's.  With a
+    measurement ``operator`` A [m, n] (``shape`` x's or y's: only its batch size is read) it is that of p(y|z),
+    C = -(m/2) log(2 pi sigma^2)."""
     B = int(shape[0])
+    if operator is not None:
+        return np.full(B, -0.5 * int(operator.shape[0]) * math.log(2.0 * math.pi * float(sigma) ** 2))
     D = int(np.prod(shape[1:]))
     l2ps = math.log(2.0 * math.pi * float(sigma) ** 2)
     if mask is None:
@@ -62,16 +67,21 @@ def _check_schedule(schedule, steps: int) -> np.ndarray:
     return b
 
 
-def _ais_chains(x, netG, netF, args, z0, *, chains, steps, betas, step_size, target_accept, mask, seed):
+def _ais_chains(x, netG, netF, args, z0, *, chains, steps, betas, step_size, target_accept, mask, seed, operator=None):
     """AIS on the plan of batch B * chains: chain c of image b is row b * chains + c.  ``z0`` [B*chains, nz] or None
-    (exact prior samples F^-1(eps)).  Returns (z_T, log w [B, chains], acceptance rate [B, chains], mask rows)."""
+    (exact prior samples F^-1(eps)).  With ``operator``, x is y [B, m].  Returns (z_T, log w [B, chains], acceptance
+    rate [B, chains])."""
     B = x.shape[0]
     n = B * chains
     sigma = float(_get(args, "g_llhd_sigma", 0.3))
     s0 = float(_get(args, "g_l_step_size", 0.1)) if step_size is None else float(step_size)
-    plan = langevin_plan(netG, netF, n, x.device, 3)
+    plan = langevin_plan(netG, netF, n, x.device, 3, meas_rows=int(operator.shape[0]) if operator is not None else 0)
     plan.ensure_generator(netG)
     plan.ensure_flow(netF, need_inverse=True)
+    if operator is not None:
+        from .plan import as_measurements
+        x = as_measurements(x, operator, B)
+        plan.ensure_operator(operator)
     xx = x.detach().float().repeat_interleave(chains, 0).contiguous()
     mm = None
     if mask is not None:
@@ -84,7 +94,10 @@ def _ais_chains(x, netG, netF, args, z0, *, chains, steps, betas, step_size, tar
         z0 = plan.flow_inverse(eps)[0]
     bt = torch.as_tensor(betas, dtype=torch.float32).to(x.device).contiguous()
     t = 0.0 if target_accept is None else float(target_accept)
-    z, lw, rate = plan.ais_run(z0.contiguous(), xx, bt, steps, s0, sigma, target_accept=t, mask=mm, seed=seed)
+    if operator is not None:
+        z, lw, rate = plan.ais_run_measured(z0.contiguous(), xx, bt, steps, s0, sigma, target_accept=t, seed=seed)
+    else:
+        z, lw, rate = plan.ais_run(z0.contiguous(), xx, bt, steps, s0, sigma, target_accept=t, mask=mm, seed=seed)
     return z, lw.view(B, chains), rate.view(B, chains)
 
 
@@ -101,23 +114,29 @@ def _validate(x, chains, steps, schedule):
 
 def ais_log_likelihood(x: torch.Tensor, netG, netF, args, *, chains: int, steps: int, schedule=None,
                        step_size: Optional[float] = None, target_accept: Optional[float] = 0.65,
-                       mask: Optional[torch.Tensor] = None, seed: Optional[int] = None):
+                       mask: Optional[torch.Tensor] = None, seed: Optional[int] = None,
+                       operator: Optional[torch.Tensor] = None):
     """Forward AIS estimate of log p(x) for every image of x [B,nc,H,W]: ``chains`` chains per image from exact prior
     samples z_0 = F^-1(eps), ``steps`` MALA transitions along ``schedule`` (steps + 1 values in [0, 1], 0 -> 1; default
     the sigmoidal schedule of Grosse et al. with delta = 4).  sigma is ``args.g_llhd_sigma``; the initial step size
     ``args.g_l_step_size`` unless ``step_size`` is given; ``target_accept`` (None or <= 0: fixed) adapts it per chain.
-    ``mask`` weights the likelihood per pixel as in ``sample_langevin_post_z_with_flow``.
+    ``mask`` weights the likelihood per pixel as in ``sample_langevin_post_z_with_flow``.  With a linear measurement
+    ``operator`` A [m, nc*H*W] (``plan.as_operator``) the first argument is y [B, m] and the estimate is log p(y) of
+    y = A vec(G(z)) + sigma noise; ``mask`` and ``operator`` together raise ValueError.
 
     Returns (log_px [B] fp64, log_w [B, chains], accept_rate [B, chains]); log_px = logmeanexp over the chains of log w
     plus the likelihood's normaliser C (``log_likelihood_constant``).  E[log_px] <= log p(x): a stochastic lower bound
     that tightens as ``steps`` grows."""
+    if mask is not None and operator is not None:
+        raise ValueError("pass either mask or operator, not both")
     betas = _validate(x, chains, steps, schedule)
     if seed is None:
         seed = (int(_get(args, "seed", 1)) << 32) ^ (0x5A15 << 16) ^ next(_call_counter)
     sigma = float(_get(args, "g_llhd_sigma", 0.3))
     _, lw, rate = _ais_chains(x, netG, netF, args, None, chains=int(chains), steps=int(steps), betas=betas,
-                              step_size=step_size, target_accept=target_accept, mask=mask, seed=seed)
-    c = torch.from_numpy(log_likelihood_constant(sigma, tuple(x.shape), mask)).to(x.device)
+                              step_size=step_size, target_accept=target_accept, mask=mask, seed=seed,
+                              operator=operator)
+    c = torch.from_numpy(log_likelihood_constant(sigma, tuple(x.shape), mask, operator)).to(x.device)
     return logmeanexp(lw, 1) + c, lw, rate
 
 

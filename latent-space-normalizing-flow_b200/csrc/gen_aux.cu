@@ -180,6 +180,99 @@ int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cud
 }
 
 // ---------------------------------------------------------------------------------------------------
+// linear measurement operator A [m, n] (lsnf_pack_measurement): the B operands of the two measurement stages,
+//   stage 2L (A x_hat):   rows i < m, K = n:  fp16 hi|lo of A[i][j] 2^k, 2^k the power of two with max|A| 2^k in [1, 2)
+//                         (wmax_kernel / wscale_finalize_kernel on the operator's scale block; the stage's epilogue
+//                         multiplies by 2^-k, exact)
+//   stage 2L+1 (A^T r):   rows j < n, K = m:  bf16 hi|lo of A[i][j] (the format of the data-gradient stages' operands)
+// Padding rows and columns are written as zeros.
+// ---------------------------------------------------------------------------------------------------
+__global__ void meas_pack_kernel(const float* __restrict__ A, int m, int n, uint16_t* __restrict__ fwd, int fwd_rows,
+                                 int kx, uint16_t* __restrict__ bwd, int bwd_rows, int km,
+                                 const float* __restrict__ scale) {
+  const float sc = *scale;
+  const long long nf = (long long)fwd_rows * kx, total = nf + (long long)bwd_rows * km;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total;
+       e += (long long)gridDim.x * blockDim.x) {
+    uint16_t hi, lo;
+    if (e < nf) {
+      const int i = (int)(e / kx), j = (int)(e % kx);
+      split16(i < m && j < n ? A[(size_t)i * n + j] * sc : 0.f, true, hi, lo);
+      fwd[(size_t)i * 2 * kx + j] = hi;
+      fwd[(size_t)i * 2 * kx + kx + j] = lo;
+    } else {
+      const int j = (int)((e - nf) / km), i = (int)((e - nf) % km);
+      split16(i < m && j < n ? A[(size_t)i * n + j] : 0.f, false, hi, lo);
+      bwd[(size_t)j * 2 * km + i] = hi;
+      bwd[(size_t)j * 2 * km + km + i] = lo;
+    }
+  }
+}
+
+int launch_meas_pack(const lsnf_plan* plan, const float* A, cudaStream_t s) {
+  const StageHost& f = plan->stages[2 * plan->n_layers];
+  const StageHost& b = plan->stages[2 * plan->n_layers + 1];
+  const int m = plan->meas_m, n = plan->cfg.nc * plan->img * plan->img;
+  unsigned int* blk = (unsigned int*)(plan->ws + plan->off_meas_scale);
+  LSNF_CUDA(cudaMemsetAsync(blk, 0, 16, s));
+  const long long na = (long long)m * n;
+  wmax_kernel<<<(int)std::min<long long>((na + 255) / 256, 148 * 8), 256, 0, s>>>(A, na, blk);
+  LSNF_CUDA(cudaGetLastError());
+  wscale_finalize_kernel<<<1, 32, 0, s>>>(blk, 1);
+  LSNF_CUDA(cudaGetLastError());
+  const long long total = (long long)f.info.b_rows * plan->meas_kx + (long long)b.info.b_rows * plan->meas_km;
+  meas_pack_kernel<<<(int)std::min<long long>((total + 255) / 256, 148 * 16), 256, 0, s>>>(
+      A, m, n, (uint16_t*)(plan->ws + f.info.b_offset), f.info.b_rows, plan->meas_kx,
+      (uint16_t*)(plan->ws + b.info.b_offset), b.info.b_rows, plan->meas_km, (const float*)(blk + 1));
+  LSNF_CUDA(cudaGetLastError());
+  return LSNF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Between the two measurement stages: r = A x_hat - y, with A x_hat the fixed-order sum of stage 2L's split-K partials
+// [S][B][n_pad] (already descaled by its epilogue).  One CTA per (256 rows of r, sample): writes r * seed_scale as the
+// bf16 hi|lo row [B][2 km] stage 2L+1 reads (seed_scale = sigma_seed_scale(sigma): the share of 1/sigma^2 the 16-bit
+// gradient tensors carry, as in the unmeasured seed) and, when epart is given, the CTA's fixed-order partial of |r|^2
+// into epart[b][blockIdx.x] (annealed importance sampling: l(z) = -|r|^2 / (2 sigma^2)).
+// ---------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) meas_finish_kernel(const float* __restrict__ part, int nsplit, int pitch,
+                                                          const float* __restrict__ y, int B, int m,
+                                                          uint16_t* __restrict__ r_hl, int km, float seed_scale,
+                                                          float* __restrict__ epart) {
+  __shared__ float red[256];
+  pdl_wait();
+  pdl_trigger();
+  const int b = blockIdx.y, i = blockIdx.x * 256 + threadIdx.x;
+  float e = 0.f;
+  if (i < m) {
+    float v = 0.f;
+    for (int q = 0; q < nsplit; ++q) v += __ldcg(part + ((size_t)q * B + b) * pitch + i);
+    const float r = v - y[(size_t)b * m + i];
+    e = r * r;
+    uint16_t hi, lo;
+    split16(r * seed_scale, false, hi, lo);
+    r_hl[(size_t)b * 2 * km + i] = hi;
+    r_hl[(size_t)b * 2 * km + km + i] = lo;
+  }
+  if (!epart) return;
+  red[threadIdx.x] = e;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) epart[(size_t)b * gridDim.x + blockIdx.x] = red[0];
+}
+
+int launch_meas_finish(const lsnf_plan* plan, const float* y, float seed_scale, float* epart, cudaStream_t s) {
+  const StageHost& f = plan->stages[2 * plan->n_layers];
+  LSNF_CUDA(launch_k(meas_finish_kernel, dim3(plan->meas_tiles, plan->cfg.batch), dim3(256), 0, s,
+                     (const float*)(plan->ws + f.info.out_offset), f.info.k_splits, f.info.n_pad, y, plan->cfg.batch,
+                     plan->meas_m, (uint16_t*)(plan->ws + plan->off_meas_r), plan->meas_km, seed_scale, epart));
+  return LSNF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // last forward layer, second half (model.py:69-70 / :90-91 / :115-116 / :149-150): the tap-GEMM left the per-tap
 // products D[b][iy][ix][tap*nc + c]; each output pixel sums the taps that land on it (fixed order), adds the bias
 // and applies tanh.   x_hat[b][c][oy][ox] = tanh(bias[c] + sum_{ky,kx} D[b][(oy+p-ky)/s][(ox+p-kx)/s][...])
@@ -188,7 +281,10 @@ template <int K, int S>
 __global__ void __launch_bounds__(256) last_gather_tanh_kernel(const float* __restrict__ d,
                                                                const float* __restrict__ bias,
                                                                float* __restrict__ xhat, int B, int nc, int img,
-                                                               int hin, int p, int n_pad, int to_unit_range) {
+                                                               int hin, int p, int n_pad, int to_unit_range,
+                                                               uint16_t* __restrict__ xhl, int kx) {
+  pdl_wait();
+  pdl_trigger();
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   const long long total = (long long)B * nc * img * img;
   if (i >= total) return;
@@ -214,22 +310,27 @@ __global__ void __launch_bounds__(256) last_gather_tanh_kernel(const float* __re
   const float t = tanhf(acc);
   // prior sampling (train.py:562, :573): to_range_0_1(x).clamp(0, 1) fused into the same store
   xhat[i] = to_unit_range ? fminf(fmaxf((t + 1.f) / 2.f, 0.f), 1.f) : t;
+  if (xhl) {
+    // the A operand of the measurement GEMM A x_hat: row b holds vec(x_hat_b) (NCHW order); |x_hat| <= 1 fits fp16
+    const long long n = (long long)nc * img * img;
+    uint16_t hi, lo;
+    split16(t, true, hi, lo);
+    uint16_t* row = xhl + (size_t)b * 2 * kx;
+    row[i - b * n] = hi;
+    row[kx + i - b * n] = lo;
+  }
 }
 
-int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s) {
+int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s, uint16_t* xhl) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const long long total = (long long)plan->cfg.batch * plan->cfg.nc * plan->img * plan->img;
   const float* d = (const float*)(plan->ws + plan->off_dlast);
   const float* bias = (const float*)(plan->ws + plan->off_bias[plan->n_layers - 1]);
   float* xh = out ? out : (float*)(plan->ws + plan->off_xhat);
   const unsigned blocks = (unsigned)((total + 255) / 256);
-  if (y.k == 3 && y.s == 1)
-    last_gather_tanh_kernel<3, 1><<<blocks, 256, 0, s>>>(d, bias, xh, plan->cfg.batch, plan->cfg.nc, plan->img, y.hin,
-                                                        y.p, plan->dlast_pad, to_unit_range);
-  else
-    last_gather_tanh_kernel<4, 2><<<blocks, 256, 0, s>>>(d, bias, xh, plan->cfg.batch, plan->cfg.nc, plan->img, y.hin,
-                                                        y.p, plan->dlast_pad, to_unit_range);
-  LSNF_CUDA(cudaGetLastError());
+  LSNF_CUDA(launch_k(y.k == 3 && y.s == 1 ? last_gather_tanh_kernel<3, 1> : last_gather_tanh_kernel<4, 2>, dim3(blocks),
+                     dim3(256), 0, s, d, bias, xh, plan->cfg.batch, plan->cfg.nc, plan->img, y.hin, y.p,
+                     plan->dlast_pad, to_unit_range, xhl, plan->meas_kx));
   return LSNF_OK;
 }
 
@@ -277,8 +378,11 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
                                                                 const float* __restrict__ mask,
                                                                 uint16_t* __restrict__ a, int B, int nc, int img,
                                                                 int hin, int k, int s, int p, float seed_scale,
-                                                                int fp16, int upstream) {
+                                                                int fp16, int upstream, const float* __restrict__ part,
+                                                                int nsplit, int pitch) {
   extern __shared__ float g[];   // [nc][k][span], span = (seg-1)*s + k
+  pdl_wait();
+  pdl_trigger();
   const int segs = (hin + IM2COL_SEG - 1) / IM2COL_SEG;
   const int seg = blockIdx.x % segs, iy = (blockIdx.x / segs) % hin, b = blockIdx.x / (segs * hin);
   const int ix0 = seg * IM2COL_SEG, nseg = min(IM2COL_SEG, hin - ix0);
@@ -291,7 +395,14 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
     if (oy >= 0 && oy < img && ox >= 0 && ox < img) {
       const size_t o = (((size_t)b * nc + c) * img + oy) * img + ox;
       const float xh = xhat[o];
-      float d = upstream ? x[o] : xh - x[o];
+      float d;
+      if (part) {   // dL/dx_hat = A^T r: its split-K partials summed in a fixed order
+        const size_t col = o - (size_t)b * nc * img * img;
+        d = 0.f;
+        for (int q = 0; q < nsplit; ++q) d += __ldcg(part + ((size_t)q * B + b) * pitch + col);
+      } else {
+        d = upstream ? x[o] : xh - x[o];
+      }
       if (mask) d = mask[o] * d;   // read only with upstream == 0 (the launcher passes null otherwise)
       v = d * seed_scale * (1.f - xh * xh);
     }
@@ -314,15 +425,15 @@ __global__ void __launch_bounds__(128) recon_grad_im2col_kernel(const float* __r
 }
 
 int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
-                             cudaStream_t s) {
+                             cudaStream_t s, const float* part, int nsplit, int pitch) {
   const auto& y = plan->layers[plan->n_layers - 1];
   const int segs = (y.hin + IM2COL_SEG - 1) / IM2COL_SEG;
   const int span = (std::min(IM2COL_SEG, y.hin) - 1) * y.s + y.k;
   const size_t smem = (size_t)plan->cfg.nc * y.k * span * 4;
-  recon_grad_im2col_kernel<<<plan->cfg.batch * y.hin * segs, 128, smem, s>>>(
-      (const float*)(plan->ws + plan->off_xhat), x, upstream ? nullptr : mask, (uint16_t*)(plan->ws + plan->off_im2col),
-      plan->cfg.batch, plan->cfg.nc, plan->img, y.hin, y.k, y.s, y.p, seed_scale, plan->cfg.bwd_passes == 1 ? 1 : 0, upstream);
-  LSNF_CUDA(cudaGetLastError());
+  LSNF_CUDA(launch_k(recon_grad_im2col_kernel, dim3(plan->cfg.batch * y.hin * segs), dim3(128), smem, s,
+                     (const float*)(plan->ws + plan->off_xhat), x, upstream ? nullptr : mask,
+                     (uint16_t*)(plan->ws + plan->off_im2col), plan->cfg.batch, plan->cfg.nc, plan->img, y.hin, y.k, y.s,
+                     y.p, seed_scale, plan->cfg.bwd_passes == 1 ? 1 : 0, upstream, part, nsplit, pitch));
   return LSNF_OK;
 }
 

@@ -100,6 +100,7 @@ struct StageHost {
   // cross8 stages: workspace offsets of the bf16 hi|lo gradient the conversion reads (the converted operand is at
   // info.a_offset) and of the two words [amax bits of that gradient, descale of the accumulator]
   size_t x8_src_off = 0, x8_off = 0;
+  int meas = 0;   // measurement-operator stage: 1 = A x_hat, 2 = A^T r (lsnf_config.meas_rows > 0); 0 otherwise
 };
 
 struct FlowLayout {
@@ -237,10 +238,10 @@ struct lsnf_plan {
   // ais_update_kernel reads it from dyn[3] under replay.  A Langevin loop keys with target = 0, an AIS loop
   // (lsnf_ais_run) with with_noise = 1, and `ais` keeps the two apart.
   struct LoopKey {
-    int steps; float step_size, sigma; int with_noise; bool masked, ais; float target;
+    int steps; float step_size, sigma; int with_noise; bool masked, ais; float target; bool measured;
     bool operator==(const LoopKey& o) const {
       return steps == o.steps && step_size == o.step_size && sigma == o.sigma && with_noise == o.with_noise &&
-             masked == o.masked && ais == o.ais && target == o.target;
+             masked == o.masked && ais == o.ais && target == o.target && measured == o.measured;
     }
   };
   struct LoopGraph { LoopKey key; cudaGraphExec_t exec; };
@@ -251,6 +252,13 @@ struct lsnf_plan {
   size_t off_ais_z = 0, off_ais_gr = 0, off_ais_gp = 0, off_ais_logw = 0, off_ais_scal = 0, off_ais_epart = 0,
          off_ais_logp = 0, off_ais_beta = 0;
   int fused_tiles = 0;   // CTAs of the fused last-layer kernel per sample
+  // linear measurements (meas_rows = m > 0): stages[2L] = A x_hat, stages[2L+1] = A^T r.  kx = n = nc*H*W and km = m,
+  // each rounded up to BLOCK_K, are the K extents of the two GEMMs; x_hat and r are stored as 16-bit hi|lo rows
+  // [B][2 kx] and [B][2 km]; y [B][m] is the graph-replayed loop's copy; epart [B][meas_tiles] the per-sample
+  // fixed-order partials of |r|^2; scale: |A|max bits, 2^k, 2^-k of the fp16 copy
+  int meas_m = 0, meas_kx = 0, meas_km = 0, meas_tiles = 0;
+  size_t off_meas_xhl = 0, off_meas_r = 0, off_meas_y = 0, off_meas_epart = 0, off_meas_scale = 0;
+  bool meas_packed = false;
   long long runs = 0;
   bool use_graphs = true;
 };
@@ -339,10 +347,17 @@ int launch_convert_fp8(const lsnf_plan* plan, const StageHost& st, cudaStream_t 
 int launch_pack_stage(const lsnf_plan* plan, const StageHost& st, const float* w, cudaStream_t s);
 int launch_split_z(const lsnf_plan* plan, const float* z, cudaStream_t s);
 int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cudaStream_t s);
-int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s);
-// mask (nullable): per-pixel likelihood weight [B,nc,H,W] of the loss-gradient seed (ignored with upstream != 0)
+// xhl (nullable): x_hat also as the fp16 hi|lo rows [B][2 meas_kx] of the measurement GEMM A x_hat
+int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cudaStream_t s, uint16_t* xhl = nullptr);
+// mask (nullable): per-pixel likelihood weight [B,nc,H,W] of the loss-gradient seed (ignored with upstream != 0).
+// part (nullable): dL/dx_hat is instead the sum of the nsplit fp32 split-K partials [nsplit][B][pitch] of A^T r
 int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
-                             cudaStream_t s);
+                             cudaStream_t s, const float* part = nullptr, int nsplit = 0, int pitch = 0);
+// A [m, n] -> the packed operands of the two measurement stages (after launch_meas_scale)
+int launch_meas_pack(const lsnf_plan* plan, const float* A, cudaStream_t s);
+// r = A x_hat - y from the split-K partials of stage 2L: bf16 hi|lo rows of r * seed_scale for stage 2L+1, and the
+// per-sample partials of |r|^2 into epart (nullable)
+int launch_meas_finish(const lsnf_plan* plan, const float* y, float seed_scale, float* epart, cudaStream_t s);
 // epart (nullable): [B][tiles] sum m (x_hat - x)^2 over the pixels each CTA owns (tiles = last_fused_tiles)
 int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float* epart, float seed_scale,
                       cudaStream_t s);

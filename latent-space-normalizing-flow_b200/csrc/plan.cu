@@ -194,6 +194,8 @@ static int check_config(lsnf_plan* p) {
     return fail(LSNF_ERR_UNSUPPORTED, "f_flow_coupling must be 0 or 1 (model.py:384-387)");
   if (c.gemm_impl != LSNF_GEMM_TCGEN05 && c.gemm_impl != LSNF_GEMM_SIMT) return fail(LSNF_ERR_INVALID, "bad gemm_impl");
   if (c.bwd_passes != 0 && c.bwd_passes != 1 && c.bwd_passes != 3) return fail(LSNF_ERR_INVALID, "bwd_passes must be 0, 1 or 3");
+  if (c.meas_rows < 0) return fail(LSNF_ERR_INVALID, "meas_rows must not be negative");
+  if (c.meas_rows > 0 && c.arch == LSNF_ARCH_NONE) return fail(LSNF_ERR_INVALID, "a measurement operator needs a generator");
 
   const int L = arch_layers(c, p->layers);
   if (L < 0) return fail(LSNF_ERR_INVALID, "unknown arch (model.py:154 raises ValueError)");
@@ -391,6 +393,16 @@ static void build_forward_stage(lsnf_plan* p, int l) {
   fill_dev(p, st);
 }
 
+// K splits of a split-K stage over `tiles` output tiles: about one wave of CTAs, at least two K blocks per split, and
+// every split non-empty
+static int split_count(int kblocks, int tiles) {
+  const int want = std::max(1, (148 + tiles - 1) / tiles);
+  int per = std::max(2, (kblocks + want - 1) / want);
+  const int s = (kblocks + per - 1) / per;
+  per = (kblocks + s - 1) / s;                            // what the kernels use (it_per_split)
+  return (kblocks + per - 1) / per;
+}
+
 // Data-gradient stage of layer l (train.py:314): stages[L + (L - 1 - l)], run from the last layer down to the first.
 // The first layer's stage writes split-K partials whose region lsnf_plan_create takes after all data-gradient stages.
 static void build_dgrad_stage(lsnf_plan* p, int l) {
@@ -417,13 +429,7 @@ static void build_dgrad_stage(lsnf_plan* p, int l) {
     I.n_taps[0] = 0;              // generated: tap t -> (dy, dx) = (t / k, t % k), B column offset t*co
     I.a_offset = p->off_gpre[0];
     b_rows = I.n_pad;
-    const int kblocks = y.k * y.k * y.co / BLOCK_K;
-    const int mtiles = (B + BLOCK_M - 1) / BLOCK_M;
-    int want = std::max(1, (148 + mtiles - 1) / mtiles);   // about one wave of CTAs
-    int per = std::max(2, (kblocks + want - 1) / want);
-    I.k_splits = (kblocks + per - 1) / per;
-    per = (kblocks + I.k_splits - 1) / I.k_splits;       // what the kernels use (it_per_split)
-    I.k_splits = (kblocks + per - 1) / per;               // every split is non-empty
+    I.k_splits = split_count(y.k * y.k * y.co / BLOCK_K, (B + BLOCK_M - 1) / BLOCK_M);
     p->ksplit_first = I.k_splits;
   } else {   // k4 s2 p1
     I.grid_h = I.grid_w = y.hin;
@@ -557,6 +563,46 @@ static void build_wgrad_layer(lsnf_plan* p, int l) {
   } else { r.nsel = 4; for (int q = 0; q < 4; ++q) r.sel[q] = 2 * q * y.co; }   // the as-is copy of every plane
 }
 
+// The two measurement-operator stages of a plan with meas_rows = m > 0, after every other region: stages[2L] = A x_hat
+// (M = B, N = m, K = n; fp16 operands, A scaled by a power of two) and stages[2L+1] = A^T r (M = B, N = n, K = m; bf16
+// operands).  Each is a plain GEMM over a flattened operand with split-K partials [S][B][n_pad] -- the kind of the
+// first layer's data-gradient stage with one generated tap of the whole K extent -- and with only one or a few
+// 128-row M tiles the K splits fill the SMs.
+static void take_meas_regions(lsnf_plan* p) {
+  const lsnf_config& c = p->cfg;
+  const int L = p->n_layers, B = c.batch, m = c.meas_rows, n = c.nc * p->img * p->img;
+  p->meas_m = m;
+  p->meas_kx = (int)align_up(n, BLOCK_K);
+  p->meas_km = (int)align_up(m, BLOCK_K);
+  p->meas_tiles = (m + 255) / 256;
+  p->off_meas_xhl = take(p, (size_t)B * 2 * p->meas_kx * 2);
+  p->off_meas_r = take(p, (size_t)B * 2 * p->meas_km * 2);
+  p->off_meas_y = take(p, (size_t)B * m * 4);
+  p->off_meas_epart = take(p, (size_t)B * p->meas_tiles * 4);
+  p->off_meas_scale = take(p, 16);
+  for (int which = 1; which <= 2; ++which) {
+    StageHost& st = p->stages[2 * L + which - 1];
+    memset(&st.info, 0, sizeof(st.info));
+    st.meas = which;
+    lsnf_stage_info& I = st.info;
+    I.kind = 3; I.layer = L - 1;
+    const int rows = which == 1 ? m : n, k = which == 1 ? p->meas_kx : p->meas_km;
+    I.grid_h = I.grid_w = 1;
+    I.k_per_tap = k;
+    I.n_valid = rows; I.block_n = 128; I.n_pad = (int)align_up(rows, 128);
+    I.n_phases = 1; I.n_taps[0] = 0; I.out_mul = 1; I.out_channels = I.n_pad; I.epilogue = EPI_PARTIAL;
+    I.a_planes = 1; I.a_h = I.a_w = 1; I.tap_gen_k = 1; I.b_k = k; I.b_rows = I.n_pad;
+    I.operand_fp16 = which == 1 ? 1 : 0; I.passes = 3;
+    make_box(1, 1, &I.box_b, &I.box_h, &I.box_w);
+    I.k_splits = split_count(k / BLOCK_K, ((B + BLOCK_M - 1) / BLOCK_M) * (I.n_pad / I.block_n));
+    I.a_offset = which == 1 ? p->off_meas_xhl : p->off_meas_r;
+    I.b_offset = take(p, (size_t)I.b_rows * 2 * k * 2);
+    I.out_offset = take(p, (size_t)I.k_splits * B * I.n_pad * 4);
+    I.flops = 2LL * B * m * (long long)n;
+    fill_dev(p, st);
+  }
+}
+
 // Annealed importance sampling (lsnf_ais_run): chain state and energies, after every other region.
 static void take_ais_regions(lsnf_plan* p) {
   const int B = p->cfg.batch, nz = p->cfg.nz;
@@ -598,6 +644,10 @@ extern "C" int lsnf_plan_create(const lsnf_config* cfg, lsnf_plan** out) {
       for (int l = 0; l < L; ++l) build_wgrad_layer(p.get(), l);
     }
     take_ais_regions(p.get());
+    if (p->cfg.meas_rows > 0) {
+      p->stages.resize(2 * L + 2);
+      take_meas_regions(p.get());
+    }
   }
   *out = p.release();
   return LSNF_OK;
@@ -687,6 +737,7 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
     const bool feeds8 = i + 1 < plan->stages.size() && plan->stages[i + 1].dev.cross8;
     d.amax_out = feeds8 ? (uint32_t*)(plan->ws + plan->stages[i + 1].x8_off) : nullptr;
     d.mbits = ((I.kind == 0 && !st.last) || (I.kind == 1 && !st.first)) ? (uint32_t*)(plan->ws + st.mbits_off) : nullptr;
+    if (st.meas) d.descale = st.meas == 1 ? (const float*)(plan->ws + plan->off_meas_scale + 8) : nullptr;
     int rc = bind_stage(plan, st, plan->cfg.gemm_impl == LSNF_GEMM_TCGEN05);
     if (rc) return rc;
   }
@@ -712,7 +763,7 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
     plan->use_graphs = !(e && e[0] == '1');
   }
   plan->bound = true;
-  plan->g_packed = plan->f_packed = false;
+  plan->g_packed = plan->f_packed = plan->meas_packed = false;
   return LSNF_OK;
 }
 
@@ -749,6 +800,7 @@ extern "C" int lsnf_pack_generator_weights(lsnf_plan* plan, const float* const* 
     if (rc) return rc;
   }
   for (auto& st : plan->stages) {
+    if (st.meas) continue;   // packed by lsnf_pack_measurement
     int rc = launch_pack_stage(plan, st, weights[st.info.layer], s);
     if (rc) return rc;
     // a cross8 stage's input amax starts at 0; from then on the stage zeroes it after each conversion
@@ -791,7 +843,8 @@ static int gen_forward(lsnf_plan* p, const float* z, float* x_hat, cudaStream_t 
   if (split && (rc = launch_split_z(p, z, s))) return rc;
   for (int l = 0; l < p->n_layers; ++l)
     if ((rc = run_stage(p, p->stages[l], s))) return rc;
-  if ((rc = launch_last_gather(p, nullptr, 0, s))) return rc;
+  uint16_t* xhl = p->meas_m ? (uint16_t*)(p->ws + p->off_meas_xhl) : nullptr;   // for lsnf_generator_dgrad_measured
+  if ((rc = launch_last_gather(p, nullptr, 0, s, xhl))) return rc;
   if (x_hat) {
     const size_t bytes = (size_t)p->cfg.batch * p->cfg.nc * p->img * p->img * 4;
     LSNF_CUDA(cudaMemcpyAsync(x_hat, p->ws + p->off_xhat, bytes, cudaMemcpyDeviceToDevice, s));
@@ -805,6 +858,53 @@ static int gen_dgrad_partial(lsnf_plan* p, const float* x, const float* mask, fl
   for (int i = p->n_layers; i < 2 * p->n_layers; ++i)
     if ((rc = run_dgrad_stage(p, p->stages[i], s))) return rc;
   return LSNF_OK;
+}
+
+// Loss-gradient seed of a measured iteration, from the last forward stage's per-tap products: x_hat (with its fp16 rows),
+// A x_hat, r = A x_hat - y (and the |r|^2 partials into epart, nullable), A^T r, and the last layer's im2col seed
+// A^T r (1 - x_hat^2).  r carries seed_scale, the share of 1/sigma^2 kept in the 16-bit tensors.
+static int meas_seed(const lsnf_plan* p, const float* y, float* epart, float seed_scale, cudaStream_t s) {
+  const int L = p->n_layers;
+  const StageHost& bw = p->stages[2 * L + 1];
+  int rc;
+  if ((rc = launch_last_gather(p, nullptr, 0, s, (uint16_t*)(p->ws + p->off_meas_xhl))) ||
+      (rc = run_stage(p, p->stages[2 * L], s)) || (rc = launch_meas_finish(p, y, seed_scale, epart, s)) ||
+      (rc = run_stage(p, bw, s)))
+    return rc;
+  return launch_recon_grad_im2col(p, nullptr, nullptr, 1.f, 1, s, (const float*)(p->ws + bw.info.out_offset),
+                                  bw.info.k_splits, bw.info.n_pad);
+}
+
+// The measured entry points' own conditions (after need()).
+static int need_measured(const lsnf_plan* p) {
+  if (p->cfg.meas_rows == 0) return fail(LSNF_ERR_UNSUPPORTED, "plan was created without lsnf_config.meas_rows");
+  if (p->cfg.bwd_passes == 1)
+    return fail(LSNF_ERR_UNSUPPORTED, "measurements need the 3-pass bf16 data gradient (bwd_passes 1 writes an fp16 "
+                                      "seed, and A^T r has no bounded range)");
+  if (!p->meas_packed) return fail(LSNF_ERR_INVALID, "no measurement operator packed (lsnf_pack_measurement)");
+  return LSNF_OK;
+}
+
+extern "C" int lsnf_pack_measurement(lsnf_plan* plan, const float* A, lsnf_stream stream) {
+  if (!plan || !plan->bound) return fail(LSNF_ERR_STATE, "plan not bound");
+  if (plan->cfg.meas_rows == 0) return fail(LSNF_ERR_UNSUPPORTED, "plan was created without lsnf_config.meas_rows");
+  if (!A) return fail(LSNF_ERR_INVALID, "null operator");
+  int rc = launch_meas_pack(plan, A, (cudaStream_t)stream);
+  if (rc) return rc;
+  plan->meas_packed = true;
+  return LSNF_OK;
+}
+
+extern "C" int lsnf_generator_dgrad_measured(lsnf_plan* plan, const float* y, float sigma, float* grad_z,
+                                             lsnf_stream stream) {
+  int rc = need(plan, true, false);
+  if (rc || (rc = need_measured(plan))) return rc;
+  if (!y || !grad_z || !(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "bad argument");
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = meas_seed(plan, y, nullptr, sigma_seed_scale(sigma), s))) return rc;
+  for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i)
+    if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
+  return launch_reduce_partial(plan, grad_z, sigma_post_scale(sigma), s);
 }
 
 extern "C" int lsnf_plan_run_stage(lsnf_plan* plan, int32_t index, lsnf_stream stream) {
@@ -1099,8 +1199,8 @@ struct LoopTrace {
 
 // With `ais` (lsnf_ais_run) the same stages also write the per-tile energy partials and log p(z), and the iteration
 // ends with the AIS update instead of the Langevin update.
-static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int steps, float step_size, float sigma,
-                         int with_noise,
+static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, bool measured, int steps, float step_size,
+                         float sigma, int with_noise,
                          const float* eps, uint64_t seed, uint64_t sample_offset, const uint64_t* dyn, float* gnorms,
                          cudaStream_t s, const AisArgs* ais) {
   const float gscale = sigma_post_scale(sigma);
@@ -1141,9 +1241,12 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
     }
     {
       PdlScope pdl(use_pdl);
-      if ((rc = launch_last_fused(plan, x, mask, ais ? ais->epart : nullptr, sigma_seed_scale(sigma), s))) return rc;
+      float* epart = ais ? ais->epart : nullptr;
+      if ((rc = measured ? meas_seed(plan, x, epart, sigma_seed_scale(sigma), s)
+                         : launch_last_fused(plan, x, mask, epart, sigma_seed_scale(sigma), s)))
+        return rc;
     }
-    tr.mark("gather + tanh + recon grad + im2col");
+    tr.mark(measured ? "gather + tanh + A x_hat + r + A^T r + im2col" : "gather + tanh + recon grad + im2col");
     for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i) {
       {
         PdlScope pdl(use_pdl);
@@ -1172,23 +1275,23 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, int
 // graph_chunk iterations: one graph per chunk length, the index of a chunk's first iteration (Philox counter) read
 // from device memory, so test mode's 8 000-step chains (train.py:606) reuse one 40-iteration graph 200 times instead
 // of instantiating 88 000 kernel nodes.  Graphs read the workspace copies of x and the mask, and an AIS graph that of
-// its chunk's schedule values, which are staged before each replay.
-static int run_chain(lsnf_plan* plan, const float* x, const float* mask, int iters, float step_size, float sigma,
-                     int with_noise, const float* eps, uint64_t seed, uint64_t sample_offset, float* gnorms,
-                     cudaStream_t s, const AisArgs* ais = nullptr) {
+// its chunk's schedule values, which are staged before each replay.  With `measured`, x is y [B][m].
+static int run_chain(lsnf_plan* plan, const float* x, const float* mask, bool measured, int iters, float step_size,
+                     float sigma, int with_noise, const float* eps, uint64_t seed, uint64_t sample_offset,
+                     float* gnorms, cudaStream_t s, const AisArgs* ais = nullptr) {
   const bool injected = eps || (ais && (ais->eps || ais->u));
   const bool graph_ok = plan->use_graphs && !injected && iters > 0 && plan->runs > 0;
   plan->runs++;
   if (!graph_ok)
-    return langevin_loop(plan, x, mask, iters, step_size, sigma, with_noise, eps, seed, sample_offset, nullptr, gnorms,
-                         s, ais);
+    return langevin_loop(plan, x, mask, measured, iters, step_size, sigma, with_noise, eps, seed, sample_offset,
+                         nullptr, gnorms, s, ais);
   const lsnf_config& c = plan->cfg;
-  float* x_ws = (float*)(plan->ws + plan->off_x);
+  float* x_ws = (float*)(plan->ws + (measured ? plan->off_meas_y : plan->off_x));
   float* mask_ws = mask ? (float*)(plan->ws + plan->off_mask) : nullptr;
   float* gn_ws = (float*)(plan->ws + plan->off_gnorms);
   float* beta_ws = (float*)(plan->ws + plan->off_ais_beta);
   const uint64_t* dyn = (const uint64_t*)(plan->ws + plan->off_dyn);
-  const size_t xbytes = (size_t)c.batch * c.nc * plan->img * plan->img * 4;
+  const size_t xbytes = (size_t)c.batch * (measured ? plan->meas_m : c.nc * plan->img * plan->img) * 4;
   LSNF_CUDA(cudaMemcpyAsync(x_ws, x, xbytes, cudaMemcpyDeviceToDevice, s));
   if (mask) LSNF_CUDA(cudaMemcpyAsync(mask_ws, mask, xbytes, cudaMemcpyDeviceToDevice, s));
   AisArgs ag = {};
@@ -1197,7 +1300,7 @@ static int run_chain(lsnf_plan* plan, const float* x, const float* mask, int ite
   for (int done = 0; done < iters;) {
     const int n = std::min(iters - done, graph_chunk);
     const lsnf_plan::LoopKey key = {n, step_size, sigma, with_noise, mask != nullptr, ais != nullptr,
-                                    ais ? ais->target : 0.f};
+                                    ais ? ais->target : 0.f, measured};
     cudaGraphExec_t exec = nullptr;
     for (auto& g : plan->graphs)
       if (g.key == key) exec = g.exec;
@@ -1205,7 +1308,7 @@ static int run_chain(lsnf_plan* plan, const float* x, const float* mask, int ite
       cudaGraph_t graph = nullptr;
       cudaStream_t cs = plan->cap_stream;
       LSNF_CUDA(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-      rc = langevin_loop(plan, x_ws, mask_ws, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs,
+      rc = langevin_loop(plan, x_ws, mask_ws, measured, n, step_size, sigma, with_noise, nullptr, 0, 0, dyn, gn_ws, cs,
                          ais ? &ag : nullptr);
       cudaError_t ce = cudaStreamEndCapture(cs, &graph);
       if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
@@ -1228,12 +1331,11 @@ static int run_chain(lsnf_plan* plan, const float* x, const float* mask, int ite
   return LSNF_OK;
 }
 
-extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const float* x, const float* mask,
-                                        int32_t steps, float step_size, float sigma, int32_t with_noise,
-                                        const float* eps, uint64_t seed, uint64_t sample_offset, float* z_out,
-                                        float* gnorms, lsnf_stream stream) {
+static int langevin_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, bool measured,
+                        int32_t steps, float step_size, float sigma, int32_t with_noise, const float* eps,
+                        uint64_t seed, uint64_t sample_offset, float* z_out, float* gnorms, lsnf_stream stream) {
   int rc = need(plan, true, true);
-  if (rc) return rc;
+  if (rc || (measured && (rc = need_measured(plan)))) return rc;
   if (!z0 || !x || !z_out || steps < 0 || !(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "bad argument");
   cudaStream_t s = (cudaStream_t)stream;
   const lsnf_config& c = plan->cfg;
@@ -1241,10 +1343,27 @@ extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const 
   const size_t zbytes = (size_t)c.batch * c.nz * 4;
   LSNF_CUDA(cudaMemcpyAsync(z, z0, zbytes, cudaMemcpyDeviceToDevice, s));
   if ((rc = launch_split_z(plan, z, s))) return rc;
-  if ((rc = run_chain(plan, x, mask, steps, step_size, sigma, with_noise, eps, seed, sample_offset, gnorms, s)))
+  if ((rc = run_chain(plan, x, mask, measured, steps, step_size, sigma, with_noise, eps, seed, sample_offset, gnorms,
+                      s)))
     return rc;
   LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
   return LSNF_OK;
+}
+
+extern "C" int lsnf_langevin_run_masked(lsnf_plan* plan, const float* z0, const float* x, const float* mask,
+                                        int32_t steps, float step_size, float sigma, int32_t with_noise,
+                                        const float* eps, uint64_t seed, uint64_t sample_offset, float* z_out,
+                                        float* gnorms, lsnf_stream stream) {
+  return langevin_run(plan, z0, x, mask, false, steps, step_size, sigma, with_noise, eps, seed, sample_offset, z_out,
+                      gnorms, stream);
+}
+
+extern "C" int lsnf_langevin_run_measured(lsnf_plan* plan, const float* z0, const float* y, int32_t steps,
+                                          float step_size, float sigma, int32_t with_noise, const float* eps,
+                                          uint64_t seed, uint64_t sample_offset, float* z_out, float* gnorms,
+                                          lsnf_stream stream) {
+  return langevin_run(plan, z0, y, nullptr, true, steps, step_size, sigma, with_noise, eps, seed, sample_offset, z_out,
+                      gnorms, stream);
 }
 
 extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* x, int32_t steps, float step_size,
@@ -1254,12 +1373,12 @@ extern "C" int lsnf_langevin_run(lsnf_plan* plan, const float* z0, const float* 
                                   z_out, gnorms, stream);
 }
 
-extern "C" int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, const float* betas,
-                            int32_t steps, float step_size, float target_accept, float sigma, const float* eps,
-                            const float* u, uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w,
-                            float* accept_rate, lsnf_stream stream) {
+static int ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, bool measured,
+                   const float* betas, int32_t steps, float step_size, float target_accept, float sigma, const float* eps,
+                   const float* u, uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w, float* accept_rate,
+                   lsnf_stream stream) {
   int rc = need(plan, true, true);
-  if (rc) return rc;
+  if (rc || (measured && (rc = need_measured(plan)))) return rc;
   if (!z0 || !x || !betas || !z_out || !log_w || !accept_rate) return fail(LSNF_ERR_INVALID, "null argument");
   if (steps < 1) return fail(LSNF_ERR_INVALID, "steps must be at least 1");
   if (!(sigma > 0.f)) return fail(LSNF_ERR_INVALID, "sigma must be positive");
@@ -1277,17 +1396,34 @@ extern "C" int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, co
   a.gp = (float*)(plan->ws + plan->off_ais_gp);
   a.scal = (float*)(plan->ws + plan->off_ais_scal);
   a.logw = (double*)(plan->ws + plan->off_ais_logw);
-  a.epart = (float*)(plan->ws + plan->off_ais_epart);
+  a.epart = (float*)(plan->ws + (measured ? plan->off_meas_epart : plan->off_ais_epart));
   a.logp = (float*)(plan->ws + plan->off_ais_logp);
   a.betas = betas; a.eps = eps; a.u = u;
-  a.tiles = plan->fused_tiles; a.total = steps;
+  a.tiles = measured ? plan->meas_tiles : plan->fused_tiles; a.total = steps;
   a.step0 = step_size; a.target = target_accept > 0.f ? target_accept : 0.f;
   a.inv2s2 = 0.5f / (sigma * sigma);
   // steps + 1 iterations: iteration 0 only initialises and proposes, the last one only decides
-  if ((rc = run_chain(plan, x, mask, steps + 1, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, s, &a)))
+  if ((rc = run_chain(plan, x, mask, measured, steps + 1, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, s,
+                      &a)))
     return rc;
   LSNF_CUDA(cudaMemcpyAsync(z_out, z, zbytes, cudaMemcpyDeviceToDevice, s));
   LSNF_CUDA(cudaMemcpyAsync(log_w, a.scal + 5 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
   LSNF_CUDA(cudaMemcpyAsync(accept_rate, a.scal + 6 * B, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
   return LSNF_OK;
+}
+
+extern "C" int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* mask, const float* betas,
+                            int32_t steps, float step_size, float target_accept, float sigma, const float* eps,
+                            const float* u, uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w,
+                            float* accept_rate, lsnf_stream stream) {
+  return ais_run(plan, z0, x, mask, false, betas, steps, step_size, target_accept, sigma, eps, u, seed, sample_offset,
+                 z_out, log_w, accept_rate, stream);
+}
+
+extern "C" int lsnf_ais_run_measured(lsnf_plan* plan, const float* z0, const float* y, const float* betas,
+                                     int32_t steps, float step_size, float target_accept, float sigma, const float* eps,
+                                     const float* u, uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w,
+                                     float* accept_rate, lsnf_stream stream) {
+  return ais_run(plan, z0, y, nullptr, true, betas, steps, step_size, target_accept, sigma, eps, u, seed,
+                 sample_offset, z_out, log_w, accept_rate, stream);
 }

@@ -28,7 +28,9 @@ def langevin_sharded(z_global, x_global, netG, netF, args, *, seed: int, rank: i
     split-K / stream-K cut points depend on the tile count).  Returns (z_shard or gathered z, |grad_g|, |grad_f|)
     with the two diagnostics averaged over the global batch when ``gather``.  ``mask`` (per-pixel likelihood weight of
     the global batch, ``plan.as_mask``) is sharded like x; a mask without a batch axis of the global batch's size
-    (e.g. [1,1,H,W] or [H,W]) is shared by every sample and passed to each rank whole."""
+    (e.g. [1,1,H,W] or [H,W]) is shared by every sample and passed to each rank whole.  With a measurement
+    ``operator`` A [m, n] in ``kw``, x_global is y [B, m]: its rows are sharded like x's and A goes to every rank
+    whole."""
     from .langevin import sample_langevin_post_z_with_flow
     rank = dist.get_rank() if rank is None else rank
     world = dist.get_world_size() if world is None else world

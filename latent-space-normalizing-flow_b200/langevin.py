@@ -9,7 +9,7 @@ from typing import Optional
 import torch
 
 from .model import _get, _netF, _netG
-from .plan import default_bwd_passes, get_plan
+from .plan import as_measurements, default_bwd_passes, get_plan
 
 _call_counter = itertools.count()
 
@@ -33,19 +33,22 @@ def make_args(**overrides) -> AttrDict:
     return a
 
 
-def langevin_plan(netG: _netG, netF: _netF, batch: int, device, bwd_passes: Optional[int] = None, train: bool = False):
+def langevin_plan(netG: _netG, netF: _netF, batch: int, device, bwd_passes: Optional[int] = None, train: bool = False,
+                  meas_rows: int = 0):
     """The plan (workspace, packed parameters, CUDA graphs) of one (netG, netF, batch) configuration; ``train=True``
-    adds the buffers of the generator parameter update so that one plan serves a whole training iteration."""
+    adds the buffers of the generator parameter update so that one plan serves a whole training iteration, and
+    ``meas_rows`` = m > 0 those of a linear measurement operator with m rows."""
     return get_plan(arch=netG.dataset, batch=batch, nz=netG.nz, ngf=netG.ngf, nc=netG.nc, f_depth=netF.f_depth,
                     f_width=netF.f_width, f_permutation=netF.f_permutation, f_coupling=netF.f_coupling,
-                    leak=netG.leak, device=device, gemm_impl=netG.gemm_impl, bwd_passes=bwd_passes, train=train)
+                    leak=netG.leak, device=device, gemm_impl=netG.gemm_impl, bwd_passes=bwd_passes, train=train,
+                    meas_rows=meas_rows)
 
 
 def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbose: bool = False, *,
                                      eps: Optional[torch.Tensor] = None, steps: Optional[int] = None,
                                      with_noise: Optional[bool] = None, seed: Optional[int] = None,
                                      sample_offset: int = 0, bwd_passes: Optional[int] = None, train: bool = False,
-                                     mask: Optional[torch.Tensor] = None):
+                                     mask: Optional[torch.Tensor] = None, operator: Optional[torch.Tensor] = None):
     """z [B,nz,1,1], x [B,nc,H,W] -> (z_k [B,nz,1,1], mean_b|grad_g|, mean_b|grad_f|) as train.py:335 returns them.
 
     ``args`` supplies g_l_steps, g_l_step_size, g_l_with_noise, g_llhd_sigma (train.py:311-326).  ``eps``
@@ -59,7 +62,14 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
     becomes 1/(2 sigma^2) sum m (G(z) - x)^2 - log p(z), with 1 = observed, 0 = missing and fractions in [0, 1]
     allowed.  Any shape that broadcasts to x's, any real or bool dtype (``plan.as_mask``).  |grad_g| is then the
     norm of the masked gradient.
+    ``operator``: a dense linear measurement operator A [m, nc*H*W] (``plan.as_operator``).  The second argument is
+    then y [B, m], the measurements y = A vec(x) + sigma noise (vec = x.view(B, -1)), and the energy
+    |A vec(G(z)) - y|^2 / (2 sigma^2) - log p(z): super-resolution, deblurring, compressed sensing.  A is packed once
+    per tensor version.  ``mask`` and ``operator`` together raise ValueError (a mask is the operator of the observed
+    pixels' identity rows).
     """
+    if mask is not None and operator is not None:
+        raise ValueError("pass either mask or operator, not both (a mask is the operator of its observed pixels)")
     if not isinstance(netG, _netG) or not isinstance(netF, _netF):
         raise TypeError("netG / netF must be lsnf_b200._netG / _netF instances")
     if not (z.is_cuda and x.is_cuda):
@@ -72,7 +82,10 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
     sigma = float(_get(args, "g_llhd_sigma", 0.3))
     noise = bool(_get(args, "g_l_with_noise", True)) if with_noise is None else bool(with_noise)
     z2 = z.detach().reshape(B, netG.nz).contiguous().float()
-    xx = x.detach().contiguous().float()
+    if operator is not None:
+        xx = as_measurements(x, operator, B)
+    else:
+        xx = x.detach().contiguous().float()
     e = None
     if eps is not None:
         e = eps.detach().reshape(T, B, netG.nz).contiguous().float()
@@ -81,11 +94,17 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
     noisy = noise or eps is not None
     if bwd_passes is None:
         bwd_passes = default_bwd_passes(noisy_chain=noisy)
-    plan = langevin_plan(netG, netF, B, z2.device, bwd_passes, train=train)
+    plan = langevin_plan(netG, netF, B, z2.device, bwd_passes, train=train,
+                         meas_rows=int(operator.shape[0]) if operator is not None else 0)
     plan.ensure_generator(netG)
     plan.ensure_flow(netF)
-    out, norms = plan.langevin_run(z2, xx, T, s, sigma, with_noise=noise, eps=e, seed=seed,
-                                   sample_offset=sample_offset, mask=mask)
+    if operator is not None:
+        plan.ensure_operator(operator)
+        out, norms = plan.langevin_run_measured(z2, xx, T, s, sigma, with_noise=noise, eps=e, seed=seed,
+                                                sample_offset=sample_offset)
+    else:
+        out, norms = plan.langevin_run(z2, xx, T, s, sigma, with_noise=noise, eps=e, seed=seed,
+                                       sample_offset=sample_offset, mask=mask)
     if verbose:
         print("Langevin posterior: z_grad_g_grad_norm={:8.3f}, z_grad_f_grad_norm={:8.3f}".format(
             norms[0].item(), norms[1].item()))
@@ -94,16 +113,17 @@ def sample_langevin_post_z_with_flow(z, x, netG: _netG, netF: _netF, args, verbo
 
 def make_sampler(args, test_mode: bool = False):
     """Closure with the reference's exact signature ``f(z, x, netG, netF, verbose=False)``, plus the keyword-only
-    ``mask`` of ``sample_langevin_post_z_with_flow``.
+    ``mask`` and ``operator`` of ``sample_langevin_post_z_with_flow``.
 
     ``test_mode=True`` reproduces the test variant: ``g_l_steps * 20`` iterations and no noise
     (train.py:606, :623-625)."""
-    def sampler(z, x, netG, netF, verbose=False, *, mask=None):
+    def sampler(z, x, netG, netF, verbose=False, *, mask=None, operator=None):
+        kw = {} if operator is None else {"operator": operator}
         if test_mode:
             return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose,
                                                     steps=int(_get(args, "g_l_steps", 20)) * 20, with_noise=False,
-                                                    mask=mask)
-        return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose, mask=mask)
+                                                    mask=mask, **kw)
+        return sample_langevin_post_z_with_flow(z, x, netG, netF, args, verbose, mask=mask, **kw)
     return sampler
 
 

@@ -67,19 +67,54 @@ def as_mask(mask, x: torch.Tensor) -> torch.Tensor:
     return mask.detach().to(torch.float32).expand(x.shape).contiguous()
 
 
+def as_operator(A, x_shape) -> torch.Tensor:
+    """The dense linear measurement operator ``A`` [m, n] of y = A vec(x) + noise as the library reads it: a contiguous
+    fp32 CUDA matrix whose columns match the images, n = nc*H*W for x of shape ``x_shape`` ([B,nc,H,W] or [nc,H,W];
+    vec is x.view(B, -1), NCHW order).  Raises TypeError for a non-tensor, ValueError for a matrix that is not 2-D, has
+    the wrong column count, a dtype that does not cast to fp32 (complex) or a non-finite value, and RuntimeError for a
+    CPU tensor.  Heteroscedastic noise: scale row i of A and of y by sigma / sigma_i."""
+    if not isinstance(A, torch.Tensor):
+        raise TypeError("operator must be a torch.Tensor")
+    n = 1
+    for d in tuple(x_shape)[-3:]:
+        n *= int(d)
+    if A.dim() != 2:
+        raise ValueError(f"operator must be a 2-D matrix [m, n] (got shape {tuple(A.shape)})")
+    if A.shape[1] != n or A.shape[0] < 1:
+        raise ValueError(f"operator of shape {tuple(A.shape)} does not act on images of {n} = nc*H*W values")
+    if A.is_complex() or A.dtype == torch.bool:
+        raise ValueError(f"operator of dtype {A.dtype} does not cast to float32")
+    if A.device.type != "meta" and not bool(torch.isfinite(A).all()):
+        raise ValueError("operator has non-finite values")
+    if A.device.type == "cpu":
+        raise RuntimeError("operator must be a CUDA tensor: the Langevin path has no CPU fallback")
+    return A.detach().to(torch.float32).contiguous()
+
+
+def as_measurements(y, A: torch.Tensor, batch: int) -> torch.Tensor:
+    """``y`` [batch, m] for the operator A [m, n] as an fp32 contiguous tensor; ValueError for another shape."""
+    if not isinstance(y, torch.Tensor):
+        raise TypeError("y must be a torch.Tensor")
+    if tuple(y.shape) != (int(batch), int(A.shape[0])):
+        raise ValueError(f"y has shape {tuple(y.shape)}, expected [B, m] = {(int(batch), int(A.shape[0]))}")
+    return y.detach().to(torch.float32).contiguous()
+
+
 class Plan:
     def __init__(self, *, arch: str, batch: int, nz: int, ngf: int, nc: int, f_depth: int, f_width: int,
                  f_permutation: int, f_coupling: int, leak: float, device, gemm_impl: int = _cabi.GEMM_TCGEN05,
-                 bwd_passes: int = 0, train: bool = False):
+                 bwd_passes: int = 0, train: bool = False, meas_rows: int = 0):
         self.lib = _cabi.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("lsnf_b200 plans live on a CUDA device; there is no CPU fallback")
         self.cfg = _cabi.Config(arch=_cabi.ARCH[arch], batch=batch, nz=nz, ngf=ngf, nc=nc, f_depth=f_depth,
                                 f_width=f_width, f_permutation=f_permutation, f_coupling=f_coupling, leak=leak,
-                                gemm_impl=gemm_impl, bwd_passes=bwd_passes, train=int(bool(train)))
+                                gemm_impl=gemm_impl, bwd_passes=bwd_passes, train=int(bool(train)),
+                                meas_rows=int(meas_rows))
         self.arch, self.batch, self.nz, self.nc = arch, batch, nz, nc
         self.train = bool(train)
+        self.meas_rows = int(meas_rows)
         self.f_depth, self.f_permutation = f_depth, f_permutation
         handle = C.c_void_p()
         _cabi.check(self.lib.lsnf_plan_create(C.byref(self.cfg), C.byref(handle)), "lsnf_plan_create")
@@ -93,6 +128,7 @@ class Plan:
         self._g_sig = None
         self._f_sig = None
         self._f_has_inv = False
+        self._a_sig = None
         self._keep = []  # tensors referenced by in-flight pack kernels
         # bumped by every call that overwrites the generator activations in the workspace (and by a re-pack, which
         # makes them stale): a backward pass that finds it moved re-runs its forward pass before lsnf_generator_vjp
@@ -210,6 +246,22 @@ class Plan:
             self._keep = keep
         self._f_sig = sig
         self._f_has_inv = need_inverse or self.f_permutation != 2
+
+    def ensure_operator(self, A: torch.Tensor) -> None:
+        """Pack the measurement operator A [meas_rows, nc*H*W] (``as_operator``) unless this very tensor, at the same
+        storage and version, is already packed: an in-place edit of A (which bumps its version) is repacked."""
+        if self._same(self._a_sig, [A]):
+            return
+        sig = self._sig([A])
+        a = as_operator(A, (self.nc, self.img, self.img))
+        if a.shape[0] != self.meas_rows or a.device != self.device:
+            raise ValueError(f"operator of shape {tuple(a.shape)} on {a.device} does not fit this plan "
+                             f"(meas_rows {self.meas_rows}, {self.device})")
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_pack_measurement(self.handle, a.data_ptr(), C.c_void_p(_stream(self.device))),
+                        "lsnf_pack_measurement")
+        self._keep_a = a   # read by the pack kernels in flight
+        self._a_sig = sig
 
     # ---- compute -------------------------------------------------------------------------------------
     def generator_forward(self, z: torch.Tensor) -> torch.Tensor:
@@ -397,6 +449,34 @@ class Plan:
                 "lsnf_langevin_run_masked")
         return out, norms
 
+    def langevin_run_measured(self, z0, y, steps, step_size, sigma, with_noise=True, eps=None, seed=0,
+                              sample_offset=0):
+        """``steps`` Langevin iterations from z0 on |A vec(G(z)) - y|^2 / (2 sigma^2) - log p(z) with the operator of
+        the last ``ensure_operator``; y [B, meas_rows].  Returns (z_T, [mean |grad_g|, mean |grad_f|])."""
+        _check_tensor(z0, "z", self.device, (self.batch, self.nz))
+        _check_tensor(y, "y", self.device, (self.batch, self.meas_rows))
+        if eps is not None:
+            _check_tensor(eps, "eps", self.device, (steps, self.batch, self.nz))
+        out = torch.empty_like(z0)
+        norms = torch.zeros(2, dtype=torch.float32, device=self.device)
+        self.act_epoch += 1
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_langevin_run_measured(
+                self.handle, z0.data_ptr(), y.data_ptr(), int(steps), float(step_size), float(sigma),
+                int(bool(with_noise)), eps.data_ptr() if eps is not None else None, int(seed) & (2 ** 64 - 1),
+                int(sample_offset), out.data_ptr(), norms.data_ptr(), _stream(self.device)),
+                "lsnf_langevin_run_measured")
+        return out, norms
+
+    def generator_dgrad_measured(self, y: torch.Tensor, sigma: float) -> torch.Tensor:
+        """d/dz [|A vec(G(z)) - y|^2 / (2 sigma^2)] at the z of the last ``generator_forward``."""
+        _check_tensor(y, "y", self.device, (self.batch, self.meas_rows))
+        g = torch.empty(self.batch, self.nz, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_generator_dgrad_measured(self.handle, y.data_ptr(), float(sigma), g.data_ptr(),
+                                                               _stream(self.device)), "lsnf_generator_dgrad_measured")
+        return g
+
     def ais_run(self, z0, x, betas, steps, step_size, sigma, *, target_accept: float = 0.0,
                 mask: Optional[torch.Tensor] = None, eps: Optional[torch.Tensor] = None,
                 u: Optional[torch.Tensor] = None, seed: int = 0, sample_offset: int = 0):
@@ -426,6 +506,30 @@ class Plan:
                 _stream(self.device)), "lsnf_ais_run")
         return z_out, log_w, rate
 
+    def ais_run_measured(self, z0, y, betas, steps, step_size, sigma, *, target_accept: float = 0.0,
+                         eps: Optional[torch.Tensor] = None, u: Optional[torch.Tensor] = None, seed: int = 0,
+                         sample_offset: int = 0):
+        """``ais_run`` on pi_beta(z) ~ p(z) exp(-beta |A vec(G(z)) - y|^2 / (2 sigma^2)), y [B, meas_rows], with the
+        operator of the last ``ensure_operator``.  log w is without -(m/2) log(2 pi sigma^2)."""
+        _check_tensor(z0, "z", self.device, (self.batch, self.nz))
+        _check_tensor(y, "y", self.device, (self.batch, self.meas_rows))
+        _check_tensor(betas, "betas", self.device, (int(steps) + 1,))
+        if eps is not None:
+            _check_tensor(eps, "eps", self.device, (steps, self.batch, self.nz))
+        if u is not None:
+            _check_tensor(u, "u", self.device, (steps, self.batch))
+        z_out = torch.empty_like(z0)
+        log_w = torch.empty(self.batch, dtype=torch.float32, device=self.device)
+        rate = torch.empty_like(log_w)
+        self.act_epoch += 1
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_ais_run_measured(
+                self.handle, z0.data_ptr(), y.data_ptr(), betas.data_ptr(), int(steps), float(step_size),
+                float(target_accept), float(sigma), eps.data_ptr() if eps is not None else None,
+                u.data_ptr() if u is not None else None, int(seed) & (2 ** 64 - 1), int(sample_offset),
+                z_out.data_ptr(), log_w.data_ptr(), rate.data_ptr(), _stream(self.device)), "lsnf_ais_run_measured")
+        return z_out, log_w, rate
+
 
 _PLANS: Dict[Tuple, Plan] = {}
 
@@ -445,21 +549,21 @@ def default_bwd_passes(noisy_chain: bool = False) -> int:
 
 
 def get_plan(*, arch, batch, nz, ngf, nc, f_depth, f_width, f_permutation, f_coupling, leak, device,
-             gemm_impl=_cabi.GEMM_TCGEN05, bwd_passes=None, train=False) -> Plan:
+             gemm_impl=_cabi.GEMM_TCGEN05, bwd_passes=None, train=False, meas_rows=0) -> Plan:
     device = torch.device(device)
     if device.type == "cuda" and device.index is None:
         device = torch.device("cuda", torch.cuda.current_device())
     if bwd_passes is None:
         bwd_passes = default_bwd_passes()
     key = (str(device), arch, batch, nz, ngf, nc, f_depth, f_width, f_permutation, f_coupling, float(leak), gemm_impl,
-           bwd_passes, bool(train))
+           bwd_passes, bool(train), int(meas_rows))
     p = _PLANS.get(key)
     if p is None:
         if len(_PLANS) > 16:
             _PLANS.pop(next(iter(_PLANS)))
         p = Plan(arch=arch, batch=batch, nz=nz, ngf=ngf, nc=nc, f_depth=f_depth, f_width=f_width,
                  f_permutation=f_permutation, f_coupling=f_coupling, leak=leak, device=device, gemm_impl=gemm_impl,
-                 bwd_passes=bwd_passes, train=train)
+                 bwd_passes=bwd_passes, train=train, meas_rows=meas_rows)
         _PLANS[key] = p
     return p
 
