@@ -272,9 +272,10 @@ int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* 
  * Workspace: A is kept as two K-major 16-bit hi|lo copies, about 8 m n bytes, plus fp32 split-K partials of
  * A x_hat and A^T r (r = A x_hat - y).  A dense operator grows fast with the image: at CelebA-HQ256 (n = 196 608) a
  * 4x-downsampling A (m = n / 16) takes 19 GB.
- * lsnf_pack_measurement: packs A (read once; the caller may free or change it afterwards) into both copies, with one
- *   power-of-two scale computed on the device for the fp16 copy of the forward product, undone exactly in fp32.
- *   Pack again after A changes.
+ * lsnf_pack_measurement: packs A (read once; the caller may free or change it afterwards) into both copies, times one
+ *   power of two 2^k computed on the device (max|A| 2^k in [1, 2)).  The 16-bit tensors of the measured path carry
+ *   2^k and 2^2k, so they do not depend on the units of A, y and sigma; 2^-2k is undone exactly in fp32.  The call
+ *   reads k back and synchronises `stream`.  Pack again after A changes.
  * lsnf_langevin_run_measured, lsnf_generator_dgrad_measured and lsnf_ais_run_measured have the contracts of
  *   lsnf_langevin_run, lsnf_generator_dgrad and lsnf_ais_run (injected noise, Philox keying, gradient norms, graph
  *   replay with y copied into the workspace before each replay; measured and unmeasured loops never share a graph)

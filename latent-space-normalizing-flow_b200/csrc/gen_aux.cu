@@ -153,13 +153,16 @@ __global__ void wmax_kernel(const float* __restrict__ w, long long n, unsigned i
   if ((threadIdx.x & 31) == 0) atomicMax(maxbits, __float_as_uint(m));  // non-negative floats order like uints
 }
 
-__global__ void wscale_finalize_kernel(unsigned int* __restrict__ blk, int n_layers) {
+// The scale exponent is clamped to [emin, emax]: [-14, 30] for the weights (whose fp16 halves must stay normal fp16
+// numbers), [-126, 126] for the measurement operator (whose scale is carried through the measured path, so 2^k and
+// 2^-k only have to be normal fp32 numbers).
+__global__ void wscale_finalize_kernel(unsigned int* __restrict__ blk, int n_layers, int emin, int emax) {
   const int l = threadIdx.x;
   if (l >= n_layers) return;
   const float m = __uint_as_float(blk[4 * l]);
   int e = 0;
   if (m > 0.f && isfinite(m)) frexpf(m, &e);      // m = f * 2^e, f in [0.5, 1)
-  e = max(-14, min(30, 1 - e));                   // scale = 2^(1-e): max|w| * scale in [1, 2)
+  e = max(emin, min(emax, 1 - e));                // scale = 2^(1-e): max|w| * scale in [1, 2)
   reinterpret_cast<float*>(blk)[4 * l + 1] = ldexpf(1.f, e);
   reinterpret_cast<float*>(blk)[4 * l + 2] = ldexpf(1.f, -e);
 }
@@ -174,7 +177,7 @@ int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cud
     wmax_kernel<<<blocks, 256, 0, s>>>(weights[l], n, blk + 4 * l);
     LSNF_CUDA(cudaGetLastError());
   }
-  wscale_finalize_kernel<<<1, 32, 0, s>>>(blk, plan->n_layers);
+  wscale_finalize_kernel<<<1, 32, 0, s>>>(blk, plan->n_layers, -14, 30);
   LSNF_CUDA(cudaGetLastError());
   return LSNF_OK;
 }
@@ -182,10 +185,12 @@ int launch_weight_scales(const lsnf_plan* plan, const float* const* weights, cud
 // ---------------------------------------------------------------------------------------------------
 // linear measurement operator A [m, n] (lsnf_pack_measurement): the B operands of the two measurement stages,
 //   stage 2L (A x_hat):   rows i < m, K = n:  fp16 hi|lo of A[i][j] 2^k, 2^k the power of two with max|A| 2^k in [1, 2)
-//                         (wmax_kernel / wscale_finalize_kernel on the operator's scale block; the stage's epilogue
-//                         multiplies by 2^-k, exact)
-//   stage 2L+1 (A^T r):   rows j < n, K = m:  bf16 hi|lo of A[i][j] (the format of the data-gradient stages' operands)
-// Padding rows and columns are written as zeros.
+//                         (wmax_kernel / wscale_finalize_kernel on the operator's scale block)
+//   stage 2L+1 (A^T r):   rows j < n, K = m:  bf16 hi|lo of A[i][j] 2^k (the format of the data-gradient stages' operands)
+// Padding rows and columns are written as zeros.  2^k is not undone in the 16-bit path: stage 2L writes A x_hat 2^k,
+// the finisher scales y by 2^k, stage 2L+1 writes A^T r 2^2k, and 2^-2k is folded into the fp32 post-scale of the
+// first layer's split-K sum and into the AIS energy (meas_post_scale, plan.cu).  So the 16-bit tensors of the
+// measured path do not depend on the units of A, y and sigma, and k is read back to the host (*k_out).
 // ---------------------------------------------------------------------------------------------------
 __global__ void meas_pack_kernel(const float* __restrict__ A, int m, int n, uint16_t* __restrict__ fwd, int fwd_rows,
                                  int kx, uint16_t* __restrict__ bwd, int bwd_rows, int km,
@@ -202,14 +207,14 @@ __global__ void meas_pack_kernel(const float* __restrict__ A, int m, int n, uint
       fwd[(size_t)i * 2 * kx + kx + j] = lo;
     } else {
       const int j = (int)((e - nf) / km), i = (int)((e - nf) % km);
-      split16(i < m && j < n ? A[(size_t)i * n + j] : 0.f, false, hi, lo);
+      split16(i < m && j < n ? A[(size_t)i * n + j] * sc : 0.f, false, hi, lo);
       bwd[(size_t)j * 2 * km + i] = hi;
       bwd[(size_t)j * 2 * km + km + i] = lo;
     }
   }
 }
 
-int launch_meas_pack(const lsnf_plan* plan, const float* A, cudaStream_t s) {
+int launch_meas_pack(const lsnf_plan* plan, const float* A, int* k_out, cudaStream_t s) {
   const StageHost& f = plan->stages[2 * plan->n_layers];
   const StageHost& b = plan->stages[2 * plan->n_layers + 1];
   const int m = plan->meas_m, n = plan->cfg.nc * plan->img * plan->img;
@@ -218,27 +223,32 @@ int launch_meas_pack(const lsnf_plan* plan, const float* A, cudaStream_t s) {
   const long long na = (long long)m * n;
   wmax_kernel<<<(int)std::min<long long>((na + 255) / 256, 148 * 8), 256, 0, s>>>(A, na, blk);
   LSNF_CUDA(cudaGetLastError());
-  wscale_finalize_kernel<<<1, 32, 0, s>>>(blk, 1);
+  wscale_finalize_kernel<<<1, 32, 0, s>>>(blk, 1, -126, 126);
   LSNF_CUDA(cudaGetLastError());
   const long long total = (long long)f.info.b_rows * plan->meas_kx + (long long)b.info.b_rows * plan->meas_km;
   meas_pack_kernel<<<(int)std::min<long long>((total + 255) / 256, 148 * 16), 256, 0, s>>>(
       A, m, n, (uint16_t*)(plan->ws + f.info.b_offset), f.info.b_rows, plan->meas_kx,
       (uint16_t*)(plan->ws + b.info.b_offset), b.info.b_rows, plan->meas_km, (const float*)(blk + 1));
   LSNF_CUDA(cudaGetLastError());
+  float sc = 0.f;
+  LSNF_CUDA(cudaMemcpyAsync(&sc, blk + 1, 4, cudaMemcpyDeviceToHost, s));
+  LSNF_CUDA(cudaStreamSynchronize(s));
+  *k_out = ilogbf(sc);
   return LSNF_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------
 // Between the two measurement stages: r = A x_hat - y, with A x_hat the fixed-order sum of stage 2L's split-K partials
-// [S][B][n_pad] (already descaled by its epilogue).  One CTA per (256 rows of r, sample): writes r * seed_scale as the
-// bf16 hi|lo row [B][2 km] stage 2L+1 reads (seed_scale = sigma_seed_scale(sigma): the share of 1/sigma^2 the 16-bit
-// gradient tensors carry, as in the unmeasured seed) and, when epart is given, the CTA's fixed-order partial of |r|^2
-// into epart[b][blockIdx.x] (annealed importance sampling: l(z) = -|r|^2 / (2 sigma^2)).
+// [S][B][n_pad], which carry the operator's scale 2^k (yscale; y is multiplied by it, exact).  One CTA per (256 rows of
+// r, sample): writes r 2^k seed_scale as the bf16 hi|lo row [B][2 km] stage 2L+1 reads (seed_scale =
+// sigma_seed_scale(sigma): the share of 1/sigma^2 the 16-bit gradient tensors carry, as in the unmeasured seed) and,
+// when epart is given, the CTA's fixed-order partial of |r 2^k|^2 into epart[b][blockIdx.x] (annealed importance
+// sampling: l(z) = -|r|^2 / (2 sigma^2), with 2^-2k in the caller's 1 / (2 sigma^2)).
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) meas_finish_kernel(const float* __restrict__ part, int nsplit, int pitch,
                                                           const float* __restrict__ y, int B, int m,
-                                                          uint16_t* __restrict__ r_hl, int km, float seed_scale,
-                                                          float* __restrict__ epart) {
+                                                          uint16_t* __restrict__ r_hl, int km, float yscale,
+                                                          float seed_scale, float* __restrict__ epart) {
   __shared__ float red[256];
   pdl_wait();
   pdl_trigger();
@@ -247,7 +257,7 @@ __global__ void __launch_bounds__(256) meas_finish_kernel(const float* __restric
   if (i < m) {
     float v = 0.f;
     for (int q = 0; q < nsplit; ++q) v += __ldcg(part + ((size_t)q * B + b) * pitch + i);
-    const float r = v - y[(size_t)b * m + i];
+    const float r = v - y[(size_t)b * m + i] * yscale;
     e = r * r;
     uint16_t hi, lo;
     split16(r * seed_scale, false, hi, lo);
@@ -268,7 +278,8 @@ int launch_meas_finish(const lsnf_plan* plan, const float* y, float seed_scale, 
   const StageHost& f = plan->stages[2 * plan->n_layers];
   LSNF_CUDA(launch_k(meas_finish_kernel, dim3(plan->meas_tiles, plan->cfg.batch), dim3(256), 0, s,
                      (const float*)(plan->ws + f.info.out_offset), f.info.k_splits, f.info.n_pad, y, plan->cfg.batch,
-                     plan->meas_m, (uint16_t*)(plan->ws + plan->off_meas_r), plan->meas_km, seed_scale, epart));
+                     plan->meas_m, (uint16_t*)(plan->ws + plan->off_meas_r), plan->meas_km,
+                     ldexpf(1.f, plan->meas_k), seed_scale, epart));
   return LSNF_OK;
 }
 

@@ -238,10 +238,11 @@ struct lsnf_plan {
   // ais_update_kernel reads it from dyn[3] under replay.  A Langevin loop keys with target = 0, an AIS loop
   // (lsnf_ais_run) with with_noise = 1, and `ais` keeps the two apart.
   struct LoopKey {
-    int steps; float step_size, sigma; int with_noise; bool masked, ais; float target; bool measured;
+    int steps; float step_size, sigma; int with_noise; bool masked, ais; float target; bool measured; int meas_k;
     bool operator==(const LoopKey& o) const {
       return steps == o.steps && step_size == o.step_size && sigma == o.sigma && with_noise == o.with_noise &&
-             masked == o.masked && ais == o.ais && target == o.target && measured == o.measured;
+             masked == o.masked && ais == o.ais && target == o.target && measured == o.measured &&
+             meas_k == o.meas_k;
     }
   };
   struct LoopGraph { LoopKey key; cudaGraphExec_t exec; };
@@ -255,8 +256,10 @@ struct lsnf_plan {
   // linear measurements (meas_rows = m > 0): stages[2L] = A x_hat, stages[2L+1] = A^T r.  kx = n = nc*H*W and km = m,
   // each rounded up to BLOCK_K, are the K extents of the two GEMMs; x_hat and r are stored as 16-bit hi|lo rows
   // [B][2 kx] and [B][2 km]; y [B][m] is the graph-replayed loop's copy; epart [B][meas_tiles] the per-sample
-  // fixed-order partials of |r|^2; scale: |A|max bits, 2^k, 2^-k of the fp16 copy
-  int meas_m = 0, meas_kx = 0, meas_km = 0, meas_tiles = 0;
+  // fixed-order partials of |r 2^k|^2; scale: |A|max bits, 2^k, 2^-k of the packed copies.  meas_k = k, read back by
+  // lsnf_pack_measurement: the 16-bit tensors of the measured path carry 2^k (r) and 2^2k (A^T r and every gradient
+  // after it), undone in fp32 (meas_post_scale, plan.cu)
+  int meas_m = 0, meas_kx = 0, meas_km = 0, meas_tiles = 0, meas_k = 0;
   size_t off_meas_xhl = 0, off_meas_r = 0, off_meas_y = 0, off_meas_epart = 0, off_meas_scale = 0;
   bool meas_packed = false;
   long long runs = 0;
@@ -353,10 +356,10 @@ int launch_last_gather(const lsnf_plan* plan, float* out, int to_unit_range, cud
 // part (nullable): dL/dx_hat is instead the sum of the nsplit fp32 split-K partials [nsplit][B][pitch] of A^T r
 int launch_recon_grad_im2col(const lsnf_plan* plan, const float* x, const float* mask, float seed_scale, int upstream,
                              cudaStream_t s, const float* part = nullptr, int nsplit = 0, int pitch = 0);
-// A [m, n] -> the packed operands of the two measurement stages (after launch_meas_scale)
-int launch_meas_pack(const lsnf_plan* plan, const float* A, cudaStream_t s);
-// r = A x_hat - y from the split-K partials of stage 2L: bf16 hi|lo rows of r * seed_scale for stage 2L+1, and the
-// per-sample partials of |r|^2 into epart (nullable)
+// A [m, n] -> the packed operands of the two measurement stages, both times 2^k; synchronises s and returns k in *k_out
+int launch_meas_pack(const lsnf_plan* plan, const float* A, int* k_out, cudaStream_t s);
+// r 2^k = A x_hat 2^k - y 2^k from the split-K partials of stage 2L (k = plan->meas_k): bf16 hi|lo rows of
+// r 2^k seed_scale for stage 2L+1, and the per-sample partials of |r 2^k|^2 into epart (nullable)
 int launch_meas_finish(const lsnf_plan* plan, const float* y, float seed_scale, float* epart, cudaStream_t s);
 // epart (nullable): [B][tiles] sum m (x_hat - x)^2 over the pixels each CTA owns (tiles = last_fused_tiles)
 int launch_last_fused(const lsnf_plan* plan, const float* x, const float* mask, float* epart, float seed_scale,

@@ -737,7 +737,7 @@ extern "C" int lsnf_plan_bind(lsnf_plan* plan, void* workspace, size_t bytes) {
     const bool feeds8 = i + 1 < plan->stages.size() && plan->stages[i + 1].dev.cross8;
     d.amax_out = feeds8 ? (uint32_t*)(plan->ws + plan->stages[i + 1].x8_off) : nullptr;
     d.mbits = ((I.kind == 0 && !st.last) || (I.kind == 1 && !st.first)) ? (uint32_t*)(plan->ws + st.mbits_off) : nullptr;
-    if (st.meas) d.descale = st.meas == 1 ? (const float*)(plan->ws + plan->off_meas_scale + 8) : nullptr;
+    if (st.meas) d.descale = nullptr;   // the operator's 2^k is carried to the fp32 post-scale (meas_post_scale)
     int rc = bind_stage(plan, st, plan->cfg.gemm_impl == LSNF_GEMM_TCGEN05);
     if (rc) return rc;
   }
@@ -862,7 +862,8 @@ static int gen_dgrad_partial(lsnf_plan* p, const float* x, const float* mask, fl
 
 // Loss-gradient seed of a measured iteration, from the last forward stage's per-tap products: x_hat (with its fp16 rows),
 // A x_hat, r = A x_hat - y (and the |r|^2 partials into epart, nullable), A^T r, and the last layer's im2col seed
-// A^T r (1 - x_hat^2).  r carries seed_scale, the share of 1/sigma^2 kept in the 16-bit tensors.
+// A^T r (1 - x_hat^2).  r carries seed_scale, the share of 1/sigma^2 kept in the 16-bit tensors, and the operator's
+// 2^k (A^T r 2^2k): see meas_post_scale.
 static int meas_seed(const lsnf_plan* p, const float* y, float* epart, float seed_scale, cudaStream_t s) {
   const int L = p->n_layers;
   const StageHost& bw = p->stages[2 * L + 1];
@@ -873,6 +874,12 @@ static int meas_seed(const lsnf_plan* p, const float* y, float* epart, float see
     return rc;
   return launch_recon_grad_im2col(p, nullptr, nullptr, 1.f, 1, s, (const float*)(p->ws + bw.info.out_offset),
                                   bw.info.k_splits, bw.info.n_pad);
+}
+
+// The fp32 factor of the first layer's split-K sum of a measured gradient: the share of 1/sigma^2 the seed did not
+// apply, and 2^-2k for the operator's scale that r (2^k) and A^T r (2^2k) carry.
+static float meas_post_scale(const lsnf_plan* p, float sigma) {
+  return ldexpf(sigma_post_scale(sigma), -2 * p->meas_k);
 }
 
 // The measured entry points' own conditions (after need()).
@@ -889,7 +896,7 @@ extern "C" int lsnf_pack_measurement(lsnf_plan* plan, const float* A, lsnf_strea
   if (!plan || !plan->bound) return fail(LSNF_ERR_STATE, "plan not bound");
   if (plan->cfg.meas_rows == 0) return fail(LSNF_ERR_UNSUPPORTED, "plan was created without lsnf_config.meas_rows");
   if (!A) return fail(LSNF_ERR_INVALID, "null operator");
-  int rc = launch_meas_pack(plan, A, (cudaStream_t)stream);
+  int rc = launch_meas_pack(plan, A, &plan->meas_k, (cudaStream_t)stream);
   if (rc) return rc;
   plan->meas_packed = true;
   return LSNF_OK;
@@ -904,7 +911,7 @@ extern "C" int lsnf_generator_dgrad_measured(lsnf_plan* plan, const float* y, fl
   if ((rc = meas_seed(plan, y, nullptr, sigma_seed_scale(sigma), s))) return rc;
   for (int i = plan->n_layers; i < 2 * plan->n_layers; ++i)
     if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
-  return launch_reduce_partial(plan, grad_z, sigma_post_scale(sigma), s);
+  return launch_reduce_partial(plan, grad_z, meas_post_scale(plan, sigma), s);
 }
 
 extern "C" int lsnf_plan_run_stage(lsnf_plan* plan, int32_t index, lsnf_stream stream) {
@@ -1203,7 +1210,7 @@ static int langevin_loop(lsnf_plan* plan, const float* x, const float* mask, boo
                          float sigma, int with_noise,
                          const float* eps, uint64_t seed, uint64_t sample_offset, const uint64_t* dyn, float* gnorms,
                          cudaStream_t s, const AisArgs* ais) {
-  const float gscale = sigma_post_scale(sigma);
+  const float gscale = measured ? meas_post_scale(plan, sigma) : sigma_post_scale(sigma);
   int rc;
   static int trace_env = -1;
   if (trace_env < 0) { const char* e = getenv("LSNF_TRACE"); trace_env = (e && e[0] == '1') ? 1 : 0; }
@@ -1300,7 +1307,7 @@ static int run_chain(lsnf_plan* plan, const float* x, const float* mask, bool me
   for (int done = 0; done < iters;) {
     const int n = std::min(iters - done, graph_chunk);
     const lsnf_plan::LoopKey key = {n, step_size, sigma, with_noise, mask != nullptr, ais != nullptr,
-                                    ais ? ais->target : 0.f, measured};
+                                    ais ? ais->target : 0.f, measured, measured ? plan->meas_k : 0};
     cudaGraphExec_t exec = nullptr;
     for (auto& g : plan->graphs)
       if (g.key == key) exec = g.exec;
@@ -1401,7 +1408,7 @@ static int ais_run(lsnf_plan* plan, const float* z0, const float* x, const float
   a.betas = betas; a.eps = eps; a.u = u;
   a.tiles = measured ? plan->meas_tiles : plan->fused_tiles; a.total = steps;
   a.step0 = step_size; a.target = target_accept > 0.f ? target_accept : 0.f;
-  a.inv2s2 = 0.5f / (sigma * sigma);
+  a.inv2s2 = measured ? ldexpf(0.5f / (sigma * sigma), -2 * plan->meas_k) : 0.5f / (sigma * sigma);   // |r 2^k|^2
   // steps + 1 iterations: iteration 0 only initialises and proposes, the last one only decides
   if ((rc = run_chain(plan, x, mask, measured, steps + 1, step_size, sigma, 1, nullptr, seed, sample_offset, nullptr, s,
                       &a)))

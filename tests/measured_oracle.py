@@ -107,3 +107,20 @@ def gaussian_operator(m: int, n: int, seed: int) -> np.ndarray:
     Langevin chain so ill-conditioned that the oracle's own fp32 and fp64 z_T differ by 9e-5 at SVHN, m = n/8, T = 20;
     with N(0, 1/n) by 3e-6.)"""
     return (np.random.default_rng(seed).standard_normal((m, n)) / np.sqrt(n)).astype(np.float32)
+
+
+def operator_scale_exp(amax) -> int:
+    """k of the operator's packed copies (csrc/gen_aux.cu, launch_meas_pack): max|A| 2^k in [1, 2), clamped to
+    [-126, 126] so that 2^k and 2^-k are normal fp32 numbers; k = 1 for an all-zero operator."""
+    a = np.float32(amax)
+    e = int(np.frexp(a)[1]) if a > 0 and np.isfinite(a) else 0   # a = f 2^e, f in [0.5, 1)
+    return max(-126, min(126, 1 - e))
+
+
+def sigma_seed_scale(sigma) -> float:
+    """csrc/lsnf_internal.cuh sigma_seed_scale: the power of two of at most 16 of 1/sigma^2 (fp32) r carries."""
+    inv = np.float32(1.0) / (np.float32(sigma) * np.float32(sigma))
+    s = np.float32(1.0)
+    while s * 2 <= inv and s < 16:
+        s = np.float32(s * 2)
+    return float(s)

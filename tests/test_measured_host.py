@@ -94,25 +94,51 @@ def test_operator_adds_two_stages_after_an_unchanged_plan(arch, nz, ngf, batch):
             assert min(st.a_offset, st.b_offset, st.out_offset) >= ws0
         assert lib.lsnf_workspace_bytes(h) >= ws0 + 8 * m * n
         assert lib.lsnf_langevin_launch_count(h, 20) == lib.lsnf_langevin_launch_count(h0, 20)
-        for st, li, rows, k in zip(s[L2:], l[L2:], (m, n), (n, m)):
-            kblocks = -(-k // 64)
-            assert st.kind == 3 and st.epilogue == 3 and st.tap_gen_k == 1 and st.k_per_tap == 64 * kblocks
-            assert st.n_valid == rows and st.n_pad % st.block_n == 0 and st.n_pad >= rows
-            assert st.b_k == st.k_per_tap and st.b_rows == st.n_pad and st.passes == 3
-            # the K splits cover every K block once, none empty
-            per = -(-kblocks // st.k_splits)
-            assert (st.k_splits - 1) * per < kblocks <= st.k_splits * per
-            # the hardware limits of tests/test_plan_tables.py
-            assert li.kernel == _cabi.KERNEL_SINGLE and li.block == 320 and li.smem_bytes <= SMEM_MAX
-            assert li.ring_stages >= 1 and li.ring_stages * li.stage_bytes + 1280 <= li.smem_bytes
-            assert li.ctas_per_sm >= 1 and li.ctas_per_sm * (li.smem_bytes + 1024) <= SMEM_PER_SM
-            assert li.ctas_per_sm * li.tmem_columns <= 512
-            assert (li.grid_x, li.grid_y, li.grid_z) == (-(-batch // 128), st.n_pad // st.block_n, st.k_splits)
-            assert not li.tma_store and not li.stream_k and not li.cross_fp8
-            # a small batch is one M tile: the splits bring the grid to about one wave or more K blocks per split
-            assert li.grid_x * li.grid_y * li.grid_z >= min(148, li.grid_x * li.grid_y * kblocks // 2) * 0.5
+        _check_operator_records(s[L2:], l[L2:], m, n, batch)
         lib.lsnf_plan_destroy(h)
     lib.lsnf_plan_destroy(h0)
+
+
+def _check_operator_records(stages, launches, m, n, batch):
+    """The two operator stages' records: shapes, K coverage of the splits, the hardware limits."""
+    for st, li, rows, k in zip(stages, launches, (m, n), (n, m)):
+        kblocks = -(-k // 64)
+        assert st.kind == 3 and st.epilogue == 3 and st.tap_gen_k == 1 and st.k_per_tap == 64 * kblocks
+        assert st.n_valid == rows and st.n_pad % st.block_n == 0 and st.n_pad >= rows
+        assert st.b_k == st.k_per_tap and st.b_rows == st.n_pad and st.passes == 3
+        # the K splits cover every K block once, none empty
+        per = -(-kblocks // st.k_splits)
+        assert (st.k_splits - 1) * per < kblocks <= st.k_splits * per
+        # the hardware limits of tests/test_plan_tables.py
+        assert li.kernel == _cabi.KERNEL_SINGLE and li.block == 320 and li.smem_bytes <= SMEM_MAX
+        assert li.ring_stages >= 1 and li.ring_stages * li.stage_bytes + 1280 <= li.smem_bytes
+        assert li.ctas_per_sm >= 1 and li.ctas_per_sm * (li.smem_bytes + 1024) <= SMEM_PER_SM
+        assert li.ctas_per_sm * li.tmem_columns <= 512
+        assert (li.grid_x, li.grid_y, li.grid_z) == (-(-batch // 128), st.n_pad // st.block_n, st.k_splits)
+        assert not li.tma_store and not li.stream_k and not li.cross_fp8
+        # a small batch is one M tile: the splits bring the grid to about one wave or more K blocks per split
+        assert li.grid_x * li.grid_y * li.grid_z >= min(148, li.grid_x * li.grid_y * kblocks // 2) * 0.5
+    return stages
+
+
+# the (m, B) grid of tests/test_gpu_measured_operator_shapes.py
+@pytest.mark.parametrize("arch,ngf,m,batch", [
+    ("svhn", 32, 1, 1), ("svhn", 32, 63, 100), ("svhn", 32, 64, 128), ("svhn", 32, 65, 129), ("svhn", 32, 129, 300),
+    ("svhn", 32, 255, 1), ("svhn", 32, 257, 129), ("svhn", 32, 773, 100), ("svhn", 32, 3072, 128),
+    ("svhn", 32, 6145, 129), ("celeba_crop", 64, 1539, 129), ("celeba_hq256", 64, 257, 3)])
+def test_operator_stage_records_across_the_shape_grid(arch, ngf, m, batch):
+    lib, h = _plan(arch, 100, ngf, batch, m)
+    n = 3 * synth.image_size(arch) ** 2
+    li = launch_infos(lib, h)[-2:]
+    fwd, bwd = _check_operator_records(stage_infos(lib, h)[-2:], li, m, n, batch)
+    lib.lsnf_plan_destroy(h)
+    assert li[0].grid_x == li[1].grid_x == (1 if batch <= 128 else 2 if batch <= 256 else 3)
+    if m == 1:        # A^T r has one K block: one split
+        assert (bwd.k_per_tap, bwd.k_splits) == (64, 1)
+    if m == 2 * n + 1:   # K of A^T r exceeds that of A x_hat: more K blocks per split there
+        assert bwd.k_per_tap == 64 * -(-m // 64) > fwd.k_per_tap and bwd.k_splits >= fwd.k_splits
+    if arch == "celeba_hq256":   # 3072 K blocks of A x_hat split about 50 ways over 3 N tiles
+        assert fwd.k_per_tap == 196608 and fwd.n_pad == 384 and 40 <= fwd.k_splits <= 60
 
 
 def test_meas_rows_is_refused_where_it_cannot_apply():
@@ -186,3 +212,22 @@ def test_langevin_sharded_hands_each_rank_its_y_shard(monkeypatch, world):
     for (zz, yy, kw), (a, b) in zip(calls, starts):
         assert torch.equal(yy, y[a:b]) and torch.equal(zz, z[a:b])
         assert kw["operator"] is A and kw["sample_offset"] == a and kw["mask"] is None
+
+
+# ---- the operator's scale rule (restated in tests/measured_oracle.py for the GPU tests) -------------------------------
+@pytest.mark.parametrize("amax,k", [(1.0, 0), (2.0, -1), (float(np.nextafter(np.float32(1), np.float32(0))), 1),
+                                    (float(np.nextafter(np.float32(2), np.float32(0))), 0), (0.5, 1), (3.0, -1),
+                                    (2.0 ** 30, -30), (2.0 ** 31, -31), (2.0 ** -15, 15), (2.0 ** -31, 31),
+                                    (2.0 ** 125, -125), (2.0 ** 127, -126), (3.4e38, -126), (2.0 ** -126, 126),
+                                    (2.0 ** -140, 126), (0.0, 1)])
+def test_operator_scale_exponent_puts_the_maximum_in_one_to_two(amax, k):
+    assert MO.operator_scale_exp(amax) == k
+    a = np.float32(amax)
+    if a > 0 and -126 < k < 126:
+        assert 1.0 <= a * np.float32(2.0 ** k) < 2.0
+    # no clamp but fp32's normal range: 2^k and 2^-k are normal fp32 numbers
+    assert np.isfinite(np.float32(2.0 ** k)) and np.float32(2.0 ** -k) >= np.finfo(np.float32).tiny
+
+
+def test_sigma_seed_scale_restatement():
+    assert [MO.sigma_seed_scale(s) for s in (0.3, 1.0, 0.6, 0.1, 2.0 ** 20)] == [8.0, 1.0, 2.0, 16.0, 1.0]
