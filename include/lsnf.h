@@ -16,6 +16,7 @@
  *   lsnf_flow_param_grads    <- loss_f = -ll.mean(); loss_f.backward()    train.py:403-411, model.py:182
  *   lsnf_adam_step           <- optG.step() / optF.step() (torch.optim.Adam) train.py:294-295, :398, :415
  *   lsnf_*_masked            <- the same three generator-loss entry points with a per-pixel likelihood weight
+ *   lsnf_*_measured          <- the same generator-loss entry points and AIS with y = A vec(G(z)) + noise in place of x
  *   lsnf_generator_vjp       <- backward of netG(z) for any loss (torch.autograd through lsnf_b200.kernel_autograd)
  *   lsnf_flow_vjp            <- backward of netF(z, objective) for any loss (same)
  *   lsnf_pack_*              <- parameters of _netG / _netF               model.py:48-157, :460-498
@@ -281,13 +282,24 @@ int lsnf_ais_run(lsnf_plan* plan, const float* z0, const float* x, const float* 
  *   replay with y copied into the workspace before each replay; measured and unmeasured loops never share a graph)
  *   with y [B, m] in place of x (and the mask).  For AIS, l(z) = -|A vec(G(z)) - y|^2 / (2 sigma^2) and the caller adds
  *   C = -(m/2) log(2 pi sigma^2).
- * The three return LSNF_ERR_UNSUPPORTED on a plan with meas_rows == 0 or bwd_passes == 1 (the single-pass data
- * gradient writes an fp16 seed and A^T r has no bounded range), and LSNF_ERR_INVALID until an operator is packed. */
+ * lsnf_generator_param_grads_measured has the contract of lsnf_generator_param_grads (flat gradient layout, part
+ *   -1 / -2 / l, loss nullable and this rank's share, GLOBAL batch, deterministic) for the measured loss
+ *     loss_g = (1 / global_batch) * sum_b |A vec(G(z_b)) - y_b|^2        (no sigma, as the unmeasured loss_g has none)
+ *   on a plan created with train != 0; y [B, m] is read by the part -1 and -2 calls only.  The 16-bit gradient tensors
+ *   carry the operator's 2^2k; the weight and bias gradients and the loss undo it in fp32, so scaling A and y by 2^j
+ *   scales loss_g and every gradient by exactly 2^2j.  Layer calls (part >= 0) must follow a part -2 call of this
+ *   entry point, not of the unmeasured one (and vice versa): LSNF_ERR_STATE otherwise.
+ * The four return LSNF_ERR_UNSUPPORTED on a plan with meas_rows == 0 or bwd_passes == 1 (the single-pass data
+ * gradient writes an fp16 seed and A^T r has no bounded range), and LSNF_ERR_INVALID until an operator is packed.
+ * lsnf_generator_param_grads_measured also returns LSNF_ERR_STATE on a plan without train and LSNF_ERR_UNSUPPORTED on
+ * the SIMT path, as lsnf_generator_param_grads_masked does. */
 int lsnf_pack_measurement(lsnf_plan* plan, const float* A, lsnf_stream stream);
 int lsnf_langevin_run_measured(lsnf_plan* plan, const float* z0, const float* y, int32_t steps, float step_size,
                                float sigma, int32_t with_noise, const float* eps, uint64_t seed, uint64_t sample_offset,
                                float* z_out, float* gnorms, lsnf_stream stream);
 int lsnf_generator_dgrad_measured(lsnf_plan* plan, const float* y, float sigma, float* grad_z, lsnf_stream stream);
+int lsnf_generator_param_grads_measured(lsnf_plan* plan, const float* z, const float* y, int32_t global_batch,
+                                        float* grads, float* loss, int32_t part, lsnf_stream stream);
 int lsnf_ais_run_measured(lsnf_plan* plan, const float* z0, const float* y, const float* betas, int32_t steps,
                           float step_size, float target_accept, float sigma, const float* eps, const float* u,
                           uint64_t seed, uint64_t sample_offset, float* z_out, float* log_w, float* accept_rate,

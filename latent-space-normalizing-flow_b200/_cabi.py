@@ -97,6 +97,8 @@ EXPORTS = {
                                              C.c_int32, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
                                              C.c_void_p]),
     "lsnf_generator_dgrad_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
+    "lsnf_generator_param_grads_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                                      C.c_void_p, C.c_int32, C.c_void_p]),
     "lsnf_ais_run_measured": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float,
                                         C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

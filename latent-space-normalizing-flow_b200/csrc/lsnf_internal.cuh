@@ -211,6 +211,7 @@ struct lsnf_plan {
   std::vector<lsnf::WgradLayer> wg;     // training plans only (cfg.train)
   size_t gen_grad_floats = 0;
   bool wg_ready = false;                // the forward pass + data-gradient chain of lsnf_generator_param_grads ran
+  bool wg_measured = false;             // ... of lsnf_generator_param_grads_measured (scale 2^-2k)
   lsnf::FlowStash fstash;
   lsnf::FlowGradLayout fgrad;
   size_t off_fstash = 0, off_fgrad = 0, off_floss = 0, off_flinalg = 0;
@@ -373,6 +374,8 @@ int launch_wgrad_finalize(const FinalizeArgs& a, cudaStream_t s);
 int launch_bias_rowsum(const RowSumArgs& a, cudaStream_t s);
 int launch_mse_sum(const float* xh, const float* x, const float* mask, long long n, float scale, float* partial,
                    unsigned int* ticket, float* out, cudaStream_t s);
+// *out = scale * the fixed-order sum of the n partials of |r 2^k|^2 (meas_finish_kernel's epart), on one CTA
+int launch_meas_loss(const float* part, int n, float scale, float* out, cudaStream_t s);
 int launch_reduce_partial(const lsnf_plan* plan, float* grad_z, float scale, cudaStream_t s);
 int launch_flow_pack(lsnf_plan* plan, const float* const* params, const int32_t* const* perm,
                      const int32_t* const* perm_inv, const float* log_abs_det, const float* const* winv,

@@ -1035,9 +1035,10 @@ extern "C" int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z
       if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
     if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
     plan->wg_ready = true;
+    plan->wg_measured = false;
     if (!layers_all) return LSNF_OK;
   }
-  if (!plan->wg_ready)
+  if (!plan->wg_ready || plan->wg_measured)
     return fail(LSNF_ERR_STATE, "a layer's gradients were requested before the forward / data-gradient part (part = -2)");
   const float scale = 2.f / (float)global_batch;
   for (int l = L - 1; l >= 0; --l) {
@@ -1050,6 +1051,49 @@ extern "C" int lsnf_generator_param_grads_masked(lsnf_plan* plan, const float* z
 extern "C" int lsnf_generator_param_grads(lsnf_plan* plan, const float* z, const float* x, int32_t global_batch,
                                           float* grads, float* loss, int32_t part, lsnf_stream stream) {
   return lsnf_generator_param_grads_masked(plan, z, x, nullptr, global_batch, grads, loss, part, stream);
+}
+
+// The measured loss loss_g = |A vec(G(z)) - y|^2 / global_batch.  The prologue is the measured Langevin iteration's
+// generator half at seed scale 1: r carries 2^k and the last layer's im2col seed A^T r (1 - x_hat^2) carries 2^2k, so
+// the factor 2 / global_batch of the loss and 2^-2k are applied together in fp32 when the gradients are finalized, and
+// 2^-2k / global_batch to the |r 2^k|^2 partials the finisher leaves in the measured regions.
+extern "C" int lsnf_generator_param_grads_measured(lsnf_plan* plan, const float* z, const float* y,
+                                                   int32_t global_batch, float* grads, float* loss, int32_t part,
+                                                   lsnf_stream stream) {
+  int rc = need(plan, true, false);
+  if (rc || (rc = need_measured(plan))) return rc;
+  if (plan->wg.empty()) return fail(LSNF_ERR_STATE, "plan was created without lsnf_config.train");
+  if (plan->cfg.gemm_impl != LSNF_GEMM_TCGEN05) return fail(LSNF_ERR_UNSUPPORTED, "weight gradients need the tcgen05 path");
+  if (part < -2 || part >= plan->n_layers) return fail(LSNF_ERR_INVALID, "part must be -1 (all), -2 (prologue) or a layer");
+  const bool prologue = part < 0, layers_all = part == -1;
+  if (!z || (prologue && !y) || !grads || global_batch <= 0) return fail(LSNF_ERR_INVALID, "bad argument");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int L = plan->n_layers;
+  if (prologue) {
+    if ((rc = launch_split_z(plan, z, s))) return rc;
+    for (int l = 0; l < L; ++l)
+      if ((rc = run_stage(plan, plan->stages[l], s))) return rc;
+    float* epart = (float*)(plan->ws + plan->off_meas_epart);
+    if ((rc = meas_seed(plan, y, epart, 1.f, s))) return rc;
+    if ((rc = sync_check(s, "generator forward and measurement seed", -1))) return rc;
+    if (loss && (rc = launch_meas_loss(epart, plan->cfg.batch * plan->meas_tiles,
+                                       ldexpf(1.f / (float)global_batch, -2 * plan->meas_k), loss, s)))
+      return rc;
+    for (int i = L; i < 2 * L - 1; ++i)
+      if ((rc = run_dgrad_stage(plan, plan->stages[i], s))) return rc;
+    if ((rc = sync_check(s, "data-gradient chain", -1))) return rc;
+    plan->wg_ready = plan->wg_measured = true;
+    if (!layers_all) return LSNF_OK;
+  }
+  if (!plan->wg_ready || !plan->wg_measured)
+    return fail(LSNF_ERR_STATE, "a layer's gradients were requested before the measured forward / data-gradient part "
+                                "(part = -2)");
+  const float scale = ldexpf(2.f / (float)global_batch, -2 * plan->meas_k);
+  for (int l = L - 1; l >= 0; --l) {
+    if (!layers_all && l != part) continue;
+    if ((rc = gen_layer_grads(plan, l, grads, scale, s))) return rc;
+  }
+  return LSNF_OK;
 }
 
 extern "C" int lsnf_generator_vjp(lsnf_plan* plan, const float* grad_x_hat, float* grad_z, float* grads,

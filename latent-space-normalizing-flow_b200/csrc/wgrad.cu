@@ -240,4 +240,29 @@ int launch_mse_sum(const float* xh, const float* x, const float* mask, long long
   return LSNF_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// loss_g of a measured update = scale * sum of the n fixed-order partials of |r 2^k|^2 that meas_finish_kernel left
+// ([B][meas_tiles]); scale = 2^-2k / global_batch.  One CTA: thread t sums partials t, t + 256, ... in index order,
+// then a fixed tree, so the result does not depend on timing (no atomics).
+// ---------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) meas_loss_kernel(const float* __restrict__ part, int n, float scale,
+                                                        float* __restrict__ out) {
+  __shared__ float red[256];
+  float acc = 0.f;
+  for (int i = threadIdx.x; i < n; i += 256) acc += part[i];
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *out = red[0] * scale;
+}
+
+int launch_meas_loss(const float* part, int n, float scale, float* out, cudaStream_t s) {
+  meas_loss_kernel<<<1, 256, 0, s>>>(part, n, scale, out);
+  LSNF_CUDA(cudaGetLastError());
+  return LSNF_OK;
+}
+
 }  // namespace lsnf

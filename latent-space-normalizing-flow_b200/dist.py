@@ -1,6 +1,7 @@
 """Data-parallel plumbing (SURVEY.md section 8e): the latent batch is sharded contiguously across ranks, one
 process per GPU; Langevin chains are independent per sample so the loop itself needs no collective.  The only
-exchange is the parameter-gradient all-reduce of the training-mode G / F updates (train.py:394, :411)."""
+exchange is the parameter-gradient all-reduce of the training-mode G / F updates (train.py:394, :411).  Training from
+linear measurements shards y [B, m] like x and hands the operator A to every rank whole (``training_iteration``)."""
 from __future__ import annotations
 
 from typing import Iterable, Tuple

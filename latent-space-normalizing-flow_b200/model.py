@@ -83,12 +83,12 @@ class _netG(nn.Module):
         self.gen = nn.Sequential(*mods)
         self.gemm_impl = 0
 
-    def _plan(self, batch, device, train=False):
+    def _plan(self, batch, device, train=False, meas_rows=0):
         # a placeholder flow the generator never runs; the shuffle permutation keeps its footprint free of nz^2, so
         # that plan creation's flow shared-memory check accepts every nz
         return get_plan(arch=self.dataset, batch=batch, nz=self.nz, ngf=self.ngf, nc=self.nc, f_depth=1, f_width=4,
                         f_permutation=1, f_coupling=1, leak=self.leak, device=device, gemm_impl=self.gemm_impl,
-                        train=train)
+                        train=train, meas_rows=meas_rows)
 
     def generate(self, z):
         """z [B,nz,1,1] or [B,nz] -> x_hat [B,nc,H,W] through the CUDA kernels (never records autograd)."""

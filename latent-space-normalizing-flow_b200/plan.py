@@ -388,6 +388,27 @@ class Plan:
                 flat.data_ptr(), loss.data_ptr(), int(part), _stream(self.device)), "lsnf_generator_param_grads_masked")
         return flat, loss
 
+    def generator_param_grads_measured(self, z: torch.Tensor, y: torch.Tensor, global_batch: int,
+                                       flat: Optional[torch.Tensor] = None, part: int = -1,
+                                       loss: Optional[torch.Tensor] = None):
+        """``generator_param_grads`` for the measured loss loss_g = |A vec(G(z)) - y|^2 / global_batch with the operator
+        of the last ``ensure_operator``; y [B, meas_rows].  Needs ``train=True`` and ``meas_rows`` > 0 at plan
+        creation; only the part -1 and -2 calls read y."""
+        _check_tensor(z, "z", self.device, (self.batch, self.nz))
+        _check_tensor(y, "y", self.device, (self.batch, self.meas_rows))
+        n = int(self.lib.lsnf_generator_grad_floats(self.handle))
+        if flat is None:
+            flat = torch.zeros(n, dtype=torch.float32, device=self.device)
+        _check_tensor(flat, "flat gradient buffer", self.device, (n,))
+        if loss is None:
+            loss = torch.empty((), dtype=torch.float32, device=self.device)
+        self.act_epoch += 1
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.lsnf_generator_param_grads_measured(
+                self.handle, z.data_ptr(), y.data_ptr(), int(global_batch), flat.data_ptr(), loss.data_ptr(), int(part),
+                _stream(self.device)), "lsnf_generator_param_grads_measured")
+        return flat, loss
+
     # ---- flow parameter update (train.py:403-415) ----------------------------------------------------
     def flow_grad_layout(self):
         """[(offset, size)] of every flow parameter gradient inside the flat buffer, step-major, in the order of

@@ -14,7 +14,7 @@ import torch.distributed as dist
 
 from .langevin import sample_langevin_post_z_with_flow
 from .optim import FusedAdam
-from .plan import as_mask, flow_step_params
+from .plan import as_mask, as_measurements, flow_step_params
 
 
 def make_optimizers(netG, netF, args):
@@ -40,14 +40,35 @@ def _comm_stream(device):
     return _comm_streams[key]
 
 
-def _gen_plan_and_buffers(netG, z_k, x, plan, mask=None):
+def _measurements(netG, y, operator, b):
+    """y [b, m] as ``plan.as_measurements`` returns it, after checking that the operator is a 2-D [m, nc*H*W] tensor for
+    netG's images (the full check, finiteness included, runs when ``Plan.ensure_operator`` packs it)."""
+    from .synth import image_size
+    if not isinstance(operator, torch.Tensor):
+        raise TypeError("operator must be a torch.Tensor")
+    n = netG.nc * image_size(netG.dataset) ** 2
+    if operator.dim() != 2 or operator.shape[0] < 1 or operator.shape[1] != n:
+        raise ValueError(f"operator of shape {tuple(operator.shape)} is not [m, n] for images of n = {n} values")
+    return as_measurements(y, operator, b)
+
+
+def _gen_plan_and_buffers(netG, z_k, x, plan, mask=None, operator=None):
+    if mask is not None and operator is not None:
+        raise ValueError("pass either mask or operator, not both (a mask is the operator of its observed pixels)")
     b = z_k.shape[0]
     z2 = z_k.detach().reshape(b, netG.nz).contiguous().float()
-    xx = x.detach().contiguous().float()
+    if operator is not None:
+        xx = _measurements(netG, x, operator, b)
+    else:
+        xx = x.detach().contiguous().float()
     m = as_mask(mask, xx) if mask is not None else None
-    if plan is None:
+    if plan is None and operator is not None:
+        plan = netG._plan(b, z2.device, train=True, meas_rows=int(operator.shape[0]))
+    elif plan is None:
         plan = netG._plan(b, z2.device, train=True)
     plan.ensure_generator(netG)
+    if operator is not None:
+        plan.ensure_operator(operator)
     flat = getattr(plan, "_ggrad_flat", None)
     if flat is None:
         flat = plan._ggrad_flat = torch.zeros(int(plan.lib.lsnf_generator_grad_floats(plan.handle)),
@@ -59,13 +80,19 @@ def _gen_plan_and_buffers(netG, z_k, x, plan, mask=None):
     return plan, z2, xx, m, flat, layout, pairs
 
 
-def generator_gradients(netG, z_k, x, global_batch, plan=None, *, mask=None):
+def generator_gradients(netG, z_k, x, global_batch, plan=None, *, mask=None, operator=None):
     """(flat gradient buffer, [(parameter, gradient view)], this rank's share of loss_g) of
     loss_g = mse_sum(G(z_k), x) / global_batch (train.py:392-394) through ``lsnf_generator_param_grads``: forward,
     data-gradient chain and one weight-gradient tap-GEMM per layer on the tensor cores.  With ``mask`` (per-pixel
-    weight m, ``plan.as_mask``) loss_g = sum m (G(z_k) - x)^2 / global_batch."""
-    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask)
-    flat, loss = plan.generator_param_grads(z2, xx, global_batch, flat, mask=m)
+    weight m, ``plan.as_mask``) loss_g = sum m (G(z_k) - x)^2 / global_batch.  With a measurement ``operator`` A
+    [m, nc*H*W] (``plan.as_operator``) x is y [B, m] and loss_g = |A vec(G(z_k)) - y|^2 / global_batch
+    (``lsnf_generator_param_grads_measured``); A is packed once per tensor version.  ``plan``, if given, must have
+    been created with ``train=True`` (and ``meas_rows`` = m with an operator)."""
+    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask, operator)
+    if operator is not None:
+        flat, loss = plan.generator_param_grads_measured(z2, xx, global_batch, flat)
+    else:
+        flat, loss = plan.generator_param_grads(z2, xx, global_batch, flat, mask=m)
     return flat, pairs, loss
 
 
@@ -93,20 +120,30 @@ class _PendingGeneratorUpdate:
         return self.loss
 
 
-def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None):
+def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None,
+                           operator=None):
     """First half of the generator step of train.py:390-398: gradients, and with several ranks their all-reduce
     started layer by layer (bucket = one layer's weight + bias gradient, last layer first) on a comm stream while the
     main stream computes the next layer's weight gradient.  ``.finish()`` completes the step.  ``mask``: per-pixel
-    weight of the loss, as in ``generator_gradients``."""
+    weight of the loss; ``operator``: a measurement operator A, x then being y [B_local, m]; both as in
+    ``generator_gradients``."""
     b_global = z_k.shape[0] if global_batch is None else int(global_batch)
-    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask)
+    plan, z2, xx, m, flat, layout, pairs = _gen_plan_and_buffers(netG, z_k, x, plan, mask, operator)
+    if operator is not None:
+        grads = lambda part, loss=None: plan.generator_param_grads_measured(z2, xx, b_global, flat, part=part, loss=loss)
     if world <= 1:
-        flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, mask=m)
+        if operator is not None:
+            flat, loss = grads(-1)
+        else:
+            flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, mask=m)
         return _PendingGeneratorUpdate(netG, optG, args, flat, pairs, loss, [])
     comm = _comm_stream(z2.device)
     main = torch.cuda.current_stream(z2.device)
     handles = []
-    flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, part=-2, mask=m)
+    if operator is not None:
+        flat, loss = grads(-2)
+    else:
+        flat, loss = plan.generator_param_grads(z2, xx, b_global, flat, part=-2, mask=m)
 
     def reduce_async(t):
         ev = torch.cuda.Event()
@@ -118,17 +155,22 @@ def generator_update_begin(netG, optG, z_k, x, args, *, global_batch=None, group
     reduce_async(loss)
     n_layers = len(layout) // 2
     for l in reversed(range(n_layers)):
-        plan.generator_param_grads(z2, xx, b_global, flat, part=l, loss=loss)
+        if operator is not None:
+            grads(l, loss)
+        else:
+            plan.generator_param_grads(z2, xx, b_global, flat, part=l, loss=loss)
         lo = layout[2 * l][0]
         hi = layout[2 * l + 1][0] + layout[2 * l + 1][1]
         reduce_async(flat[lo:hi])
     return _PendingGeneratorUpdate(netG, optG, args, flat, pairs, loss, handles)
 
 
-def generator_update(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None):
-    """The generator step of train.py:390-398 without autograd.  Returns loss_g."""
+def generator_update(netG, optG, z_k, x, args, *, global_batch=None, group=None, world=1, plan=None, mask=None,
+                     operator=None):
+    """The generator step of train.py:390-398 without autograd.  Returns loss_g.  ``mask`` / ``operator``: as in
+    ``generator_gradients``."""
     return generator_update_begin(netG, optG, z_k, x, args, global_batch=global_batch, group=group, world=world,
-                                  plan=plan, mask=mask).finish()
+                                  plan=plan, mask=mask, operator=operator).finish()
 
 
 def flow_params_in_order(netF):
@@ -184,10 +226,14 @@ _iter_counter = [0]
 
 
 def training_iteration(x, netG, netF, optG, optF, args, *, global_batch=None, sample_offset=None, seed=None,
-                       z0=None, group=None, data_parallel=None, mask=None):
+                       z0=None, group=None, data_parallel=None, mask=None, operator=None):
     """x: this rank's shard [B_local, nc, H, W] on the GPU.  Returns (loss_g, loss_f, |grad_g|, |grad_f|, z_k).
     ``mask``: this rank's shard of a per-pixel likelihood weight (any shape that broadcasts to x's, ``plan.as_mask``)
     for training on partly observed images: both the Langevin energy and loss_g weight (G(z) - x)^2 by it.
+    ``operator``: a dense linear measurement operator A [m, nc*H*W] (``plan.as_operator``), the whole matrix on every
+    rank, for training from measurements only: x is then this rank's shard of y [B_local, m], the Langevin energy is
+    |A vec(G(z)) - y|^2 / (2 sigma^2) - log p(z) and loss_g = |A vec(G(z_k)) - y|^2 / B (compressed sensing,
+    low-resolution or blurred observations).  ``mask`` and ``operator`` together raise ValueError.
 
     Mirrors train.py:378-415: z_0 ~ N(0, I); z_k = Langevin(z_0, x); generator step on mse_sum(G(z_k), x) / B;
     flow step on -mean log p(z_k) (with the f_is_grad_clamp / f_max_norm clipping of train.py:411-412).  With several
@@ -198,6 +244,8 @@ def training_iteration(x, netG, netF, optG, optF, args, *, global_batch=None, sa
     (seed, global sample index, step) and z_0 is the rank's slice of ONE global draw from a generator seeded with
     ``seed``, so an N-rank iteration reproduces the single-process one.  ``seed`` defaults to
     (args.seed << 32) ^ iteration counter -- identical on every rank, as it must be."""
+    if mask is not None and operator is not None:
+        raise ValueError("pass either mask or operator, not both (a mask is the operator of its observed pixels)")
     b_local = x.shape[0]
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     if data_parallel is False:
@@ -226,13 +274,18 @@ def training_iteration(x, netG, netF, optG, optF, args, *, global_batch=None, sa
     if z0 is None:                                                                       # train.py:384
         gen = torch.Generator(x.device).manual_seed(int(seed) & (2 ** 63 - 1))
         z0 = torch.randn(b_global, netG.nz, 1, 1, device=x.device, generator=gen)[sample_offset:sample_offset + b_local]
+    # an iteration without a mask or an operator makes exactly the calls it makes without these keywords
+    measured = {} if operator is None else {"operator": operator}
     z_k, gn, fn = sample_langevin_post_z_with_flow(z0, x, netG, netF, args, seed=seed,
-                                                   sample_offset=sample_offset, train=True, mask=mask)   # train.py:387
+                                                   sample_offset=sample_offset, train=True, mask=mask,
+                                                   **measured)   # train.py:387
     from .langevin import langevin_plan
     from .plan import default_bwd_passes
-    plan = langevin_plan(netG, netF, b_local, x.device, default_bwd_passes(), train=True)  # the plan that call used
+    rows = {} if operator is None else {"meas_rows": int(operator.shape[0])}
+    plan = langevin_plan(netG, netF, b_local, x.device, default_bwd_passes(), train=True, **rows)  # the plan that call used
     # generator update (train.py:390-398): weight-gradient tap-GEMMs, per-layer all-reduces on the comm stream ...
-    masked = {} if mask is None else {"mask": mask}   # an unmasked iteration makes exactly the unmasked call
+    masked = {} if mask is None else {"mask": mask}
+    masked.update(measured)
     pending = generator_update_begin(netG, optG, z_k, x, args, global_batch=b_global, group=group, world=world,
                                      plan=plan, **masked)
     # ... overlapped with the flow update (train.py:403-415): gradient kernels + one flat all-reduce + fused Adam.
